@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the headline benchmark of BASELINE.json: Mrays/s (and samples/s) of the path-tracing hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1|c4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c1|c4] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -13,9 +13,10 @@ path) — the reference's `render_scene(cam, spp, scene)` (lib.rs:75-124).  Rays
              K x collective render_scene (shard render -> per-GPU finalise (1/spp, sqrt, x256, saturating u8) -> gather on rank 0,
              all inside librbrt_gpu.so), with --frames-in-flight groups (default 2) of --frames-per-batch frames (default 4, THE SAME
              at every N) in flight on their own streams (rbrt_b200.FramePipeline): the sparse, latency-bound last bounces of one
-             group overlap the dense first bounces of the next.  The K-step region is repeated (>= ~0.6 s in total) and the median
-             region is reported.  `single_frame` is one frame at a time, `frames_per_batch_1` the pipelined figure with one frame
-             per batch.  The last pipelined image is checked against the single-frame one.
+             group overlap the dense first bounces of the next.  Every timed arm runs exactly K steps after its warm-up.
+             `single_frame` is one frame at a time, `frames_per_batch_1` the pipelined figure with one frame per batch.  The last
+             pipelined image is checked against the single-frame one; --dump-outputs DIR writes it as DIR/image.npy (float32,
+             H x W x 3, values 0..255; above 64 MB a fixed seeded pixel sample, image_sample.npy + image_sample_index.npy).
   e2e        the same metric through the reference-facing call with HOST buffers: every step uploads the
              triangle soup from pinned host memory (rbrt_gpu_scene_create: H2D + LBVH build on rank 0, NCCL broadcast of the
              scene block to the other ranks), renders and copies the RGB8 image back to the host.
@@ -114,6 +115,24 @@ def pin_meshes(meshes):
         keep.append(t)
         out.append(t.numpy())
     return out, keep
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, image):
+    """The RGB8 image of the last timed step as out_dir/image.npy (float32 [H, W, 3], values 0..255, exact).  An image above
+    DUMP_BYTES as float32 is written as a fixed sample of 2^21 pixels drawn with SEED: image_sample.npy (float32 [n, 3]) and
+    image_sample_index.npy (float64 [n], the flat pixel index y * W + x, ascending)."""
+    os.makedirs(out_dir, exist_ok=True)
+    px = image.astype(np.float32)
+    if px.nbytes <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, "image.npy"), px)
+        return
+    px = px.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(SEED).choice(len(px), 1 << 21, replace=False))
+    np.save(os.path.join(out_dir, "image_sample.npy"), px[idx])
+    np.save(os.path.join(out_dir, "image_sample_index.npy"), idx.astype(np.float64))
 
 
 class ClockSampler:
@@ -394,7 +413,7 @@ def run_gpu(args):
     for _ in range(max(args.warmup, 3)):
         step_single(dict(time_kernels=True), _abi.StatsC())
     barrier()
-    n_single = 5
+    n_single = args.steps
     single_ms = []
     for _ in range(n_single):
         st = _abi.StatsC()
@@ -425,52 +444,43 @@ def run_gpu(args):
 
     # ---- resident arm (timed region): `steps` frames through the FramePipeline, `frames_in_flight` groups in flight on their own
     #      streams and wavefront pools, `frames_per_batch` frames per group — THE SAME at every N (a rank's launches on 8 GPUs
-    #      then have about the size they have on one GPU with one frame).  The K-step region is repeated until >= ~0.6 s have been
-    #      timed, each repeat bracketed by barrier + synchronize; the MEDIAN region is reported.
+    #      then have about the size they have on one GPU with one frame).  The region is bracketed by barrier + synchronize.
     # 4 frames per batch at every N — unless ONE frame of the workload already fills a wavefront pool (2^27 paths: C4, C5), where
     # batching frames only cuts each frame's samples into more, smaller batches (measured on C4: 59.1 ms with 4, 52.0 with 1)
     fpb = args.frames_per_batch or (1 if (args.workload in SAMPLE_SHARDED or W * H * spp > (1 << 27)) else 4)
 
-    def timed_pipeline(fpb_, budget_s):
+    def timed_pipeline(fpb_):
         pipe = R.FramePipeline(W, H, depth=args.frames_in_flight, host_output=False, shard_mode=shard_mode, frames_per_batch=fpb_)
         for _ in range(max(args.warmup, 3) * fpb_):
             pipe.submit(cam_c, spp, scene, seed=SEED)
         pipe.drain()
         barrier()
-        regions = []
-        t_all = time.perf_counter()
-        while True:
-            e0.record(stream)
-            for _ in range(args.steps):
-                pipe.submit(cam_c, spp, scene, seed=SEED)
-            pipe.flush()                                      # a last, partially filled group of frames
-            pipe.wait_on(stream)
-            e1.record(stream)
-            last = pipe.drain()[-1][0]
-            barrier()
-            regions.append(e0.elapsed_time(e1))
-            go = torch.tensor([1.0 if (time.perf_counter() - t_all < budget_s and len(regions) < 60) else 0.0], device="cuda")
-            if world > 1:
-                dist.broadcast(go, src=0)                     # every rank runs the same number of repeats
-            if go.item() == 0.0:
-                break
-        return regions, last
+        e0.record(stream)
+        for _ in range(args.steps):
+            pipe.submit(cam_c, spp, scene, seed=SEED)
+        pipe.flush()                                          # a last, partially filled group of frames
+        pipe.wait_on(stream)
+        e1.record(stream)
+        last = pipe.drain()[-1][0]
+        barrier()
+        return e0.elapsed_time(e1), last
 
     with ClockSampler(local) as clk:
         time.sleep(0.3)                                       # let nvidia-smi deliver its first samples
         clk.mark_begin()
-        regions, last = timed_pipeline(fpb, 0.7)
+        ms, last = timed_pipeline(fpb)
         clk.mark_end()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last.cpu().numpy().reshape(H, W, 3))
     check_images = not os.environ.get("RBRT_DEBUG_NO_GATHER")   # (a timing experiment of csrc/multi.cu that leaves rank 0's image incomplete)
     if rank == 0 and check_images:
         assert torch.equal(last, rgb_ref), "pipelined frame differs from the single-frame render"
-    ms = statistics.median(regions)
-    regions1 = None
+    ms_fpb1 = None
     if fpb != 1:                                              # the same measurement with ONE frame per batch, for the record
-        regions1, last1 = timed_pipeline(1, 0.4)
+        ms_fpb1, last1 = timed_pipeline(1)
         if rank == 0 and check_images:
             assert torch.equal(last1, rgb_ref), "pipelined frame (1 per batch) differs from the single-frame render"
-    t = torch.tensor([ms, ms_single, statistics.median(regions1) if regions1 else 0.0, min(regions), max(regions), ms_single_one_lane], dtype=torch.float64, device="cuda")
+    t = torch.tensor([ms, ms_single, ms_fpb1 or 0.0, ms_single_one_lane], dtype=torch.float64, device="cuda")
     agg = torch.tensor([frame["rays"] * args.steps, frame["paths"] * args.steps, (frame["launches"]) * args.steps,
                         counts["node_visits"] - counts["tail_node_visits"], counts["tri_tests"] - counts["tail_tri_tests"], counts["rays"],
                         counts["traversed_rays"] - counts["tail_traversed_rays"]], dtype=torch.float64, device="cuda")
@@ -479,7 +489,7 @@ def run_gpu(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dist.all_reduce(agg, op=dist.ReduceOp.SUM)
         dist.all_reduce(trace_ms, op=dist.ReduceOp.MAX)
-    ms, ms_single, ms_fpb1, ms_min, ms_max, ms_single_one_lane = (float(x) for x in t.tolist())
+    ms, ms_single, ms_fpb1, ms_single_one_lane = (float(x) for x in t.tolist())
     rays, paths, launches, V, T, Rc, Cc = (float(x) for x in agg.tolist())
     trace_ms = float(trace_ms.item())
     clocks = clk.summary()
@@ -512,45 +522,34 @@ def run_gpu(args):
         t_c = time.perf_counter()
         return (t_b - t_a) * 1e3, (t_c - t_b) * 1e3
 
-    e_steps = max(2, min(args.steps, 5))
-
-    def timed_e2e(budget_s):
+    def timed_e2e():
         for _ in range(max(2, args.frames_in_flight + 1)):
             step_e2e()
         for fin in pipe_e.drain():
             retire(fin)
         barrier()
-        regs = []
-        t_all = time.perf_counter()
-        while True:
-            t0 = time.perf_counter()
-            e0.record(stream)
-            for _ in range(e_steps):
-                ms_create, ms_render = step_e2e()
-            for fin in pipe_e.drain():                        # every image of the timed steps is on the host when the clock stops
-                retire(fin)
-            e1.record(stream)
-            barrier()
-            regs.append(max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3))   # host-side work (malloc, sync copies) counts too
-            go = torch.tensor([1.0 if (time.perf_counter() - t_all < budget_s and len(regs) < 30) else 0.0], device="cuda")
-            if world > 1:
-                dist.broadcast(go, src=0)
-            if go.item() == 0.0:
-                break
+        t0 = time.perf_counter()
+        e0.record(stream)
+        for _ in range(args.steps):
+            ms_create, ms_render = step_e2e()
+        for fin in pipe_e.drain():                            # every image of the timed steps is on the host when the clock stops
+            retire(fin)
+        e1.record(stream)
+        barrier()
+        ms_ = max(e0.elapsed_time(e1), (time.perf_counter() - t0) * 1e3)   # host-side work (malloc, sync copies) counts too
         print(f"[e2e rank {rank}] broadcast={e2e_broadcast[0]} last step: scene_create {ms_create:.1f} ms, submit (+ wait for the frame {args.frames_in_flight} steps back) "
-              f"{ms_render:.1f} ms; {len(regs)} regions of {e_steps} steps", file=sys.stderr)
-        return regs
+              f"{ms_render:.1f} ms; {args.steps} steps", file=sys.stderr)
+        return ms_
 
-    e_regions = timed_e2e(0.6)
-    e_ms = statistics.median(e_regions)
+    e_ms = timed_e2e()
     e_ms_bcast = None
     if world > 1:                                             # for the record: rank 0 alone uploads + builds, NCCL broadcast of the scene block
         e2e_broadcast[0] = True
-        e_ms_bcast = statistics.median(timed_e2e(0.4))
+        e_ms_bcast = timed_e2e()
         e2e_broadcast[0] = False
     if rank == 0 and check_images:
         assert np.array_equal(e2e_last[0].pixels.reshape(-1), rgb_ref.cpu().numpy()), "e2e image differs from the single-frame render"
-    e_rays = frame["rays"] * e_steps
+    e_rays = frame["rays"] * args.steps
     te = torch.tensor([e_ms, e_ms_bcast or 0.0], dtype=torch.float64, device="cuda")
     re = torch.tensor([float(e_rays)], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -622,19 +621,19 @@ def run_gpu(args):
         "warmup": max(args.warmup, 3), "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "strong",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": dict(workload_config(args.workload, spheres, meshes, world), frames_in_flight=args.frames_in_flight, frames_per_batch=fpb),
-        "timed_region": {"repeats": len(regions), "steps_per_repeat": args.steps, "ms_median": ms, "ms_min": ms_min, "ms_max": ms_max,
-                         "note": "the K-step region (barrier + synchronize on both sides, CUDA events, max over ranks) is repeated; value uses the median region"},
+        "timed_region": {"steps": args.steps, "ms": ms,
+                         "note": "one region of K steps (barrier + synchronize on both sides, CUDA events, max over ranks)"},
         "single_frame": {"ms_per_step": ms_single, "value": rays / args.steps / (ms_single / 1e3) / 1e6, "unit": "Mrays/s",
                          "ms_per_step_one_lane": ms_single_one_lane, "two_lanes": bool(use_split),
                          "note": "one frame at a time, host waits for each (latency of a lone render_scene call, gather on rank 0 included), the frame's "
                                  "sample batches on two lanes when it has >= 2^26 paths per GPU, as rbrt_gpu_render issues it (RBRT_OPT_SPLIT_BATCHES; one lane: ms_per_step_one_lane); `value` "
                                  "keeps `frames_in_flight` groups of `frames_per_batch` frames in flight on separate streams"},
-        "frames_per_batch_1": ({"ms_per_step": ms_fpb1 / args.steps, "value": rays / (ms_fpb1 / 1e3) / 1e6, "unit": "Mrays/s"} if regions1 else None),
+        "frames_per_batch_1": ({"ms_per_step": ms_fpb1 / args.steps, "value": rays / (ms_fpb1 / 1e3) / 1e6, "unit": "Mrays/s"} if ms_fpb1 else None),
         "samples_per_s": paths / (ms / 1e3), "rays_per_step": rays / args.steps, "rays_per_sample": rays / max(paths, 1),
         "clocks": clocks,
-        "e2e": {"value": e_val, "unit": "Mrays/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h), "steps": e_steps, "repeats": len(e_regions),
-                "ms_per_step": e_ms_max / e_steps,
-                "ms_per_step_scene_broadcast": (e_ms_bcast_max / e_steps) if e_ms_bcast else None,
+        "e2e": {"value": e_val, "unit": "Mrays/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h), "steps": args.steps,
+                "ms_per_step": e_ms_max / args.steps,
+                "ms_per_step_scene_broadcast": (e_ms_bcast_max / args.steps) if e_ms_bcast else None,
                 "includes": "scene upload from pinned host memory + LBVH build (every rank its own replica, the library's default with one process per GPU; "
                             "ms_per_step_scene_broadcast: rank 0 alone + ncclBroadcast of the 168 MB block) + render + RGB8 image to pinned host memory, per step; "
                             "frames_in_flight frames overlap (FramePipeline), all images on the host when the clock stops"},
@@ -681,7 +680,12 @@ def main():
                     help="frames rendered together in the same wavefront batches in the timed region (0 = 4 at EVERY N; sample-sharded workloads 1)")
     ap.add_argument("--frames-in-flight", type=int, default=2, choices=[1, 2, 3, 4],
                     help="groups of frames kept in flight on separate streams in the timed region (1 = one group at a time)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the image of the last timed step as DIR/<name>.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU arm computed; the reference arm has no such output")
     # exactly ONE line goes to stdout (the JSON); the host mirror's progress prints (lib.rs:80,114, mesh.rs:115) go to stderr
     # (NCCL and the host mirror also write to fd 1 from C: redirect the descriptor itself, keep a private duplicate for the JSON)
     global _STDOUT
