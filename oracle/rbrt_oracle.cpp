@@ -482,9 +482,10 @@ bool scatter(const Material& m, const Ray& in, const HitInfo& h, PathRng& rng, V
 struct Counters { uint64_t rays = 0, nan_rays = 0; };
 
 // Iterative form of the recursion: the product att_1 * (att_2 * (... * leaf)) is evaluated
-// innermost-first exactly as the recursion unwinds (lib.rs:62).
-V3 colorize(Ray ray, const Scene& sc, V3 bg, uint32_t depth, PathRng& rng, std::vector<float>& scratch, Counters& cnt) {
-    V3 atts[64]; int n_att = 0;
+// innermost-first exactly as the recursion unwinds (lib.rs:62).  `atts` holds at least `depth` entries:
+// a path scatters at most `depth` times.
+V3 colorize(Ray ray, const Scene& sc, V3 bg, uint32_t depth, PathRng& rng, std::vector<float>& scratch, std::vector<V3>& atts, Counters& cnt) {
+    int n_att = 0;
     V3 leaf;
     for (;;) {
         HitInfo h; h.tri = 0;
@@ -537,6 +538,7 @@ int render_sum(const Scene& sc, const rbrt_camera& cam, uint32_t spp, const rbrt
     if (!W || !H || !spp) return fail(RBRT_E_INVALID, "empty image or zero samples");
     uint64_t seed = o ? o->seed : 0;
     uint32_t depth = (o && o->max_depth) ? o->max_depth : 50;
+    if (depth > 1024) return fail(RBRT_E_INVALID, "max_depth > 1024");     // the product's limit (render.cu)
     ShardPlan sp{0, spp, false, 0, 1};
     if (o && o->shard_count > 1) {
         if (o->shard_rank >= o->shard_count) return fail(RBRT_E_INVALID, "shard_rank >= shard_count");
@@ -553,7 +555,7 @@ int render_sum(const Scene& sc, const rbrt_camera& cam, uint32_t spp, const rbrt
     std::atomic<uint64_t> rays{0}, nans{0}, paths{0};
     auto t0 = std::chrono::steady_clock::now();
     auto worker = [&]() {
-        std::vector<float> scratch; Counters cnt; uint64_t np = 0;
+        std::vector<float> scratch; std::vector<V3> atts(depth); Counters cnt; uint64_t np = 0;
         V3 bg = v3(0.05f, 0.05f, 0.8f);                              // lib.rs:89-93
         for (;;) {
             uint32_t col = next_col.fetch_add(stride_x);
@@ -564,7 +566,7 @@ int render_sum(const Scene& sc, const rbrt_camera& cam, uint32_t spp, const rbrt
                 for (uint32_t s = sp.s0; s < sp.s1; ++s) {
                     PathRng rng{{(uint32_t)seed, (uint32_t)(seed >> 32)}, row * W + col, s, 0, 0};
                     Ray ray = get_ray_through_pixel(cam, row, col, rng);
-                    V3 c = colorize(ray, sc, bg, depth, rng, scratch, cnt);
+                    V3 c = colorize(ray, sc, bg, depth, rng, scratch, atts, cnt);
                     color = color + c;                                // lib.rs:99
                     ++np;
                 }

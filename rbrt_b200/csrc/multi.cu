@@ -108,10 +108,12 @@ void release_dist_buffers() {
 // the caller has made `device` current
 static int ensure_dist(DistBuffers& d, int device, size_t n_px, uint32_t n_frames, size_t slab_bytes) {
     if (d.device != device) { free_dist(d); cudaSetDevice(device); d.device = device; }
-    if (d.accum_px < n_px) { for (auto& p : d.accum) { cudaFree(p); p = nullptr; } d.accum_px = 0; d.accum_n = 0; }
+    // every allocated accumulator holds accum_px pixels: one added for a further frame gets the size of those already there, not
+    // n_px (a smaller image), or a later, larger image with that many frames would pass the size check and not fit in it
+    if (d.accum_px < n_px) { for (auto& p : d.accum) { cudaFree(p); p = nullptr; } d.accum_px = n_px; d.accum_n = 0; }
     for (uint32_t f = 0; f < n_frames; ++f)
-        if (!d.accum[f]) { CKM(cudaMalloc(&d.accum[f], 16 * n_px)); }
-    d.accum_px = std::max(d.accum_px, n_px); d.accum_n = std::max(d.accum_n, n_frames);
+        if (!d.accum[f]) { CKM(cudaMalloc(&d.accum[f], 16 * d.accum_px)); }
+    d.accum_n = std::max(d.accum_n, n_frames);
     if (d.slab_bytes < slab_bytes) { cudaFree(d.slab); d.slab = nullptr; d.slab_bytes = 0; CKM(cudaMalloc(&d.slab, slab_bytes)); d.slab_bytes = slab_bytes; }
     if (!d.ev_start) { CKM(cudaEventCreateWithFlags(&d.ev_start, cudaEventDisableTiming)); CKM(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming)); }
     return RBRT_OK;

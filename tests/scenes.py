@@ -61,6 +61,58 @@ def quirk_camera(width, height):
     return R.Camera.new(Vec3(0.0, 1.5, 3.0), Vec3(0.0, -0.05, -1.0), Vec3(0.0, 1.0, 0.0), height, width, 24.0)
 
 
+def _quads(quads, inward):
+    """Two triangles per quad (corners in order around it), wound so that the normal (triangle.rs:30-34) points along `inward`."""
+    tris = []
+    for q, n in zip(np.asarray(quads, np.float32), np.asarray(inward, np.float32)):
+        a, b, c, d = q
+        tris += [(a, b, c), (a, c, d)] if np.dot(np.cross(b - a, c - a), n) > 0 else [(a, c, b), (a, d, c)]
+    return np.array(tris, np.float32)
+
+
+def deep_path_scene(length=12.0, hole=0.3, **kw):
+    """A long 2 x 2 box along -z, its walls facing inwards, open only through a `2 hole` x `2 hole` window in the front wall at z = 0:
+    Lambertian floor, ceiling, left wall, far end and front wall (albedo 0.95), a metal right wall (fuzz 0.05) in four segments and a glass sphere
+    in the middle.  A path has to diffuse back to the window to reach the sky, so most paths scatter well over 64 times and still
+    end with radiance > 0.  Both meshes have N % 8 == 0 triangles (every triangle is tested)."""
+    L, h = -float(length), float(hole)
+    lam = _quads([[(-1, -1, 0), (1, -1, 0), (1, -1, L), (-1, -1, L)],          # floor
+                  [(-1, 1, 0), (1, 1, 0), (1, 1, L), (-1, 1, L)],              # ceiling
+                  [(-1, -1, 0), (-1, 1, 0), (-1, 1, L), (-1, -1, L)],          # left wall
+                  [(-1, -1, L), (1, -1, L), (1, 1, L), (-1, 1, L)],            # far end
+                  [(-1, -1, 0), (1, -1, 0), (1, -h, 0), (-1, -h, 0)],          # front wall: four frames around the window
+                  [(-1, h, 0), (1, h, 0), (1, 1, 0), (-1, 1, 0)],
+                  [(-1, -h, 0), (-h, -h, 0), (-h, h, 0), (-1, h, 0)],
+                  [(h, -h, 0), (1, -h, 0), (1, h, 0), (h, h, 0)]],
+                 [(0, 1, 0), (0, -1, 0), (1, 0, 0), (0, 0, 1)] + [(0, 0, -1)] * 4)
+    seg = [L * k / 4 for k in range(5)]
+    metal = _quads([[(1, -1, z0), (1, 1, z0), (1, 1, z1), (1, -1, z1)] for z0, z1 in zip(seg, seg[1:])], [(-1, 0, 0)] * 4)
+    scene = R.Scene(**kw)
+    scene.elements.append(R.Sphere(Vec3(0.2, -0.3, L / 2), 0.5, R.Dielectric(1.5)))
+    scene.triangle_meshes += [R.TriangleMesh.from_triangles(lam, R.Lambertian(Vec3(0.95, 0.95, 0.95))),
+                              R.TriangleMesh.from_triangles(metal, R.Metal(Vec3(0.95, 0.9, 0.95), 0.05))]
+    return scene
+
+
+def deep_path_camera(width, height):
+    """Just inside the opening of deep_path_scene, looking down the box."""
+    return R.Camera.new(Vec3(0.0, 0.0, -0.2), Vec3(0.05, 0.02, -1.0), Vec3(0.0, 1.0, 0.0), height, width, 24.0)
+
+
+def two_mirror_scene():
+    """Two facing perfect mirrors, 10 apart, eight copies of each triangle: every path of two_mirror_camera bounces until its depth
+    budget is gone, so a render gives exactly (max_depth + 1) rays per path and a black image (lib.rs:54-66)."""
+    sc = R.Scene()
+    tris = np.array([((-50, -50, -5), (50, -50, -5), (0, 50, -5))] * 8 + [((-50, -50, 5), (0, 50, 5), (50, -50, 5))] * 8, np.float32)
+    sc.triangle_meshes.append(R.TriangleMesh.from_triangles(tris, R.Metal(Vec3(1, 1, 1), 0.0)))
+    return sc
+
+
+def two_mirror_camera(width=2, height=2):
+    """A long lens on the axis between the mirrors of two_mirror_scene: the rays stay between them."""
+    return R.Camera.new(Vec3(0, 0, 0), Vec3(0, 0, -1), Vec3(0, 1, 0), height, width, 28000.0)
+
+
 def random_rays(n, center, spread, seed=0):
     """Secondary-like rays: origins scattered around `center`, random unit directions, plus degenerate
     ones (axis-aligned directions with exact zeros, un-normalised and tiny directions)."""

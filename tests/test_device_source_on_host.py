@@ -189,6 +189,26 @@ def test_renders_against_the_oracle(hd, oracle):
                     assert np.array_equal(bits(hdr_b), bits(want)) and rays_b == rays, (k, seed, depth, leaf)
 
 
+def test_deep_paths_against_the_oracle(hd, oracle):
+    """Depth budgets past 64 up to the product's limit of 1024 on a scene whose paths scatter far more than 64 times: every bit of the HDR
+    image, the u8 image and the ray count; depth 200 also with every closest hit through the voted BVH traversal."""
+    scene, cam = S.deep_path_scene(), S.deep_path_camera(12, 8)
+    osc = oracle.OracleScene.from_scene(scene)
+    for depth in (64, 65, 200, 1024):
+        st = {}
+        want = osc.render_hdr(cam.to_c(), 2, _abi.RenderOptsC(seed=41, max_depth=depth), st)
+        hdr, rgb, rays, nans = hd_render(hd, scene, cam, 2, 41, depth)
+        assert np.array_equal(bits(hdr), bits(want)), (depth, int((bits(hdr) != bits(want)).any(axis=2).sum()))
+        assert rays == st["rays"] and nans == st["nan_rays"] == 0
+        assert np.array_equal(rgb, osc.render(cam.to_c(), 2, _abi.RenderOptsC(seed=41, max_depth=depth)))
+        assert (want > 0).any(axis=2).sum() >= want.shape[0] * want.shape[1] // 4           # not a black image
+        if depth >= 200:
+            assert st["rays"] > 65 * st["paths"], st                                          # the regime this is about
+        if depth == 200:
+            hdr_b, _, rays_b, _ = hd_render(hd, scene, cam, 2, 41, depth, 17)
+            assert np.array_equal(bits(hdr_b), bits(want)) and rays_b == rays
+
+
 def test_scatter_against_the_oracle(hd, oracle):
     """scatter() alone on the inputs of tests/test_gpu_scatter.py (random + grazing + normal incidence, ref_idx 0.2 ... 3.5)."""
     from .test_gpu_scatter import oracle_scatter

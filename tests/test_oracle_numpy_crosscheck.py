@@ -261,20 +261,47 @@ def scatter(mat, d, point, normal, key, pixel, sample, bounce):   # -> (attenuat
     return np.ones(3, F), (refl if u < prob else (refr if refr is not None else np.zeros(3, F)))
 
 
-def colorize(o, d, depth, world, key, pixel, sample):       # lib.rs:43-73, the recursion itself
+def colorize(o, d, max_depth, world, key, pixel, sample):   # lib.rs:43-73: the recursion unrolled into a loop
     spheres, meshes, mats = world
-    kind, elem, tri, t, dist = scene_hit(spheres, meshes, o, d)
-    if kind >= 0:
+    atts = []                                               # the attenuations in path order: the recursion's pending factors
+    depth = max_depth
+    while True:
+        kind, elem, tri, t, dist = scene_hit(spheres, meshes, o, d)
+        if kind < 0:
+            tt = F(F(0.5) * F(d[1] + F(1.0)))               # lib.rs:68-71
+            leaf = ((tt * np.ones(3, F)).astype(F) + (F(F(1.0) - tt) * np.array([0.05, 0.05, 0.8], F)).astype(F)).astype(F)
+            break
         point = (o + t * d).astype(F)
         normal = meshes[elem].normals[tri] if kind == 1 else (point - spheres[elem][0]).astype(F)
         mat = mats[elem if kind == 0 else len(spheres) + elem]
-        if depth > 0:
-            sc = scatter(mat, d, point, normal, key, pixel, sample, 50 - depth + 1)
-            if sc is not None:
-                return (sc[0] * colorize(point, sc[1], depth - 1, world, key, pixel, sample)).astype(F)
-        return np.zeros(3, F)
-    tt = F(F(0.5) * F(d[1] + F(1.0)))                       # lib.rs:68-71
-    return ((tt * np.ones(3, F)).astype(F) + (F(F(1.0) - tt) * np.array([0.05, 0.05, 0.8], F)).astype(F)).astype(F)
+        sc = scatter(mat, d, point, normal, key, pixel, sample, max_depth - depth + 1) if depth > 0 else None
+        if sc is None:
+            leaf = np.zeros(3, F)
+            break
+        atts.append(sc[0])
+        o, d, depth = point, sc[1], depth - 1
+    for a in reversed(atts):                                # att_1 * (att_2 * (... * leaf)): innermost first, as the recursion returns
+        leaf = (a * leaf).astype(F)
+    return leaf
+
+
+def numpy_render(scene, cam, spp, seed, max_depth=50):
+    """render_scene (lib.rs:75-124) by the numpy restatement: the HDR image (pre-gamma mean colour)."""
+    W, H = cam.img_width_pix, cam.img_height_pix
+    meshes = [NpMesh(np.asarray(m.triangles, dtype=F).reshape(-1, 3, 3), scene.simd_lanes) for m in scene.triangle_meshes]
+    spheres = [(vec(e.center), F(e.radius)) for e in scene.elements]
+    mats = [e.material for e in scene.elements] + [m.material for m in scene.triangle_meshes]
+    key = [seed & 0xFFFFFFFF, seed >> 32]
+    got = np.zeros((H, W, 3), F)
+    inv = F(F(1.0) / F(spp))                                # lib.rs:101
+    for row in range(H):
+        for col in range(W):
+            color = np.zeros(3, F)
+            for s in range(spp):                            # lib.rs:96-100
+                o, d = camera_ray(cam, row, col, key, s)
+                color = (color + colorize(o, d, max_depth, (spheres, meshes, mats), key, row * W + col, s)).astype(F)
+            got[row, col] = (color * inv).astype(F)
+    return got
 
 
 def test_numpy_render_agrees_with_the_oracle(oracle):
@@ -285,22 +312,23 @@ def test_numpy_render_agrees_with_the_oracle(oracle):
     scene = S.small_mesh_scene(2)
     cam = S.example_camera(20, 15)
     W, H, spp = 20, 15, 3
-    mesh = NpMesh(np.asarray(scene.triangle_meshes[0].triangles, dtype=F).reshape(-1, 3, 3))
-    spheres = [(vec(e.center), F(e.radius)) for e in scene.elements]
-    mats = [e.material for e in scene.elements] + [m.material for m in scene.triangle_meshes]
-    key = [seed & 0xFFFFFFFF, seed >> 32]
     want = oracle.OracleScene.from_scene(scene).render_hdr(cam.to_c(), spp, _abi.RenderOptsC(seed=seed))
-    got = np.zeros((H, W, 3), F)
-    inv = F(F(1.0) / F(spp))                                # lib.rs:101
-    for row in range(H):
-        for col in range(W):
-            color = np.zeros(3, F)
-            for s in range(spp):                            # lib.rs:96-100
-                o, d = camera_ray(cam, row, col, key, s)
-                color = (color + colorize(o, d, 50, (spheres, [mesh], mats), key, row * W + col, s)).astype(F)
-            got[row, col] = (color * inv).astype(F)
+    got = numpy_render(scene, cam, spp, seed)
     bad = (got.view(np.uint32) != want.view(np.uint32)).any(axis=2)
     assert not bad.any(), f"{int(bad.sum())} of {W * H} pixels differ, first at {np.argwhere(bad)[:3].tolist()}"
     # every arm of the path was exercised
     assert COVER.get("Lambertian", 0) > 50 and COVER.get("Metal", 0) > 10 and COVER.get("Dielectric", 0) > 20, COVER
     assert COVER.get("refracted", 0) > 5 and COVER.get("total_reflection", 0) > 0 and COVER["max_bounce"] >= 5, COVER
+
+
+def test_numpy_render_of_deep_paths_agrees_with_the_oracle(oracle):
+    """Paths that scatter far more than 64 times (tests/scenes.py deep_path_scene) at max_depth 300: the bounce index of the Philox
+    stream runs to max_depth - depth + 1 past 64, and the oracle's attenuation store holds every factor of such a path."""
+    COVER.clear()
+    scene, cam = S.deep_path_scene(), S.deep_path_camera(6, 4)
+    st = {}
+    want = oracle.OracleScene.from_scene(scene).render_hdr(cam.to_c(), 2, _abi.RenderOptsC(seed=77, max_depth=300), st)
+    got = numpy_render(scene, cam, 2, 77, max_depth=300)
+    bad = (got.view(np.uint32) != want.view(np.uint32)).any(axis=2)
+    assert not bad.any(), f"{int(bad.sum())} of 24 pixels differ, first at {np.argwhere(bad)[:3].tolist()}"
+    assert st["rays"] > 65 * st["paths"] and COVER["max_bounce"] > 100 and (want > 0).any(axis=2).sum() >= 8, (st, COVER)

@@ -2,6 +2,7 @@
 Q1-Q15).  The reference has no test for these; each case below is derived by hand from the cited lines,
 so that the oracle (the only pin for these rows) is itself pinned to a reading of the source."""
 import numpy as np
+import pytest
 
 import rbrt_b200 as R
 from rbrt_b200 import _abi
@@ -195,6 +196,21 @@ def test_q11_q15_depth_and_output(oracle):  # lib.rs:54-66,99,101,118-120
     assert np.allclose(hdr, 1.0, atol=1e-5), hdr
     rgb = osc.render(cam.to_c(), 4, _abi.RenderOptsC(seed=0))
     assert (rgb >= 254).all()
+
+
+def test_depth_budget_up_to_the_limit(oracle):  # lib.rs:54-66; the product accepts max_depth <= 1024
+    """Past 64 bounces (the size of a fixed attenuation store the oracle once had) up to the product's limit, and the limit itself."""
+    osc = oracle.OracleScene.from_scene(S.two_mirror_scene())
+    cam = S.two_mirror_camera()
+    for depth in (64, 65, 1024):
+        st = {}
+        img = osc.render_hdr(cam.to_c(), 1, _abi.RenderOptsC(seed=3, max_depth=depth), st)
+        assert st["rays"] == 4 * (depth + 1) and st["paths"] == 4 and not img.any()
+    for depth in (1025, 2 ** 32 - 1):
+        with pytest.raises(RuntimeError, match="max_depth"):
+            osc.render_hdr(cam.to_c(), 1, _abi.RenderOptsC(seed=3, max_depth=depth))
+        with pytest.raises(RuntimeError, match="max_depth"):
+            osc.render(cam.to_c(), 1, _abi.RenderOptsC(seed=3, max_depth=depth))
 
 
 def test_basic_triangle_element(oracle):  # triangle.rs:9-28, 92-130, 412-441
