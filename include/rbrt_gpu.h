@@ -270,6 +270,35 @@ int rbrt_gpu_scene_create_elements(const rbrt_element_ref* order, uint32_t num_e
 int rbrt_gpu_scene_info(const rbrt_scene* scene, rbrt_scene_info* out);
 int rbrt_gpu_scene_destroy(rbrt_scene* scene);
 
+/* ---- updating a scene in place (animation) ------------------------------------------------
+ * New vertices for a mesh, new values for Scene.elements, without creating the scene again.  The scene keeps its counts, its element
+ * kinds, its device block and, by default, each mesh's tree topology.  Every update is ordered after every render / trace already
+ * enqueued against the scene (on any stream, any replica) and before every one enqueued afterwards; replicas under a communicator
+ * are updated too (one process: replica 0 is updated and copied again; process per GPU: the call is collective like the creation,
+ * every rank updates its own replica from its own arrays, or with RBRT_SCENE_BROADCAST rank 0 updates and broadcasts and the other
+ * ranks may pass NULL data).  rbrt_scene_info keeps describing the creation.  Images and hits are bit-exact for the new geometry
+ * whatever the tree's shape (DESIGN.md section 10); a refit tree may only be slower to traverse.
+ * Refused with RBRT_E_INVALID, the scene untouched: a triangle or element count, or element kinds, that differ from the creation,
+ * a bad mesh index, an unknown material kind, NULL data, a scene with a mesh whose tree was refused as too deep. */
+enum {
+    RBRT_UPDATE_REFIT = 0,     /* keep the mesh's tree topology, recompute every box on the device (default; librbrt_gpu_update.so) */
+    RBRT_UPDATE_REBUILD = 1    /* full LBVH build of the new vertices into the same slots (the creation's build) */
+};
+/* New world-space positions for mesh `mesh_index`: num_triangles * 9 floats in the creation's triangle order, num_triangles equal to
+ * the count it was created with (the SIMD tail rule, N_eff, the block layout and the triangle order do not change); material NULL =
+ * keep.  HOST pointer: returns once it has been read. */
+int rbrt_gpu_scene_update_mesh(rbrt_scene* scene, uint32_t mesh_index, const float* tri_vertices, uint64_t num_triangles,
+                               const rbrt_material* material, uint32_t flags);
+/* The same with a DEVICE pointer on the scene's first device, read in stream order on cuda_stream; cuda_stream then waits for the
+ * update, so the caller may overwrite the buffer with work enqueued later on that stream.  Returns without synchronising. */
+int rbrt_gpu_scene_update_mesh_device(rbrt_scene* scene, uint32_t mesh_index, const void* d_tri_vertices, uint64_t num_triangles,
+                                      const rbrt_material* material, uint32_t flags, void* cuda_stream);
+/* New values for Scene.elements: the same count and the same kinds in the same order as at creation (centres, radii, corners and
+ * materials may change, material kinds included).  HOST pointers: returns once they have been read. */
+int rbrt_gpu_scene_update_elements(rbrt_scene* scene, const rbrt_element_ref* order, uint32_t num_elements,
+                                   const rbrt_sphere_desc* spheres, uint32_t num_spheres,
+                                   const rbrt_triangle_desc* triangles, uint32_t num_triangles);
+
 /* = render_scene (lib.rs:75-124).  rgb_out: caller-allocated W*H*3 bytes, row-major RGB8 =
  *   the layout of image::ImageBuffer<Rgb<u8>>.  opts / stats may be NULL.  HOST pointers.
  *   Under a communicator (scene created collectively, opts->shard_count == 0) the call is collective: every rank makes

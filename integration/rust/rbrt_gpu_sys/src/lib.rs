@@ -42,6 +42,8 @@ pub const RBRT_TRANSPORT_NCCL: c_int = 1;
 pub const RBRT_TRANSPORT_PEER: c_int = 2;
 pub const RBRT_SCENE_LOCAL: u32 = 1;
 pub const RBRT_SCENE_NO_SAH: u32 = 2;
+pub const RBRT_UPDATE_REFIT: u32 = 0;
+pub const RBRT_UPDATE_REBUILD: u32 = 1;
 pub const RBRT_SCENE_BROADCAST: u32 = 4;
 pub const RBRT_OPT_COUNT_VISITS: u32 = 1;
 pub const RBRT_OPT_TIME_KERNELS: u32 = 2;
@@ -73,6 +75,16 @@ extern "C" {
                                           triangles: *const RbrtTriangleDesc, num_triangles: u32, meshes: *const RbrtMeshDesc, num_meshes: u32,
                                           opts: *const c_void, out: *mut *mut RbrtScene) -> c_int;
     pub fn rbrt_gpu_scene_destroy(scene: *mut RbrtScene) -> c_int;
+    /// Animation: new vertices for one mesh (same triangle count; the tree is refit, or rebuilt with RBRT_UPDATE_REBUILD), from host
+    /// memory or from device memory read in order on `stream`, and new values for Scene.elements (same count and kinds).  Ordered
+    /// after every render already enqueued against the scene and before every one enqueued afterwards.
+    pub fn rbrt_gpu_scene_update_mesh(scene: *mut RbrtScene, mesh_index: u32, tri_vertices: *const f32, num_triangles: u64,
+                                      material: *const RbrtMaterial, flags: u32) -> c_int;
+    pub fn rbrt_gpu_scene_update_mesh_device(scene: *mut RbrtScene, mesh_index: u32, d_tri_vertices: *const c_void, num_triangles: u64,
+                                             material: *const RbrtMaterial, flags: u32, stream: *mut c_void) -> c_int;
+    pub fn rbrt_gpu_scene_update_elements(scene: *mut RbrtScene, order: *const RbrtElementRef, num_elements: u32,
+                                          spheres: *const RbrtSphereDesc, num_spheres: u32, triangles: *const RbrtTriangleDesc,
+                                          num_triangles: u32) -> c_int;
     pub fn rbrt_gpu_render(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, opts: *const RbrtRenderOpts,
                            rgb_out: *mut u8, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_render_hdr(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, opts: *const RbrtRenderOpts,

@@ -115,6 +115,7 @@ OPT_COUNT_VISITS, OPT_TIME_KERNELS, OPT_NO_TAIL_KERNEL, OPT_POOL_SHIFT, OPT_SPLI
 MAX_FRAMES = 4          # frames one wavefront batch can hold (rbrt_gpu_render_accum_device_frames)
 HIT_NONE, HIT_SPHERE, HIT_MESH, HIT_TRIANGLE = -1, 0, 1, 2
 ELEM_SPHERE, ELEM_TRIANGLE = 0, 1
+UPDATE_REFIT, UPDATE_REBUILD = 0, 1
 E_INVALID, E_CUDA, E_NODEVICE = 1, 2, 3
 
 P = C.POINTER
@@ -138,6 +139,10 @@ GPU_SIGNATURES = {
     "rbrt_gpu_scene_create_elements": (C.c_int, [P(ElementRefC), C.c_uint32, P(SphereDescC), C.c_uint32, P(TriangleDescC), C.c_uint32,
                                                 P(MeshDescC), C.c_uint32, P(SceneOptsC), P(C.c_void_p)]),
     "rbrt_gpu_scene_info": (C.c_int, [C.c_void_p, P(SceneInfoC)]),
+    "rbrt_gpu_scene_update_mesh": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, P(MaterialC), C.c_uint32]),
+    "rbrt_gpu_scene_update_mesh_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, P(MaterialC), C.c_uint32, C.c_void_p]),
+    "rbrt_gpu_scene_update_elements": (C.c_int, [C.c_void_p, P(ElementRefC), C.c_uint32, P(SphereDescC), C.c_uint32, P(TriangleDescC),
+                                                C.c_uint32]),
     "rbrt_gpu_scene_destroy": (C.c_int, [C.c_void_p]),
     "rbrt_gpu_render": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, P(RenderOptsC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_render_hdr": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, P(RenderOptsC), C.c_void_p, P(StatsC)]),

@@ -3,6 +3,7 @@
 // RBRT_E_NODEVICE / RBRT_E_CUDA and a message.
 // Every entry point takes the process-wide lock (api_mutex): the library keeps per-device pools (scene blocks,
 // wavefront state, build scratch), and the reference's render_scene may be called from any thread.
+#include <dlfcn.h>
 #include <chrono>
 #include <cstdarg>
 #include <cstdio>
@@ -10,6 +11,7 @@
 #include "bvh_build.cuh"
 #include "engine.cuh"
 #include "multi.cuh"
+#include "update.cuh"
 
 namespace rbrt {
 
@@ -113,6 +115,9 @@ static void* pinned_get(size_t bytes) {
 static void pinned_put(void* p, size_t bytes) { if (!p) return; if (bytes <= 4096 && g_pinned_free.size() < 16) g_pinned_free.push_back(p); else cudaFreeHost(p); }
 
 void wait_scene_ready(const Scene& sc, int li, cudaStream_t st) { if (sc.rep[li].ready) cudaStreamWaitEvent(st, sc.rep[li].ready, 0); }
+void wait_scene_uses(const Scene& sc, int device, cudaStream_t st) {
+    for (const SceneUse& u : sc.uses) if (u.ev && (device < 0 || u.device == device)) cudaStreamWaitEvent(st, u.ev, 0);
+}
 
 int resolve_scene_info(const Scene& sc, bool wait) {
     Scene& m = const_cast<Scene&>(sc);                                     // lazily filled cache behind the handle (under the API lock)
@@ -133,6 +138,14 @@ int resolve_scene_info(const Scene& sc, bool wait) {
         m.info.ms_upload = up; m.info.ms_build = bu;                       // device times: H2D of the triangle soup / build kernels
         m.info_resolved = true;
     }
+    if (m.rebuild_pending && (wait || cudaEventQuery(m.rebuild_ev) == cudaSuccess)) {   // a mesh rebuilt by an update (RBRT_UPDATE_REBUILD)
+        cudaGetLastError();
+        cudaError_t e = cudaEventSynchronize(m.rebuild_ev);
+        if (e != cudaSuccess) return cuda_fail(e, "scene update");
+        const BuildResult* r = (const BuildResult*)m.res_h;
+        for (uint32_t i = 0; i < m.n_meshes; ++i) if (r[i].error && !m.build_error) m.build_error = (int)i + 1;
+        m.rebuild_pending = false;
+    }
     if (m.build_error) { set_error("mesh %d: BVH deeper than the traversal stack allows (the mesh was left out of the scene)", m.build_error - 1); return RBRT_E_INVALID; }
     return RBRT_OK;
 }
@@ -140,7 +153,13 @@ int resolve_scene_info(const Scene& sc, bool wait) {
 void destroy_scene(Scene* sc) {
     if (!sc) return;
     int cur = 0; cudaGetDevice(&cur);
-    for (cudaEvent_t* e : {&sc->info_ev, &sc->t_up0, &sc->t_up1, &sc->t_b0, &sc->t_b1}) if (*e) { cudaEventSynchronize(*e); cudaEventDestroy(*e); *e = nullptr; }
+    for (cudaEvent_t* e : {&sc->info_ev, &sc->t_up0, &sc->t_up1, &sc->t_b0, &sc->t_b1, &sc->upd_in, &sc->upd_out, &sc->rebuild_ev})
+        if (*e) { cudaEventSynchronize(*e); cudaEventDestroy(*e); *e = nullptr; }
+    for (Scene::Staging& s : sc->stage) {
+        if (s.done) { cudaEventSynchronize(s.done); cudaEventDestroy(s.done); }
+        if (s.p) cudaFreeHost(s.p);
+        s = Scene::Staging();
+    }
     pinned_put(sc->res_h, 16ull * sc->n_meshes); sc->res_h = nullptr;
     for (Replica& r : sc->rep) {
         if (!r.arena) { if (r.ready) cudaEventDestroy(r.ready); continue; }
@@ -172,6 +191,179 @@ SceneDev make_scene_dev(char* base, const ArenaLayout& lay, uint32_t n_elems, ui
 static uint64_t tested_triangles(uint64_t n, uint32_t lanes) {
     uint64_t r = n % lanes, total = n + r, tested = (total / lanes) * lanes;
     return tested < n ? tested : n;
+}
+
+// Scene.elements -> the block's element arrays: per element a sphere record or {bits(index into etris)}, its material and kind; per
+// BasicTriangle four etris records.  mat / kind / ekind hold at least ns entries (the mesh materials follow in mat / kind).
+static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt_sphere_desc* spheres, const rbrt_triangle_desc* triangles,
+                          std::vector<float4>& sph, std::vector<float4>& etris, std::vector<float4>& mat, std::vector<uint32_t>& kind,
+                          std::vector<uint32_t>& ekind) {
+    for (uint32_t i = 0; i < ns; ++i) {
+        rbrt_material m;
+        if (order[i].kind == RBRT_ELEM_SPHERE) {
+            const rbrt_sphere_desc& sp = spheres[order[i].index];
+            sph[i] = make_float4(sp.center.x, sp.center.y, sp.center.z, sp.radius);
+            m = sp.material; ekind[i] = RBRT_ELEM_SPHERE;
+        } else {                                                          // BasicTriangle::new (triangle.rs:19-27), host f32, no contraction
+            const rbrt_triangle_desc& t = triangles[order[i].index];
+            const rbrt_vec3 &a = t.corners[0], &b = t.corners[1], &c = t.corners[2];
+            float e1[3] = {b.x - a.x, b.y - a.y, b.z - a.z}, e2[3] = {c.x - a.x, c.y - a.y, c.z - a.z};
+            float cx = e1[1] * e2[2] - e1[2] * e2[1], cy = e1[2] * e2[0] - e1[0] * e2[2], cz = e1[0] * e2[1] - e1[1] * e2[0];
+            float len = sqrtf(cx * cx + cy * cy + cz * cz);
+            uint32_t ti = (uint32_t)(etris.size() / 4);
+            float tif; memcpy(&tif, &ti, 4);
+            sph[i] = make_float4(tif, 0.0f, 0.0f, 0.0f);
+            etris.push_back(make_float4(a.x, a.y, a.z, 0.0f)); etris.push_back(make_float4(e1[0], e1[1], e1[2], 0.0f));
+            etris.push_back(make_float4(e2[0], e2[1], e2[2], 0.0f)); etris.push_back(make_float4(cx / len, cy / len, cz / len, 0.0f));
+            m = t.material; ekind[i] = RBRT_ELEM_TRIANGLE;
+        }
+        mat[i] = make_float4(m.albedo.x, m.albedo.y, m.albedo.z, m.param);
+        kind[i] = m.kind;
+    }
+}
+
+// ------------------------------------------------------------------ scene updates (rbrt_gpu_scene_update_*)
+// The refit kernels live in their own device module, librbrt_gpu_update.so, loaded from this library's directory
+// (RBRT_GPU_UPDATE_LIB: another path).  Without it a refit is refused: there is no other implementation.
+struct UpdateModule { void* h = nullptr; rbrt_update_scratch_bytes_fn scratch_bytes = nullptr; rbrt_update_refit_fn refit = nullptr; };
+static int update_module(const UpdateModule** out) {
+    static UpdateModule m;
+    if (!m.h) {
+        std::string path;
+        const char* env = getenv("RBRT_GPU_UPDATE_LIB");
+        if (env && *env) path = env;
+        else {
+            Dl_info di;
+            if (!dladdr((void*)&update_module, &di) || !di.dli_fname) { set_error("cannot locate librbrt_gpu.so to find librbrt_gpu_update.so"); return RBRT_E_CUDA; }
+            path = di.dli_fname;
+            const size_t slash = path.find_last_of('/');
+            path = (slash == std::string::npos ? std::string(".") : path.substr(0, slash)) + "/librbrt_gpu_update.so";
+        }
+        void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
+        if (!h) { set_error("the refit module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", path.c_str(), dlerror()); return RBRT_E_CUDA; }
+        UpdateModule n; n.h = h;
+        *(void**)(&n.scratch_bytes) = dlsym(h, "rbrt_update_scratch_bytes");
+        *(void**)(&n.refit) = dlsym(h, "rbrt_update_refit");
+        if (!n.scratch_bytes || !n.refit) { set_error("%s lacks the refit entry points", path.c_str()); dlclose(h); return RBRT_E_CUDA; }
+        m = n;
+    }
+    *out = &m;
+    return RBRT_OK;
+}
+
+// Opens an update: the device's build stream, made to wait for every read of the scene enqueued so far on replica 0's device.
+// Every write of the update is enqueued on ctx->build after this.
+static int update_begin(Scene* sc, BuildCtx* ctx) {
+    CKA(cudaSetDevice(sc->rep[0].device));
+    CKA(build_begin(sc->rep[0].device, ctx));
+    wait_scene_uses(*sc, sc->rep[0].device, ctx->build);
+    return RBRT_OK;
+}
+// Publishes it: the other replicas are copied again (each behind its own readers), and every replica's `ready` is recorded
+// behind the writes, so that reads enqueued from now on see the new values.
+static int update_end(Scene* sc, BuildCtx& ctx) {
+    if (sc->replicated) return replicate_scene(sc, ctx.build);
+    CKA(cudaEventRecord(sc->rep[0].ready, ctx.build));
+    return RBRT_OK;
+}
+// Pinned host staging for `bytes` of element / material values (copied to the block on the build stream, behind the scene's readers):
+// one of two alternating buffers, once its previous copy has run.  The caller records s->done behind its copies.
+static int stage_get(Scene* sc, size_t bytes, Scene::Staging** out) {
+    Scene::Staging& s = sc->stage[sc->stage_next];
+    sc->stage_next ^= 1;
+    if (s.done) CKA(cudaEventSynchronize(s.done));
+    else CKA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+    if (s.bytes < bytes) {
+        if (s.p) cudaFreeHost(s.p);
+        s.p = nullptr; s.bytes = 0;
+        CKA(cudaMallocHost(&s.p, bytes < 4096 ? 4096 : bytes)); s.bytes = bytes < 4096 ? 4096 : bytes;
+    }
+    *out = &s;
+    return RBRT_OK;
+}
+static int ensure_event(cudaEvent_t* e) { if (!*e) CKA(cudaEventCreateWithFlags(e, cudaEventDisableTiming)); return RBRT_OK; }
+
+// rbrt_gpu_scene_update_mesh(_device).  `user_st` is the caller's stream for device vertices (on_device), unused otherwise.
+static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool on_device, uint64_t n, const rbrt_material* mat,
+                       uint32_t flags, cudaStream_t user_st) {
+    if (!scene) { set_error("null argument"); return RBRT_E_INVALID; }
+    Scene* sc = reinterpret_cast<Scene*>(scene);
+    if (flags > RBRT_UPDATE_REBUILD) { set_error("unknown update flags %u", flags); return RBRT_E_INVALID; }
+    if (mi >= sc->n_meshes) { set_error("mesh index %u out of range (the scene has %u meshes)", mi, sc->n_meshes); return RBRT_E_INVALID; }
+    if (n != sc->mesh_n_all[mi]) {
+        set_error("mesh %u: %llu triangles, created with %llu (an update keeps the count)", mi, (unsigned long long)n, (unsigned long long)sc->mesh_n_all[mi]);
+        return RBRT_E_INVALID;
+    }
+    if (mat && mat->kind > 2) { set_error("mesh %u: unknown material kind", mi); return RBRT_E_INVALID; }
+    const bool receiver = sc->replicated && comm().multi_process && comm().rank != 0;   // RBRT_SCENE_BROADCAST: rank 0's update arrives by broadcast
+    if (n && !verts && !receiver) { set_error("mesh %u: null tri_vertices", mi); return RBRT_E_INVALID; }
+    {   // a mesh whose tree was refused (too deep) is out of the scene: nothing to update
+        int rc = resolve_scene_info(*sc, true);
+        if (rc) return rc;
+    }
+    const UpdateModule* um = nullptr;
+    if (flags == RBRT_UPDATE_REFIT && !receiver) { int rc = update_module(&um); if (rc) return rc; }
+
+    BuildCtx ctx;
+    { int rc = update_begin(sc, &ctx); if (rc) return rc; }
+    if (on_device && !receiver) {
+        { int rc = ensure_event(&sc->upd_in); if (rc) return rc; }
+        CKA(cudaEventRecord(sc->upd_in, user_st));                      // the vertices are ready in stream order on the caller's stream
+    }
+    cudaEvent_t uploaded = nullptr;                                       // host vertices: completes when they have been read
+    if (!receiver) {
+        const MeshDev& md = sc->meshes_h[mi];
+        const uint32_t n_eff = md.n_tris;
+        char* const base = sc->rep[0].arena;
+        MeshDev* d_mesh = (MeshDev*)(base + sc->lay.mesh) + mi;
+        float4* d_tris = (float4*)(base + sc->lay.tris) + 3ull * md.tri_base;
+        float4* d_normals = (float4*)(base + sc->lay.nrm) + md.nrm_base;
+        float4* d_nodes = (float4*)(base + sc->lay.nodes) + 4ull * md.node_base;
+        BuildResult* d_res = (BuildResult*)(base + sc->lay.result) + mi;
+        if (mat) {
+            Scene::Staging* sg = nullptr;
+            { int rc = stage_get(sc, 32, &sg); if (rc) return rc; }
+            const float4 m4 = make_float4(mat->albedo.x, mat->albedo.y, mat->albedo.z, mat->param);
+            memcpy(sg->p, &m4, 16); memcpy((char*)sg->p + 16, &mat->kind, 4);
+            const size_t e = sc->n_elems + mi;
+            CKA(cudaMemcpyAsync(base + sc->lay.mat + 16 * e, sg->p, 16, cudaMemcpyHostToDevice, ctx.build));
+            CKA(cudaMemcpyAsync(base + sc->lay.kind + 4 * e, (char*)sg->p + 16, 4, cudaMemcpyHostToDevice, ctx.build));
+            CKA(cudaEventRecord(sg->done, ctx.build));
+        }
+        if (flags == RBRT_UPDATE_REBUILD) {                               // the creation's build into the mesh's own slots (<= n_eff - 1 nodes)
+            CKA(build_mesh(ctx, verts, n, n_eff, sc->pad_rel, sc->leaf_size, sc->sah, md, d_mesh, d_tris, d_normals, d_nodes, d_res,
+                           on_device ? sc->upd_in : nullptr));
+            if (!on_device) {
+                { int rc = ensure_event(&sc->t_up1); if (rc) return rc; }
+                CKA(build_uploads_done(ctx, sc->t_up1)); uploaded = sc->t_up1;
+            }
+            { int rc = ensure_event(&sc->rebuild_ev); if (rc) return rc; }   // a too-deep tree is reported like the creation's (resolve_scene_info)
+            CKA(cudaMemcpyAsync((BuildResult*)sc->res_h + mi, d_res, sizeof(BuildResult), cudaMemcpyDeviceToHost, ctx.build));
+            CKA(cudaEventRecord(sc->rebuild_ev, ctx.build));
+            sc->rebuild_pending = true;
+        } else {
+            const size_t raw_bytes = on_device ? 0 : (36ull * n + 255) & ~255ull;
+            char* sbase = nullptr;
+            CKA(build_slot_acquire(ctx, raw_bytes + um->scratch_bytes(n_eff), &sbase));
+            if (!on_device && n) CKA(cudaMemcpyAsync(sbase, verts, 36ull * n, cudaMemcpyHostToDevice, ctx.copy));
+            CKA(build_slot_uploaded(ctx, &uploaded));
+            if (on_device) CKA(cudaStreamWaitEvent(ctx.build, sc->upd_in, 0));
+            RefitArgs a;
+            a.raw = on_device ? verts : (const float*)sbase; a.n_all = n; a.n_eff = n_eff; a.pad_rel = sc->pad_rel;
+            a.mesh = d_mesh; a.tris = d_tris; a.normals = d_normals; a.nodes = reinterpret_cast<uint4*>(d_nodes); a.res = d_res;
+            CKA((cudaError_t)um->refit(&a, sbase + raw_bytes, ctx.build));
+            CKA(build_slot_release(ctx));
+            if (on_device) uploaded = nullptr;
+        }
+    }
+    { int rc = update_end(sc, ctx); if (rc) return rc; }
+    if (on_device && !receiver) {                                         // the caller's stream continues behind the update
+        { int rc = ensure_event(&sc->upd_out); if (rc) return rc; }
+        CKA(cudaEventRecord(sc->upd_out, ctx.build));
+        CKA(cudaStreamWaitEvent(user_st, sc->upd_out, 0));
+    }
+    if (uploaded) CKA(cudaEventSynchronize(uploaded));                    // the caller's array has been read (copy engine: no wait for busy SMs)
+    return RBRT_OK;
 }
 
 }  // namespace rbrt
@@ -257,6 +449,11 @@ int rbrt_gpu_scene_create_elements(const rbrt_element_ref* order, uint32_t ne, c
     sc->n_elems = ns; sc->n_meshes = nm; sc->n_etris = n_et;
     sc->info.num_spheres = ns; sc->info.num_meshes = nm;
     sc->info.num_triangles = total_tris; sc->info.num_triangles_tested = total_eff;
+    sc->pad_rel = pad_rel; sc->leaf_size = leaf_size; sc->sah = !(sflags & RBRT_SCENE_NO_SAH); sc->replicated = replicate;
+    sc->mesh_n_all.resize(nm);
+    for (uint32_t i = 0; i < nm; ++i) sc->mesh_n_all[i] = meshes[i].num_triangles;
+    sc->elem_kind_h.resize(ns);
+    for (uint32_t i = 0; i < ns; ++i) sc->elem_kind_h[i] = order[i].kind;
     double t0 = now_ms();
 
 #define CKS(x) do { int rc_ = (x); if (rc_) { destroy_scene(sc); return rc_; } } while (0)
@@ -310,28 +507,7 @@ int rbrt_gpu_scene_create_elements(const rbrt_element_ref* order, uint32_t ne, c
         // ---- elements: spheres + per-element materials (flattened SoA, 16-byte records)
         std::vector<float4> sph(ns), mat(ns + nm), etris;
         std::vector<uint32_t> kind(ns + nm), ekind(ns);
-        for (uint32_t i = 0; i < ns; ++i) {
-            rbrt_material m;
-            if (order[i].kind == RBRT_ELEM_SPHERE) {
-                const rbrt_sphere_desc& sp = spheres[order[i].index];
-                sph[i] = make_float4(sp.center.x, sp.center.y, sp.center.z, sp.radius);
-                m = sp.material; ekind[i] = RBRT_ELEM_SPHERE;
-            } else {                                                          // BasicTriangle::new (triangle.rs:19-27), host f32, no contraction
-                const rbrt_triangle_desc& t = triangles[order[i].index];
-                const rbrt_vec3 &a = t.corners[0], &b = t.corners[1], &c = t.corners[2];
-                float e1[3] = {b.x - a.x, b.y - a.y, b.z - a.z}, e2[3] = {c.x - a.x, c.y - a.y, c.z - a.z};
-                float cx = e1[1] * e2[2] - e1[2] * e2[1], cy = e1[2] * e2[0] - e1[0] * e2[2], cz = e1[0] * e2[1] - e1[1] * e2[0];
-                float len = sqrtf(cx * cx + cy * cy + cz * cz);
-                uint32_t ti = (uint32_t)(etris.size() / 4);
-                float tif; memcpy(&tif, &ti, 4);
-                sph[i] = make_float4(tif, 0.0f, 0.0f, 0.0f);
-                etris.push_back(make_float4(a.x, a.y, a.z, 0.0f)); etris.push_back(make_float4(e1[0], e1[1], e1[2], 0.0f));
-                etris.push_back(make_float4(e2[0], e2[1], e2[2], 0.0f)); etris.push_back(make_float4(cx / len, cy / len, cz / len, 0.0f));
-                m = t.material; ekind[i] = RBRT_ELEM_TRIANGLE;
-            }
-            mat[i] = make_float4(m.albedo.x, m.albedo.y, m.albedo.z, m.param);
-            kind[i] = m.kind;
-        }
+        pack_elements(order, ns, spheres, triangles, sph, etris, mat, kind, ekind);
         for (uint32_t i = 0; i < nm; ++i) {
             mat[ns + i] = make_float4(meshes[i].material.albedo.x, meshes[i].material.albedo.y, meshes[i].material.albedo.z, meshes[i].material.param);
             kind[ns + i] = meshes[i].material.kind;
@@ -395,6 +571,57 @@ int rbrt_gpu_scene_destroy(rbrt_scene* scene) {
     if (!scene) return RBRT_OK;
     destroy_scene(reinterpret_cast<Scene*>(scene));
     return RBRT_OK;
+}
+
+int rbrt_gpu_scene_update_mesh(rbrt_scene* scene, uint32_t mesh_index, const float* tri_vertices, uint64_t num_triangles,
+                               const rbrt_material* material, uint32_t flags) {
+    LOCK;
+    return update_mesh(scene, mesh_index, tri_vertices, false, num_triangles, material, flags, nullptr);
+}
+
+int rbrt_gpu_scene_update_mesh_device(rbrt_scene* scene, uint32_t mesh_index, const void* d_tri_vertices, uint64_t num_triangles,
+                                      const rbrt_material* material, uint32_t flags, void* cuda_stream) {
+    LOCK;
+    return update_mesh(scene, mesh_index, (const float*)d_tri_vertices, true, num_triangles, material, flags, (cudaStream_t)cuda_stream);
+}
+
+int rbrt_gpu_scene_update_elements(rbrt_scene* scene, const rbrt_element_ref* order, uint32_t ne, const rbrt_sphere_desc* spheres,
+                                   uint32_t n_sph, const rbrt_triangle_desc* triangles, uint32_t n_bt) {
+    LOCK;
+    if (!scene) { set_error("null argument"); return RBRT_E_INVALID; }
+    Scene* sc = reinterpret_cast<Scene*>(scene);
+    const bool receiver = sc->replicated && comm().multi_process && comm().rank != 0;   // RBRT_SCENE_BROADCAST: rank 0's values arrive by broadcast
+    if (ne != sc->n_elems) { set_error("%u elements, the scene was created with %u (an update keeps them)", ne, sc->n_elems); return RBRT_E_INVALID; }
+    const bool have = !receiver || order;
+    if (have) {
+        if ((ne && !order) || (n_sph && !spheres) || (n_bt && !triangles)) { set_error("null argument"); return RBRT_E_INVALID; }
+        for (uint32_t i = 0; i < ne; ++i) {
+            if (order[i].kind != sc->elem_kind_h[i]) { set_error("element %u: kind %u, created as %u (an update keeps the kinds)", i, order[i].kind, sc->elem_kind_h[i]); return RBRT_E_INVALID; }
+            if (order[i].kind == RBRT_ELEM_SPHERE ? order[i].index >= n_sph : order[i].index >= n_bt) { set_error("element %u: bad index", i); return RBRT_E_INVALID; }
+            const rbrt_material& m = order[i].kind == RBRT_ELEM_SPHERE ? spheres[order[i].index].material : triangles[order[i].index].material;
+            if (m.kind > 2) { set_error("element %u: unknown material kind", i); return RBRT_E_INVALID; }
+        }
+    }
+    BuildCtx ctx;
+    { int rc = update_begin(sc, &ctx); if (rc) return rc; }
+    if (have && ne) {
+        std::vector<float4> sph(ne), mat(ne), etris;
+        std::vector<uint32_t> kind(ne), ekind(ne);
+        pack_elements(order, ne, spheres, triangles, sph, etris, mat, kind, ekind);
+        const size_t b_sph = 16ull * ne, b_et = 16ull * etris.size(), b_mat = 16ull * ne, b_kind = 4ull * ne;
+        Scene::Staging* sg = nullptr;
+        { int rc = stage_get(sc, b_sph + b_et + b_mat + b_kind, &sg); if (rc) return rc; }
+        char* h = (char*)sg->p;
+        memcpy(h, sph.data(), b_sph); memcpy(h + b_sph, etris.data(), b_et);
+        memcpy(h + b_sph + b_et, mat.data(), b_mat); memcpy(h + b_sph + b_et + b_mat, kind.data(), b_kind);
+        char* const base = sc->rep[0].arena;
+        CKA(cudaMemcpyAsync(base + sc->lay.sph, h, b_sph, cudaMemcpyHostToDevice, ctx.build));
+        if (b_et) CKA(cudaMemcpyAsync(base + sc->lay.etris, h + b_sph, b_et, cudaMemcpyHostToDevice, ctx.build));
+        CKA(cudaMemcpyAsync(base + sc->lay.mat, h + b_sph + b_et, b_mat, cudaMemcpyHostToDevice, ctx.build));
+        CKA(cudaMemcpyAsync(base + sc->lay.kind, h + b_sph + b_et + b_mat, b_kind, cudaMemcpyHostToDevice, ctx.build));
+        CKA(cudaEventRecord(sg->done, ctx.build));
+    }
+    return update_end(sc, ctx);
 }
 
 int rbrt_gpu_render_accum_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t spp, const rbrt_render_opts* opts,

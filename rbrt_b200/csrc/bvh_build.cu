@@ -431,8 +431,38 @@ cudaError_t build_begin(int device, BuildCtx* ctx) {
 cudaError_t build_uploads_done(BuildCtx& ctx, cudaEvent_t ev) { return cudaEventRecord(ev, ctx.copy); }
 
 
+static cudaError_t slot_reserve(ScratchSlot& S, cudaStream_t cs, size_t bytes) {
+    if (S.bytes < bytes) {                                                 // grow (rare): nothing may still be using the slot
+        CK(cudaEventSynchronize(S.busy));
+        CK(cudaStreamSynchronize(cs));
+        cudaFree(S.p); S.p = nullptr; S.bytes = 0;
+        const size_t want = bytes + bytes / 8 + (1u << 20);
+        CK(cudaMalloc(&S.p, want)); S.bytes = want;
+    }
+    return cudaSuccess;
+}
+
+cudaError_t build_slot_acquire(BuildCtx& ctx, size_t bytes, char** base) {
+    ScratchSlot& S = g_build[ctx.device & 63].slot[ctx.slot];
+    CK(slot_reserve(S, ctx.copy, bytes));
+    CK(cudaStreamWaitEvent(ctx.copy, S.busy, 0));
+    *base = (char*)S.p;
+    return cudaSuccess;
+}
+
+cudaError_t build_slot_uploaded(BuildCtx& ctx, cudaEvent_t* uploaded) {
+    ScratchSlot& S = g_build[ctx.device & 63].slot[ctx.slot];
+    CK(cudaEventRecord(S.up, ctx.copy));
+    CK(cudaStreamWaitEvent(ctx.build, S.up, 0));
+    *uploaded = S.up;
+    return cudaSuccess;
+}
+
+cudaError_t build_slot_release(BuildCtx& ctx) { return cudaEventRecord(g_build[ctx.device & 63].slot[ctx.slot].busy, ctx.build); }
+
 cudaError_t build_mesh(BuildCtx& ctx, const float* h_tris, uint64_t n_all, uint32_t n, float pad_rel, uint32_t leaf_size, bool sah,
-                       const MeshDev& proto, MeshDev* d_mesh, float4* d_tris, float4* d_normals, float4* d_nodes, BuildResult* d_res) {
+                       const MeshDev& proto, MeshDev* d_mesh, float4* d_tris, float4* d_normals, float4* d_nodes, BuildResult* d_res,
+                       cudaEvent_t src_ready) {
     DeviceBuild& B = g_build[ctx.device & 63];
     ScratchSlot& S = B.slot[ctx.slot];
     cudaStream_t cs = ctx.copy, st = ctx.build;
@@ -449,17 +479,12 @@ cudaError_t build_mesh(BuildCtx& ctx, const float* h_tris, uint64_t n_all, uint3
     const size_t o_children = take_off(8ull * ni), o_range = take_off(8ull * ni), o_parent_int = take_off(4ull * ni), o_parent_leaf = take_off(4ull * n);
     const size_t o_flags = take_off(4ull * ni), o_height = take_off(4ull * ni), o_queue = take_off(4ull * ni), o_cstate = take_off(sizeof(CollapseState));
     const size_t o_tmp = take_off(tmp_bytes ? tmp_bytes : 16);
-    if (S.bytes < off) {                                                   // grow (rare): nothing may still be using the slot
-        CK(cudaEventSynchronize(S.busy));
-        CK(cudaStreamSynchronize(cs));
-        cudaFree(S.p); S.p = nullptr; S.bytes = 0;
-        const size_t want = off + off / 8 + (1u << 20);
-        CK(cudaMalloc(&S.p, want)); S.bytes = want;
-    }
+    CK(slot_reserve(S, cs, off));
     char* base = (char*)S.p;
-    // ---- upload (copy stream): after the previous build that read this slot
+    // ---- upload (copy stream): after the previous build that read this slot (and, for device vertices, after their producer)
     CK(cudaStreamWaitEvent(cs, S.busy, 0));
-    if (n_all) CK(cudaMemcpyAsync(base, h_tris, 36ull * n_all, cudaMemcpyHostToDevice, cs));
+    if (src_ready) CK(cudaStreamWaitEvent(cs, src_ready, 0));
+    if (n_all) CK(cudaMemcpyAsync(base, h_tris, 36ull * n_all, cudaMemcpyDefault, cs));
     CK(cudaEventRecord(S.up, cs));
     // ---- build (build stream)
     CK(cudaStreamWaitEvent(st, S.up, 0));

@@ -66,9 +66,23 @@ struct Scene {
     mutable bool info_resolved = false;
     mutable int build_error = 0; // mesh index + 1 whose tree was refused (deeper than the traversal stack), 0 = none
     double ms_host_create = 0;
+    // ---- what an update (rbrt_gpu_scene_update_*) needs to know about the creation
+    std::vector<uint64_t> mesh_n_all;       // real triangles per mesh (the count an update must hand in)
+    std::vector<uint32_t> elem_kind_h;      // RBRT_ELEM_* per element, in order
+    float pad_rel = 0.0f;
+    uint32_t leaf_size = 1;
+    bool sah = true;
+    bool replicated = false;                // replicas are copies of replica 0 (one process; or RBRT_SCENE_BROADCAST)
+    cudaEvent_t upd_in = nullptr, upd_out = nullptr;   // device-pointer updates: caller's stream -> build stream -> caller's stream
+    cudaEvent_t rebuild_ev = nullptr;       // RBRT_UPDATE_REBUILD: the rebuilt mesh's BuildResult has reached res_h
+    mutable bool rebuild_pending = false;
+    struct Staging { void* p = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
+    Staging stage[2];                       // pinned host staging of element / material values, alternating; `done`: its copy has run
+    int stage_next = 0;
 };
 int resolve_scene_info(const Scene& sc, bool wait);   // api.cu: fills info from the build results once they are there (wait: block for them); returns RBRT_E_* if the build refused a mesh
 void wait_scene_ready(const Scene& sc, int li, cudaStream_t st);   // makes `st` wait for replica li's data
+void wait_scene_uses(const Scene& sc, int device, cudaStream_t st);   // makes `st` wait for every read of the scene enqueued so far on `device` (< 0: any)
 
 // Everything a wavefront kernel needs, passed by value (kernel parameter space).
 struct WaveParams {

@@ -178,6 +178,7 @@ int replicate_scene(Scene* sc, cudaStream_t bs) {
     const size_t bytes = sc->lay.total;
     if (C.multi_process) {
         CKM(cudaSetDevice(C.devices[0]));
+        wait_scene_uses(*sc, C.devices[0], bs);
         CKN(g_nccl.Broadcast(sc->rep[0].arena, sc->rep[0].arena, bytes, ncclChar, 0, (ncclComm_t)C.nccl[0], bs));
         CKM(cudaEventRecord(sc->rep[0].ready, bs));
         return RBRT_OK;
@@ -190,7 +191,12 @@ int replicate_scene(Scene* sc, cudaStream_t bs) {
         if (e != cudaSuccess) return cuda_fail(e, "build_begin");
         s_of[li] = other.build;
     }
+    for (int li = 0; li < C.local_n; ++li) {                              // readers of the replica this copy overwrites
+        CKM(cudaSetDevice(C.devices[li]));
+        if (s_of[li] != bs) wait_scene_uses(*sc, C.devices[li], s_of[li]);
+    }
     CKM(cudaSetDevice(C.devices[0]));
+    wait_scene_uses(*sc, -1, bs);                                         // the peer copies below run on bs
     if (C.transport == RBRT_TRANSPORT_NCCL) {
         CKN(g_nccl.GroupStart());
         for (int li = 0; li < C.local_n; ++li)

@@ -24,7 +24,8 @@ void destroy_scene(Scene* sc);
 
 // multi.cu
 // Enqueues, behind the build on `build_stream`, the copy of replica 0's block to the scene's other replicas / ranks and records
-// every replica's `ready` event.
+// every replica's `ready` event.  Each copy first waits for the reads of the scene enqueued so far on its replica's device (an
+// update replicates again while frames of the old geometry may be in flight).
 int replicate_scene(Scene* sc, cudaStream_t build_stream);
 // The collective render (or, without a communicator, render + finalise on one GPU) with device outputs on rank 0.
 int render_frames(const Scene& sc, const rbrt_camera* cams, const uint64_t* seeds, uint32_t n_frames, uint32_t spp,

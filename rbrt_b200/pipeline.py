@@ -20,14 +20,30 @@ Every frame is computed by the same kernels on the same inputs as a lone render_
             ...
     rest = pipe.drain()
 
+Scene updates: a frame renders the scene as it was when the frame was SUBMITTED.  The library orders every update after the
+frames already enqueued against the scene, but a group that is still being collected (frames_per_batch > 1) has not been
+enqueued yet; so Scene.update_mesh / update_mesh_device / update_elements first launch the pending group of every live pipeline
+that holds frames of that scene.  The frames that left a pipeline on that occasion are returned by its next submit / flush / drain.
+
 Multi-GPU: under a library communicator (rbrt_gpu_init_multi, or rbrt_b200.dist.init_comm() for one process per GPU) every
 rank calls submit() in the same order; a group is ONE call of rbrt_gpu_render_frames_device — shard render, per-GPU
 finalise, gather on rank 0, all enqueued on the group's stream — and rank 0 gets the images.
 """
 import ctypes as C
+import weakref
 
 from . import _abi
 from .render import ImageBuffer, make_opts
+
+_live = weakref.WeakSet()      # every FramePipeline, for launch_pending
+
+
+def launch_pending(handle):
+    """Launch the pending group of every pipeline that holds frames of the scene with this library handle (before an update)."""
+    hv = handle.value if hasattr(handle, "value") else handle
+    for p in list(_live):
+        if p._pending and p._pending_hv == hv:
+            p._early = [*p._early, *p._launch()]
 
 
 class _Slot:
@@ -42,6 +58,8 @@ class _Slot:
 
 
 class FramePipeline:
+    _early = ()                  # frames that left the pipeline while an update launched the pending group (launch_pending)
+
     def __init__(self, width, height, depth=2, host_output=True, hdr=False, shard_mode=_abi.SHARD_TILES, frames_per_batch=1):
         import torch
         if depth not in (1, 2, 3, 4):
@@ -61,6 +79,7 @@ class FramePipeline:
         self._pending = []           # frames of the group being collected: (cam_c, seed, tag)
         self._pending_key = None     # (scene, spp, opts) the pending frames share
         self._pending_hv = None
+        _live.add(self)
 
     # ------------------------------------------------------------------ internals
     def _make_slot(self, host_output):
@@ -131,7 +150,7 @@ class FramePipeline:
         h = scene.handle() if hasattr(scene, "handle") else scene
         hv = h.value if hasattr(h, "value") else int(h)       # the same scene = the same library handle
         key = (scene, int(num_samples), tuple(sorted(opts.items())))
-        finished = []
+        finished, self._early = list(self._early), ()
         if self._pending and (self._pending_hv != hv or self._pending_key[1:] != key[1:]):
             finished += self._launch()
         self._pending_hv = hv
@@ -143,7 +162,8 @@ class FramePipeline:
 
     def flush(self):
         """Launch a partially filled group now; returns the frames that left the pipeline meanwhile."""
-        return self._launch() if self._pending else []
+        early, self._early = list(self._early), ()
+        return early + (self._launch() if self._pending else [])
 
     def drain(self):
         """Launch what is pending and wait for everything in flight; returns the (image, tag) in submission order."""

@@ -1,11 +1,34 @@
 """Scene — host mirror of rbrt_lib::scene::Scene (scene.rs:12-16): `elements` (spheres and BasicTriangles, any `Intersectable` of the reference that has a GPU twin),
 `triangle_meshes`, `lights` (dead in the reference, scene.rs:7-10).  The GPU scene (flattened SoA buffers
-+ one LBVH per mesh) is created lazily on first use and owned by this object."""
++ one LBVH per mesh) is created lazily on first use and owned by this object.
+
+Animation: `update_mesh` / `update_mesh_device` / `update_elements` change the scene in place (rbrt_gpu_scene_update_*): same
+triangle counts, same element kinds, no new device block and, by default, each mesh's tree refit rather than rebuilt.  Frames
+submitted before an update render the old geometry, frames submitted after it the new one (also through a FramePipeline, whose
+pending group is launched first).  The host mirror (`triangle_meshes`, `elements`) follows, so the CPU oracle sees the new scene."""
 import ctypes as C
 
 import numpy as np
 
 from . import _abi
+from .mesh import TriangleMesh
+
+
+class _DeviceTriangles(TriangleMesh):
+    """Host mirror of vertices handed in on the device (update_mesh_device): a device snapshot, copied to the host when first read."""
+
+    def __init__(self, snapshot, stream, material):
+        self._snap, self._stream, self._host = snapshot, stream, None
+        self.material = material
+
+    @property
+    def triangles(self):
+        if self._host is None:
+            import torch
+            with torch.cuda.stream(self._stream):
+                self._host = self._snap.cpu().numpy().reshape(-1, 3, 3)
+            self._snap = self._stream = None
+        return self._host
 
 
 def element_arrays(elements):
@@ -62,6 +85,55 @@ class Scene:
             self.close()
         except Exception:
             pass
+
+    # ---- updates in place (rbrt_gpu_scene_update_*) ----------------------------------------------
+    def _before_update(self):
+        from .pipeline import launch_pending
+        launch_pending(self._handle)                                   # frames already submitted keep the old geometry
+
+    def update_mesh(self, i, triangles, material=None, rebuild=False):
+        """New world-space vertices [N,3,3] for mesh i (N = its triangle count), optionally a new material; rebuild=True builds the
+        mesh's tree afresh instead of refitting it.  Returns once the vertices have been read."""
+        tris = np.ascontiguousarray(triangles, dtype=np.float32).reshape(-1, 3, 3)   # (held by the mirror like TriangleMesh holds it)
+        i = int(i)
+        mat = material if material is not None else (self.triangle_meshes[i].material if 0 <= i < len(self.triangle_meshes) else None)
+        if self._handle is not None:
+            self._before_update()
+            _abi.check(_abi.lib().rbrt_gpu_scene_update_mesh(self._handle, i, tris.ctypes.data, len(tris),
+                                                             C.byref(material.to_c()) if material is not None else None,
+                                                             _abi.UPDATE_REBUILD if rebuild else _abi.UPDATE_REFIT))
+        self.triangle_meshes[i] = TriangleMesh(tris, mat)
+
+    def update_mesh_device(self, i, tensor, material=None, rebuild=False, stream=None):
+        """The same from a CUDA float32 tensor [N,3,3] on the scene's device, read in order on `stream` (default: the current stream),
+        which then waits for the update: the tensor may be overwritten by work enqueued on that stream afterwards."""
+        import torch
+        if not (isinstance(tensor, torch.Tensor) and tensor.is_cuda and tensor.dtype == torch.float32):
+            raise TypeError("update_mesh_device takes a CUDA float32 tensor of shape [N,3,3]")
+        t = tensor.reshape(-1, 3, 3)
+        stream = stream or torch.cuda.current_stream()
+        i = int(i)
+        mat = material if material is not None else (self.triangle_meshes[i].material if 0 <= i < len(self.triangle_meshes) else None)
+        with torch.cuda.stream(stream):
+            t = t.contiguous()
+            snap = t.clone()                                           # the mirror's copy, taken before the caller may overwrite `tensor`
+        if self._handle is not None:
+            self._before_update()
+            _abi.check(_abi.lib().rbrt_gpu_scene_update_mesh_device(self._handle, i, t.data_ptr(), t.shape[0],
+                                                                    C.byref(material.to_c()) if material is not None else None,
+                                                                    _abi.UPDATE_REBUILD if rebuild else _abi.UPDATE_REFIT,
+                                                                    stream.cuda_stream))
+        self.triangle_meshes[i] = _DeviceTriangles(snap, stream, mat)
+
+    def update_elements(self, elements):
+        """New Scene.elements: the same number, the same kinds (Sphere / BasicTriangle) in the same order; positions, sizes and
+        materials may change."""
+        elements = list(elements)
+        if self._handle is not None:
+            self._before_update()
+            order, spheres, tris, ne, ns, nt = element_arrays(elements)
+            _abi.check(_abi.lib().rbrt_gpu_scene_update_elements(self._handle, order, ne, spheres, ns, tris, nt))
+        self.elements = elements
 
     # ---- Scene::hit (scene.rs:19-43) for caller-supplied rays ----------------------------------
     def hit(self, rays, trace_mode=_abi.TRACE_BVH, stats=None):
