@@ -84,7 +84,11 @@ typedef struct rbrt_element_ref { uint32_t kind; uint32_t index; } rbrt_element_
 
 /* = what TriangleMesh::new (mesh.rs:41-74) holds after load_mesh_vertices_from_file
  * (mesh.rs:78-121): world-space triangle soup, 9 floats per triangle (v0 v1 v2), already
- * scale -> rotate_point -> translate'd in f32.  One material per mesh (mesh.rs:24). */
+ * scale -> rotate_point -> translate'd in f32.  One material per mesh (mesh.rs:24).
+ * Coordinates: any f32 value, inf and NaN included; hits are the reference's at every extent.  The BVH culls on an axis only while
+ * its node grid step, (padded extent) / 65 500, is at most 2e6, i.e. up to a padded extent of about 1.3e11 on that axis (the padding is
+ * 2e-5 of the mesh's largest coordinate).  Beyond that the axis is not culled; from a largest coordinate or extent of about 3.3e15 on
+ * the padding alone exceeds it on every axis and the mesh is traversed like a brute-force sweep: exact, but slow. */
 typedef struct rbrt_mesh_desc {
     const float*  tri_vertices;   /* num_triangles * 9 floats, caller keeps ownership */
     uint64_t      num_triangles;

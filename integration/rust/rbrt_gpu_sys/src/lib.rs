@@ -21,6 +21,8 @@ pub const RBRT_MAT_DIELECTRIC: u32 = 2;
 #[repr(C)] #[derive(Copy, Clone, Debug)] pub struct RbrtSphereDesc { pub center: RbrtVec3, pub radius: f32, pub material: RbrtMaterial }
 #[repr(C)] #[derive(Copy, Clone, Debug)] pub struct RbrtTriangleDesc { pub corners: [RbrtVec3; 3], pub material: RbrtMaterial }
 #[repr(C)] #[derive(Copy, Clone, Debug)] pub struct RbrtElementRef { pub kind: u32, pub index: u32 }   // 0 sphere, 1 BasicTriangle
+/// A triangle soup, 9 f32 per triangle.  Any coordinate value is accepted (inf and NaN too) and hits stay exact; the BVH culls on an
+/// axis only while the padded extent there is at most about 1.3e11 (grid step 2e6), beyond that the axis is not culled (slower).
 #[repr(C)] #[derive(Copy, Clone, Debug)] pub struct RbrtMeshDesc { pub tri_vertices: *const f32, pub num_triangles: u64, pub material: RbrtMaterial }
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct RbrtRenderOpts { pub seed: u64, pub max_depth: u32, pub trace_mode: u32, pub shard_mode: u32, pub shard_rank: u32,

@@ -361,7 +361,8 @@ __global__ void k_mesh_setup(const int* __restrict__ mm, MeshDev proto, float pa
         float step = ext / 65500.0f;
         if (!(step > 1e-30f)) step = 1e-30f;
         bp->grid.step[k] = step; bp->grid.org[k] = (lo[k] - pad) - 8.0f * step;
-        md.qstep[k] = md.n_tris ? step : 0.0f; md.qorg[k] = md.n_tris ? bp->grid.org[k] : 0.0f;
+        // a step the slab test cannot take without overflow (huge extents, inf coordinates): NaN, the axis is not culled (common.cuh)
+        md.qstep[k] = md.n_tris ? (step <= RBRT_QSTEP_MAX ? step : __int_as_float(0x7FFFFFFF)) : 0.0f; md.qorg[k] = md.n_tris ? bp->grid.org[k] : 0.0f;
         bp->lo[k] = lo[k]; bp->inv_ext[k] = hi[k] > lo[k] ? 1.0f / (hi[k] - lo[k]) : 0.0f;
     }
     *out = md;

@@ -78,8 +78,16 @@ struct MeshDev {
     int32_t  root_ref;         // >=0 node index (relative to node_base), <0 leaf reference
     uint32_t nrm_base;         // first normal of this mesh in SceneDev::normals (original order)
     uint32_t elem;             // element id = num_spheres + mesh index (material lookup)
-    float qorg[3], qstep[3];   // 16-bit grid of this mesh's BVH node boxes: bound = qorg + q * qstep (bvh_build.cu)
+    float qorg[3], qstep[3];   // 16-bit grid of this mesh's BVH node boxes: bound = qorg + q * qstep (bvh_build.cu); qstep NaN: see below
 };
+
+// Largest grid step the slab test of intersect.cuh (ray_slabs / bvh4_step) evaluates without overflow.  It forms -2^23 * qstep * (1/d) with
+// |1/d| up to its clamp of 1e25 (a direction component of 0 or |d| <= 1e-25), and the node decode adds (2^23 + q) * qstep / d to that.
+// Above ~4.05e6 (a padded extent of ~2.65e11 on the axis) the product overflows to inf, every t of the axis becomes -inf or +inf and the
+// traversal rejects boxes the ray is inside: hits were lost.  2e6 keeps 2^23 * 2e6 * 1e25 = 1.68e38 below half of FLT_MAX, so nothing
+// overflows for an origin anywhere in the grid.  On an axis whose step is larger (or inf / NaN), the mesh set-up stores qstep = NaN: every
+// slab t of that axis is NaN, fminf / fmaxf ignore it, and the traversal culls on the other axes only (on none: every box is entered).
+#define RBRT_QSTEP_MAX 2.0e6f
 
 struct SceneDev {
     const float4* spheres;     // per ELEMENT of Scene.elements, in order: sphere {cx, cy, cz, r}; BasicTriangle {bits(index into etris), 0, 0, 0}

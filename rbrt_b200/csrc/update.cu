@@ -37,7 +37,7 @@ __global__ void k_upd_aabb(const float* __restrict__ raw, uint64_t n_vertices, i
     }
 }
 
-// ------------------------------------------------------------------ 2. MeshDev box + grid (= k_mesh_setup, bvh_build.cu:341-368)
+// ------------------------------------------------------------------ 2. MeshDev box + grid (= k_mesh_setup, bvh_build.cu:341-369)
 // Only lo/hi/qorg/qstep change; tri_base, n_tris, node_base, root_ref, nrm_base and elem are the device record's own.
 __global__ void k_upd_setup(const int* __restrict__ mm, uint32_t n_eff, float pad_rel, MeshDev* __restrict__ md_io, RefitParams* __restrict__ rp) {
     if (threadIdx.x || blockIdx.x) return;
@@ -51,13 +51,13 @@ __global__ void k_upd_setup(const int* __restrict__ mm, uint32_t n_eff, float pa
     // the relative padding with its floor of 2^-21 * (mx + 1000) (bvh_build.cu:357; profiles/r2_device_code.md)
     const float pad = pad_rel > 0.0f ? fmaxf(pad_rel * mx, 4.7683716e-7f * (mx + 1000.0f)) : 0.0f;
     rp->pad = pad;
-    for (int k = 0; k < 3; ++k) {                                          // bvh_build.cu:359-366
+    for (int k = 0; k < 3; ++k) {                                          // bvh_build.cu:359-367
         float ext = (hi[k] + pad) - (lo[k] - pad);
         float step = ext / 65500.0f;
         if (!(step > 1e-30f)) step = 1e-30f;
         const float org = (lo[k] - pad) - 8.0f * step;
         rp->step[k] = step; rp->org[k] = org;
-        md.qstep[k] = n_eff ? step : 0.0f; md.qorg[k] = n_eff ? org : 0.0f;
+        md.qstep[k] = n_eff ? (step <= RBRT_QSTEP_MAX ? step : __int_as_float(0x7FFFFFFF)) : 0.0f; md.qorg[k] = n_eff ? org : 0.0f;   // bvh_build.cu:365
     }
     *md_io = md;
 }
@@ -210,7 +210,7 @@ int rbrt_update_refit(const RefitArgs* a, void* scratch, cudaStream_t st) {
     float4* cbox = (float4*)(base + c.cbox);
     const int Bk = 256;
     k_upd_aabb_init<<<1, 32, 0, st>>>(mm);
-    if (a->n_all) k_upd_aabb<<<148 * 4, 256, 0, st>>>(a->raw, a->n_all * 3, mm);    // the build's grid (bvh_build.cu:470)
+    if (a->n_all) k_upd_aabb<<<148 * 4, 256, 0, st>>>(a->raw, a->n_all * 3, mm);    // the build's grid (bvh_build.cu:496)
     k_upd_setup<<<1, 32, 0, st>>>(mm, a->n_eff, a->pad_rel, a->mesh, rp);
     if (a->n_eff) k_upd_tris<<<(a->n_eff + Bk - 1) / Bk, Bk, 0, st>>>(a->raw, a->n_eff, rp, a->tris, a->normals, leaf_lo, leaf_hi);
     if (a->n_eff > 1) {                                                   // live_nodes (0 for a one-leaf mesh) is read on the device

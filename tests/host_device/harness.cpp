@@ -75,6 +75,7 @@ struct TreeBuilder {
     const std::vector<Box>& tb;                                // per triangle (already padded), in the order `order` lists them
     std::vector<uint32_t>& order;
     uint32_t leaf_size;
+    const float* step;                                         // the grid step of k_mesh_setup's BuildParams (md.qstep may be NaN)
     const MeshDev& md;
     std::vector<uint4>& out; size_t base;                      // nodes of this mesh start at out[4 * base]
     struct Part { uint32_t a, b; Box box; };                   // triangles order[a..b)
@@ -102,7 +103,7 @@ struct TreeBuilder {
         uint32_t q[4][3]; int32_t refs[4];
         for (size_t k = 0; k < 4; ++k) {
             if (k < kids.size()) {
-                for (int c = 0; c < 3; ++c) q[k][c] = quant_lo(kids[k].box.lo[c], md.qorg[c], md.qstep[c]) | (quant_hi(kids[k].box.hi[c], md.qorg[c], md.qstep[c]) << 16);
+                for (int c = 0; c < 3; ++c) q[k][c] = quant_lo(kids[k].box.lo[c], md.qorg[c], step[c]) | (quant_hi(kids[k].box.hi[c], md.qorg[c], step[c]) << 16);
                 if (kids[k].b - kids[k].a > leaf_size) { const uint32_t child = (uint32_t)(out.size() / 4 - base); out.resize(out.size() + 4); refs[k] = (int32_t)child; node(kids[k], child); }
                 else refs[k] = make_leaf_ref(kids[k].a, kids[k].b - kids[k].a);
             } else { q[k][0] = q[k][1] = q[k][2] = 0x0000FFFFu; refs[k] = make_leaf_ref(0, 1); }      // unused slot: inverted box
@@ -142,7 +143,7 @@ void flatten(HostScene& hs, const rbrt_element_ref* order, uint32_t ne, const rb
         MeshDev md; memset(&md, 0, sizeof(md));
         const uint64_t n_eff = tested_triangles(m.num_triangles, lanes);
         md.tri_base = (uint32_t)(hs.tris.size() / 3); md.n_tris = (uint32_t)n_eff; md.nrm_base = (uint32_t)hs.normals.size(); md.elem = ne + mi;
-        for (int k = 0; k < 3; ++k) { md.lo[k] = INFINITY; md.hi[k] = -INFINITY; }
+        for (int k = 0; k < 3; ++k) { md.lo[k] = 3.40282347e+38f; md.hi[k] = -3.40282347e+38f; }        // k_aabb_init: an axis with no number keeps them
         for (uint64_t t = 0; t < m.num_triangles; ++t) {
             const float* v = m.tri_vertices + 9 * t;
             for (int c = 0; c < 3; ++c) for (int k = 0; k < 3; ++k) { md.lo[k] = fminf(md.lo[k], v[3 * c + k]); md.hi[k] = fmaxf(md.hi[k], v[3 * c + k]); }   // aabbox.rs:62-88
@@ -151,23 +152,26 @@ void flatten(HostScene& hs, const rbrt_element_ref* order, uint32_t ne, const rb
         for (uint32_t t = 0; t < n_eff; ++t) order[t] = t;
         md.node_base = (uint32_t)(hs.nodes.size() / 4); md.root_ref = make_leaf_ref(0, 1);
         if (leaf_size && n_eff) {                                    // grid as k_mesh_setup lays it, then the tree; triangles go out in tree order
-            float mx = 0.0f;
+            float mx = 0.0f, grid_step[3];
             for (int k = 0; k < 3; ++k) { mx = fmaxf(mx, fmaxf(fabsf(md.lo[k]), fabsf(md.hi[k]))); mx = fmaxf(mx, md.hi[k] - md.lo[k]); }
             const float pad = pad_rel() > 0.0f ? fmaxf(pad_rel() * mx, (getenv("HD_NO_PAD_FLOOR") ? 0.0f : (getenv("HD_PAD_FLOOR") ? (float)atof(getenv("HD_PAD_FLOOR")) : 4.7683716e-7f) * (mx + 1000.0f))) : 0.0f;   // k_mesh_setup
             for (int k = 0; k < 3; ++k) {
                 float ext = (md.hi[k] + pad) - (md.lo[k] - pad), step = ext / 65500.0f;
                 if (!(step > 1e-30f)) step = 1e-30f;
-                md.qstep[k] = step; md.qorg[k] = (md.lo[k] - pad) - 8.0f * step;
+                md.qorg[k] = (md.lo[k] - pad) - 8.0f * step;
+                grid_step[k] = step;                                                                                  // the nodes are quantised on this grid...
+                md.qstep[k] = step <= RBRT_QSTEP_MAX ? step : NAN;                                                    // ...the traversal reads NaN where it would overflow
             }
             std::vector<Box> tb(n_eff);
             for (uint32_t t = 0; t < n_eff; ++t) {
                 const float* v = m.tri_vertices + 9 * (size_t)t;
-                Box b = empty_box();
-                for (int c = 0; c < 3; ++c) for (int k = 0; k < 3; ++k) { b.lo[k] = fminf(b.lo[k], v[3 * c + k]); b.hi[k] = fmaxf(b.hi[k], v[3 * c + k]); }
-                for (int k = 0; k < 3; ++k) { b.lo[k] -= pad; b.hi[k] += pad; }
+                Box b;
+                for (int k = 0; k < 3; ++k) {                                                                         // k_emit_tris' padded box
+                    b.lo[k] = fminf(v[k], fminf(v[3 + k], v[6 + k])) - pad; b.hi[k] = fmaxf(v[k], fmaxf(v[3 + k], v[6 + k])) + pad;
+                }
                 tb[t] = b;
             }
-            TreeBuilder B{tb, order, leaf_size, md, hs.nodes, md.node_base};
+            TreeBuilder B{tb, order, leaf_size, grid_step, md, hs.nodes, md.node_base};
             if (n_eff <= leaf_size) md.root_ref = make_leaf_ref(0, (uint32_t)n_eff);
             else { hs.nodes.resize(hs.nodes.size() + 4); md.root_ref = 0; B.node(B.part(0, (uint32_t)n_eff), 0); }
         }

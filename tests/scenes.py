@@ -180,3 +180,46 @@ def edge_aimed_rays(tris, n, dist, seed=0):
     d = target - o.astype(np.float64)
     d /= np.linalg.norm(d, axis=1, keepdims=True)
     return np.concatenate([o, d.astype(np.float32)], 1).astype(np.float32)
+
+
+EXTENT_CENTRE = (5.0, 1.4, -12.5)
+
+
+def far_triangle_mesh(far, axis=0):
+    """The 1280-triangle icosphere of small_mesh_scene, one small triangle whose corners lie at coordinate `far` on `axis` (inf and -inf
+    too), and seven copies of the first triangles: 1288 = 161 x 8, so the 8-lane tail rule drops nothing and every triangle is in the tree.
+    The far triangle stretches the mesh box, its padding and the node grid on that axis; the icosphere, where the rays hit, stays put."""
+    base = synth.displaced_icosphere(3, 3.0, EXTENT_CENTRE)
+    tri = np.zeros((1, 3, 3), np.float32)
+    tri[0, :, axis] = np.float32(far)
+    tri[0, 1, (axis + 1) % 3] = 1.0
+    tri[0, 2, (axis + 2) % 3] = 1.0
+    return np.concatenate([base, tri, base[:7]], 0).astype(np.float32)
+
+
+def scaled_mesh(extent):
+    """The icosphere of far_triangle_mesh scaled about the world origin until its box is `extent` wide; returns (triangles, scale)."""
+    base = synth.displaced_icosphere(3, 3.0, EXTENT_CENTRE).astype(np.float64)
+    s = extent / float(np.ptp(base.reshape(-1, 3), axis=0).max())
+    return (base * s).astype(np.float32), s
+
+
+def extent_rays(n, seed=0, tris=None):
+    """Four kinds of rays at the icosphere of far_triangle_mesh, n of each: random (random_rays: also axis-aligned, zero components,
+    un-normalised), edge-aimed from 30 units away, exactly axis-parallel (two zero components, either sign) and directions with one or two
+    components scaled down to 1e-30 ... 1e-5."""
+    rng = np.random.default_rng(seed)
+    c = np.asarray(EXTENT_CENTRE, np.float32)
+    tris = synth.displaced_icosphere(3, 3.0, EXTENT_CENTRE) if tris is None else tris
+    axis = np.zeros((n, 6), np.float32)
+    axis[:, :3] = c + rng.uniform(-3.5, 3.5, (n, 3)).astype(np.float32)
+    k = rng.integers(0, 3, n)
+    axis[np.arange(n), k] = c[k] - np.float32(20.0) * np.sign(rng.uniform(-1, 1, n)).astype(np.float32)
+    axis[np.arange(n), 3 + k] = np.sign(c[k] - axis[np.arange(n), k])
+    tiny = random_rays(n, EXTENT_CENTRE, 4.0, seed + 1)
+    tiny[:, 3:] = rng.normal(size=(n, 3)).astype(np.float32)
+    scale = (10.0 ** rng.uniform(-30, -5, (n, 2))).astype(np.float32)
+    tiny[np.arange(n), 3 + k] *= scale[:, 0]
+    two = rng.random(n) < 0.3
+    tiny[np.arange(n)[two], 3 + (k[two] + 1) % 3] *= scale[two, 1]
+    return np.concatenate([random_rays(n, EXTENT_CENTRE, 4.0, seed + 2), edge_aimed_rays(tris, n, 30.0, seed + 3), axis, tiny], 0).astype(np.float32)

@@ -434,3 +434,46 @@ def test_traversal_in_awkward_regimes(hd, oracle):
     assert set(np.unique(want["elem_idx"][want["kind"] == 1]).tolist()) == {0, 1} and (want["kind"] == 0).sum() > 100     # mesh 3 never beats its twin, mesh 1
     for leaf in (1, 17, 4):
         assert_hits(hd_hit(hd, several, rays, leaf), want, f"several meshes leaf {leaf}")
+
+
+EXTENT_FAR = (1e6, 1e9, 1e11, 1.4e11, 2.6e11, 3e11, 1e12, 1e15, 1e20, 1e25, 1e30, 1e35, 2e38, 3.4e38, np.inf)
+
+
+def test_traversal_at_extreme_mesh_extents(hd, oracle):
+    """Meshes whose box is huge on one axis: the icosphere of tests/scenes.py with ONE small triangle at coordinate `far` (1e6 ... 3.4e38, inf,
+    and negative) on each axis, and the icosphere scaled to extents 1e8 ... 1e36; rays of scenes.extent_rays (random, edge-aimed, exactly
+    axis-parallel, direction components down to 1e-30).  The BVH traversals must return the oracle's hits.
+
+    What went wrong first: ray_slabs (intersect.cuh) forms B' = (qorg - o) / d - 2^23 * qstep / d, with 1/d clamped to 1e25 for a direction
+    component of 0 or |d| <= 1e-25.  Once the grid step of an axis exceeds ~4.05e6 (a padded extent of ~2.65e11: far = 3e11 here) that product
+    overflows to inf, every slab t of the axis becomes -inf and rays with such a component reject the boxes they are in: before the fix, far =
+    2.6e11 (step 3.97e6) still passed and far = 3e11 lost 384 of these 4000 hits.  For other directions the same happens when
+    qstep / |d| > 4e31 (far = 2e38: every hit lost).  Up to step 2e6 (far = 1.3e11) the arithmetic stays finite and the one-step margin of the
+    quantisation covers B's rounding.  Beyond it k_mesh_setup stores qstep = NaN for the axis: its slab t is NaN, fminf / fmaxf drop it, and the
+    traversal culls on the remaining axes (common.cuh, RBRT_QSTEP_MAX).  The harness' builder applies the same rule."""
+    rays = S.extent_rays(1000, 5)
+    cases = [(far, 0) for far in EXTENT_FAR] + [(-far, 0) for far in (1e12, 1e20, 3.4e38, np.inf)]
+    cases += [(far, ax) for ax in (1, 2) for far in (1e11, 1e12, 1e20, 1e30, 2e38, -np.inf)]
+    for far, ax in cases:
+        scene = R.Scene()
+        scene.triangle_meshes.append(R.TriangleMesh.from_triangles(S.far_triangle_mesh(far, ax), R.Lambertian(Vec3(0.5, 0.5, 0.5))))
+        want = oracle.OracleScene.from_scene(scene).hit(rays)
+        assert (want["kind"] == 1).sum() > 1500, (far, ax)                  # the icosphere is hit
+        assert ((want["kind"] == 1)[2000:3000]).sum() > 300                  # ... also by the axis-parallel rays
+        for leaf in (1, 4, 17):
+            assert_hits(hd_hit(hd, scene, rays, leaf), want, f"far {far:g} on axis {ax} leaf {leaf}")
+    rng = np.random.default_rng(6)
+    for extent in (1e8, 1e12, 1e16, 1e20, 1e24, 1e28, 1e32, 1e36):
+        tris, _ = S.scaled_mesh(extent)
+        scene = R.Scene()
+        scene.triangle_meshes.append(R.TriangleMesh.from_triangles(tris, R.Lambertian(Vec3(0.5, 0.5, 0.5))))
+        # a hit counts up to dist 2000 (lib.rs:45): edge-aimed rays from 500 away, and axis-parallel ones at triangle centres from 500 away
+        target = tris[rng.integers(0, len(tris), 1500)].astype(np.float64).mean(1)
+        k = rng.integers(0, 3, 1500)
+        d = np.zeros((1500, 3)); d[np.arange(1500), k] = rng.choice([-1.0, 1.0], 1500)
+        r = np.concatenate([S.edge_aimed_rays(tris, 2500, 500.0, 7), np.concatenate([target - 500.0 * d, d], 1).astype(np.float32)], 0)
+        want = oracle.OracleScene.from_scene(scene).hit(r)
+        if extent <= 1e8:
+            assert (want["kind"] == 1).sum() > 1500, extent                  # (from ~1e10 on, ulp(|o|) > 500 and the origins snap onto the surface)
+        for leaf in (1, 4, 17):
+            assert_hits(hd_hit(hd, scene, r, leaf), want, f"mesh scaled to {extent:g} leaf {leaf}")
