@@ -376,6 +376,47 @@ int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rb
 int rbrt_gpu_primary_rays(const rbrt_camera* cam, uint64_t seed, uint32_t sample_idx,
                           rbrt_ray* rays_out);
 
+/* ---- first-hit AOVs (DESIGN.md section 11) -------------------------------------------------
+ * Geometric passes of the render's own camera rays: depth, shading normal, albedo, coverage and the ids of what each pixel sees.
+ * For pixel px = row*W + col and samples s = 0 .. num_samples-1 (S = num_samples):
+ *   r[px,s] = the camera ray rbrt_gpu_primary_rays(cam, seed, s) returns for px, bit for bit;
+ *   h[px,s] = Scene::hit(r), bit for bit what rbrt_gpu_trace_rays reports for that ray with RBRT_TRACE_BVH.
+ * A sample hits when h.kind != RBRT_HIT_NONE; a NaN ray, where the reference panics, is a miss and is counted in stats->nan_rays.
+ * With n_hit hit samples, every sum below is an f32 sum starting from +0, left to right in sample order over the hit samples only,
+ * followed by ONE IEEE division by the float n_hit:
+ *   coverage = n_hit / S (both as float);
+ *   depth    = sum of h.dist / n_hit, +inf when n_hit = 0;
+ *   normal   = sum of n / n_hit per component, 0 when n_hit = 0.  Mesh and BasicTriangle normals as stored (unit); a sphere's normal
+ *              p - c is divided per component by its length sqrt((x*x + y*y) + z*z).  No normal is flipped toward the ray, and the
+ *              mean is not renormalised;
+ *   albedo   = sum of a / n_hit per component, 0 when n_hit = 0: the hit element's material albedo for Lambertian and Metal (a mesh's
+ *              material for a mesh hit), (1,1,1) for Dielectric, the attenuation rbrt_gpu_scatter reports;
+ *   hit_kind, elem_idx, tri_idx = sample 0's hit as rbrt_hit reports it (RBRT_HIT_NONE, 0, 0 for a miss).
+ * The planes are row-major, W*H values (W*H*3 for normal and albedo, xyz per pixel).  A NULL member is not produced and not written. */
+typedef struct rbrt_aov_out {
+    float*    depth;      /* W*H */
+    float*    normal;     /* W*H*3 */
+    float*    albedo;     /* W*H*3 */
+    float*    coverage;   /* W*H */
+    int32_t*  hit_kind;   /* W*H, sample 0: RBRT_HIT_* */
+    uint32_t* elem_idx;   /* W*H, sample 0 */
+    uint32_t* tri_idx;    /* W*H, sample 0 */
+} rbrt_aov_out;
+/* HOST pointers; blocks until the passes are on the host.  The kernel lives in librbrt_gpu_aov.so, loaded at run time from this
+ * library's directory (RBRT_GPU_AOV_LIB: another path); without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL scene, camera or out, every member of out NULL, num_samples = 0, an empty image,
+ * a scene with a mesh whose tree was refused as too deep (the call waits for the scene's build to know).
+ * Ordered like a render: the call sees every update of the scene enqueued before it, and every later update waits for it.
+ * stats may be NULL; it reports rays = W*H*S, nan_rays, node_visits / tri_tests, ms_device, ms_d2h, ms_total and launches.
+ * Under a communicator the call is NOT collective: it runs on this process's first device (replica 0) over the whole image;
+ * AOVs are not sharded over GPUs. */
+int rbrt_gpu_render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint64_t seed,
+                        const rbrt_aov_out* out, rbrt_stats* stats);
+/* The same with DEVICE pointers on the scene's first device, enqueued on cuda_stream (0 = default stream).  stats == NULL: enqueue
+ * only, no synchronisation; with stats the call waits for the kernel and fills them. */
+int rbrt_gpu_render_aov_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint64_t seed,
+                               const rbrt_aov_out* d_out, void* cuda_stream, rbrt_stats* stats);
+
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
  * between renders and across scenes; this releases it (and the pooled scene blocks and the build scratch). */
 int rbrt_gpu_release_cache(void);

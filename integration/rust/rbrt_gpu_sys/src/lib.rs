@@ -36,6 +36,10 @@ pub struct RbrtSceneOpts { pub simd_lanes: u32, pub leaf_size: u32, pub box_pad_
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct RbrtCommInfo { pub active: i32, pub world: i32, pub rank: i32, pub local_devices: i32, pub transport: i32, pub nccl_version: i32,
                           pub devices: [i32; 16] }
+/// First-hit AOV planes (row-major, W*H values; W*H*3 for normal and albedo); a null member is not produced.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtAovOut { pub depth: *mut f32, pub normal: *mut f32, pub albedo: *mut f32, pub coverage: *mut f32, pub hit_kind: *mut i32,
+                        pub elem_idx: *mut u32, pub tri_idx: *mut u32 }
 pub enum RbrtScene {}
 pub const RBRT_MAX_FRAMES: u32 = 4;
 pub const RBRT_COMM_ID_BYTES: usize = 128;
@@ -106,6 +110,12 @@ extern "C" {
                                          stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_finalize_device(d_accum: *const c_void, width: u32, height: u32, num_samples: u32, d_rgb: *mut c_void,
                                     d_hdr: *mut c_void, stream: *mut c_void) -> c_int;
+    /// First-hit AOVs of the render's camera rays (depth, normal, albedo, coverage, sample 0's ids), host planes; the device variant
+    /// takes device planes and enqueues on `stream` (stats = null: no synchronisation).  Not collective: replica 0, whole image.
+    pub fn rbrt_gpu_render_aov(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, seed: u64, out: *const RbrtAovOut,
+                               stats: *mut RbrtStats) -> c_int;
+    pub fn rbrt_gpu_render_aov_device(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, seed: u64, d_out: *const RbrtAovOut,
+                                      stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

@@ -93,6 +93,11 @@ class StatsC(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class AovOutC(C.Structure):  # rbrt_aov_out: device or host planes, NULL = pass not produced
+    _fields_ = [("depth", C.c_void_p), ("normal", C.c_void_p), ("albedo", C.c_void_p), ("coverage", C.c_void_p),
+                ("hit_kind", C.c_void_p), ("elem_idx", C.c_void_p), ("tri_idx", C.c_void_p)]
+
+
 class SceneInfoC(C.Structure):
     _fields_ = [("num_spheres", C.c_uint32), ("num_meshes", C.c_uint32), ("num_triangles", C.c_uint64),
                 ("num_triangles_tested", C.c_uint64), ("num_bvh_nodes", C.c_uint64),
@@ -152,6 +157,8 @@ GPU_SIGNATURES = {
     "rbrt_gpu_finalize_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rbrt_gpu_trace_rays": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_primary_rays": (C.c_int, [P(CameraC), C.c_uint64, C.c_uint32, C.c_void_p]),
+    "rbrt_gpu_render_aov": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), P(StatsC)]),
+    "rbrt_gpu_render_aov_device": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

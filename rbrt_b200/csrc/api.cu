@@ -8,6 +8,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include "aov.cuh"
 #include "bvh_build.cuh"
 #include "engine.cuh"
 #include "multi.cuh"
@@ -225,20 +226,24 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
 // ------------------------------------------------------------------ scene updates (rbrt_gpu_scene_update_*)
 // The refit kernels live in their own device module, librbrt_gpu_update.so, loaded from this library's directory
 // (RBRT_GPU_UPDATE_LIB: another path).  Without it a refit is refused: there is no other implementation.
+// Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
+static int module_path(const char* env, const char* file, std::string* path) {
+    const char* e = getenv(env);
+    if (e && *e) { *path = e; return RBRT_OK; }
+    Dl_info di;
+    if (!dladdr((void*)&module_path, &di) || !di.dli_fname) { set_error("cannot locate librbrt_gpu.so to find %s", file); return RBRT_E_CUDA; }
+    *path = di.dli_fname;
+    const size_t slash = path->find_last_of('/');
+    *path = (slash == std::string::npos ? std::string(".") : path->substr(0, slash)) + "/" + file;
+    return RBRT_OK;
+}
+
 struct UpdateModule { void* h = nullptr; rbrt_update_scratch_bytes_fn scratch_bytes = nullptr; rbrt_update_refit_fn refit = nullptr; };
 static int update_module(const UpdateModule** out) {
     static UpdateModule m;
     if (!m.h) {
         std::string path;
-        const char* env = getenv("RBRT_GPU_UPDATE_LIB");
-        if (env && *env) path = env;
-        else {
-            Dl_info di;
-            if (!dladdr((void*)&update_module, &di) || !di.dli_fname) { set_error("cannot locate librbrt_gpu.so to find librbrt_gpu_update.so"); return RBRT_E_CUDA; }
-            path = di.dli_fname;
-            const size_t slash = path.find_last_of('/');
-            path = (slash == std::string::npos ? std::string(".") : path.substr(0, slash)) + "/librbrt_gpu_update.so";
-        }
+        { int rc = module_path("RBRT_GPU_UPDATE_LIB", "librbrt_gpu_update.so", &path); if (rc) return rc; }
         void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
         if (!h) { set_error("the refit module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", path.c_str(), dlerror()); return RBRT_E_CUDA; }
         UpdateModule n; n.h = h;
@@ -363,6 +368,119 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
         CKA(cudaStreamWaitEvent(user_st, sc->upd_out, 0));
     }
     if (uploaded) CKA(cudaEventSynchronize(uploaded));                    // the caller's array has been read (copy engine: no wait for busy SMs)
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ first-hit AOVs (rbrt_gpu_render_aov*)
+// The AOV kernel lives in its own device module, librbrt_gpu_aov.so (RBRT_GPU_AOV_LIB: another path), like the refit.
+struct AovModule { void* h = nullptr; rbrt_aov_launch_fn launch = nullptr; };
+static int aov_module(const AovModule** out) {
+    static AovModule m;
+    if (!m.h) {
+        std::string path;
+        { int rc = module_path("RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", &path); if (rc) return rc; }
+        void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
+        if (!h) { set_error("the AOV module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", path.c_str(), dlerror()); return RBRT_E_CUDA; }
+        AovModule n; n.h = h;
+        *(void**)(&n.launch) = dlsym(h, "rbrt_aov_launch");
+        if (!n.launch) { set_error("%s lacks the AOV entry point", path.c_str()); dlclose(h); return RBRT_E_CUDA; }
+        m = n;
+    }
+    *out = &m;
+    return RBRT_OK;
+}
+
+// Per device: the planes of the host-pointer variant (grown, never shrunk, until rbrt_gpu_release_cache), the counters and the
+// events.  Only calls that synchronise before returning use them, so one set per device serves every call.
+struct AovPool { char* buf = nullptr; size_t bytes = 0; unsigned long long* ctr = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr; };
+static AovPool g_aov[64];
+static void aov_release_all() {
+    int cur = 0; cudaGetDevice(&cur);
+    for (int d = 0; d < 64; ++d) {
+        AovPool& p = g_aov[d];
+        if (!p.buf && !p.ctr && !p.e0) continue;
+        cudaSetDevice(d);
+        cudaFree(p.buf); cudaFree(p.ctr);
+        if (p.e0) cudaEventDestroy(p.e0);
+        if (p.e1) cudaEventDestroy(p.e1);
+        p = AovPool();
+    }
+    cudaSetDevice(cur);
+}
+
+static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t spp, uint64_t seed, const rbrt_aov_out* out, bool host,
+                      cudaStream_t st, rbrt_stats* stats) {
+    if (!scene || !cam || !out) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!out->depth && !out->normal && !out->albedo && !out->coverage && !out->hit_kind && !out->elem_idx && !out->tri_idx) {
+        set_error("no AOV requested (every member of the output is NULL)"); return RBRT_E_INVALID;
+    }
+    const uint64_t n = (uint64_t)cam->img_width_pix * cam->img_height_pix;
+    if (!n || !spp) { set_error("empty image or zero samples"); return RBRT_E_INVALID; }
+    if (n > 0xFFFFFFFFull) { set_error("more than 2^32 - 1 pixels"); return RBRT_E_INVALID; }
+    const Scene& sc = *reinterpret_cast<const Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device, whole image
+    CKA(cudaSetDevice(rp.device));
+    const double t0 = now_ms();
+    if (stats) memset(stats, 0, sizeof(*stats));
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    const AovModule* am = nullptr;
+    { int rc = aov_module(&am); if (rc) return rc; }
+
+    AovPool& pool = g_aov[rp.device & 63];
+    AovArgs a;
+    memset(&a, 0, sizeof(a));
+    a.S = rp.dev; a.cam = make_cam(*cam); a.key0 = (uint32_t)seed; a.key1 = (uint32_t)(seed >> 32); a.n_samples = spp;
+    a.tiles_x = (cam->img_width_pix + 7) / 8; a.tiles_total = a.tiles_x * ((cam->img_height_pix + 3) / 4);
+    a.out = *out;
+    if (host) {                                                           // the requested planes, carved from the pooled block
+        const size_t b1 = a256(4 * n), b3 = a256(12 * n);
+        const size_t need = (out->depth ? b1 : 0) + (out->normal ? b3 : 0) + (out->albedo ? b3 : 0) + (out->coverage ? b1 : 0) +
+                            (out->hit_kind ? b1 : 0) + (out->elem_idx ? b1 : 0) + (out->tri_idx ? b1 : 0);
+        if (pool.bytes < need) {
+            cudaFree(pool.buf); pool.buf = nullptr; pool.bytes = 0;
+            CKA(cudaMalloc(&pool.buf, need)); pool.bytes = need;
+        }
+        char* p = pool.buf;
+        auto take = [&](const void* want, size_t b) -> char* { if (!want) return nullptr; char* q = p; p += b; return q; };
+        a.out.depth = (float*)take(out->depth, b1); a.out.normal = (float*)take(out->normal, b3); a.out.albedo = (float*)take(out->albedo, b3);
+        a.out.coverage = (float*)take(out->coverage, b1); a.out.hit_kind = (int32_t*)take(out->hit_kind, b1);
+        a.out.elem_idx = (uint32_t*)take(out->elem_idx, b1); a.out.tri_idx = (uint32_t*)take(out->tri_idx, b1);
+    }
+    if (stats) {
+        if (!pool.ctr) CKA(cudaMalloc(&pool.ctr, 8 * AOV_ST_COUNT));
+        if (!pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
+        a.stats = pool.ctr;
+    }
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    if (stats) { CKA(cudaMemsetAsync(pool.ctr, 0, 8 * AOV_ST_COUNT, st)); CKA(cudaEventRecord(pool.e0, st)); }
+    CKA((cudaError_t)am->launch(&a, st));
+    if (stats) CKA(cudaEventRecord(pool.e1, st));
+    note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
+    if (!host && !stats) return RBRT_OK;                                  // enqueue only
+
+    if (stats) CKA(cudaEventSynchronize(pool.e1));
+    const double t1 = now_ms();
+    if (host) {
+        if (out->depth) CKA(cudaMemcpyAsync(out->depth, a.out.depth, 4 * n, cudaMemcpyDeviceToHost, st));
+        if (out->normal) CKA(cudaMemcpyAsync(out->normal, a.out.normal, 12 * n, cudaMemcpyDeviceToHost, st));
+        if (out->albedo) CKA(cudaMemcpyAsync(out->albedo, a.out.albedo, 12 * n, cudaMemcpyDeviceToHost, st));
+        if (out->coverage) CKA(cudaMemcpyAsync(out->coverage, a.out.coverage, 4 * n, cudaMemcpyDeviceToHost, st));
+        if (out->hit_kind) CKA(cudaMemcpyAsync(out->hit_kind, a.out.hit_kind, 4 * n, cudaMemcpyDeviceToHost, st));
+        if (out->elem_idx) CKA(cudaMemcpyAsync(out->elem_idx, a.out.elem_idx, 4 * n, cudaMemcpyDeviceToHost, st));
+        if (out->tri_idx) CKA(cudaMemcpyAsync(out->tri_idx, a.out.tri_idx, 4 * n, cudaMemcpyDeviceToHost, st));
+        CKA(cudaStreamSynchronize(st));
+    }
+    const double t2 = now_ms();
+    if (stats) {
+        unsigned long long h[AOV_ST_COUNT];
+        CKA(cudaMemcpyAsync(h, pool.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+        CKA(cudaStreamSynchronize(st));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+        stats->rays = n * spp; stats->paths = n * spp; stats->nan_rays = h[AOV_ST_NAN];
+        stats->node_visits = h[AOV_ST_NODES]; stats->tri_tests = h[AOV_ST_TRIS];
+        stats->ms_device = ms; stats->ms_d2h = host ? t2 - t1 : 0.0; stats->launches = 1;
+        stats->ms_total = now_ms() - t0;
+    }
     return RBRT_OK;
 }
 
@@ -663,6 +781,7 @@ int rbrt_gpu_release_cache(void) {
     release_device_wave_buffers();
     release_dist_buffers();
     release_build_scratch();
+    aov_release_all();
     arena_release_all();
     for (void* p : g_pinned_free) cudaFreeHost(p);
     g_pinned_free.clear();
@@ -797,6 +916,18 @@ done:
     if (e1) cudaEventDestroy(e1);
     cudaFree(d_rays); cudaFree(d_hits); cudaFree(d_stats);
     return rc;
+}
+
+int rbrt_gpu_render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint64_t seed, const rbrt_aov_out* out,
+                        rbrt_stats* stats) {
+    LOCK;
+    return render_aov(scene, cam, num_samples, seed, out, true, 0, stats);
+}
+
+int rbrt_gpu_render_aov_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint64_t seed, const rbrt_aov_out* d_out,
+                               void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return render_aov(scene, cam, num_samples, seed, d_out, false, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

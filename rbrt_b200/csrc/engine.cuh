@@ -137,6 +137,7 @@ int finalize(const float4* d_accum, uint32_t W, uint32_t H, uint32_t spp, uint8_
 int trace_rays_device(const Scene& sc, const rbrt_ray* d_rays, uint64_t n, uint32_t mode, rbrt_hit* d_hits,
                       unsigned long long* d_stats, cudaStream_t st);
 int primary_rays_device(const rbrt_camera& cam, uint64_t seed, uint32_t sample, rbrt_ray* d_rays, cudaStream_t st);
+CamDev make_cam(const rbrt_camera& c);       // the kernels' view of a camera
 void free_wave_buffers(WaveBuffers& wb);
 // Per-device pool of wavefront state, shared by every scene of the process and kept between renders (allocating and
 // freeing tens of GB per render would cost more than the render).  The library is single-threaded per device.

@@ -225,6 +225,22 @@ bool save_image(const std::string& path, const std::vector<uint8_t>& rgb, uint32
     return fclose(fp) == 0 && ok;
 }
 
+// Portable float map (little-endian): "PF" (3 channels) or "Pf" (1), width height, scale -1 (negative = little-endian), rows bottom to top.
+bool save_pfm(const std::string& path, const float* v, uint32_t w, uint32_t h, int channels) {
+    FILE* fp = fopen(path.c_str(), "wb");
+    if (!fp) return false;
+    bool ok = fprintf(fp, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", w, h) > 0;
+    const uint16_t probe = 1;
+    const bool little = *(const uint8_t*)&probe == 1;
+    std::vector<float> row((size_t)w * channels);
+    for (uint32_t y = h; ok && y-- > 0;) {
+        memcpy(row.data(), v + (size_t)y * w * channels, row.size() * 4);
+        if (!little) for (float& f : row) { uint32_t u; memcpy(&u, &f, 4); u = __builtin_bswap32(u); memcpy(&f, &u, 4); }
+        ok = fwrite(row.data(), 4, row.size(), fp) == row.size();
+    }
+    return fclose(fp) == 0 && ok;
+}
+
 void usage() {
     printf("a lighweight raytracer written in rust\n\nUsage: rbrt [OPTIONS]\n\nOptions:\n"
            "  -t, --target_file <target_file>  file that will be created witht he rendered output [default: dbg_out.png]\n"
@@ -239,6 +255,9 @@ void usage() {
            "      --check                      (extension) parse the scene, print a summary and exit without rendering\n"
            "      --dump                       (extension, with --check) also print every blueprint field as read (f32 bit patterns)\n"
            "      --from-ppm <file>            (extension) no rendering: read a binary PPM (P6) and save it as --target_file (format by extension)\n"
+           "      --aov <prefix>               (extension) after the render also write first-hit AOVs of the same camera and --seed:\n"
+           "                                   <prefix>.depth.pfm, <prefix>.normal.pfm, <prefix>.albedo.pfm, <prefix>.coverage.pfm\n"
+           "      --aov-samples <n>            (extension) samples per pixel of the AOVs [default: --samples]\n"
            "  -h, --help                       Print help\n  -V, --version                    Print version\n");
 }
 
@@ -256,7 +275,8 @@ int main(int argc, char** argv) {
     uint32_t height = 600, width = 800, samples = 5;
     uint64_t seed = 0; int device = 0; bool check_only = false, dump = false;
     uint32_t gpus = 1; int transport = RBRT_TRANSPORT_AUTO;
-    std::string from_ppm;
+    std::string from_ppm, aov;
+    uint32_t aov_samples = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         auto value = [&](const char* name) -> const char* {
@@ -282,6 +302,8 @@ int main(int argc, char** argv) {
         else if (key == "--check") check_only = true;
         else if (key == "--dump") dump = true;
         else if (key == "--from-ppm") from_ppm = value("--from-ppm");
+        else if (key == "--aov") aov = value("--aov");
+        else if (key == "--aov-samples") aov_samples = parse_u32(value("--aov-samples"), "--aov-samples");
         else if (key == "-h" || key == "--help") { usage(); return 0; }
         else if (key == "-V" || key == "--version") { printf("rbrt 0.1 (%s)\n", rbrt_gpu_version()); return 0; }
         else { fprintf(stderr, "error: unexpected argument '%s' found\n", a.c_str()); return 2; }
@@ -353,9 +375,26 @@ int main(int argc, char** argv) {
     rbrt_stats st;
     if (rbrt_gpu_render(scene, &cam, samples, &opts, rgb.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
     printf("\rRendering 100%% complete!\n");                                        // lib.rs:114
+    std::vector<float> depth, normal, albedo, coverage;
+    if (!aov.empty()) {                                                            // first-hit AOVs of the same camera rays (include/rbrt_gpu.h)
+        const size_t n = (size_t)width * height;
+        depth.resize(n); normal.resize(3 * n); albedo.resize(3 * n); coverage.resize(n);
+        rbrt_aov_out ao; memset(&ao, 0, sizeof(ao));
+        ao.depth = depth.data(); ao.normal = normal.data(); ao.albedo = albedo.data(); ao.coverage = coverage.data();
+        if (rbrt_gpu_render_aov(scene, &cam, aov_samples ? aov_samples : samples, seed, &ao, nullptr) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
+    }
     rbrt_gpu_scene_destroy(scene);
     printf("Saving rendered image to %s\n", target.c_str());                        // main.rs:84
     if (!save_image(target, rgb, width, height)) die("Unable to save target img to " + target + "! Maybe the directory does not exist?");   // main.rs:86-91
+    if (!aov.empty()) {
+        const struct { const char* name; const std::vector<float>& v; int ch; } planes[] = {
+            {"depth", depth, 1}, {"normal", normal, 3}, {"albedo", albedo, 3}, {"coverage", coverage, 1}};
+        for (const auto& p : planes) {
+            const std::string path = aov + "." + p.name + ".pfm";
+            printf("Saving %s AOV to %s\n", p.name, path.c_str());
+            if (!save_pfm(path, p.v.data(), width, height, p.ch)) die("Unable to save AOV to " + path + "! Maybe the directory does not exist?");
+        }
+    }
     fprintf(stderr, "[rbrt_b200] %llu rays, %llu samples in %.1f ms on %u GPU%s (%.1f Mrays/s)\n", (unsigned long long)st.rays,
             (unsigned long long)st.paths, st.ms_device, gpus, gpus > 1 ? "s" : "", st.ms_device > 0 ? st.rays / st.ms_device / 1e3 : 0.0);
     return 0;

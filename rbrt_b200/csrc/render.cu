@@ -870,7 +870,7 @@ __global__ void __launch_bounds__(256) k_rays_collect(WaveParams P, const rbrt_r
 }
 
 // ====================================================================== host side
-static CamDev make_cam(const rbrt_camera& c) {
+CamDev make_cam(const rbrt_camera& c) {
     CamDev d;
     d.pos[0] = c.position.x; d.pos[1] = c.position.y; d.pos[2] = c.position.z;
     d.right[0] = c.right.x; d.right[1] = c.right.y; d.right[2] = c.right.z;

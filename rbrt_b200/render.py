@@ -142,3 +142,53 @@ def primary_rays(cam, seed=0, sample_idx=0):
     rays = np.empty((cam.img_width_pix * cam.img_height_pix, 6), dtype=np.float32)
     _abi.check(_abi.lib().rbrt_gpu_primary_rays(cam.to_c(), int(seed), int(sample_idx), rays.ctypes.data))
     return rays
+
+
+# ---- first-hit AOVs (rbrt_gpu_render_aov*, include/rbrt_gpu.h and DESIGN.md section 11) ----------------------------------
+AOV_PASSES = ("depth", "normal", "albedo", "coverage", "ids")
+# pass -> [(plane, numpy dtype, components)]; "ids" is sample 0's hit_kind / elem_idx / tri_idx
+_AOV_PLANES = {"depth": [("depth", np.float32, 1)], "normal": [("normal", np.float32, 3)], "albedo": [("albedo", np.float32, 3)],
+               "coverage": [("coverage", np.float32, 1)],
+               "ids": [("hit_kind", np.int32, 1), ("elem_idx", np.uint32, 1), ("tri_idx", np.uint32, 1)]}
+
+
+def _aov_planes(passes):
+    if isinstance(passes, str):
+        passes = (passes,)
+    unknown = [p for p in passes if p not in _AOV_PLANES]
+    if unknown:
+        raise ValueError(f"unknown AOV pass(es) {unknown}; choose from {AOV_PASSES}")
+    return [pl for p in dict.fromkeys(passes) for pl in _AOV_PLANES[p]]
+
+
+def render_aovs(cam, num_samples, scene, seed=0, passes=AOV_PASSES, stats=None):
+    """First-hit AOVs of the render's own camera rays: a dict of numpy arrays, [H,W] for depth / coverage / hit_kind / elem_idx /
+    tri_idx and [H,W,3] for normal / albedo ("ids" gives the last three).  Blocks until they are on the host."""
+    W, H = cam.img_width_pix, cam.img_height_pix
+    out, arrays = _abi.AovOutC(), {}
+    for name, dt, k in _aov_planes(passes):
+        arrays[name] = np.empty((H, W, k) if k > 1 else (H, W), dtype=dt)
+        setattr(out, name, arrays[name].ctypes.data)
+    st = _abi.StatsC()
+    _abi.check(_abi.lib().rbrt_gpu_render_aov(scene.handle(), cam.to_c(), int(num_samples), int(seed) & 0xFFFFFFFFFFFFFFFF, out, st))
+    if stats is not None:
+        stats.update(st.as_dict())
+    return arrays
+
+
+def render_aovs_device(cam, num_samples, scene, seed=0, passes=AOV_PASSES, stream=None):
+    """The same as CUDA tensors on the scene's first device, enqueued on `stream` (default: the current stream); returns without
+    synchronising."""
+    import torch
+    stream = stream or torch.cuda.current_stream()
+    W, H = cam.img_width_pix, cam.img_height_pix
+    tdt = {np.float32: torch.float32, np.int32: torch.int32, np.uint32: torch.uint32}
+    out, tensors = _abi.AovOutC(), {}
+    handle = scene.handle()
+    with torch.cuda.stream(stream):
+        for name, dt, k in _aov_planes(passes):
+            tensors[name] = torch.empty((H, W, k) if k > 1 else (H, W), dtype=tdt[dt], device=stream.device)
+            setattr(out, name, tensors[name].data_ptr())
+    _abi.check(_abi.lib().rbrt_gpu_render_aov_device(handle, cam.to_c(), int(num_samples), int(seed) & 0xFFFFFFFFFFFFFFFF, out,
+                                                     stream.cuda_stream, None))
+    return tensors
