@@ -417,8 +417,41 @@ int rbrt_gpu_render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_
 int rbrt_gpu_render_aov_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint64_t seed,
                                const rbrt_aov_out* d_out, void* cuda_stream, rbrt_stats* stats);
 
+/* ---- ray queries on device memory (DESIGN.md section 12) -----------------------------------
+ * Scene::hit for rays the caller made, with rays and results in device memory, enqueued on the caller's stream.  Let h[i] be what
+ * rbrt_gpu_trace_rays(scene, rays, n, RBRT_TRACE_BVH, ...) reports for ray i.
+ *   closest:  each requested plane holds, bit for bit, the matching field of h[i] (kind RBRT_HIT_*, the sphere normal un-normalised,
+ *             zeros and RBRT_HIT_NONE for a miss).  A NaN ray (a NaN sphere discriminant, where the reference panics) is a miss and
+ *             is counted in stats->nan_rays.
+ *   occluded: d_occluded[i] = 1 when h[i] is a hit and h[i].dist < max_dist[i] (strict; a NaN max_dist gives 0), 2 when ray i is a NaN
+ *             ray whatever else it hits, 0 otherwise.  The traversal may stop at the first triangle that proves it.
+ * Rays, bounds and planes are DEVICE memory on the scene's first device.  Both calls are enqueued on cuda_stream (0 = default stream):
+ * stats == NULL returns without synchronising; with stats the call waits and fills rays, nan_rays, node_visits, tri_tests, ms_device,
+ * ms_total and launches.  Ordered like a render: a call sees every update of the scene enqueued before it, and every later update waits
+ * for it.  Under a communicator the call runs on replica 0 and is not collective.  n = 0 returns RBRT_OK, nothing written.
+ * The kernels live in librbrt_gpu_query.so, loaded at run time from this library's directory (RBRT_GPU_QUERY_LIB: another path); without
+ * it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL scene, rays or output with n > 0, every plane of the output NULL, n > 2^32 - 1,
+ * rays or outputs in another device's memory or in unregistered host memory, a scene with a mesh whose tree was refused as too deep. */
+typedef struct rbrt_query_out {      /* device planes, n entries each (point / normal: n*3); NULL = not produced, not written */
+    float*    t;
+    float*    dist;
+    int32_t*  kind;                  /* RBRT_HIT_* */
+    uint32_t* elem_idx;
+    uint32_t* tri_idx;
+    float*    point;
+    float*    normal;
+} rbrt_query_out;
+int rbrt_gpu_query_closest_device(const rbrt_scene* scene, const rbrt_ray* d_rays, uint64_t n,
+                                  const rbrt_query_out* d_out, void* cuda_stream, rbrt_stats* stats);
+/* d_max_dist: n values, or NULL = +inf for every ray.  d_occluded[i]: one of */
+enum { RBRT_QUERY_CLEAR = 0, RBRT_QUERY_OCCLUDED = 1, RBRT_QUERY_NAN_RAY = 2 };
+int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_rays, uint64_t n,
+                                   const float* d_max_dist,
+                                   uint8_t* d_occluded, void* cuda_stream, rbrt_stats* stats);
+
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
- * between renders and across scenes; this releases it (and the pooled scene blocks and the build scratch). */
+ * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch and the query counters). */
 int rbrt_gpu_release_cache(void);
 
 /* Upper bound, in bytes, of ONE pool of wavefront state (there are up to four per device, one per frame in flight).

@@ -40,7 +40,20 @@ pub struct RbrtCommInfo { pub active: i32, pub world: i32, pub rank: i32, pub lo
 #[repr(C)] #[derive(Copy, Clone, Debug)]
 pub struct RbrtAovOut { pub depth: *mut f32, pub normal: *mut f32, pub albedo: *mut f32, pub coverage: *mut f32, pub hit_kind: *mut i32,
                         pub elem_idx: *mut u32, pub tri_idx: *mut u32 }
+/// Ray-query planes in device memory (n values each; n*3 for point and normal); a null member is not produced.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtQueryOut { pub t: *mut f32, pub dist: *mut f32, pub kind: *mut i32, pub elem_idx: *mut u32, pub tri_idx: *mut u32,
+                          pub point: *mut f32, pub normal: *mut f32 }
 pub enum RbrtScene {}
+/// `kind` of a hit (rbrt_hit, rbrt_query_out)
+pub const RBRT_HIT_NONE: i32 = -1;
+pub const RBRT_HIT_SPHERE: i32 = 0;
+pub const RBRT_HIT_MESH: i32 = 1;
+pub const RBRT_HIT_TRIANGLE: i32 = 2;
+/// values of rbrt_gpu_query_occluded_device's output
+pub const RBRT_QUERY_CLEAR: u8 = 0;
+pub const RBRT_QUERY_OCCLUDED: u8 = 1;
+pub const RBRT_QUERY_NAN_RAY: u8 = 2;
 pub const RBRT_MAX_FRAMES: u32 = 4;
 pub const RBRT_COMM_ID_BYTES: usize = 128;
 pub const RBRT_TRANSPORT_AUTO: c_int = 0;
@@ -116,6 +129,14 @@ extern "C" {
                                stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_render_aov_device(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, seed: u64, d_out: *const RbrtAovOut,
                                       stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// Scene::hit for rays in device memory, each requested plane bit for bit the field rbrt_gpu_trace_rays reports; enqueued on `stream`
+    /// (stats = null: no synchronisation).  Not collective: replica 0.
+    pub fn rbrt_gpu_query_closest_device(scene: *const RbrtScene, d_rays: *const RbrtRay, n: u64, d_out: *const RbrtQueryOut,
+                                         stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// Occlusion for rays in device memory: RBRT_QUERY_OCCLUDED where Scene::hit is a hit with dist < max_dist (null = +inf),
+    /// RBRT_QUERY_NAN_RAY for a NaN ray, else RBRT_QUERY_CLEAR.
+    pub fn rbrt_gpu_query_occluded_device(scene: *const RbrtScene, d_rays: *const RbrtRay, n: u64, d_max_dist: *const f32,
+                                          d_occluded: *mut u8, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

@@ -98,6 +98,11 @@ class AovOutC(C.Structure):  # rbrt_aov_out: device or host planes, NULL = pass 
                 ("hit_kind", C.c_void_p), ("elem_idx", C.c_void_p), ("tri_idx", C.c_void_p)]
 
 
+class QueryOutC(C.Structure):  # rbrt_query_out: device planes, NULL = not produced
+    _fields_ = [("t", C.c_void_p), ("dist", C.c_void_p), ("kind", C.c_void_p), ("elem_idx", C.c_void_p), ("tri_idx", C.c_void_p),
+                ("point", C.c_void_p), ("normal", C.c_void_p)]
+
+
 class SceneInfoC(C.Structure):
     _fields_ = [("num_spheres", C.c_uint32), ("num_meshes", C.c_uint32), ("num_triangles", C.c_uint64),
                 ("num_triangles_tested", C.c_uint64), ("num_bvh_nodes", C.c_uint64),
@@ -120,6 +125,7 @@ OPT_COUNT_VISITS, OPT_TIME_KERNELS, OPT_NO_TAIL_KERNEL, OPT_POOL_SHIFT, OPT_SPLI
 MAX_FRAMES = 4          # frames one wavefront batch can hold (rbrt_gpu_render_accum_device_frames)
 HIT_NONE, HIT_SPHERE, HIT_MESH, HIT_TRIANGLE = -1, 0, 1, 2
 ELEM_SPHERE, ELEM_TRIANGLE = 0, 1
+QUERY_CLEAR, QUERY_OCCLUDED, QUERY_NAN_RAY = 0, 1, 2
 UPDATE_REFIT, UPDATE_REBUILD = 0, 1
 E_INVALID, E_CUDA, E_NODEVICE = 1, 2, 3
 
@@ -159,6 +165,8 @@ GPU_SIGNATURES = {
     "rbrt_gpu_primary_rays": (C.c_int, [P(CameraC), C.c_uint64, C.c_uint32, C.c_void_p]),
     "rbrt_gpu_render_aov": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), P(StatsC)]),
     "rbrt_gpu_render_aov_device": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_query_closest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, P(QueryOutC), C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_query_occluded_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

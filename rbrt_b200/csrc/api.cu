@@ -12,6 +12,7 @@
 #include "bvh_build.cuh"
 #include "engine.cuh"
 #include "multi.cuh"
+#include "query.cuh"
 #include "update.cuh"
 
 namespace rbrt {
@@ -371,25 +372,26 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
     return RBRT_OK;
 }
 
-// ------------------------------------------------------------------ first-hit AOVs (rbrt_gpu_render_aov*)
-// The AOV kernel lives in its own device module, librbrt_gpu_aov.so (RBRT_GPU_AOV_LIB: another path), like the refit.
-struct AovModule { void* h = nullptr; rbrt_aov_launch_fn launch = nullptr; };
-static int aov_module(const AovModule** out) {
-    static AovModule m;
-    if (!m.h) {
+// ------------------------------------------------------------------ device modules with one launch entry point
+// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path) and the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB) live
+// in their own device modules, like the refit; each is opened once, on first use.
+struct LaunchModule { const char* env; const char* file; const char* what; const char* symbol; void* launch; };
+static LaunchModule g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", "rbrt_aov_launch", nullptr};
+static LaunchModule g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", "rbrt_query_launch", nullptr};
+static int load_module(LaunchModule& m) {
+    if (!m.launch) {
         std::string path;
-        { int rc = module_path("RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", &path); if (rc) return rc; }
+        { int rc = module_path(m.env, m.file, &path); if (rc) return rc; }
         void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
-        if (!h) { set_error("the AOV module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", path.c_str(), dlerror()); return RBRT_E_CUDA; }
-        AovModule n; n.h = h;
-        *(void**)(&n.launch) = dlsym(h, "rbrt_aov_launch");
-        if (!n.launch) { set_error("%s lacks the AOV entry point", path.c_str()); dlclose(h); return RBRT_E_CUDA; }
-        m = n;
+        if (!h) { set_error("the %s module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", m.what, path.c_str(), dlerror()); return RBRT_E_CUDA; }
+        void* f = dlsym(h, m.symbol);
+        if (!f) { set_error("%s lacks the %s entry point", path.c_str(), m.what); dlclose(h); return RBRT_E_CUDA; }
+        m.launch = f;
     }
-    *out = &m;
     return RBRT_OK;
 }
 
+// ------------------------------------------------------------------ first-hit AOVs (rbrt_gpu_render_aov*)
 // Per device: the planes of the host-pointer variant (grown, never shrunk, until rbrt_gpu_release_cache), the counters and the
 // events.  Only calls that synchronise before returning use them, so one set per device serves every call.
 struct AovPool { char* buf = nullptr; size_t bytes = 0; unsigned long long* ctr = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr; };
@@ -423,8 +425,8 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
     const double t0 = now_ms();
     if (stats) memset(stats, 0, sizeof(*stats));
     { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
-    const AovModule* am = nullptr;
-    { int rc = aov_module(&am); if (rc) return rc; }
+    { int rc = load_module(g_aov_module); if (rc) return rc; }
+    const rbrt_aov_launch_fn launch = reinterpret_cast<rbrt_aov_launch_fn>(g_aov_module.launch);
 
     AovPool& pool = g_aov[rp.device & 63];
     AovArgs a;
@@ -453,7 +455,7 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
     }
     wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
     if (stats) { CKA(cudaMemsetAsync(pool.ctr, 0, 8 * AOV_ST_COUNT, st)); CKA(cudaEventRecord(pool.e0, st)); }
-    CKA((cudaError_t)am->launch(&a, st));
+    CKA((cudaError_t)launch(&a, st));
     if (stats) CKA(cudaEventRecord(pool.e1, st));
     note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
     if (!host && !stats) return RBRT_OK;                                  // enqueue only
@@ -481,6 +483,98 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
         stats->ms_device = ms; stats->ms_d2h = host ? t2 - t1 : 0.0; stats->launches = 1;
         stats->ms_total = now_ms() - t0;
     }
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ ray queries on device memory (rbrt_gpu_query_*_device)
+// Per device: a ring of QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
+// block, zeroes it on its own stream and records an event behind its kernel, so calls on different streams never share a cursor.  A block
+// is reused QRY_RING calls later; the host waits for its previous call only if that one has still not run by then.
+#define QRY_RING 256
+struct QueryPool { unsigned long long* ctr = nullptr; cudaEvent_t used[QRY_RING] = {}; uint32_t next = 0; cudaEvent_t e0 = nullptr, e1 = nullptr; };
+static QueryPool g_query[64];
+static void query_release_all() {
+    int cur = 0; cudaGetDevice(&cur);
+    for (int d = 0; d < 64; ++d) {
+        QueryPool& p = g_query[d];
+        if (!p.ctr) continue;
+        cudaSetDevice(d);
+        for (cudaEvent_t& e : p.used) if (e) { cudaEventSynchronize(e); cudaEventDestroy(e); }
+        if (p.e0) cudaEventDestroy(p.e0);
+        if (p.e1) cudaEventDestroy(p.e1);
+        cudaFree(p.ctr);
+        p = QueryPool();
+    }
+    cudaSetDevice(cur);
+}
+
+// Device memory on `device` (or managed / registered host memory the device can read)?  Unregistered host memory or another device's
+// memory would fault in the kernel.
+static bool usable_on(const void* p, int device) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (a.type == cudaMemoryTypeDevice) return a.device == device;
+    return a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeHost && a.devicePointer == p);
+}
+
+// occ: an occlusion query into occluded[]; else a closest query into *out.
+static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool occ, const rbrt_query_out* out, const float* max_dist,
+                 uint8_t* occluded, cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!n) return RBRT_OK;
+    if (!scene || !rays || (occ ? !occluded : !out)) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!occ && !out->t && !out->dist && !out->kind && !out->elem_idx && !out->tri_idx && !out->point && !out->normal) {
+        set_error("no output requested (every plane of the output is NULL)"); return RBRT_E_INVALID;
+    }
+    if (n > 0xFFFFFFFFull) { set_error("more than 2^32 - 1 rays"); return RBRT_E_INVALID; }
+    const Scene& sc = *reinterpret_cast<const Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device
+    CKA(cudaSetDevice(rp.device));
+    const double t0 = now_ms();
+    {
+        const void* ptrs[10] = {rays, max_dist, occluded};
+        if (!occ) { ptrs[3] = out->t; ptrs[4] = out->dist; ptrs[5] = out->kind; ptrs[6] = out->elem_idx; ptrs[7] = out->tri_idx; ptrs[8] = out->point; ptrs[9] = out->normal; }
+        for (const void* p : ptrs)
+            if (p && !usable_on(p, rp.device)) { set_error("rays and outputs must be device memory on the scene's device %d", rp.device); return RBRT_E_INVALID; }
+    }
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    { int rc = load_module(g_query_module); if (rc) return rc; }
+    const rbrt_query_launch_fn launch = reinterpret_cast<rbrt_query_launch_fn>(g_query_module.launch);
+
+    QueryPool& pool = g_query[rp.device & 63];
+    if (!pool.ctr) CKA(cudaMalloc(&pool.ctr, 8ull * QRY_ST_COUNT * QRY_RING));
+    const uint32_t slot = pool.next++ % QRY_RING;
+    cudaEvent_t& used = pool.used[slot];
+    if (used) CKA(cudaEventSynchronize(used));
+    else CKA(cudaEventCreateWithFlags(&used, cudaEventDisableTiming));
+    if (stats && !pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
+
+    QueryArgs a;
+    memset(&a, 0, sizeof(a));
+    a.S = rp.dev; a.rays = rays; a.n = n; a.max_dist = max_dist; a.occluded = occluded; a.ctr = pool.ctr + QRY_ST_COUNT * slot;
+    if (!occ) a.out = *out;
+    a.count = stats != nullptr;
+    {
+        const uint64_t blocks = (n + 127) / 128;                          // persistent: at most the resident blocks (8 per SM, query.cu)
+        const uint64_t resident = 8ull * (uint64_t)rp.sm_count;
+        a.blocks = (uint32_t)(blocks < resident ? blocks : resident);
+    }
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    CKA(cudaMemsetAsync(a.ctr, 0, 8 * QRY_ST_COUNT, st));
+    if (stats) CKA(cudaEventRecord(pool.e0, st));
+    CKA((cudaError_t)launch(&a, st));
+    if (stats) CKA(cudaEventRecord(pool.e1, st));
+    CKA(cudaEventRecord(used, st));
+    note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
+    if (!stats) return RBRT_OK;                                           // enqueue only
+
+    unsigned long long h[QRY_ST_COUNT];
+    CKA(cudaMemcpyAsync(h, a.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CKA(cudaStreamSynchronize(st));
+    float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+    stats->rays = n; stats->nan_rays = h[QRY_ST_NAN]; stats->node_visits = h[QRY_ST_NODES]; stats->tri_tests = h[QRY_ST_TRIS];
+    stats->ms_device = ms; stats->launches = 1;
+    stats->ms_total = now_ms() - t0;
     return RBRT_OK;
 }
 
@@ -782,6 +876,7 @@ int rbrt_gpu_release_cache(void) {
     release_dist_buffers();
     release_build_scratch();
     aov_release_all();
+    query_release_all();
     arena_release_all();
     for (void* p : g_pinned_free) cudaFreeHost(p);
     g_pinned_free.clear();
@@ -928,6 +1023,18 @@ int rbrt_gpu_render_aov_device(const rbrt_scene* scene, const rbrt_camera* cam, 
                                void* cuda_stream, rbrt_stats* stats) {
     LOCK;
     return render_aov(scene, cam, num_samples, seed, d_out, false, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_query_closest_device(const rbrt_scene* scene, const rbrt_ray* d_rays, uint64_t n, const rbrt_query_out* d_out, void* cuda_stream,
+                                  rbrt_stats* stats) {
+    LOCK;
+    return query(scene, d_rays, n, false, d_out, nullptr, nullptr, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_rays, uint64_t n, const float* d_max_dist, uint8_t* d_occluded,
+                                   void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return query(scene, d_rays, n, true, nullptr, d_max_dist, d_occluded, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

@@ -46,6 +46,9 @@ def element_arrays(elements):
             (_abi.TriangleDescC * max(len(tri), 1))(*[t.to_c() for t in tri]), len(order), len(sph), len(tri))
 
 
+QUERY_PASSES = ("t", "dist", "kind", "elem_idx", "tri_idx", "point", "normal")
+
+
 class Scene:
     def __init__(self, elements=None, triangle_meshes=None, lights=None, simd_lanes=8, leaf_size=0, box_pad_rel=0.0, local=False, sah=True, broadcast=False):
         self.elements = list(elements or [])
@@ -146,6 +149,66 @@ class Scene:
         if stats is not None:
             stats.update(st.as_dict())
         return hits
+
+    # ---- ray queries on device memory (rbrt_gpu_query_*_device, DESIGN.md section 12) ---------------
+    def _query_rays(self, rays, stream):
+        import torch
+        if not (isinstance(rays, torch.Tensor) and rays.is_cuda and rays.dtype == torch.float32 and rays.dim() == 2 and rays.shape[1] == 6
+                and rays.is_contiguous()):
+            raise ValueError("rays must be a contiguous float32 CUDA tensor of shape [N,6] (origin xyz, direction xyz)")
+        stream = stream or torch.cuda.current_stream(rays.device)
+        if stream.device != rays.device:
+            raise ValueError(f"rays are on {rays.device}, the stream on {stream.device}")
+        return stream
+
+    @staticmethod
+    def _query_check(rc, stats, st):
+        if rc == _abi.E_INVALID:                                       # a refused argument (rays or outputs on another device, ...)
+            raise ValueError(_abi.lib().rbrt_last_error().decode("utf-8", "replace"))
+        _abi.check(rc)
+        if stats is not None:
+            stats.update(st.as_dict())
+
+    def intersect_device(self, rays, passes=None, stream=None, stats=None):
+        """Scene::hit for the rays of a CUDA tensor [N,6] on the scene's device: a dict of CUDA tensors t, dist, kind (RBRT_HIT_*),
+        elem_idx, tri_idx [N] and point, normal [N,3], each bit for bit the field `hit` reports (`passes`: a subset of those names).
+        Enqueued on `stream` (default: the rays' current stream); returns without synchronising unless `stats` (a dict) is given."""
+        import torch
+        stream = self._query_rays(rays, stream)
+        names = QUERY_PASSES if passes is None else ((passes,) if isinstance(passes, str) else tuple(dict.fromkeys(passes)))
+        unknown = [p for p in names if p not in QUERY_PASSES]
+        if unknown or not names:
+            raise ValueError(f"unknown or no pass(es) {unknown}; choose from {QUERY_PASSES}")
+        n = rays.shape[0]
+        handle = self.handle()
+        out, tensors = _abi.QueryOutC(), {}
+        with torch.cuda.stream(stream):
+            for name in names:
+                dt = torch.int32 if name == "kind" else (torch.uint32 if name in ("elem_idx", "tri_idx") else torch.float32)
+                tensors[name] = torch.empty((n, 3) if name in ("point", "normal") else (n,), dtype=dt, device=rays.device)
+                setattr(out, name, tensors[name].data_ptr())
+        st = _abi.StatsC()
+        rc = _abi.lib().rbrt_gpu_query_closest_device(handle, rays.data_ptr(), n, out, stream.cuda_stream, st if stats is not None else None)
+        self._query_check(rc, stats, st)
+        return tensors
+
+    def occluded_device(self, rays, max_dist=None, stream=None, stats=None):
+        """Occlusion for the rays of a CUDA tensor [N,6]: a uint8 CUDA tensor [N], 1 where `hit` reports a hit with dist < max_dist
+        (strict; max_dist a float32 CUDA tensor [N], None = +inf), 2 for a NaN ray, 0 otherwise.  Enqueued like intersect_device."""
+        import torch
+        stream = self._query_rays(rays, stream)
+        n = rays.shape[0]
+        if max_dist is not None and not (isinstance(max_dist, torch.Tensor) and max_dist.device == rays.device and max_dist.dtype == torch.float32
+                                         and tuple(max_dist.shape) == (n,) and max_dist.is_contiguous()):
+            raise ValueError("max_dist must be None or a contiguous float32 CUDA tensor [N] on the rays' device")
+        handle = self.handle()
+        with torch.cuda.stream(stream):
+            occ = torch.empty(n, dtype=torch.uint8, device=rays.device)
+        st = _abi.StatsC()
+        rc = _abi.lib().rbrt_gpu_query_occluded_device(handle, rays.data_ptr(), n, max_dist.data_ptr() if max_dist is not None else None,
+                                                         occ.data_ptr(), stream.cuda_stream, st if stats is not None else None)
+        self._query_check(rc, stats, st)
+        return occ
 
 
 def scatter(items, seed=0):
