@@ -354,7 +354,9 @@ int rbrt_gpu_finalize_device(const void* d_accum_rgba_f32, uint32_t width, uint3
 
 /* Parity hook = Scene::hit (scene.rs:19-43) for caller-supplied rays; the reference's nearest
  * public analogue is do_intersection_soa (mesh.rs:183-190).  HOST pointers.
- * trace_mode: RBRT_TRACE_BVH or RBRT_TRACE_BRUTE (every triangle, the reference's own loop). */
+ * trace_mode: RBRT_TRACE_BVH or RBRT_TRACE_BRUTE (every triangle, the reference's own loop).
+ * Refused with RBRT_E_INVALID, nothing written: a scene with a mesh whose tree was refused as too deep (the call waits for the
+ * scene's build to know). */
 int rbrt_gpu_trace_rays(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n,
                         uint32_t trace_mode, rbrt_hit* hits_out, rbrt_stats* stats);
 

@@ -973,6 +973,7 @@ int rbrt_gpu_trace_rays(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t 
     const Scene& sc = *reinterpret_cast<const Scene*>(scene);
     CKA(cudaSetDevice(sc.device));
     if (stats) memset(stats, 0, sizeof(*stats));
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh: the hits would not be Scene::hit's
     if (!n) return RBRT_OK;
     double t0 = now_ms();
     rbrt_ray* d_rays = nullptr; rbrt_hit* d_hits = nullptr; unsigned long long* d_stats = nullptr;
