@@ -452,8 +452,55 @@ int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_ra
                                    const float* d_max_dist,
                                    uint8_t* d_occluded, void* cuda_stream, rbrt_stats* stats);
 
+/* ---- guided denoising (DESIGN.md section 13) -----------------------------------------------
+ * An edge-aware à-trous filter of the HDR mean colour, guided by the first-hit AOVs of the same camera and seed (the spatial filter of
+ * SVGF, Schied et al. 2017, without variance or temporal terms).  Inputs are row-major W x H planes: c = hdr (W*H*3, what
+ * rbrt_gpu_render_hdr returns), and from `guides` the depth z (W*H), normal n and albedo a (W*H*3) as rbrt_gpu_render_aov fills them.
+ * Every operation below is one IEEE f32 operation, correctly rounded, products and sums left to right as written; rbrt_b200/csrc/denoise.cuh
+ * holds the per-pixel code.  Per pixel p:
+ *   1. d = max(a, 2^-10) per component (a NaN albedo gives 2^-10); e = c / d; l(e) = (0.2126 e.r + 0.7152 e.g) + 0.0722 e.b.
+ *      p is VALID when c, d and z are all finite (not NaN, not +-inf).
+ *   2. levels L (default 4), level i = 0 .. L-1 with step s = 2^i, filters the previous level's e (level 0: step 1's).  For a valid p,
+ *      over the 5x5 taps q = p + (dx*s, dy*s), dx, dy in -2..2, in row-major order (dy outer, dx inner):
+ *        skipped: q outside the image; q not valid; w_n == 0;
+ *        centre (dx = dy = 0): w = 9/64;
+ *        other:  w_n = max(0, (n_p.x*n_q.x + n_p.y*n_q.y) + n_p.z*n_q.z) ^ 128, by seven squarings (a NaN dot gives 0);
+ *                x_z = |z_p - z_q| * r_p,          r_p  = 1 / ((σ_z * z_p) * s),        σ_z = sigma_depth     (default 0.01)
+ *                x_l = (l_p - l_q) * r'_p,         r'_p = 1 / (σ_l * l_p + 2^-7),       σ_l = sigma_luminance (default 0.25)
+ *                w   = (h[dx]*h[dy] * w_n) / ((1 + x_z*x_z) * (1 + x_l*x_l)),   h = {1/16, 1/4, 3/8, 1/4, 1/16}  (h[dx]*h[dy] exact)
+ *      with l_p, l_q the luminances of this level's input.  Σw and Σ w*e_q (per channel) are f32 sums from +0 in tap order; the
+ *      output is e' = Σ w*e_q / Σw (one division per channel).  An invalid p keeps its e.
+ *   3. hdr_out = e_L * d per channel for a valid p, c unchanged for an invalid one; rgb_out = (sqrt(hdr_out) * 256) as u8, saturating
+ *      (NaN -> 0): the tonemap of rbrt_gpu_finalize_device.
+ * A miss has depth +inf and normal 0, so it is passed through and never mixes with anything.  The guides line up with the colour when
+ * they come from the same camera and seed with at most as many samples (section 11: their samples are the colour's first camera rays). */
+typedef struct rbrt_denoise_opts {
+    uint32_t levels;           /* à-trous levels, steps 1, 2, 4, ...; 0 = default (4); at most 8 */
+    float    sigma_depth;      /* σ_z; 0 = default */
+    float    sigma_luminance;  /* σ_l; 0 = default */
+} rbrt_denoise_opts;
+/* guides: an rbrt_aov_out as rbrt_gpu_render_aov* filled it; depth, normal and albedo are read, the other members are ignored.  opts may
+ * be NULL.  Outputs: hdr_out (W*H*3 f32) and / or rgb_out (W*H*3 u8); either may be NULL, not both.
+ * The calls run on this process's current render device (rbrt_gpu_init; under a communicator its first device) and are not collective.
+ * The kernels live in librbrt_gpu_denoise.so, loaded at run time from this library's directory (RBRT_GPU_DENOISE_LIB: another path);
+ * without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL hdr, guides, guide depth, normal or albedo; both outputs NULL; W or H = 0 or
+ * W*H > 2^31 - 1 (as rbrt_gpu_render_hdr); levels > 8; a negative, NaN or infinite sigma; an output that overlaps an input or the
+ * other output.
+ * stats may be NULL; it reports ms_device, ms_total and launches (1 + levels). */
+/* HOST pointers; blocks until the outputs are on the host. */
+int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,
+                     float* hdr_out, uint8_t* rgb_out, rbrt_stats* stats);
+/* DEVICE pointers on the current render device, enqueued on cuda_stream (0 = default stream); the scratch (48 bytes per pixel) is
+ * allocated and freed in stream order on that stream, so calls in flight on different streams never share it.  stats == NULL: enqueue
+ * only, no synchronisation; with stats the call waits for its kernels and fills them.  Also refused: inputs or outputs in another
+ * device's memory or in unregistered host memory. */
+int rbrt_gpu_denoise_device(uint32_t width, uint32_t height, const float* d_hdr, const rbrt_aov_out* d_guides, const rbrt_denoise_opts* opts,
+                            float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats);
+
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
- * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch and the query counters). */
+ * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters and the
+ * denoiser's host-call block). */
 int rbrt_gpu_release_cache(void);
 
 /* Upper bound, in bytes, of ONE pool of wavefront state (there are up to four per device, one per frame in flight).

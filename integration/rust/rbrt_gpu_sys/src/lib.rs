@@ -44,6 +44,9 @@ pub struct RbrtAovOut { pub depth: *mut f32, pub normal: *mut f32, pub albedo: *
 #[repr(C)] #[derive(Copy, Clone, Debug)]
 pub struct RbrtQueryOut { pub t: *mut f32, pub dist: *mut f32, pub kind: *mut i32, pub elem_idx: *mut u32, pub tri_idx: *mut u32,
                           pub point: *mut f32, pub normal: *mut f32 }
+/// Options of the guided denoiser (rbrt_gpu_denoise*); 0 = default (4 levels, at most 8).
+#[repr(C)] #[derive(Copy, Clone, Debug, Default)]
+pub struct RbrtDenoiseOpts { pub levels: u32, pub sigma_depth: f32, pub sigma_luminance: f32 }
 pub enum RbrtScene {}
 /// `kind` of a hit (rbrt_hit, rbrt_query_out)
 pub const RBRT_HIT_NONE: i32 = -1;
@@ -137,6 +140,13 @@ extern "C" {
     /// RBRT_QUERY_NAN_RAY for a NaN ray, else RBRT_QUERY_CLEAR.
     pub fn rbrt_gpu_query_occluded_device(scene: *const RbrtScene, d_rays: *const RbrtRay, n: u64, d_max_dist: *const f32,
                                           d_occluded: *mut u8, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// Edge-aware à-trous denoise of a render_hdr image guided by render_aov depth / normal / albedo of the same camera and seed; HOST
+    /// pointers, blocks.  hdr_out (W*H*3 f32) and / or rgb_out (W*H*3 u8, k_finalize's tonemap); opts may be null.
+    pub fn rbrt_gpu_denoise(width: u32, height: u32, hdr: *const f32, guides: *const RbrtAovOut, opts: *const RbrtDenoiseOpts,
+                            hdr_out: *mut f32, rgb_out: *mut u8, stats: *mut RbrtStats) -> c_int;
+    /// The same on DEVICE planes of the current render device, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_denoise_device(width: u32, height: u32, d_hdr: *const f32, d_guides: *const RbrtAovOut, opts: *const RbrtDenoiseOpts,
+                                   d_hdr_out: *mut f32, d_rgb_out: *mut u8, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

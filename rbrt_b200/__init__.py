@@ -15,7 +15,8 @@ from .cam import Camera
 from .materials import Dielectric, Lambertian, Metal
 from .mesh import TriangleMesh, load_mesh_vertices_from_file
 from .pipeline import FramePipeline
-from .render import AOV_PASSES, ImageBuffer, primary_rays, render_aovs, render_aovs_device, render_scene, render_scene_hdr
+from .render import (AOV_PASSES, ImageBuffer, denoise, denoise_device, primary_rays, render_aovs, render_aovs_device, render_scene,
+                     render_scene_hdr)
 from .scene import Scene
 from .sphere import Sphere
 from .triangle import BasicTriangle

@@ -103,6 +103,10 @@ class QueryOutC(C.Structure):  # rbrt_query_out: device planes, NULL = not produ
                 ("point", C.c_void_p), ("normal", C.c_void_p)]
 
 
+class DenoiseOptsC(C.Structure):  # rbrt_denoise_opts: 0 = default
+    _fields_ = [("levels", C.c_uint32), ("sigma_depth", C.c_float), ("sigma_luminance", C.c_float)]
+
+
 class SceneInfoC(C.Structure):
     _fields_ = [("num_spheres", C.c_uint32), ("num_meshes", C.c_uint32), ("num_triangles", C.c_uint64),
                 ("num_triangles_tested", C.c_uint64), ("num_bvh_nodes", C.c_uint64),
@@ -167,6 +171,9 @@ GPU_SIGNATURES = {
     "rbrt_gpu_render_aov_device": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_closest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, P(QueryOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_occluded_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_denoise": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_denoise_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, C.c_void_p,
+                                          P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

@@ -8,8 +8,10 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <cfloat>
 #include "aov.cuh"
 #include "bvh_build.cuh"
+#include "denoise.cuh"
 #include "engine.cuh"
 #include "multi.cuh"
 #include "query.cuh"
@@ -373,11 +375,12 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
 }
 
 // ------------------------------------------------------------------ device modules with one launch entry point
-// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path) and the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB) live
-// in their own device modules, like the refit; each is opened once, on first use.
+// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path), the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB) and the
+// denoiser (librbrt_gpu_denoise.so, RBRT_GPU_DENOISE_LIB) live in their own device modules, like the refit; each is opened once, on first use.
 struct LaunchModule { const char* env; const char* file; const char* what; const char* symbol; void* launch; };
 static LaunchModule g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", "rbrt_aov_launch", nullptr};
 static LaunchModule g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", "rbrt_query_launch", nullptr};
+static LaunchModule g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", "rbrt_denoise_launch", nullptr};
 static int load_module(LaunchModule& m) {
     if (!m.launch) {
         std::string path;
@@ -575,6 +578,120 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     stats->rays = n; stats->nan_rays = h[QRY_ST_NAN]; stats->node_visits = h[QRY_ST_NODES]; stats->tri_tests = h[QRY_ST_TRIS];
     stats->ms_device = ms; stats->launches = 1;
     stats->ms_total = now_ms() - t0;
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ guided denoising (rbrt_gpu_denoise*)
+// Per device: the block the host-pointer variant copies its planes into and carves its scratch from (grown, never shrunk, until
+// rbrt_gpu_release_cache), and the events of calls with stats.  Only calls that synchronise before returning use them.  The device
+// variant takes its scratch from the stream-ordered allocator on the call's stream instead, so calls in flight never share it.
+struct DenoisePool { char* buf = nullptr; size_t bytes = 0; cudaEvent_t e0 = nullptr, e1 = nullptr; };
+static DenoisePool g_denoise[64];
+static void denoise_release_all() {
+    int cur = 0; cudaGetDevice(&cur);
+    for (int d = 0; d < 64; ++d) {
+        DenoisePool& p = g_denoise[d];
+        if (!p.buf && !p.e0) continue;
+        cudaSetDevice(d);
+        cudaFree(p.buf);
+        if (p.e0) cudaEventDestroy(p.e0);
+        if (p.e1) cudaEventDestroy(p.e1);
+        p = DenoisePool();
+    }
+    cudaSetDevice(cur);
+}
+
+static bool overlap(const void* a, size_t na, const void* b, size_t nb) {
+    if (!a || !b) return false;
+    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+    return x < y + nb && y < x + na;
+}
+
+static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts, float* hdr_out,
+                   uint8_t* rgb_out, bool host, cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!hdr || !guides) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!guides->depth || !guides->normal || !guides->albedo) { set_error("null guide plane: depth, normal and albedo are read"); return RBRT_E_INVALID; }
+    if (!hdr_out && !rgb_out) { set_error("no output requested (hdr_out and rgb_out are both NULL)"); return RBRT_E_INVALID; }
+    if (!W || !H) { set_error("empty image"); return RBRT_E_INVALID; }
+    const size_t n = (size_t)W * H;
+    if (n > 0x7FFFFFFFull) { set_error("image too large"); return RBRT_E_INVALID; }
+    DenoiseArgs a;
+    memset(&a, 0, sizeof(a));
+    a.W = W; a.H = H;
+    a.levels = opts && opts->levels ? opts->levels : DN_DEFAULT_LEVELS;
+    if (a.levels > DN_MAX_LEVELS) { set_error("levels must be at most %u", DN_MAX_LEVELS); return RBRT_E_INVALID; }
+    const float sz = opts ? opts->sigma_depth : 0.0f, sl = opts ? opts->sigma_luminance : 0.0f;
+    if (!(sz >= 0.0f && sz <= FLT_MAX) || !(sl >= 0.0f && sl <= FLT_MAX)) { set_error("a sigma must be finite and >= 0 (0 = default)"); return RBRT_E_INVALID; }
+    a.sigma_z = sz > 0.0f ? sz : DN_SIGMA_DEPTH;
+    a.sigma_l = sl > 0.0f ? sl : DN_SIGMA_LUMINANCE;
+    {
+        const struct { const void* p; size_t b; } in[4] = {{hdr, 12 * n}, {guides->depth, 4 * n}, {guides->normal, 12 * n}, {guides->albedo, 12 * n}};
+        for (const auto& i : in) {
+            if (overlap(hdr_out, 12 * n, i.p, i.b) || overlap(rgb_out, 3 * n, i.p, i.b)) { set_error("an output overlaps an input"); return RBRT_E_INVALID; }
+        }
+        if (overlap(hdr_out, 12 * n, rgb_out, 3 * n)) { set_error("hdr_out and rgb_out overlap"); return RBRT_E_INVALID; }
+    }
+    { int rc = ensure_device(); if (rc) return rc; }
+    const int dev = g_device;
+    if (!host) {
+        const void* ptrs[6] = {hdr, guides->depth, guides->normal, guides->albedo, hdr_out, rgb_out};
+        for (const void* p : ptrs)
+            if (p && !usable_on(p, dev)) { set_error("planes must be device memory on the current device %d", dev); return RBRT_E_INVALID; }
+    }
+    { int rc = load_module(g_denoise_module); if (rc) return rc; }
+    const rbrt_denoise_launch_fn launch = reinterpret_cast<rbrt_denoise_launch_fn>(g_denoise_module.launch);
+    const double t0 = now_ms();
+
+    DenoisePool& pool = g_denoise[dev & 63];
+    if (stats && !pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
+    a.hdr = hdr; a.depth = guides->depth; a.normal = guides->normal; a.albedo = guides->albedo; a.hdr_out = hdr_out; a.rgb_out = rgb_out;
+    if (host) {                                                           // inputs, outputs and scratch carved from the pooled block
+        const size_t b1 = a256(4 * n), b3 = a256(12 * n), bs = a256(48 * n);
+        const size_t need = bs + 3 * b3 + b1 + (hdr_out ? b3 : 0) + (rgb_out ? a256(3 * n) : 0);
+        if (pool.bytes < need) {
+            cudaFree(pool.buf); pool.buf = nullptr; pool.bytes = 0;
+            CKA(cudaMalloc(&pool.buf, need)); pool.bytes = need;
+        }
+        char* p = pool.buf;
+        a.scratch = (float4*)p; p += bs;
+        float* d_hdr = (float*)p; p += b3;
+        float* d_nrm = (float*)p; p += b3;
+        float* d_alb = (float*)p; p += b3;
+        float* d_dep = (float*)p; p += b1;
+        CKA(cudaMemcpyAsync(d_hdr, hdr, 12 * n, cudaMemcpyHostToDevice, st));
+        CKA(cudaMemcpyAsync(d_nrm, guides->normal, 12 * n, cudaMemcpyHostToDevice, st));
+        CKA(cudaMemcpyAsync(d_alb, guides->albedo, 12 * n, cudaMemcpyHostToDevice, st));
+        CKA(cudaMemcpyAsync(d_dep, guides->depth, 4 * n, cudaMemcpyHostToDevice, st));
+        a.hdr = d_hdr; a.normal = d_nrm; a.albedo = d_alb; a.depth = d_dep;
+        if (hdr_out) { a.hdr_out = (float*)p; p += b3; }
+        if (rgb_out) a.rgb_out = (uint8_t*)p;
+    } else {
+        CKA(cudaMallocAsync((void**)&a.scratch, 48 * n, st));
+    }
+    if (stats) {
+        cudaError_t e = cudaEventRecord(pool.e0, st);
+        if (e != cudaSuccess) { if (!host) cudaFreeAsync(a.scratch, st); return cuda_fail(e, "cudaEventRecord"); }
+    }
+    {
+        cudaError_t e = (cudaError_t)launch(&a, st);
+        if (e == cudaSuccess && stats) e = cudaEventRecord(pool.e1, st);
+        if (!host) { cudaError_t f = cudaFreeAsync(a.scratch, st); if (e == cudaSuccess) e = f; }
+        if (e != cudaSuccess) return cuda_fail(e, "rbrt_denoise_launch");
+    }
+    if (host) {
+        if (hdr_out) CKA(cudaMemcpyAsync(hdr_out, a.hdr_out, 12 * n, cudaMemcpyDeviceToHost, st));
+        if (rgb_out) CKA(cudaMemcpyAsync(rgb_out, a.rgb_out, 3 * n, cudaMemcpyDeviceToHost, st));
+        CKA(cudaStreamSynchronize(st));
+    } else if (!stats) {
+        return RBRT_OK;                                                   // enqueue only
+    }
+    if (stats) {
+        CKA(cudaEventSynchronize(pool.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+        stats->ms_device = ms; stats->launches = 1 + a.levels;
+        stats->ms_total = now_ms() - t0;
+    }
     return RBRT_OK;
 }
 
@@ -877,6 +994,7 @@ int rbrt_gpu_release_cache(void) {
     release_build_scratch();
     aov_release_all();
     query_release_all();
+    denoise_release_all();
     arena_release_all();
     for (void* p : g_pinned_free) cudaFreeHost(p);
     g_pinned_free.clear();
@@ -1036,6 +1154,18 @@ int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_ra
                                    void* cuda_stream, rbrt_stats* stats) {
     LOCK;
     return query(scene, d_rays, n, true, nullptr, d_max_dist, d_occluded, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,
+                     float* hdr_out, uint8_t* rgb_out, rbrt_stats* stats) {
+    LOCK;
+    return denoise(width, height, hdr, guides, opts, hdr_out, rgb_out, true, 0, stats);
+}
+
+int rbrt_gpu_denoise_device(uint32_t width, uint32_t height, const float* d_hdr, const rbrt_aov_out* d_guides, const rbrt_denoise_opts* opts,
+                            float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return denoise(width, height, d_hdr, d_guides, opts, d_hdr_out, d_rgb_out, false, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

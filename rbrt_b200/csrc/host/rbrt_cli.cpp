@@ -258,6 +258,7 @@ void usage() {
            "      --aov <prefix>               (extension) after the render also write first-hit AOVs of the same camera and --seed:\n"
            "                                   <prefix>.depth.pfm, <prefix>.normal.pfm, <prefix>.albedo.pfm, <prefix>.coverage.pfm\n"
            "      --aov-samples <n>            (extension) samples per pixel of the AOVs [default: --samples]\n"
+           "      --denoise                    (extension) save the image denoised on the GPU, guided by AOVs of the same camera and --seed [--aov-samples default: min(--samples, 4)]\n"
            "  -h, --help                       Print help\n  -V, --version                    Print version\n");
 }
 
@@ -273,7 +274,7 @@ uint32_t parse_u32(const char* s, const char* what) {
 int main(int argc, char** argv) {
     std::string target = "dbg_out.png", config = "scenes/example_scene.yaml";      // main.rs:14-50
     uint32_t height = 600, width = 800, samples = 5;
-    uint64_t seed = 0; int device = 0; bool check_only = false, dump = false;
+    uint64_t seed = 0; int device = 0; bool check_only = false, dump = false, denoise = false;
     uint32_t gpus = 1; int transport = RBRT_TRANSPORT_AUTO;
     std::string from_ppm, aov;
     uint32_t aov_samples = 0;
@@ -304,11 +305,17 @@ int main(int argc, char** argv) {
         else if (key == "--from-ppm") from_ppm = value("--from-ppm");
         else if (key == "--aov") aov = value("--aov");
         else if (key == "--aov-samples") aov_samples = parse_u32(value("--aov-samples"), "--aov-samples");
+        else if (key == "--denoise") denoise = true;
         else if (key == "-h" || key == "--help") { usage(); return 0; }
         else if (key == "-V" || key == "--version") { printf("rbrt 0.1 (%s)\n", rbrt_gpu_version()); return 0; }
         else { fprintf(stderr, "error: unexpected argument '%s' found\n", a.c_str()); return 2; }
     }
 
+    if (denoise) {
+        if (!from_ppm.empty()) die("error: '--denoise' cannot be used with '--from-ppm' (there is no render to denoise)");
+        if (aov_samples > samples) die("error: '--aov-samples' must not exceed '--samples' with '--denoise': the guides must be the image's first camera rays");
+        if (!aov_samples) aov_samples = std::min<uint32_t>(samples, 4);
+    }
     if (!from_ppm.empty()) {                                                        // the image writers on their own (main.rs:84-91)
         std::ifstream f(from_ppm, std::ios::binary);
         std::string magic; uint32_t w = 0, h = 0, maxv = 0;
@@ -373,15 +380,21 @@ int main(int argc, char** argv) {
     std::vector<uint8_t> rgb((size_t)width * height * 3);
     rbrt_render_opts opts; memset(&opts, 0, sizeof(opts)); opts.seed = seed;
     rbrt_stats st;
-    if (rbrt_gpu_render(scene, &cam, samples, &opts, rgb.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
+    std::vector<float> hdr;
+    if (denoise) {                                                                 // the mean colour, denoised below into rgb
+        hdr.resize((size_t)width * height * 3);
+        if (rbrt_gpu_render_hdr(scene, &cam, samples, &opts, hdr.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
+    } else if (rbrt_gpu_render(scene, &cam, samples, &opts, rgb.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
     printf("\rRendering 100%% complete!\n");                                        // lib.rs:114
     std::vector<float> depth, normal, albedo, coverage;
-    if (!aov.empty()) {                                                            // first-hit AOVs of the same camera rays (include/rbrt_gpu.h)
+    if (!aov.empty() || denoise) {                                                 // first-hit AOVs of the same camera rays (include/rbrt_gpu.h)
         const size_t n = (size_t)width * height;
         depth.resize(n); normal.resize(3 * n); albedo.resize(3 * n); coverage.resize(n);
         rbrt_aov_out ao; memset(&ao, 0, sizeof(ao));
         ao.depth = depth.data(); ao.normal = normal.data(); ao.albedo = albedo.data(); ao.coverage = coverage.data();
         if (rbrt_gpu_render_aov(scene, &cam, aov_samples ? aov_samples : samples, seed, &ao, nullptr) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
+        if (denoise && rbrt_gpu_denoise(width, height, hdr.data(), &ao, nullptr, nullptr, rgb.data(), nullptr) != RBRT_OK)   // on the first device
+            die(std::string("rbrt_gpu: ") + rbrt_last_error());
     }
     rbrt_gpu_scene_destroy(scene);
     printf("Saving rendered image to %s\n", target.c_str());                        // main.rs:84

@@ -192,3 +192,66 @@ def render_aovs_device(cam, num_samples, scene, seed=0, passes=AOV_PASSES, strea
     _abi.check(_abi.lib().rbrt_gpu_render_aov_device(handle, cam.to_c(), int(num_samples), int(seed) & 0xFFFFFFFFFFFFFFFF, out,
                                                      stream.cuda_stream, None))
     return tensors
+
+
+# ---- guided denoising (rbrt_gpu_denoise*, include/rbrt_gpu.h and DESIGN.md section 13) --------------------------------------
+def _denoise_inputs(hdr, aovs, is_tensor):
+    """(H, W) of the colour [H,W,3] and the guides depth [H,W], normal and albedo [H,W,3]: contiguous float32 (CUDA tensors for the device
+    variant, numpy arrays otherwise), or ValueError."""
+    planes = {"hdr": hdr}
+    for k in ("depth", "normal", "albedo"):
+        if k not in aovs:
+            raise ValueError(f"the guides need the {k!r} AOV (render_aovs with passes including it)")
+        planes[k] = aovs[k]
+    if getattr(hdr, "ndim", 0) != 3 or hdr.shape[2] != 3:
+        raise ValueError("hdr must be [H, W, 3]")
+    H, W = hdr.shape[:2]
+    for k, v in planes.items():
+        want = (H, W) if k == "depth" else (H, W, 3)
+        if is_tensor(v) is not True or tuple(v.shape) != want:
+            raise ValueError(f"{k} must be a contiguous float32 {'CUDA tensor' if is_tensor is _is_cuda_f32 else 'numpy array'} of shape {want}")
+    return H, W
+
+
+def _is_numpy_f32(v):
+    return isinstance(v, np.ndarray) and v.dtype == np.float32 and v.flags.c_contiguous
+
+
+def _is_cuda_f32(v):
+    import torch
+    return isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == torch.float32 and v.is_contiguous()
+
+
+def _denoise_opts(levels, sigma_depth, sigma_luminance):
+    return _abi.DenoiseOptsC(int(levels), float(sigma_depth), float(sigma_luminance))
+
+
+def denoise(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stats=None):
+    """Denoise a render_scene_hdr image [H,W,3] guided by render_aovs planes of the same camera and seed (depth, normal, albedo; guides
+    with at most the image's samples line up with it pixel for pixel).  Returns (hdr_out [H,W,3] float32, ImageBuffer of its tonemap).
+    levels / sigmas: 0 = the defaults (4 levels).  Blocks until the result is on the host."""
+    H, W = _denoise_inputs(hdr, aovs, _is_numpy_f32)
+    out = np.empty((H, W, 3), dtype=np.float32)
+    rgb = np.empty((H, W, 3), dtype=np.uint8)
+    g = _abi.AovOutC(depth=aovs["depth"].ctypes.data, normal=aovs["normal"].ctypes.data, albedo=aovs["albedo"].ctypes.data)
+    st = _abi.StatsC()
+    _abi.check(_abi.lib().rbrt_gpu_denoise(W, H, hdr.ctypes.data, g, _denoise_opts(levels, sigma_depth, sigma_luminance), out.ctypes.data,
+                                           rgb.ctypes.data, st))
+    if stats is not None:
+        stats.update(st.as_dict())
+    return out, ImageBuffer(rgb)
+
+
+def denoise_device(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stream=None):
+    """The same on CUDA tensors (render_aovs_device's planes) of the current render device: returns (hdr_out [H,W,3] float32,
+    rgb [H,W,3] uint8) tensors, enqueued on `stream` (default: the current stream) without synchronising."""
+    import torch
+    H, W = _denoise_inputs(hdr, aovs, _is_cuda_f32)
+    stream = stream or torch.cuda.current_stream()
+    with torch.cuda.stream(stream):
+        out = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
+        rgb = torch.empty((H, W, 3), dtype=torch.uint8, device=stream.device)
+    g = _abi.AovOutC(depth=aovs["depth"].data_ptr(), normal=aovs["normal"].data_ptr(), albedo=aovs["albedo"].data_ptr())
+    _abi.check(_abi.lib().rbrt_gpu_denoise_device(W, H, hdr.data_ptr(), g, _denoise_opts(levels, sigma_depth, sigma_luminance),
+                                                  out.data_ptr(), rgb.data_ptr(), stream.cuda_stream, None))
+    return out, rgb
