@@ -498,9 +498,68 @@ int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rb
 int rbrt_gpu_denoise_device(uint32_t width, uint32_t height, const float* d_hdr, const rbrt_aov_out* d_guides, const rbrt_denoise_opts* opts,
                             float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats);
 
+/* ---- per-pixel variance and variance-guided denoising (DESIGN.md section 14) ------------------
+ * VARIANCE OF A RENDER.  S = num_samples, K = splits, n = S / K.  The call renders shard k = 0 .. K-1 as rbrt_gpu_render_accum_device
+ * does with shard_mode = RBRT_SHARD_SAMPLES, shard_rank = k, shard_count = K: samples [k*n, (k+1)*n) of the frame's Philox stream into
+ * a per-pixel sum A_k.  K shards of one seed are K independent estimates of each pixel's mean.  Per pixel and channel, in f32, each
+ * operation correctly rounded, sums from +0 in shard order (rbrt_b200/csrc/variance.cuh holds the code):
+ *   hdr_out = (((A_0 + A_1) + A_2) + ... + A_{K-1}) * (1.0f / (float)S)
+ *             — the arithmetic of the PEER sample-sharded rbrt_gpu_render_hdr on K ranks (rank order sum, then the finalise), and the
+ *             same bits; within 1e-5 relative of the unsharded rbrt_gpu_render_hdr, whose per-pixel sum runs over the samples in one chain;
+ *   m_k     = A_k * (1.0f / (float)n);
+ *   var_out = (Σ_k (m_k - hdr_out) * (m_k - hdr_out)) / (float)(K * (K - 1))
+ *             — the unbiased variance of the mean hdr_out (the K-buffer estimate: its expectation is the pixel's sample variance / S).
+ * Outputs W*H*3 f32 each, row-major; either may be NULL, not both.  opts as a render (seed, max_depth, trace_mode, batch_paths, pool).
+ * Refused with RBRT_E_INVALID, nothing written: splits < 2 or > 16; num_samples = 0 or not a multiple of splits; opts->shard_count > 1
+ * (the call shards by itself); a NULL scene or camera; both outputs NULL; an empty image or W*H > 2^31 - 1; the outputs overlapping;
+ * a scene with a mesh whose tree was refused as too deep (the call waits for the scene's build to know); opts a render refuses.
+ * Ordered against scene updates like a render.  Under a communicator the call is not collective: it runs on this process's first
+ * device (replica 0).  The shards alternate between two lanes: the calling stream with the wavefront pool of opts->flags (p), and an
+ * internal stream of the device with pool 4 + p (the second lane of RBRT_OPT_SPLIT_BATCHES, which the call does not use otherwise);
+ * calls in flight at the same time use different pools.  The K accumulators (16 bytes per pixel each) are allocated and freed in stream
+ * order on the calling stream.  The kernel that forms the moments lives in librbrt_gpu_variance.so (RBRT_GPU_VARIANCE_LIB: another path).
+ * stats may be NULL; it reports rays, paths and nan_rays summed over the shards, ms_device (all shards and the moments), ms_total and
+ * launches; with stats the call also waits after each pair of shards to read their counters. */
+/* HOST pointers; blocks until the outputs are on the host. */
+int rbrt_gpu_render_hdr_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint32_t splits,
+                                 const rbrt_render_opts* opts, float* hdr_out, float* var_out, rbrt_stats* stats);
+/* DEVICE pointers on the scene's first device, enqueued on cuda_stream (0 = default stream); stats == NULL: enqueue only, no
+ * synchronisation.  Also refused: outputs in another device's memory or in unregistered host memory. */
+int rbrt_gpu_render_hdr_variance_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint32_t splits,
+                                        const rbrt_render_opts* opts, float* d_hdr_out, float* d_var_out, void* cuda_stream,
+                                        rbrt_stats* stats);
+
+/* VARIANCE-GUIDED FILTER: rbrt_gpu_denoise with the variance of the colour steering the luminance term (the spatial filter of SVGF with
+ * its variance estimate and propagation, Schied et al. 2017, without temporal terms).  Inputs as rbrt_gpu_denoise, plus var (W*H*3, as
+ * var_out above).  rbrt_denoise_opts is read with this filter's defaults: levels 5, σ_z = 0.01, σ_l = 4.  Per pixel p, each operation one
+ * correctly rounded f32 operation, products and sums left to right as written:
+ *   1. d, e, l and validity as rbrt_gpu_denoise step 1; p is also INVALID when a component of var is NaN, +-inf or negative (-0 is not).
+ *      σ² = sd * sd with sd = ((0.2126 / d.r) * sqrt(v.r) + (0.7152 / d.g) * sqrt(v.g)) + (0.0722 / d.b) * sqrt(v.b).  This adds the
+ *      channels' standard deviations: an upper bound of the deviation of l(e) (Cauchy-Schwarz), exact for fully correlated channels, as
+ *      path-tracing noise mostly is.  Per-channel variances cannot give the covariances that the exact value needs.
+ *   2. levels L, level i = 0 .. L-1 with step s = 2^i, filters the previous level's e and σ² (level 0: step 1's).  For a valid p:
+ *        g_p  = (Σ k[dx]*k[dy] * σ²_q) / (Σ k[dx]*k[dy]) over the 3x3 neighbours q = p + (dx, dy), dx, dy in -1..1, inside the image and
+ *               valid, row-major, sums from +0, k = {1/4, 1/2, 1/4} (products exact);
+ *        r'_p = 1 / (σ_l * sqrt(g_p) + 2^-10);  x_l = (l_p - l_q) * r'_p;
+ *        taps, skips, w_n, x_z, r_p and the centre weight 9/64 as rbrt_gpu_denoise step 2, and for a tap other than the centre
+ *        w    = (h[dx]*h[dy] * w_n) / ((1 + x_z*x_z) * ((1 + x_l*x_l) * (1 + x_l*x_l)));
+ *        e'   = Σ w*e_q / Σw per channel;  σ²' = (Σ (w*w) * σ²_q) / (Σw * Σw), sums from +0 in tap order.
+ *      An invalid p keeps its e and σ².
+ *   3. hdr_out and rgb_out as rbrt_gpu_denoise step 3.
+ * A pixel whose variance is 0 (a converged or constant region) takes no tap whose luminance differs: a well-sampled frame is not blurred.
+ * Refusals, devices, stats and the scratch's stream-ordered allocation as rbrt_gpu_denoise*, plus a NULL var and an output that overlaps
+ * var; the scratch is 56 bytes per pixel.  The kernels live in librbrt_gpu_variance.so (RBRT_GPU_VARIANCE_LIB: another path). */
+/* HOST pointers; blocks until the outputs are on the host. */
+int rbrt_gpu_denoise_variance(uint32_t width, uint32_t height, const float* hdr, const float* var, const rbrt_aov_out* guides,
+                              const rbrt_denoise_opts* opts, float* hdr_out, uint8_t* rgb_out, rbrt_stats* stats);
+/* DEVICE pointers on the current render device, enqueued on cuda_stream; stats == NULL: enqueue only. */
+int rbrt_gpu_denoise_variance_device(uint32_t width, uint32_t height, const float* d_hdr, const float* d_var, const rbrt_aov_out* d_guides,
+                                     const rbrt_denoise_opts* opts, float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream,
+                                     rbrt_stats* stats);
+
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
- * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters and the
- * denoiser's host-call block). */
+ * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters, the
+ * denoiser's host-call block and the variance call's internal stream). */
 int rbrt_gpu_release_cache(void);
 
 /* Upper bound, in bytes, of ONE pool of wavefront state (there are up to four per device, one per frame in flight).

@@ -147,6 +147,22 @@ extern "C" {
     /// The same on DEVICE planes of the current render device, enqueued on `stream` (stats = null: no synchronisation).
     pub fn rbrt_gpu_denoise_device(width: u32, height: u32, d_hdr: *const f32, d_guides: *const RbrtAovOut, opts: *const RbrtDenoiseOpts,
                                    d_hdr_out: *mut f32, d_rgb_out: *mut u8, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// The mean colour of num_samples samples rendered as `splits` (2..16) sample-range shards, and the unbiased variance of that mean
+    /// per pixel and channel (W*H*3 f32 each, either may be null); HOST pointers, blocks.
+    pub fn rbrt_gpu_render_hdr_variance(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, splits: u32,
+                                        opts: *const RbrtRenderOpts, hdr_out: *mut f32, var_out: *mut f32, stats: *mut RbrtStats) -> c_int;
+    /// The same into DEVICE buffers, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_render_hdr_variance_device(scene: *const RbrtScene, cam: *const RbrtCamera, num_samples: u32, splits: u32,
+                                               opts: *const RbrtRenderOpts, d_hdr_out: *mut f32, d_var_out: *mut f32, stream: *mut c_void,
+                                               stats: *mut RbrtStats) -> c_int;
+    /// Variance-guided à-trous denoise of a render_hdr_variance frame and its variance, guided by render_aov depth / normal / albedo of
+    /// the same camera and seed; HOST pointers, blocks.  opts may be null (5 levels).
+    pub fn rbrt_gpu_denoise_variance(width: u32, height: u32, hdr: *const f32, var: *const f32, guides: *const RbrtAovOut,
+                                     opts: *const RbrtDenoiseOpts, hdr_out: *mut f32, rgb_out: *mut u8, stats: *mut RbrtStats) -> c_int;
+    /// The same on DEVICE planes of the current render device, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_denoise_variance_device(width: u32, height: u32, d_hdr: *const f32, d_var: *const f32, d_guides: *const RbrtAovOut,
+                                            opts: *const RbrtDenoiseOpts, d_hdr_out: *mut f32, d_rgb_out: *mut u8, stream: *mut c_void,
+                                            stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

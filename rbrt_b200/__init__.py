@@ -15,8 +15,8 @@ from .cam import Camera
 from .materials import Dielectric, Lambertian, Metal
 from .mesh import TriangleMesh, load_mesh_vertices_from_file
 from .pipeline import FramePipeline
-from .render import (AOV_PASSES, ImageBuffer, denoise, denoise_device, primary_rays, render_aovs, render_aovs_device, render_scene,
-                     render_scene_hdr)
+from .render import (AOV_PASSES, ImageBuffer, denoise, denoise_device, denoise_variance, denoise_variance_device, primary_rays, render_aovs,
+                     render_aovs_device, render_hdr_variance_device, render_scene, render_scene_hdr, render_scene_hdr_variance)
 from .scene import Scene
 from .sphere import Sphere
 from .triangle import BasicTriangle

@@ -174,6 +174,14 @@ GPU_SIGNATURES = {
     "rbrt_gpu_denoise": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, C.c_void_p,
                                           P(StatsC)]),
+    "rbrt_gpu_render_hdr_variance": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint32, P(RenderOptsC), C.c_void_p, C.c_void_p,
+                                               P(StatsC)]),
+    "rbrt_gpu_render_hdr_variance_device": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint32, P(RenderOptsC), C.c_void_p,
+                                                      C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_denoise_variance": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p,
+                                            C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_denoise_variance_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, P(AovOutC), P(DenoiseOptsC),
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

@@ -16,6 +16,7 @@
 #include "multi.cuh"
 #include "query.cuh"
 #include "update.cuh"
+#include "variance.cuh"
 
 namespace rbrt {
 
@@ -375,12 +376,15 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
 }
 
 // ------------------------------------------------------------------ device modules with one launch entry point
-// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path), the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB) and the
-// denoiser (librbrt_gpu_denoise.so, RBRT_GPU_DENOISE_LIB) live in their own device modules, like the refit; each is opened once, on first use.
+// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path), the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB), the
+// denoiser (librbrt_gpu_denoise.so, RBRT_GPU_DENOISE_LIB) and the variance kernels (librbrt_gpu_variance.so, RBRT_GPU_VARIANCE_LIB) live in
+// their own device modules, like the refit; each is opened once, on first use.
 struct LaunchModule { const char* env; const char* file; const char* what; const char* symbol; void* launch; };
 static LaunchModule g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", "rbrt_aov_launch", nullptr};
 static LaunchModule g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", "rbrt_query_launch", nullptr};
 static LaunchModule g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", "rbrt_denoise_launch", nullptr};
+static LaunchModule g_moments_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", "rbrt_variance_moments_launch", nullptr};
+static LaunchModule g_vfilter_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", "rbrt_variance_filter_launch", nullptr};
 static int load_module(LaunchModule& m) {
     if (!m.launch) {
         std::string path;
@@ -581,7 +585,7 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     return RBRT_OK;
 }
 
-// ------------------------------------------------------------------ guided denoising (rbrt_gpu_denoise*)
+// ------------------------------------------------------------------ guided denoising (rbrt_gpu_denoise*, rbrt_gpu_denoise_variance*)
 // Per device: the block the host-pointer variant copies its planes into and carves its scratch from (grown, never shrunk, until
 // rbrt_gpu_release_cache), and the events of calls with stats.  Only calls that synchronise before returning use them.  The device
 // variant takes its scratch from the stream-ordered allocator on the call's stream instead, so calls in flight never share it.
@@ -607,10 +611,11 @@ static bool overlap(const void* a, size_t na, const void* b, size_t nb) {
     return x < y + nb && y < x + na;
 }
 
-static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts, float* hdr_out,
-                   uint8_t* rgb_out, bool host, cudaStream_t st, rbrt_stats* stats) {
+// var: the variance-guided filter of librbrt_gpu_variance.so with that variance plane; NULL: rbrt_gpu_denoise's filter.
+static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,
+                   float* hdr_out, uint8_t* rgb_out, bool with_var, bool host, cudaStream_t st, rbrt_stats* stats) {
     if (stats) memset(stats, 0, sizeof(*stats));
-    if (!hdr || !guides) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!hdr || !guides || (with_var && !var)) { set_error("null argument"); return RBRT_E_INVALID; }
     if (!guides->depth || !guides->normal || !guides->albedo) { set_error("null guide plane: depth, normal and albedo are read"); return RBRT_E_INVALID; }
     if (!hdr_out && !rgb_out) { set_error("no output requested (hdr_out and rgb_out are both NULL)"); return RBRT_E_INVALID; }
     if (!W || !H) { set_error("empty image"); return RBRT_E_INVALID; }
@@ -619,14 +624,15 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out*
     DenoiseArgs a;
     memset(&a, 0, sizeof(a));
     a.W = W; a.H = H;
-    a.levels = opts && opts->levels ? opts->levels : DN_DEFAULT_LEVELS;
+    a.levels = opts && opts->levels ? opts->levels : (with_var ? VR_DEFAULT_LEVELS : DN_DEFAULT_LEVELS);
     if (a.levels > DN_MAX_LEVELS) { set_error("levels must be at most %u", DN_MAX_LEVELS); return RBRT_E_INVALID; }
     const float sz = opts ? opts->sigma_depth : 0.0f, sl = opts ? opts->sigma_luminance : 0.0f;
     if (!(sz >= 0.0f && sz <= FLT_MAX) || !(sl >= 0.0f && sl <= FLT_MAX)) { set_error("a sigma must be finite and >= 0 (0 = default)"); return RBRT_E_INVALID; }
-    a.sigma_z = sz > 0.0f ? sz : DN_SIGMA_DEPTH;
-    a.sigma_l = sl > 0.0f ? sl : DN_SIGMA_LUMINANCE;
+    a.sigma_z = sz > 0.0f ? sz : (with_var ? VR_SIGMA_DEPTH : DN_SIGMA_DEPTH);
+    a.sigma_l = sl > 0.0f ? sl : (with_var ? VR_SIGMA_LUMINANCE : DN_SIGMA_LUMINANCE);
     {
-        const struct { const void* p; size_t b; } in[4] = {{hdr, 12 * n}, {guides->depth, 4 * n}, {guides->normal, 12 * n}, {guides->albedo, 12 * n}};
+        const struct { const void* p; size_t b; } in[5] = {{hdr, 12 * n}, {guides->depth, 4 * n}, {guides->normal, 12 * n}, {guides->albedo, 12 * n},
+                                                           {var, 12 * n}};
         for (const auto& i : in) {
             if (overlap(hdr_out, 12 * n, i.p, i.b) || overlap(rgb_out, 3 * n, i.p, i.b)) { set_error("an output overlaps an input"); return RBRT_E_INVALID; }
         }
@@ -635,20 +641,22 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out*
     { int rc = ensure_device(); if (rc) return rc; }
     const int dev = g_device;
     if (!host) {
-        const void* ptrs[6] = {hdr, guides->depth, guides->normal, guides->albedo, hdr_out, rgb_out};
+        const void* ptrs[7] = {hdr, guides->depth, guides->normal, guides->albedo, hdr_out, rgb_out, var};
         for (const void* p : ptrs)
             if (p && !usable_on(p, dev)) { set_error("planes must be device memory on the current device %d", dev); return RBRT_E_INVALID; }
     }
-    { int rc = load_module(g_denoise_module); if (rc) return rc; }
+    { int rc = load_module(with_var ? g_vfilter_module : g_denoise_module); if (rc) return rc; }
     const rbrt_denoise_launch_fn launch = reinterpret_cast<rbrt_denoise_launch_fn>(g_denoise_module.launch);
+    const rbrt_variance_filter_launch_fn vlaunch = reinterpret_cast<rbrt_variance_filter_launch_fn>(g_vfilter_module.launch);
+    const size_t scratch = (with_var ? 56 : 48) * n;                      // guides and two planes of (e.rgb, l); with var two planes of σ²
     const double t0 = now_ms();
 
     DenoisePool& pool = g_denoise[dev & 63];
     if (stats && !pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
     a.hdr = hdr; a.depth = guides->depth; a.normal = guides->normal; a.albedo = guides->albedo; a.hdr_out = hdr_out; a.rgb_out = rgb_out;
     if (host) {                                                           // inputs, outputs and scratch carved from the pooled block
-        const size_t b1 = a256(4 * n), b3 = a256(12 * n), bs = a256(48 * n);
-        const size_t need = bs + 3 * b3 + b1 + (hdr_out ? b3 : 0) + (rgb_out ? a256(3 * n) : 0);
+        const size_t b1 = a256(4 * n), b3 = a256(12 * n), bs = a256(scratch);
+        const size_t need = bs + 3 * b3 + b1 + (with_var ? b3 : 0) + (hdr_out ? b3 : 0) + (rgb_out ? a256(3 * n) : 0);
         if (pool.bytes < need) {
             cudaFree(pool.buf); pool.buf = nullptr; pool.bytes = 0;
             CKA(cudaMalloc(&pool.buf, need)); pool.bytes = need;
@@ -664,20 +672,25 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out*
         CKA(cudaMemcpyAsync(d_alb, guides->albedo, 12 * n, cudaMemcpyHostToDevice, st));
         CKA(cudaMemcpyAsync(d_dep, guides->depth, 4 * n, cudaMemcpyHostToDevice, st));
         a.hdr = d_hdr; a.normal = d_nrm; a.albedo = d_alb; a.depth = d_dep;
+        if (with_var) {
+            float* d_var = (float*)p; p += b3;
+            CKA(cudaMemcpyAsync(d_var, var, 12 * n, cudaMemcpyHostToDevice, st));
+            var = d_var;
+        }
         if (hdr_out) { a.hdr_out = (float*)p; p += b3; }
         if (rgb_out) a.rgb_out = (uint8_t*)p;
     } else {
-        CKA(cudaMallocAsync((void**)&a.scratch, 48 * n, st));
+        CKA(cudaMallocAsync((void**)&a.scratch, scratch, st));
     }
     if (stats) {
         cudaError_t e = cudaEventRecord(pool.e0, st);
         if (e != cudaSuccess) { if (!host) cudaFreeAsync(a.scratch, st); return cuda_fail(e, "cudaEventRecord"); }
     }
     {
-        cudaError_t e = (cudaError_t)launch(&a, st);
+        cudaError_t e = (cudaError_t)(with_var ? vlaunch(&a, var, st) : launch(&a, st));
         if (e == cudaSuccess && stats) e = cudaEventRecord(pool.e1, st);
         if (!host) { cudaError_t f = cudaFreeAsync(a.scratch, st); if (e == cudaSuccess) e = f; }
-        if (e != cudaSuccess) return cuda_fail(e, "rbrt_denoise_launch");
+        if (e != cudaSuccess) return cuda_fail(e, with_var ? "rbrt_variance_filter_launch" : "rbrt_denoise_launch");
     }
     if (host) {
         if (hdr_out) CKA(cudaMemcpyAsync(hdr_out, a.hdr_out, 12 * n, cudaMemcpyDeviceToHost, st));
@@ -691,6 +704,114 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const rbrt_aov_out*
         float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
         stats->ms_device = ms; stats->launches = 1 + a.levels;
         stats->ms_total = now_ms() - t0;
+    }
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ variance of a render from sample shards (rbrt_gpu_render_hdr_variance*)
+// Shard k renders samples [k*n, (k+1)*n) into its own accumulator.  The shards alternate between two lanes: the caller's stream with the
+// wavefront pool p of opts->flags, and an internal stream of the device with pool 4 + p (the second lane of RBRT_OPT_SPLIT_BATCHES).  No
+// shard waits for another (each has its own accumulator), so the sparse last bounces of one shard run under the dense first bounces of the
+// shard on the other lane.  The moments kernel then runs on the caller's stream behind both lanes.
+struct VariancePool { cudaStream_t aux = nullptr; cudaEvent_t fork = nullptr, join = nullptr, e0 = nullptr, e1 = nullptr; };
+static VariancePool g_variance[64];
+static void variance_release_all() {
+    int cur = 0; cudaGetDevice(&cur);
+    for (int d = 0; d < 64; ++d) {
+        VariancePool& p = g_variance[d];
+        if (!p.aux) continue;
+        cudaSetDevice(d);
+        cudaStreamSynchronize(p.aux); cudaStreamDestroy(p.aux);
+        for (cudaEvent_t e : {p.fork, p.join, p.e0, p.e1}) if (e) cudaEventDestroy(e);
+        p = VariancePool();
+    }
+    cudaSetDevice(cur);
+}
+
+static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t S, uint32_t K, const rbrt_render_opts* opts,
+                           float* hdr_out, float* var_out, bool host, cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!scene || !cam) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!hdr_out && !var_out) { set_error("no output requested (hdr_out and var_out are both NULL)"); return RBRT_E_INVALID; }
+    if (K < 2 || K > VR_MAX_SPLITS) { set_error("splits must be 2..%u", VR_MAX_SPLITS); return RBRT_E_INVALID; }
+    if (!S || S % K) { set_error("num_samples must be a positive multiple of splits"); return RBRT_E_INVALID; }
+    rbrt_render_opts o{}; if (opts) o = *opts;
+    if (o.shard_count > 1) { set_error("shard_count > 1: the call shards the samples itself"); return RBRT_E_INVALID; }
+    const size_t n = (size_t)cam->img_width_pix * cam->img_height_pix;
+    if (!n) { set_error("empty image"); return RBRT_E_INVALID; }
+    if (n > 0x7FFFFFFFull) { set_error("image too large"); return RBRT_E_INVALID; }
+    if (overlap(hdr_out, 12 * n, var_out, 12 * n)) { set_error("hdr_out and var_out overlap"); return RBRT_E_INVALID; }
+    const Scene& sc = *reinterpret_cast<const Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device, whole image
+    CKA(cudaSetDevice(rp.device));
+    if (!host)
+        for (const void* p : {(const void*)hdr_out, (const void*)var_out})
+            if (p && !usable_on(p, rp.device)) { set_error("outputs must be device memory on the scene's device %d", rp.device); return RBRT_E_INVALID; }
+    const double t0 = now_ms();
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    { int rc = load_module(g_moments_module); if (rc) return rc; }
+    const rbrt_variance_moments_launch_fn launch = reinterpret_cast<rbrt_variance_moments_launch_fn>(g_moments_module.launch);
+    VariancePool& vp = g_variance[rp.device & 63];
+    if (!vp.aux) {
+        CKA(cudaStreamCreateWithFlags(&vp.aux, cudaStreamNonBlocking));
+        CKA(cudaEventCreateWithFlags(&vp.fork, cudaEventDisableTiming)); CKA(cudaEventCreateWithFlags(&vp.join, cudaEventDisableTiming));
+        CKA(cudaEventCreate(&vp.e0)); CKA(cudaEventCreate(&vp.e1));
+    }
+    const uint32_t pool = (o.flags & RBRT_OPT_POOL_MASK) >> RBRT_OPT_POOL_SHIFT;
+    o.flags &= ~(uint32_t)RBRT_OPT_SPLIT_BATCHES;                         // the two lanes are the shards'
+    o.shard_mode = RBRT_SHARD_SAMPLES; o.shard_count = K;
+
+    // K accumulators, then (host variant) the two output planes, from the stream-ordered allocator on the call's stream
+    const size_t b_acc = 16 * n * K, b3 = a256(12 * n);
+    char* block = nullptr;
+    CKA(cudaMallocAsync((void**)&block, b_acc + (host ? 2 * b3 : 0), st));
+    MomentsArgs m;
+    memset(&m, 0, sizeof(m));
+    m.W = cam->img_width_pix; m.H = cam->img_height_pix; m.K = K;
+    m.inv_S = 1.0f / (float)S; m.inv_n = 1.0f / (float)(S / K);
+    m.acc = (const float4*)block;
+    m.hdr_out = hdr_out ? (host ? (float*)(block + b_acc) : hdr_out) : nullptr;
+    m.var_out = var_out ? (host ? (float*)(block + b_acc + b3) : var_out) : nullptr;
+    std::vector<RenderJob> jobs(stats ? K : 0);
+    uint32_t launches = 0;
+    cudaError_t e = cudaSuccess;
+    int rc = RBRT_OK;
+    if (stats) e = cudaEventRecord(vp.e0, st);
+    if (e == cudaSuccess) e = cudaEventRecord(vp.fork, st);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(vp.aux, vp.fork, 0);
+    for (uint32_t k = 0; k < K && e == cudaSuccess && !rc; ++k) {
+        const int lane = (int)(k & 1);
+        o.shard_rank = k;
+        float4* acc1[1] = {(float4*)(block + 16 * n * k)};
+        rc = render_accum(sc, 0, cam, nullptr, 1, S, &o, acc1, lane ? vp.aux : st, nullptr, stats ? &jobs[k] : nullptr, (int)pool + 4 * lane);
+        if (rc || !stats || (lane == 0 && k + 1 < K)) continue;
+        for (uint32_t j = k - lane; j <= k && !rc; ++j) {                 // this round's counters, before the next round resets its pools
+            rbrt_stats one; memset(&one, 0, sizeof(one));
+            rc = collect_stats(jobs[j], &one);
+            stats->rays += one.rays; stats->paths += one.paths; stats->nan_rays += one.nan_rays; launches += one.launches;
+        }
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(vp.join, vp.aux);           // (also when a shard was refused: the block is freed behind both lanes)
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, vp.join, 0);
+    if (e == cudaSuccess && !rc) e = (cudaError_t)launch(&m, st);
+    if (e == cudaSuccess && !rc && stats) e = cudaEventRecord(vp.e1, st);
+    if (e == cudaSuccess && !rc && host) {
+        if (hdr_out) e = cudaMemcpyAsync(hdr_out, m.hdr_out, 12 * n, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess && var_out) e = cudaMemcpyAsync(var_out, m.var_out, 12 * n, cudaMemcpyDeviceToHost, st);
+    }
+    {
+        const cudaError_t f = cudaFreeAsync(block, st);
+        if (e == cudaSuccess) e = f;
+    }
+    if (rc) return rc;
+    if (e != cudaSuccess) return cuda_fail(e, "rbrt_gpu_render_hdr_variance");
+    if (host) CKA(cudaStreamSynchronize(st));
+    if (stats) {
+        CKA(cudaEventSynchronize(vp.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, vp.e0, vp.e1));
+        stats->ms_device = ms; stats->launches = launches + 1;
+        stats->ms_total = now_ms() - t0;
+        return resolve_scene_info(sc, true);
     }
     return RBRT_OK;
 }
@@ -995,6 +1116,7 @@ int rbrt_gpu_release_cache(void) {
     aov_release_all();
     query_release_all();
     denoise_release_all();
+    variance_release_all();
     arena_release_all();
     for (void* p : g_pinned_free) cudaFreeHost(p);
     g_pinned_free.clear();
@@ -1159,13 +1281,37 @@ int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_ra
 int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,
                      float* hdr_out, uint8_t* rgb_out, rbrt_stats* stats) {
     LOCK;
-    return denoise(width, height, hdr, guides, opts, hdr_out, rgb_out, true, 0, stats);
+    return denoise(width, height, hdr, nullptr, guides, opts, hdr_out, rgb_out, false, true, 0, stats);
 }
 
 int rbrt_gpu_denoise_device(uint32_t width, uint32_t height, const float* d_hdr, const rbrt_aov_out* d_guides, const rbrt_denoise_opts* opts,
                             float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats) {
     LOCK;
-    return denoise(width, height, d_hdr, d_guides, opts, d_hdr_out, d_rgb_out, false, (cudaStream_t)cuda_stream, stats);
+    return denoise(width, height, d_hdr, nullptr, d_guides, opts, d_hdr_out, d_rgb_out, false, false, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_render_hdr_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint32_t splits,
+                                 const rbrt_render_opts* opts, float* hdr_out, float* var_out, rbrt_stats* stats) {
+    LOCK;
+    return render_variance(scene, cam, num_samples, splits, opts, hdr_out, var_out, true, 0, stats);
+}
+
+int rbrt_gpu_render_hdr_variance_device(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t num_samples, uint32_t splits,
+                                        const rbrt_render_opts* opts, float* d_hdr_out, float* d_var_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return render_variance(scene, cam, num_samples, splits, opts, d_hdr_out, d_var_out, false, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_denoise_variance(uint32_t width, uint32_t height, const float* hdr, const float* var, const rbrt_aov_out* guides,
+                              const rbrt_denoise_opts* opts, float* hdr_out, uint8_t* rgb_out, rbrt_stats* stats) {
+    LOCK;
+    return denoise(width, height, hdr, var, guides, opts, hdr_out, rgb_out, true, true, 0, stats);
+}
+
+int rbrt_gpu_denoise_variance_device(uint32_t width, uint32_t height, const float* d_hdr, const float* d_var, const rbrt_aov_out* d_guides,
+                                     const rbrt_denoise_opts* opts, float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return denoise(width, height, d_hdr, d_var, d_guides, opts, d_hdr_out, d_rgb_out, true, false, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

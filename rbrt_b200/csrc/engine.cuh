@@ -127,8 +127,10 @@ struct RenderJob {
 int make_shard(const rbrt_render_opts& o, uint32_t W, uint32_t H, uint32_t spp, ShardDev* out);
 // Renders replica `li` of the scene on that replica's device (the caller has made it current).  With `job` the call only
 // enqueues and fills *job (collect_stats later); without, stats (may be NULL = enqueue only) are collected before returning.
+// pool: the wavefront pool, 0..7 (4 + p: the second lane of pool p, see RBRT_OPT_SPLIT_BATCHES); -1 = the one opts->flags name.
 int render_accum(const Scene& sc, int li, const rbrt_camera* cams, const uint64_t* seeds, uint32_t n_frames, uint32_t spp,
-                 const rbrt_render_opts* opts, float4* const* d_accum, cudaStream_t st, rbrt_stats* stats, RenderJob* job = nullptr);
+                 const rbrt_render_opts* opts, float4* const* d_accum, cudaStream_t st, rbrt_stats* stats, RenderJob* job = nullptr,
+                 int pool = -1);
 int collect_stats(RenderJob& job, rbrt_stats* stats);
 int trace_rays_wavefront(const Scene& sc, const rbrt_ray* d_rays, uint64_t n, rbrt_hit* d_hits, unsigned long long* d_stats, cudaStream_t st);
 int scatter_device(const rbrt_scatter_in* d_in, uint64_t n, uint64_t seed, rbrt_scatter_out* d_out, cudaStream_t st);

@@ -259,6 +259,8 @@ void usage() {
            "                                   <prefix>.depth.pfm, <prefix>.normal.pfm, <prefix>.albedo.pfm, <prefix>.coverage.pfm\n"
            "      --aov-samples <n>            (extension) samples per pixel of the AOVs [default: --samples]\n"
            "      --denoise                    (extension) save the image denoised on the GPU, guided by AOVs of the same camera and --seed [--aov-samples default: min(--samples, 4)]\n"
+           "      --denoise-splits <k>         (extension, with --denoise) render the image as k sample shards (2..16, dividing --samples) for its per-pixel\n"
+           "                                   variance, and denoise with the variance-guided filter [--aov-samples default: min(--samples / k, 4)]\n"
            "  -h, --help                       Print help\n  -V, --version                    Print version\n");
 }
 
@@ -277,7 +279,7 @@ int main(int argc, char** argv) {
     uint64_t seed = 0; int device = 0; bool check_only = false, dump = false, denoise = false;
     uint32_t gpus = 1; int transport = RBRT_TRANSPORT_AUTO;
     std::string from_ppm, aov;
-    uint32_t aov_samples = 0;
+    uint32_t aov_samples = 0, denoise_splits = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         auto value = [&](const char* name) -> const char* {
@@ -306,11 +308,20 @@ int main(int argc, char** argv) {
         else if (key == "--aov") aov = value("--aov");
         else if (key == "--aov-samples") aov_samples = parse_u32(value("--aov-samples"), "--aov-samples");
         else if (key == "--denoise") denoise = true;
+        else if (key == "--denoise-splits") denoise_splits = parse_u32(value("--denoise-splits"), "--denoise-splits");
         else if (key == "-h" || key == "--help") { usage(); return 0; }
         else if (key == "-V" || key == "--version") { printf("rbrt 0.1 (%s)\n", rbrt_gpu_version()); return 0; }
         else { fprintf(stderr, "error: unexpected argument '%s' found\n", a.c_str()); return 2; }
     }
 
+    if (denoise_splits) {
+        if (!denoise) die("error: '--denoise-splits' needs '--denoise'");
+        if (denoise_splits < 2 || denoise_splits > 16) die("error: '--denoise-splits' must be 2..16");
+        if (!samples || samples % denoise_splits) die("error: '--denoise-splits' must divide '--samples'");
+        if (aov_samples > samples / denoise_splits)
+            die("error: '--aov-samples' must not exceed '--samples' / '--denoise-splits' with '--denoise-splits': the guides must be the first camera rays of shard 0");
+        if (!aov_samples) aov_samples = std::min<uint32_t>(samples / denoise_splits, 4);
+    }
     if (denoise) {
         if (!from_ppm.empty()) die("error: '--denoise' cannot be used with '--from-ppm' (there is no render to denoise)");
         if (aov_samples > samples) die("error: '--aov-samples' must not exceed '--samples' with '--denoise': the guides must be the image's first camera rays");
@@ -380,8 +391,12 @@ int main(int argc, char** argv) {
     std::vector<uint8_t> rgb((size_t)width * height * 3);
     rbrt_render_opts opts; memset(&opts, 0, sizeof(opts)); opts.seed = seed;
     rbrt_stats st;
-    std::vector<float> hdr;
-    if (denoise) {                                                                 // the mean colour, denoised below into rgb
+    std::vector<float> hdr, var;
+    if (denoise_splits) {                                                          // the mean colour and its variance (on the first device)
+        hdr.resize((size_t)width * height * 3); var.resize(hdr.size());
+        if (rbrt_gpu_render_hdr_variance(scene, &cam, samples, denoise_splits, &opts, hdr.data(), var.data(), &st) != RBRT_OK)
+            die(std::string("rbrt_gpu: ") + rbrt_last_error());
+    } else if (denoise) {                                                          // the mean colour, denoised below into rgb
         hdr.resize((size_t)width * height * 3);
         if (rbrt_gpu_render_hdr(scene, &cam, samples, &opts, hdr.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
     } else if (rbrt_gpu_render(scene, &cam, samples, &opts, rgb.data(), &st) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
@@ -393,7 +408,10 @@ int main(int argc, char** argv) {
         rbrt_aov_out ao; memset(&ao, 0, sizeof(ao));
         ao.depth = depth.data(); ao.normal = normal.data(); ao.albedo = albedo.data(); ao.coverage = coverage.data();
         if (rbrt_gpu_render_aov(scene, &cam, aov_samples ? aov_samples : samples, seed, &ao, nullptr) != RBRT_OK) die(std::string("rbrt_gpu: ") + rbrt_last_error());
-        if (denoise && rbrt_gpu_denoise(width, height, hdr.data(), &ao, nullptr, nullptr, rgb.data(), nullptr) != RBRT_OK)   // on the first device
+        if (denoise_splits) {
+            if (rbrt_gpu_denoise_variance(width, height, hdr.data(), var.data(), &ao, nullptr, nullptr, rgb.data(), nullptr) != RBRT_OK)
+                die(std::string("rbrt_gpu: ") + rbrt_last_error());
+        } else if (denoise && rbrt_gpu_denoise(width, height, hdr.data(), &ao, nullptr, nullptr, rgb.data(), nullptr) != RBRT_OK)   // on the first device
             die(std::string("rbrt_gpu: ") + rbrt_last_error());
     }
     rbrt_gpu_scene_destroy(scene);

@@ -976,7 +976,8 @@ int make_shard(const rbrt_render_opts& o, uint32_t W, uint32_t H, uint32_t spp, 
 }
 
 int render_accum(const Scene& sc, int li, const rbrt_camera* cams, const uint64_t* seeds, uint32_t n_frames, uint32_t spp,
-                 const rbrt_render_opts* opts, float4* const* d_accum, cudaStream_t st, rbrt_stats* stats, RenderJob* job_out) {
+                 const rbrt_render_opts* opts, float4* const* d_accum, cudaStream_t st, rbrt_stats* stats, RenderJob* job_out,
+                 int pool_arg) {
     const Replica& rp = sc.rep[li];
     RenderJob local_job;
     RenderJob& job = job_out ? *job_out : local_job;
@@ -999,16 +1000,16 @@ int render_accum(const Scene& sc, int li, const rbrt_camera* cams, const uint64_
     wait_scene_ready(sc, li, st);                                         // the scene's build / replication is asynchronous
     for (uint32_t f = 0; f < n_frames; ++f) CKR(cudaMemsetAsync(d_accum[f], 0, 16ull * W * H, st));
     uint32_t launches = 0, iterations = 0, batch_iters = 0;
-    const int pool = (int)((o.flags & RBRT_OPT_POOL_MASK) >> RBRT_OPT_POOL_SHIFT);
+    const int pool = pool_arg >= 0 ? pool_arg & 7 : (int)((o.flags & RBRT_OPT_POOL_MASK) >> RBRT_OPT_POOL_SHIFT);
     // TWO LANES (RBRT_OPT_SPLIT_BATCHES).  A batch ends sparsely: its last bounce iterations and the tail kernel are latency chains
     // that leave most SMs idle (1/8 shard of C3: ~2.3 of 6.3 ms), and for a LONE frame no other frame is there to fill them.  So the
     // frame's samples are cut into at least two batches that alternate between two lanes — the caller's stream with pool p, an
     // internal stream with pool 4 + p — and the dense start of one batch runs under the sparse end of the previous one.  The
     // per-pixel sums keep their sample order: a batch's k_accumulate waits (event) for the previous batch's.
-    const bool split = (o.flags & RBRT_OPT_SPLIT_BATCHES) && !(o.flags & RBRT_OPT_TIME_KERNELS) && sh.s1 - sh.s0 >= 2;
+    const bool split = (o.flags & RBRT_OPT_SPLIT_BATCHES) && !(o.flags & RBRT_OPT_TIME_KERNELS) && sh.s1 - sh.s0 >= 2 && pool < 4;
     WaveBuffers* wbs[2] = {&device_wave_buffers(rp.device, pool), split ? &device_wave_buffers(rp.device, 4 + pool) : nullptr};
     WaveBuffers& wb = *wbs[0];
-    SplitLane& SL = g_lane[pool][rp.device & 63];
+    SplitLane& SL = g_lane[pool & 3][rp.device & 63];
     if (split) { int rc_l = ensure_lane(SL); if (rc_l) return rc_l; }
     cudaStream_t lane_st[2] = {st, split ? SL.aux : st};
     uint32_t lane_iters[2] = {0, 0};

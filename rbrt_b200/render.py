@@ -255,3 +255,72 @@ def denoise_device(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, st
     _abi.check(_abi.lib().rbrt_gpu_denoise_device(W, H, hdr.data_ptr(), g, _denoise_opts(levels, sigma_depth, sigma_luminance),
                                                   out.data_ptr(), rgb.data_ptr(), stream.cuda_stream, None))
     return out, rgb
+
+
+# ---- per-pixel variance and variance-guided denoising (rbrt_gpu_render_hdr_variance*, rbrt_gpu_denoise_variance*; DESIGN.md section 14)
+def render_scene_hdr_variance(cam, num_samples, scene, splits=4, stats=None, **opts):
+    """The pre-gamma mean colour [H,W,3] f32 of num_samples samples, rendered as `splits` sample-range shards (2..16, dividing
+    num_samples), and the unbiased variance of that mean per pixel and channel [H,W,3] f32, from the spread of the shards' means.
+    Returns (hdr, var); blocks until both are on the host."""
+    W, H = cam.img_width_pix, cam.img_height_pix
+    hdr = np.empty((H, W, 3), dtype=np.float32)
+    var = np.empty((H, W, 3), dtype=np.float32)
+    st = _abi.StatsC()
+    _abi.check(_abi.lib().rbrt_gpu_render_hdr_variance(scene.handle(), cam.to_c(), int(num_samples), int(splits), make_opts(**opts),
+                                                       hdr.ctypes.data, var.ctypes.data, st))
+    if stats is not None:
+        stats.update(st.as_dict())
+    return hdr, var
+
+
+def render_hdr_variance_device(cam, num_samples, scene, splits=4, stream=None, **opts):
+    """The same as CUDA tensors on the scene's first device, enqueued on `stream` (default: the current stream) without synchronising."""
+    import torch
+    stream = stream or torch.cuda.current_stream()
+    W, H = cam.img_width_pix, cam.img_height_pix
+    handle = scene.handle()
+    with torch.cuda.stream(stream):
+        hdr = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
+        var = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
+    _abi.check(_abi.lib().rbrt_gpu_render_hdr_variance_device(handle, cam.to_c(), int(num_samples), int(splits), make_opts(**opts),
+                                                              hdr.data_ptr(), var.data_ptr(), stream.cuda_stream, None))
+    return hdr, var
+
+
+def _variance_input(var, hdr, is_tensor):
+    if is_tensor(var) is not True or tuple(var.shape) != tuple(hdr.shape):
+        raise ValueError(f"var must be a contiguous float32 {'CUDA tensor' if is_tensor is _is_cuda_f32 else 'numpy array'} of the shape of hdr")
+
+
+def denoise_variance(hdr, var, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stats=None):
+    """Denoise a render_scene_hdr_variance frame [H,W,3] with its variance [H,W,3], guided by render_aovs planes of the same camera and
+    seed (depth, normal, albedo).  Returns (hdr_out [H,W,3] float32, ImageBuffer of its tonemap).  levels / sigmas: 0 = this filter's
+    defaults (5 levels).  Blocks until the result is on the host."""
+    H, W = _denoise_inputs(hdr, aovs, _is_numpy_f32)
+    _variance_input(var, hdr, _is_numpy_f32)
+    out = np.empty((H, W, 3), dtype=np.float32)
+    rgb = np.empty((H, W, 3), dtype=np.uint8)
+    g = _abi.AovOutC(depth=aovs["depth"].ctypes.data, normal=aovs["normal"].ctypes.data, albedo=aovs["albedo"].ctypes.data)
+    st = _abi.StatsC()
+    _abi.check(_abi.lib().rbrt_gpu_denoise_variance(W, H, hdr.ctypes.data, var.ctypes.data, g, _denoise_opts(levels, sigma_depth, sigma_luminance),
+                                                    out.ctypes.data, rgb.ctypes.data, st))
+    if stats is not None:
+        stats.update(st.as_dict())
+    return out, ImageBuffer(rgb)
+
+
+def denoise_variance_device(hdr, var, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stream=None):
+    """The same on CUDA tensors of the current render device: returns (hdr_out [H,W,3] float32, rgb [H,W,3] uint8) tensors, enqueued on
+    `stream` (default: the current stream) without synchronising."""
+    import torch
+    H, W = _denoise_inputs(hdr, aovs, _is_cuda_f32)
+    _variance_input(var, hdr, _is_cuda_f32)
+    stream = stream or torch.cuda.current_stream()
+    with torch.cuda.stream(stream):
+        out = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
+        rgb = torch.empty((H, W, 3), dtype=torch.uint8, device=stream.device)
+    g = _abi.AovOutC(depth=aovs["depth"].data_ptr(), normal=aovs["normal"].data_ptr(), albedo=aovs["albedo"].data_ptr())
+    _abi.check(_abi.lib().rbrt_gpu_denoise_variance_device(W, H, hdr.data_ptr(), var.data_ptr(), g,
+                                                           _denoise_opts(levels, sigma_depth, sigma_luminance), out.data_ptr(),
+                                                           rgb.data_ptr(), stream.cuda_stream, None))
+    return out, rgb
