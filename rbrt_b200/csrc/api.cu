@@ -227,9 +227,11 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
     }
 }
 
-// ------------------------------------------------------------------ scene updates (rbrt_gpu_scene_update_*)
-// The refit kernels live in their own device module, librbrt_gpu_update.so, loaded from this library's directory
-// (RBRT_GPU_UPDATE_LIB: another path).  Without it a refit is refused: there is no other implementation.
+// ------------------------------------------------------------------ device modules
+// The refit kernels (librbrt_gpu_update.so), the AOV kernel (librbrt_gpu_aov.so), the ray queries (librbrt_gpu_query.so), the denoiser
+// (librbrt_gpu_denoise.so) and the variance kernels (librbrt_gpu_variance.so) live in their own device modules, loaded from this library's
+// directory (or the path in the module's environment variable) on first use.  Without a module its calls are refused: there is no other
+// implementation.
 // Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
 static int module_path(const char* env, const char* file, std::string* path) {
     const char* e = getenv(env);
@@ -242,24 +244,28 @@ static int module_path(const char* env, const char* file, std::string* path) {
     return RBRT_OK;
 }
 
-struct UpdateModule { void* h = nullptr; rbrt_update_scratch_bytes_fn scratch_bytes = nullptr; rbrt_update_refit_fn refit = nullptr; };
-static int update_module(const UpdateModule** out) {
-    static UpdateModule m;
+// `what` names the module in messages; `h` is its handle once opened.
+struct Module { const char* env; const char* file; const char* what; void* h; };
+static Module g_update_module = {"RBRT_GPU_UPDATE_LIB", "librbrt_gpu_update.so", "refit", nullptr};
+static Module g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", nullptr};
+static Module g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", nullptr};
+static Module g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", nullptr};
+static Module g_variance_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", nullptr};
+// The entry point `symbol` of module m, which is opened on first use.  A failed dlopen is not remembered: the next call tries again.
+template <class F> static int module_entry(Module& m, const char* symbol, F* fn) {
     if (!m.h) {
         std::string path;
-        { int rc = module_path("RBRT_GPU_UPDATE_LIB", "librbrt_gpu_update.so", &path); if (rc) return rc; }
-        void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
-        if (!h) { set_error("the refit module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", path.c_str(), dlerror()); return RBRT_E_CUDA; }
-        UpdateModule n; n.h = h;
-        *(void**)(&n.scratch_bytes) = dlsym(h, "rbrt_update_scratch_bytes");
-        *(void**)(&n.refit) = dlsym(h, "rbrt_update_refit");
-        if (!n.scratch_bytes || !n.refit) { set_error("%s lacks the refit entry points", path.c_str()); dlclose(h); return RBRT_E_CUDA; }
-        m = n;
+        { int rc = module_path(m.env, m.file, &path); if (rc) return rc; }
+        m.h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
+        if (!m.h) { set_error("the %s module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", m.what, path.c_str(), dlerror()); return RBRT_E_CUDA; }
     }
-    *out = &m;
+    void* p = dlsym(m.h, symbol);
+    if (!p) { set_error("the %s module lacks the entry point %s; rebuild it with make -C rbrt_b200/csrc", m.what, symbol); return RBRT_E_CUDA; }
+    *fn = reinterpret_cast<F>(p);
     return RBRT_OK;
 }
 
+// ------------------------------------------------------------------ scene updates (rbrt_gpu_scene_update_*)
 // Opens an update: the device's build stream, made to wait for every read of the scene enqueued so far on replica 0's device.
 // Every write of the update is enqueued on ctx->build after this.
 static int update_begin(Scene* sc, BuildCtx* ctx) {
@@ -310,8 +316,13 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
         int rc = resolve_scene_info(*sc, true);
         if (rc) return rc;
     }
-    const UpdateModule* um = nullptr;
-    if (flags == RBRT_UPDATE_REFIT && !receiver) { int rc = update_module(&um); if (rc) return rc; }
+    rbrt_update_scratch_bytes_fn scratch_bytes = nullptr;
+    rbrt_update_refit_fn refit = nullptr;
+    if (flags == RBRT_UPDATE_REFIT && !receiver) {
+        int rc = module_entry(g_update_module, "rbrt_update_scratch_bytes", &scratch_bytes);
+        if (!rc) rc = module_entry(g_update_module, "rbrt_update_refit", &refit);
+        if (rc) return rc;
+    }
 
     BuildCtx ctx;
     { int rc = update_begin(sc, &ctx); if (rc) return rc; }
@@ -353,14 +364,14 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
         } else {
             const size_t raw_bytes = on_device ? 0 : (36ull * n + 255) & ~255ull;
             char* sbase = nullptr;
-            CKA(build_slot_acquire(ctx, raw_bytes + um->scratch_bytes(n_eff), &sbase));
+            CKA(build_slot_acquire(ctx, raw_bytes + scratch_bytes(n_eff), &sbase));
             if (!on_device && n) CKA(cudaMemcpyAsync(sbase, verts, 36ull * n, cudaMemcpyHostToDevice, ctx.copy));
             CKA(build_slot_uploaded(ctx, &uploaded));
             if (on_device) CKA(cudaStreamWaitEvent(ctx.build, sc->upd_in, 0));
             RefitArgs a;
             a.raw = on_device ? verts : (const float*)sbase; a.n_all = n; a.n_eff = n_eff; a.pad_rel = sc->pad_rel;
             a.mesh = d_mesh; a.tris = d_tris; a.normals = d_normals; a.nodes = reinterpret_cast<uint4*>(d_nodes); a.res = d_res;
-            CKA((cudaError_t)um->refit(&a, sbase + raw_bytes, ctx.build));
+            CKA((cudaError_t)refit(&a, sbase + raw_bytes, ctx.build));
             CKA(build_slot_release(ctx));
             if (on_device) uploaded = nullptr;
         }
@@ -375,48 +386,71 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
     return RBRT_OK;
 }
 
-// ------------------------------------------------------------------ device modules with one launch entry point
-// The AOV kernel (librbrt_gpu_aov.so, RBRT_GPU_AOV_LIB: another path), the ray queries (librbrt_gpu_query.so, RBRT_GPU_QUERY_LIB), the
-// denoiser (librbrt_gpu_denoise.so, RBRT_GPU_DENOISE_LIB) and the variance kernels (librbrt_gpu_variance.so, RBRT_GPU_VARIANCE_LIB) live in
-// their own device modules, like the refit; each is opened once, on first use.
-struct LaunchModule { const char* env; const char* file; const char* what; const char* symbol; void* launch; };
-static LaunchModule g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", "rbrt_aov_launch", nullptr};
-static LaunchModule g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", "rbrt_query_launch", nullptr};
-static LaunchModule g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", "rbrt_denoise_launch", nullptr};
-static LaunchModule g_moments_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", "rbrt_variance_moments_launch", nullptr};
-static LaunchModule g_vfilter_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", "rbrt_variance_filter_launch", nullptr};
-static int load_module(LaunchModule& m) {
-    if (!m.launch) {
-        std::string path;
-        { int rc = module_path(m.env, m.file, &path); if (rc) return rc; }
-        void* h = dlopen(path.c_str(), RTLD_NOW | RTLD_LOCAL);
-        if (!h) { set_error("the %s module is missing (dlopen %s: %s); build it with make -C rbrt_b200/csrc", m.what, path.c_str(), dlerror()); return RBRT_E_CUDA; }
-        void* f = dlsym(h, m.symbol);
-        if (!f) { set_error("%s lacks the %s entry point", path.c_str(), m.what); dlclose(h); return RBRT_E_CUDA; }
-        m.launch = f;
+// ------------------------------------------------------------------ per-device state of the calls into the device modules
+// Created on first use, freed by rbrt_gpu_release_cache.
+//  - The staging block that the host-pointer AOV and denoise calls carve their device planes from (grown, never shrunk).  One block
+//    serves both: each such call runs on the legacy default stream and synchronises it before returning.
+//  - The timing events of calls with stats (AOV, query, denoise, variance).  Each such call waits for `e1` or its stream before returning.
+//  - The AOV counters, used by calls with stats.
+//  - The query ring: QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
+//    block, zeroes it on its own stream and records `qry_used` behind its kernel, so calls on different streams never share a cursor.  A
+//    block is reused QRY_RING calls later; the host waits for its previous call only if that one has still not run by then.
+//  - The variance lane: an internal stream and the events that fork a call's shards onto it and join them back (render_variance).
+//    Calls without stats return before their shards run, so the lane is ordered by those events, not by the host.
+#define QRY_RING 256
+struct DeviceCache {
+    char* buf = nullptr; size_t bytes = 0;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    unsigned long long* aov_ctr = nullptr;
+    unsigned long long* qry_ctr = nullptr; cudaEvent_t qry_used[QRY_RING] = {}; uint32_t qry_next = 0;
+    cudaStream_t aux = nullptr; cudaEvent_t fork = nullptr, join = nullptr;
+};
+static DeviceCache g_cache[64];
+static void cache_release_all() {
+    int cur = 0; cudaGetDevice(&cur);
+    for (int d = 0; d < 64; ++d) {
+        DeviceCache& c = g_cache[d];
+        if (!c.buf && !c.e0 && !c.e1 && !c.aov_ctr && !c.qry_ctr && !c.aux) continue;
+        cudaSetDevice(d);
+        for (cudaEvent_t& e : c.qry_used) if (e) { cudaEventSynchronize(e); cudaEventDestroy(e); }
+        if (c.aux) { cudaStreamSynchronize(c.aux); cudaStreamDestroy(c.aux); }
+        for (cudaEvent_t e : {c.e0, c.e1, c.fork, c.join}) if (e) cudaEventDestroy(e);
+        cudaFree(c.buf); cudaFree(c.aov_ctr); cudaFree(c.qry_ctr);
+        c = DeviceCache();
     }
+    cudaSetDevice(cur);
+}
+// The device's staging block, grown to at least `need` bytes.
+static int staging_block(DeviceCache& c, size_t need, char** out) {
+    if (c.bytes < need) {
+        cudaFree(c.buf); c.buf = nullptr; c.bytes = 0;
+        CKA(cudaMalloc(&c.buf, need)); c.bytes = need;
+    }
+    *out = c.buf;
+    return RBRT_OK;
+}
+static int timing_events(DeviceCache& c) {
+    if (!c.e0) CKA(cudaEventCreate(&c.e0));
+    if (!c.e1) CKA(cudaEventCreate(&c.e1));
+    return RBRT_OK;
+}
+
+// Device memory on `device` (or managed / registered host memory the device can read)?  Unregistered host memory or another device's
+// memory would fault in the kernel.
+static bool usable_on(const void* p, int device) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (a.type == cudaMemoryTypeDevice) return a.device == device;
+    return a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeHost && a.devicePointer == p);
+}
+// RBRT_E_INVALID with the message `msg` (formatted with the device) unless every non-NULL pointer of `ptrs` is usable on `device`.
+static int check_usable_on(std::initializer_list<const void*> ptrs, int device, const char* msg) {
+    for (const void* p : ptrs)
+        if (p && !usable_on(p, device)) { set_error(msg, device); return RBRT_E_INVALID; }
     return RBRT_OK;
 }
 
 // ------------------------------------------------------------------ first-hit AOVs (rbrt_gpu_render_aov*)
-// Per device: the planes of the host-pointer variant (grown, never shrunk, until rbrt_gpu_release_cache), the counters and the
-// events.  Only calls that synchronise before returning use them, so one set per device serves every call.
-struct AovPool { char* buf = nullptr; size_t bytes = 0; unsigned long long* ctr = nullptr; cudaEvent_t e0 = nullptr, e1 = nullptr; };
-static AovPool g_aov[64];
-static void aov_release_all() {
-    int cur = 0; cudaGetDevice(&cur);
-    for (int d = 0; d < 64; ++d) {
-        AovPool& p = g_aov[d];
-        if (!p.buf && !p.ctr && !p.e0) continue;
-        cudaSetDevice(d);
-        cudaFree(p.buf); cudaFree(p.ctr);
-        if (p.e0) cudaEventDestroy(p.e0);
-        if (p.e1) cudaEventDestroy(p.e1);
-        p = AovPool();
-    }
-    cudaSetDevice(cur);
-}
-
 static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t spp, uint64_t seed, const rbrt_aov_out* out, bool host,
                       cudaStream_t st, rbrt_stats* stats) {
     if (!scene || !cam || !out) { set_error("null argument"); return RBRT_E_INVALID; }
@@ -432,42 +466,39 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
     const double t0 = now_ms();
     if (stats) memset(stats, 0, sizeof(*stats));
     { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
-    { int rc = load_module(g_aov_module); if (rc) return rc; }
-    const rbrt_aov_launch_fn launch = reinterpret_cast<rbrt_aov_launch_fn>(g_aov_module.launch);
+    rbrt_aov_launch_fn launch = nullptr;
+    { int rc = module_entry(g_aov_module, "rbrt_aov_launch", &launch); if (rc) return rc; }
 
-    AovPool& pool = g_aov[rp.device & 63];
+    DeviceCache& c = g_cache[rp.device & 63];
     AovArgs a;
     memset(&a, 0, sizeof(a));
     a.S = rp.dev; a.cam = make_cam(*cam); a.key0 = (uint32_t)seed; a.key1 = (uint32_t)(seed >> 32); a.n_samples = spp;
     a.tiles_x = (cam->img_width_pix + 7) / 8; a.tiles_total = a.tiles_x * ((cam->img_height_pix + 3) / 4);
     a.out = *out;
-    if (host) {                                                           // the requested planes, carved from the pooled block
+    if (host) {                                                           // the requested planes, carved from the staging block
         const size_t b1 = a256(4 * n), b3 = a256(12 * n);
         const size_t need = (out->depth ? b1 : 0) + (out->normal ? b3 : 0) + (out->albedo ? b3 : 0) + (out->coverage ? b1 : 0) +
                             (out->hit_kind ? b1 : 0) + (out->elem_idx ? b1 : 0) + (out->tri_idx ? b1 : 0);
-        if (pool.bytes < need) {
-            cudaFree(pool.buf); pool.buf = nullptr; pool.bytes = 0;
-            CKA(cudaMalloc(&pool.buf, need)); pool.bytes = need;
-        }
-        char* p = pool.buf;
+        char* p = nullptr;
+        { int rc = staging_block(c, need, &p); if (rc) return rc; }
         auto take = [&](const void* want, size_t b) -> char* { if (!want) return nullptr; char* q = p; p += b; return q; };
         a.out.depth = (float*)take(out->depth, b1); a.out.normal = (float*)take(out->normal, b3); a.out.albedo = (float*)take(out->albedo, b3);
         a.out.coverage = (float*)take(out->coverage, b1); a.out.hit_kind = (int32_t*)take(out->hit_kind, b1);
         a.out.elem_idx = (uint32_t*)take(out->elem_idx, b1); a.out.tri_idx = (uint32_t*)take(out->tri_idx, b1);
     }
     if (stats) {
-        if (!pool.ctr) CKA(cudaMalloc(&pool.ctr, 8 * AOV_ST_COUNT));
-        if (!pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
-        a.stats = pool.ctr;
+        if (!c.aov_ctr) CKA(cudaMalloc(&c.aov_ctr, 8 * AOV_ST_COUNT));
+        { int rc = timing_events(c); if (rc) return rc; }
+        a.stats = c.aov_ctr;
     }
     wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
-    if (stats) { CKA(cudaMemsetAsync(pool.ctr, 0, 8 * AOV_ST_COUNT, st)); CKA(cudaEventRecord(pool.e0, st)); }
+    if (stats) { CKA(cudaMemsetAsync(c.aov_ctr, 0, 8 * AOV_ST_COUNT, st)); CKA(cudaEventRecord(c.e0, st)); }
     CKA((cudaError_t)launch(&a, st));
-    if (stats) CKA(cudaEventRecord(pool.e1, st));
+    if (stats) CKA(cudaEventRecord(c.e1, st));
     note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
     if (!host && !stats) return RBRT_OK;                                  // enqueue only
 
-    if (stats) CKA(cudaEventSynchronize(pool.e1));
+    if (stats) CKA(cudaEventSynchronize(c.e1));
     const double t1 = now_ms();
     if (host) {
         if (out->depth) CKA(cudaMemcpyAsync(out->depth, a.out.depth, 4 * n, cudaMemcpyDeviceToHost, st));
@@ -482,9 +513,9 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
     const double t2 = now_ms();
     if (stats) {
         unsigned long long h[AOV_ST_COUNT];
-        CKA(cudaMemcpyAsync(h, pool.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+        CKA(cudaMemcpyAsync(h, c.aov_ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
         CKA(cudaStreamSynchronize(st));
-        float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
         stats->rays = n * spp; stats->paths = n * spp; stats->nan_rays = h[AOV_ST_NAN];
         stats->node_visits = h[AOV_ST_NODES]; stats->tri_tests = h[AOV_ST_TRIS];
         stats->ms_device = ms; stats->ms_d2h = host ? t2 - t1 : 0.0; stats->launches = 1;
@@ -494,36 +525,6 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
 }
 
 // ------------------------------------------------------------------ ray queries on device memory (rbrt_gpu_query_*_device)
-// Per device: a ring of QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
-// block, zeroes it on its own stream and records an event behind its kernel, so calls on different streams never share a cursor.  A block
-// is reused QRY_RING calls later; the host waits for its previous call only if that one has still not run by then.
-#define QRY_RING 256
-struct QueryPool { unsigned long long* ctr = nullptr; cudaEvent_t used[QRY_RING] = {}; uint32_t next = 0; cudaEvent_t e0 = nullptr, e1 = nullptr; };
-static QueryPool g_query[64];
-static void query_release_all() {
-    int cur = 0; cudaGetDevice(&cur);
-    for (int d = 0; d < 64; ++d) {
-        QueryPool& p = g_query[d];
-        if (!p.ctr) continue;
-        cudaSetDevice(d);
-        for (cudaEvent_t& e : p.used) if (e) { cudaEventSynchronize(e); cudaEventDestroy(e); }
-        if (p.e0) cudaEventDestroy(p.e0);
-        if (p.e1) cudaEventDestroy(p.e1);
-        cudaFree(p.ctr);
-        p = QueryPool();
-    }
-    cudaSetDevice(cur);
-}
-
-// Device memory on `device` (or managed / registered host memory the device can read)?  Unregistered host memory or another device's
-// memory would fault in the kernel.
-static bool usable_on(const void* p, int device) {
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-    if (a.type == cudaMemoryTypeDevice) return a.device == device;
-    return a.type == cudaMemoryTypeManaged || (a.type == cudaMemoryTypeHost && a.devicePointer == p);
-}
-
 // occ: an occlusion query into occluded[]; else a closest query into *out.
 static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool occ, const rbrt_query_out* out, const float* max_dist,
                  uint8_t* occluded, cudaStream_t st, rbrt_stats* stats) {
@@ -538,28 +539,25 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device
     CKA(cudaSetDevice(rp.device));
     const double t0 = now_ms();
-    {
-        const void* ptrs[10] = {rays, max_dist, occluded};
-        if (!occ) { ptrs[3] = out->t; ptrs[4] = out->dist; ptrs[5] = out->kind; ptrs[6] = out->elem_idx; ptrs[7] = out->tri_idx; ptrs[8] = out->point; ptrs[9] = out->normal; }
-        for (const void* p : ptrs)
-            if (p && !usable_on(p, rp.device)) { set_error("rays and outputs must be device memory on the scene's device %d", rp.device); return RBRT_E_INVALID; }
-    }
+    const rbrt_query_out o = occ ? rbrt_query_out{} : *out;
+    { int rc = check_usable_on({rays, max_dist, occluded, o.t, o.dist, o.kind, o.elem_idx, o.tri_idx, o.point, o.normal}, rp.device,
+                               "rays and outputs must be device memory on the scene's device %d"); if (rc) return rc; }
     { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
-    { int rc = load_module(g_query_module); if (rc) return rc; }
-    const rbrt_query_launch_fn launch = reinterpret_cast<rbrt_query_launch_fn>(g_query_module.launch);
+    rbrt_query_launch_fn launch = nullptr;
+    { int rc = module_entry(g_query_module, "rbrt_query_launch", &launch); if (rc) return rc; }
 
-    QueryPool& pool = g_query[rp.device & 63];
-    if (!pool.ctr) CKA(cudaMalloc(&pool.ctr, 8ull * QRY_ST_COUNT * QRY_RING));
-    const uint32_t slot = pool.next++ % QRY_RING;
-    cudaEvent_t& used = pool.used[slot];
+    DeviceCache& c = g_cache[rp.device & 63];
+    if (!c.qry_ctr) CKA(cudaMalloc(&c.qry_ctr, 8ull * QRY_ST_COUNT * QRY_RING));
+    const uint32_t slot = c.qry_next++ % QRY_RING;
+    cudaEvent_t& used = c.qry_used[slot];
     if (used) CKA(cudaEventSynchronize(used));
     else CKA(cudaEventCreateWithFlags(&used, cudaEventDisableTiming));
-    if (stats && !pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
 
     QueryArgs a;
     memset(&a, 0, sizeof(a));
-    a.S = rp.dev; a.rays = rays; a.n = n; a.max_dist = max_dist; a.occluded = occluded; a.ctr = pool.ctr + QRY_ST_COUNT * slot;
-    if (!occ) a.out = *out;
+    a.S = rp.dev; a.rays = rays; a.n = n; a.max_dist = max_dist; a.occluded = occluded; a.ctr = c.qry_ctr + QRY_ST_COUNT * slot;
+    a.out = o;
     a.count = stats != nullptr;
     {
         const uint64_t blocks = (n + 127) / 128;                          // persistent: at most the resident blocks (8 per SM, query.cu)
@@ -568,9 +566,9 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     }
     wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
     CKA(cudaMemsetAsync(a.ctr, 0, 8 * QRY_ST_COUNT, st));
-    if (stats) CKA(cudaEventRecord(pool.e0, st));
+    if (stats) CKA(cudaEventRecord(c.e0, st));
     CKA((cudaError_t)launch(&a, st));
-    if (stats) CKA(cudaEventRecord(pool.e1, st));
+    if (stats) CKA(cudaEventRecord(c.e1, st));
     CKA(cudaEventRecord(used, st));
     note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
     if (!stats) return RBRT_OK;                                           // enqueue only
@@ -578,7 +576,7 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     unsigned long long h[QRY_ST_COUNT];
     CKA(cudaMemcpyAsync(h, a.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
     CKA(cudaStreamSynchronize(st));
-    float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+    float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
     stats->rays = n; stats->nan_rays = h[QRY_ST_NAN]; stats->node_visits = h[QRY_ST_NODES]; stats->tri_tests = h[QRY_ST_TRIS];
     stats->ms_device = ms; stats->launches = 1;
     stats->ms_total = now_ms() - t0;
@@ -586,25 +584,8 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
 }
 
 // ------------------------------------------------------------------ guided denoising (rbrt_gpu_denoise*, rbrt_gpu_denoise_variance*)
-// Per device: the block the host-pointer variant copies its planes into and carves its scratch from (grown, never shrunk, until
-// rbrt_gpu_release_cache), and the events of calls with stats.  Only calls that synchronise before returning use them.  The device
-// variant takes its scratch from the stream-ordered allocator on the call's stream instead, so calls in flight never share it.
-struct DenoisePool { char* buf = nullptr; size_t bytes = 0; cudaEvent_t e0 = nullptr, e1 = nullptr; };
-static DenoisePool g_denoise[64];
-static void denoise_release_all() {
-    int cur = 0; cudaGetDevice(&cur);
-    for (int d = 0; d < 64; ++d) {
-        DenoisePool& p = g_denoise[d];
-        if (!p.buf && !p.e0) continue;
-        cudaSetDevice(d);
-        cudaFree(p.buf);
-        if (p.e0) cudaEventDestroy(p.e0);
-        if (p.e1) cudaEventDestroy(p.e1);
-        p = DenoisePool();
-    }
-    cudaSetDevice(cur);
-}
-
+// The host-pointer variant copies its planes into the device's staging block and carves its scratch from it.  The device variant takes
+// its scratch from the stream-ordered allocator on the call's stream instead, so calls in flight never share it.
 static bool overlap(const void* a, size_t na, const void* b, size_t nb) {
     if (!a || !b) return false;
     const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
@@ -641,27 +622,28 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
     { int rc = ensure_device(); if (rc) return rc; }
     const int dev = g_device;
     if (!host) {
-        const void* ptrs[7] = {hdr, guides->depth, guides->normal, guides->albedo, hdr_out, rgb_out, var};
-        for (const void* p : ptrs)
-            if (p && !usable_on(p, dev)) { set_error("planes must be device memory on the current device %d", dev); return RBRT_E_INVALID; }
+        int rc = check_usable_on({hdr, guides->depth, guides->normal, guides->albedo, hdr_out, rgb_out, var}, dev,
+                                 "planes must be device memory on the current device %d");
+        if (rc) return rc;
     }
-    { int rc = load_module(with_var ? g_vfilter_module : g_denoise_module); if (rc) return rc; }
-    const rbrt_denoise_launch_fn launch = reinterpret_cast<rbrt_denoise_launch_fn>(g_denoise_module.launch);
-    const rbrt_variance_filter_launch_fn vlaunch = reinterpret_cast<rbrt_variance_filter_launch_fn>(g_vfilter_module.launch);
+    rbrt_denoise_launch_fn launch = nullptr;
+    rbrt_variance_filter_launch_fn vlaunch = nullptr;
+    {
+        int rc = with_var ? module_entry(g_variance_module, "rbrt_variance_filter_launch", &vlaunch)
+                          : module_entry(g_denoise_module, "rbrt_denoise_launch", &launch);
+        if (rc) return rc;
+    }
     const size_t scratch = (with_var ? 56 : 48) * n;                      // guides and two planes of (e.rgb, l); with var two planes of σ²
     const double t0 = now_ms();
 
-    DenoisePool& pool = g_denoise[dev & 63];
-    if (stats && !pool.e0) { CKA(cudaEventCreate(&pool.e0)); CKA(cudaEventCreate(&pool.e1)); }
+    DeviceCache& c = g_cache[dev & 63];
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
     a.hdr = hdr; a.depth = guides->depth; a.normal = guides->normal; a.albedo = guides->albedo; a.hdr_out = hdr_out; a.rgb_out = rgb_out;
-    if (host) {                                                           // inputs, outputs and scratch carved from the pooled block
+    if (host) {                                                           // inputs, outputs and scratch carved from the staging block
         const size_t b1 = a256(4 * n), b3 = a256(12 * n), bs = a256(scratch);
         const size_t need = bs + 3 * b3 + b1 + (with_var ? b3 : 0) + (hdr_out ? b3 : 0) + (rgb_out ? a256(3 * n) : 0);
-        if (pool.bytes < need) {
-            cudaFree(pool.buf); pool.buf = nullptr; pool.bytes = 0;
-            CKA(cudaMalloc(&pool.buf, need)); pool.bytes = need;
-        }
-        char* p = pool.buf;
+        char* p = nullptr;
+        { int rc = staging_block(c, need, &p); if (rc) return rc; }
         a.scratch = (float4*)p; p += bs;
         float* d_hdr = (float*)p; p += b3;
         float* d_nrm = (float*)p; p += b3;
@@ -683,12 +665,12 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
         CKA(cudaMallocAsync((void**)&a.scratch, scratch, st));
     }
     if (stats) {
-        cudaError_t e = cudaEventRecord(pool.e0, st);
+        cudaError_t e = cudaEventRecord(c.e0, st);
         if (e != cudaSuccess) { if (!host) cudaFreeAsync(a.scratch, st); return cuda_fail(e, "cudaEventRecord"); }
     }
     {
         cudaError_t e = (cudaError_t)(with_var ? vlaunch(&a, var, st) : launch(&a, st));
-        if (e == cudaSuccess && stats) e = cudaEventRecord(pool.e1, st);
+        if (e == cudaSuccess && stats) e = cudaEventRecord(c.e1, st);
         if (!host) { cudaError_t f = cudaFreeAsync(a.scratch, st); if (e == cudaSuccess) e = f; }
         if (e != cudaSuccess) return cuda_fail(e, with_var ? "rbrt_variance_filter_launch" : "rbrt_denoise_launch");
     }
@@ -700,8 +682,8 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
         return RBRT_OK;                                                   // enqueue only
     }
     if (stats) {
-        CKA(cudaEventSynchronize(pool.e1));
-        float ms = 0; CKA(cudaEventElapsedTime(&ms, pool.e0, pool.e1));
+        CKA(cudaEventSynchronize(c.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
         stats->ms_device = ms; stats->launches = 1 + a.levels;
         stats->ms_total = now_ms() - t0;
     }
@@ -713,21 +695,6 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
 // wavefront pool p of opts->flags, and an internal stream of the device with pool 4 + p (the second lane of RBRT_OPT_SPLIT_BATCHES).  No
 // shard waits for another (each has its own accumulator), so the sparse last bounces of one shard run under the dense first bounces of the
 // shard on the other lane.  The moments kernel then runs on the caller's stream behind both lanes.
-struct VariancePool { cudaStream_t aux = nullptr; cudaEvent_t fork = nullptr, join = nullptr, e0 = nullptr, e1 = nullptr; };
-static VariancePool g_variance[64];
-static void variance_release_all() {
-    int cur = 0; cudaGetDevice(&cur);
-    for (int d = 0; d < 64; ++d) {
-        VariancePool& p = g_variance[d];
-        if (!p.aux) continue;
-        cudaSetDevice(d);
-        cudaStreamSynchronize(p.aux); cudaStreamDestroy(p.aux);
-        for (cudaEvent_t e : {p.fork, p.join, p.e0, p.e1}) if (e) cudaEventDestroy(e);
-        p = VariancePool();
-    }
-    cudaSetDevice(cur);
-}
-
 static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t S, uint32_t K, const rbrt_render_opts* opts,
                            float* hdr_out, float* var_out, bool host, cudaStream_t st, rbrt_stats* stats) {
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -744,19 +711,20 @@ static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint
     const Scene& sc = *reinterpret_cast<const Scene*>(scene);
     const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device, whole image
     CKA(cudaSetDevice(rp.device));
-    if (!host)
-        for (const void* p : {(const void*)hdr_out, (const void*)var_out})
-            if (p && !usable_on(p, rp.device)) { set_error("outputs must be device memory on the scene's device %d", rp.device); return RBRT_E_INVALID; }
+    if (!host) {
+        int rc = check_usable_on({hdr_out, var_out}, rp.device, "outputs must be device memory on the scene's device %d");
+        if (rc) return rc;
+    }
     const double t0 = now_ms();
     { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
-    { int rc = load_module(g_moments_module); if (rc) return rc; }
-    const rbrt_variance_moments_launch_fn launch = reinterpret_cast<rbrt_variance_moments_launch_fn>(g_moments_module.launch);
-    VariancePool& vp = g_variance[rp.device & 63];
-    if (!vp.aux) {
-        CKA(cudaStreamCreateWithFlags(&vp.aux, cudaStreamNonBlocking));
-        CKA(cudaEventCreateWithFlags(&vp.fork, cudaEventDisableTiming)); CKA(cudaEventCreateWithFlags(&vp.join, cudaEventDisableTiming));
-        CKA(cudaEventCreate(&vp.e0)); CKA(cudaEventCreate(&vp.e1));
+    rbrt_variance_moments_launch_fn launch = nullptr;
+    { int rc = module_entry(g_variance_module, "rbrt_variance_moments_launch", &launch); if (rc) return rc; }
+    DeviceCache& c = g_cache[rp.device & 63];
+    if (!c.aux) {
+        CKA(cudaStreamCreateWithFlags(&c.aux, cudaStreamNonBlocking));
+        CKA(cudaEventCreateWithFlags(&c.fork, cudaEventDisableTiming)); CKA(cudaEventCreateWithFlags(&c.join, cudaEventDisableTiming));
     }
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
     const uint32_t pool = (o.flags & RBRT_OPT_POOL_MASK) >> RBRT_OPT_POOL_SHIFT;
     o.flags &= ~(uint32_t)RBRT_OPT_SPLIT_BATCHES;                         // the two lanes are the shards'
     o.shard_mode = RBRT_SHARD_SAMPLES; o.shard_count = K;
@@ -776,14 +744,14 @@ static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint
     uint32_t launches = 0;
     cudaError_t e = cudaSuccess;
     int rc = RBRT_OK;
-    if (stats) e = cudaEventRecord(vp.e0, st);
-    if (e == cudaSuccess) e = cudaEventRecord(vp.fork, st);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(vp.aux, vp.fork, 0);
+    if (stats) e = cudaEventRecord(c.e0, st);
+    if (e == cudaSuccess) e = cudaEventRecord(c.fork, st);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(c.aux, c.fork, 0);
     for (uint32_t k = 0; k < K && e == cudaSuccess && !rc; ++k) {
         const int lane = (int)(k & 1);
         o.shard_rank = k;
         float4* acc1[1] = {(float4*)(block + 16 * n * k)};
-        rc = render_accum(sc, 0, cam, nullptr, 1, S, &o, acc1, lane ? vp.aux : st, nullptr, stats ? &jobs[k] : nullptr, (int)pool + 4 * lane);
+        rc = render_accum(sc, 0, cam, nullptr, 1, S, &o, acc1, lane ? c.aux : st, nullptr, stats ? &jobs[k] : nullptr, (int)pool + 4 * lane);
         if (rc || !stats || (lane == 0 && k + 1 < K)) continue;
         for (uint32_t j = k - lane; j <= k && !rc; ++j) {                 // this round's counters, before the next round resets its pools
             rbrt_stats one; memset(&one, 0, sizeof(one));
@@ -791,10 +759,10 @@ static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint
             stats->rays += one.rays; stats->paths += one.paths; stats->nan_rays += one.nan_rays; launches += one.launches;
         }
     }
-    if (e == cudaSuccess) e = cudaEventRecord(vp.join, vp.aux);           // (also when a shard was refused: the block is freed behind both lanes)
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, vp.join, 0);
+    if (e == cudaSuccess) e = cudaEventRecord(c.join, c.aux);           // (also when a shard was refused: the block is freed behind both lanes)
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, c.join, 0);
     if (e == cudaSuccess && !rc) e = (cudaError_t)launch(&m, st);
-    if (e == cudaSuccess && !rc && stats) e = cudaEventRecord(vp.e1, st);
+    if (e == cudaSuccess && !rc && stats) e = cudaEventRecord(c.e1, st);
     if (e == cudaSuccess && !rc && host) {
         if (hdr_out) e = cudaMemcpyAsync(hdr_out, m.hdr_out, 12 * n, cudaMemcpyDeviceToHost, st);
         if (e == cudaSuccess && var_out) e = cudaMemcpyAsync(var_out, m.var_out, 12 * n, cudaMemcpyDeviceToHost, st);
@@ -807,8 +775,8 @@ static int render_variance(const rbrt_scene* scene, const rbrt_camera* cam, uint
     if (e != cudaSuccess) return cuda_fail(e, "rbrt_gpu_render_hdr_variance");
     if (host) CKA(cudaStreamSynchronize(st));
     if (stats) {
-        CKA(cudaEventSynchronize(vp.e1));
-        float ms = 0; CKA(cudaEventElapsedTime(&ms, vp.e0, vp.e1));
+        CKA(cudaEventSynchronize(c.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
         stats->ms_device = ms; stats->launches = launches + 1;
         stats->ms_total = now_ms() - t0;
         return resolve_scene_info(sc, true);
@@ -1113,10 +1081,7 @@ int rbrt_gpu_release_cache(void) {
     release_device_wave_buffers();
     release_dist_buffers();
     release_build_scratch();
-    aov_release_all();
-    query_release_all();
-    denoise_release_all();
-    variance_release_all();
+    cache_release_all();
     arena_release_all();
     for (void* p : g_pinned_free) cudaFreeHost(p);
     g_pinned_free.clear();

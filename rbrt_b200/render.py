@@ -226,35 +226,49 @@ def _denoise_opts(levels, sigma_depth, sigma_luminance):
     return _abi.DenoiseOptsC(int(levels), float(sigma_depth), float(sigma_luminance))
 
 
-def denoise(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stats=None):
-    """Denoise a render_scene_hdr image [H,W,3] guided by render_aovs planes of the same camera and seed (depth, normal, albedo; guides
-    with at most the image's samples line up with it pixel for pixel).  Returns (hdr_out [H,W,3] float32, ImageBuffer of its tonemap).
-    levels / sigmas: 0 = the defaults (4 levels).  Blocks until the result is on the host."""
-    H, W = _denoise_inputs(hdr, aovs, _is_numpy_f32)
-    out = np.empty((H, W, 3), dtype=np.float32)
-    rgb = np.empty((H, W, 3), dtype=np.uint8)
-    g = _abi.AovOutC(depth=aovs["depth"].ctypes.data, normal=aovs["normal"].ctypes.data, albedo=aovs["albedo"].ctypes.data)
-    st = _abi.StatsC()
-    _abi.check(_abi.lib().rbrt_gpu_denoise(W, H, hdr.ctypes.data, g, _denoise_opts(levels, sigma_depth, sigma_luminance), out.ctypes.data,
-                                           rgb.ctypes.data, st))
+def _denoise(hdr, var, aovs, levels, sigma_depth, sigma_luminance, device, stats=None, stream=None):
+    """denoise (var None) and denoise_variance, on numpy arrays or, with device=True, on CUDA tensors enqueued on `stream`."""
+    is_tensor = _is_cuda_f32 if device else _is_numpy_f32
+    H, W = _denoise_inputs(hdr, aovs, is_tensor)
+    if var is not None:
+        _variance_input(var, hdr, is_tensor)
+    if device:
+        import torch
+        stream = stream or torch.cuda.current_stream()
+        with torch.cuda.stream(stream):
+            out = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
+            rgb = torch.empty((H, W, 3), dtype=torch.uint8, device=stream.device)
+        ptr, tail = (lambda a: a.data_ptr()), (stream.cuda_stream, None)
+    else:
+        out = np.empty((H, W, 3), dtype=np.float32)
+        rgb = np.empty((H, W, 3), dtype=np.uint8)
+        st = _abi.StatsC()
+        ptr, tail = (lambda a: a.ctypes.data), (st,)
+    lib = _abi.lib()
+    if var is None:
+        call, planes = (lib.rbrt_gpu_denoise_device if device else lib.rbrt_gpu_denoise), (ptr(hdr),)
+    else:
+        call, planes = (lib.rbrt_gpu_denoise_variance_device if device else lib.rbrt_gpu_denoise_variance), (ptr(hdr), ptr(var))
+    g = _abi.AovOutC(depth=ptr(aovs["depth"]), normal=ptr(aovs["normal"]), albedo=ptr(aovs["albedo"]))
+    _abi.check(call(W, H, *planes, g, _denoise_opts(levels, sigma_depth, sigma_luminance), ptr(out), ptr(rgb), *tail))
+    if device:
+        return out, rgb
     if stats is not None:
         stats.update(st.as_dict())
     return out, ImageBuffer(rgb)
 
 
+def denoise(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stats=None):
+    """Denoise a render_scene_hdr image [H,W,3] guided by render_aovs planes of the same camera and seed (depth, normal, albedo; guides
+    with at most the image's samples line up with it pixel for pixel).  Returns (hdr_out [H,W,3] float32, ImageBuffer of its tonemap).
+    levels / sigmas: 0 = the defaults (4 levels).  Blocks until the result is on the host."""
+    return _denoise(hdr, None, aovs, levels, sigma_depth, sigma_luminance, False, stats=stats)
+
+
 def denoise_device(hdr, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stream=None):
     """The same on CUDA tensors (render_aovs_device's planes) of the current render device: returns (hdr_out [H,W,3] float32,
     rgb [H,W,3] uint8) tensors, enqueued on `stream` (default: the current stream) without synchronising."""
-    import torch
-    H, W = _denoise_inputs(hdr, aovs, _is_cuda_f32)
-    stream = stream or torch.cuda.current_stream()
-    with torch.cuda.stream(stream):
-        out = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
-        rgb = torch.empty((H, W, 3), dtype=torch.uint8, device=stream.device)
-    g = _abi.AovOutC(depth=aovs["depth"].data_ptr(), normal=aovs["normal"].data_ptr(), albedo=aovs["albedo"].data_ptr())
-    _abi.check(_abi.lib().rbrt_gpu_denoise_device(W, H, hdr.data_ptr(), g, _denoise_opts(levels, sigma_depth, sigma_luminance),
-                                                  out.data_ptr(), rgb.data_ptr(), stream.cuda_stream, None))
-    return out, rgb
+    return _denoise(hdr, None, aovs, levels, sigma_depth, sigma_luminance, True, stream=stream)
 
 
 # ---- per-pixel variance and variance-guided denoising (rbrt_gpu_render_hdr_variance*, rbrt_gpu_denoise_variance*; DESIGN.md section 14)
@@ -296,31 +310,10 @@ def denoise_variance(hdr, var, aovs, levels=0, sigma_depth=0.0, sigma_luminance=
     """Denoise a render_scene_hdr_variance frame [H,W,3] with its variance [H,W,3], guided by render_aovs planes of the same camera and
     seed (depth, normal, albedo).  Returns (hdr_out [H,W,3] float32, ImageBuffer of its tonemap).  levels / sigmas: 0 = this filter's
     defaults (5 levels).  Blocks until the result is on the host."""
-    H, W = _denoise_inputs(hdr, aovs, _is_numpy_f32)
-    _variance_input(var, hdr, _is_numpy_f32)
-    out = np.empty((H, W, 3), dtype=np.float32)
-    rgb = np.empty((H, W, 3), dtype=np.uint8)
-    g = _abi.AovOutC(depth=aovs["depth"].ctypes.data, normal=aovs["normal"].ctypes.data, albedo=aovs["albedo"].ctypes.data)
-    st = _abi.StatsC()
-    _abi.check(_abi.lib().rbrt_gpu_denoise_variance(W, H, hdr.ctypes.data, var.ctypes.data, g, _denoise_opts(levels, sigma_depth, sigma_luminance),
-                                                    out.ctypes.data, rgb.ctypes.data, st))
-    if stats is not None:
-        stats.update(st.as_dict())
-    return out, ImageBuffer(rgb)
+    return _denoise(hdr, var, aovs, levels, sigma_depth, sigma_luminance, False, stats=stats)
 
 
 def denoise_variance_device(hdr, var, aovs, levels=0, sigma_depth=0.0, sigma_luminance=0.0, stream=None):
     """The same on CUDA tensors of the current render device: returns (hdr_out [H,W,3] float32, rgb [H,W,3] uint8) tensors, enqueued on
     `stream` (default: the current stream) without synchronising."""
-    import torch
-    H, W = _denoise_inputs(hdr, aovs, _is_cuda_f32)
-    _variance_input(var, hdr, _is_cuda_f32)
-    stream = stream or torch.cuda.current_stream()
-    with torch.cuda.stream(stream):
-        out = torch.empty((H, W, 3), dtype=torch.float32, device=stream.device)
-        rgb = torch.empty((H, W, 3), dtype=torch.uint8, device=stream.device)
-    g = _abi.AovOutC(depth=aovs["depth"].data_ptr(), normal=aovs["normal"].data_ptr(), albedo=aovs["albedo"].data_ptr())
-    _abi.check(_abi.lib().rbrt_gpu_denoise_variance_device(W, H, hdr.data_ptr(), var.data_ptr(), g,
-                                                           _denoise_opts(levels, sigma_depth, sigma_luminance), out.data_ptr(),
-                                                           rgb.data_ptr(), stream.cuda_stream, None))
-    return out, rgb
+    return _denoise(hdr, var, aovs, levels, sigma_depth, sigma_luminance, True, stream=stream)
