@@ -557,6 +557,71 @@ int rbrt_gpu_denoise_variance_device(uint32_t width, uint32_t height, const floa
                                      const rbrt_denoise_opts* opts, float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream,
                                      rbrt_stats* stats);
 
+/* ---- temporal accumulation (DESIGN.md section 15) ----------------------------------------------
+ * Carries a frame sequence's samples from frame to frame: each pixel's history, aligned to the previous camera, is reprojected through
+ * that camera and blended with the current frame (the temporal part of SVGF, Schied et al. 2017, with its variance propagation).
+ * Current frame at camera cam, W x H pixels, row-major: hdr c (W*H*3, the mean colour), optionally var v (W*H*3, its variance, as
+ * rbrt_gpu_render_hdr_variance* returns it), and from `guides` (rbrt_gpu_render_aov* with the same camera and seed) the depth z (W*H),
+ * normal n (W*H*3), hit_kind and elem_idx (W*H).  The history is the previous call's outputs and that frame's guides and camera; the
+ * caller ping-pongs two sets of buffers, and the current guides become the next call's history guides.  Per pixel p = (x, y), each
+ * operation one correctly rounded f32 operation, products and sums left to right as written (rbrt_b200/csrc/temporal.cuh holds the code):
+ *   1. p is VALID when c and z are finite and, with var, every component of v is finite and >= 0 (-0 is).  A miss (z = +inf) is not
+ *      valid.  An invalid p gives hdr_out = c, var_out = v, len_out = 0.
+ *   2. Without a history (history NULL), or when steps 3-4 find none: hdr_out = c, var_out = v, len_out = 1.
+ *   3. X = pos + z * d, per component, with d = the direction of rbrt_gpu_primary_rays for p with both jitter draws at 0.5 (the pixel
+ *      centre); D = X - pos', r = sqrt((D.x*D.x + D.y*D.y) + D.z*D.z) (primes: the history's camera).  X is projected into that camera
+ *      by solving pos' + s*D = center' + a*right' - b*up' with Cramer's rule (up' as stored: it need not be orthogonal to right'):
+ *        C = center' - pos';  det = D . (right' x up');  s = (C . (right' x up')) / det;  a = (D . (up' x C)) / det;
+ *        b = (D . (right' x C)) / det   (u . v = (u.x*v.x + u.y*v.y) + u.z*v.z, the cross product as rbrt_vec3's);
+ *        px = (a / 0.001) / mm_per_pix_hor' + (float)(W / 2),  py = (b / 0.001) / mm_per_pix_vert' + (float)(H / 2)
+ *      (integers are pixel centres).  No history when r is not finite, s <= 0 or NaN, or px or py is outside [0, W-1] x [0, H-1] or not
+ *      finite.  When the history's camera equals cam field for field, bit for bit, (px, py) = (x, y) exactly and s is not formed: a
+ *      static camera accumulates each pixel from itself alone.
+ *   4. x0 = floor(px), fx = px - x0, y0 = floor(py), fy = py - y0; the taps (x0, y0), (x0+1, y0), (x0, y0+1), (x0+1, y0+1) in that order,
+ *      with weights w = (1-fx)*(1-fy), fx*(1-fy), (1-fx)*fy, fx*fy.  A tap q is skipped when w = 0 or q is outside the image, and unless
+ *      it is CONSISTENT: length'_q > 0, hit_kind'_q = hit_kind_p, elem_idx'_q = elem_idx_p, |z'_q - r| <= σ_z * r and
+ *      n_p . n'_q >= n_min * (|n_p| * |n'_q|), |n| = sqrt(n . n) (the AOV normals are sample means, shorter than 1 at edges).
+ *      Σw, Σ w*c'_q, Σ (w*w)*v'_q and Σ w*length'_q are sums from +0 in tap order.  Σw < 2^-6: no history.
+ *      c_h = Σ w*c'_q / Σw;  v_h = Σ (w*w)*v'_q / (Σw * Σw);  n_h = Σ w*length'_q / Σw.
+ *   5. α = max(1 / (n_h + 1), α_min);  hdr_out = c_h + α * (c - c_h);  var_out = ((1-α)*(1-α)) * v_h + (α*α) * v;  len_out = n_h + 1.
+ * With α_min = 0, a static camera and scene, and independent frames (different seeds), hdr_out is the running mean of the frames and
+ * var_out the variance of that mean.  A surface moving under a static camera keeps its history where id, depth and normal still agree,
+ * so its shading lags by up to about 1 / α_min frames; there are no per-object motion vectors. */
+typedef struct rbrt_temporal_opts {
+    float alpha_min;           /* α_min, in [0, 1] (default 0.1) */
+    float sigma_depth;         /* σ_z, >= 0 (default 0.02) */
+    float normal_min;          /* n_min, >= 0 (default 0.9) */
+} rbrt_temporal_opts;
+/* The previous call's outputs, aligned to cam: hdr (W*H*3), var (W*H*3; read only when var_out is requested) and length (W*H, the
+ * frames folded in), and that frame's guides: depth, normal, hit_kind and elem_idx are read, the other members are ignored. */
+typedef struct rbrt_temporal_history {
+    rbrt_camera  cam;
+    const float* hdr;
+    const float* var;
+    const float* length;
+    rbrt_aov_out guides;
+} rbrt_temporal_history;
+/* history NULL: the first frame.  opts NULL: the defaults; otherwise every member is used as given.  Outputs hdr_out, var_out (W*H*3)
+ * and len_out (W*H), f32; any may be NULL, not all.  The calls run on this process's current render device (rbrt_gpu_init; under a
+ * communicator its first device) and are not collective.  The kernel lives in librbrt_gpu_temporal.so, loaded at run time from this
+ * library's directory (RBRT_GPU_TEMPORAL_LIB: another path); without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL cam, hdr, guides or guide depth, normal, hit_kind or elem_idx (and the same in a
+ * history, with its hdr and length); every output NULL; var_out without var, or with a history without var; W or H = 0 or
+ * W*H > 2^31 - 1; a camera (cam or the history's) whose image is not W x H; an option that is NaN, infinite or negative, or
+ * α_min > 1; an output that overlaps an input or another output (so no call accumulates in place: ping-pong two sets of buffers).
+ * stats may be NULL; it reports ms_device, ms_total and launches (1). */
+/* HOST pointers; blocks until the outputs are on the host. */
+int rbrt_gpu_temporal_accumulate(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* hdr, const float* var,
+                                 const rbrt_aov_out* guides, const rbrt_temporal_history* history, const rbrt_temporal_opts* opts,
+                                 float* hdr_out, float* var_out, float* len_out, rbrt_stats* stats);
+/* DEVICE pointers on the current render device, enqueued on cuda_stream (0 = default stream); stats == NULL: enqueue only, no
+ * synchronisation; with stats the call waits for its kernel and fills them.  Also refused: planes in another device's memory or in
+ * unregistered host memory. */
+int rbrt_gpu_temporal_accumulate_device(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* d_hdr, const float* d_var,
+                                        const rbrt_aov_out* d_guides, const rbrt_temporal_history* d_history,
+                                        const rbrt_temporal_opts* opts, float* d_hdr_out, float* d_var_out, float* d_len_out,
+                                        void* cuda_stream, rbrt_stats* stats);
+
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
  * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters, the
  * denoiser's host-call block and the variance call's internal stream). */

@@ -47,6 +47,12 @@ pub struct RbrtQueryOut { pub t: *mut f32, pub dist: *mut f32, pub kind: *mut i3
 /// Options of the guided denoiser (rbrt_gpu_denoise*); 0 = default (4 levels, at most 8).
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct RbrtDenoiseOpts { pub levels: u32, pub sigma_depth: f32, pub sigma_luminance: f32 }
+/// Options of the temporal accumulation, every member used as given (a null pointer gives 0.1, 0.02, 0.9).
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtTemporalOpts { pub alpha_min: f32, pub sigma_depth: f32, pub normal_min: f32 }
+/// The previous temporal call's outputs (hdr, var, length), aligned to `cam`, and that frame's guides.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtTemporalHistory { pub cam: RbrtCamera, pub hdr: *const f32, pub var: *const f32, pub length: *const f32, pub guides: RbrtAovOut }
 pub enum RbrtScene {}
 /// `kind` of a hit (rbrt_hit, rbrt_query_out)
 pub const RBRT_HIT_NONE: i32 = -1;
@@ -163,6 +169,17 @@ extern "C" {
     pub fn rbrt_gpu_denoise_variance_device(width: u32, height: u32, d_hdr: *const f32, d_var: *const f32, d_guides: *const RbrtAovOut,
                                             opts: *const RbrtDenoiseOpts, d_hdr_out: *mut f32, d_rgb_out: *mut u8, stream: *mut c_void,
                                             stats: *mut RbrtStats) -> c_int;
+    /// Temporal accumulation: the frame hdr (and its variance var, may be null) at camera `cam`, guided by render_aov depth / normal /
+    /// hit_kind / elem_idx of the same camera and seed, blended with the history reprojected from its camera (null: the first frame).
+    /// hdr_out, var_out (W*H*3) and len_out (W*H), any may be null, not all, none overlapping an input; HOST pointers, blocks.
+    pub fn rbrt_gpu_temporal_accumulate(width: u32, height: u32, cam: *const RbrtCamera, hdr: *const f32, var: *const f32,
+                                        guides: *const RbrtAovOut, history: *const RbrtTemporalHistory, opts: *const RbrtTemporalOpts,
+                                        hdr_out: *mut f32, var_out: *mut f32, len_out: *mut f32, stats: *mut RbrtStats) -> c_int;
+    /// The same on DEVICE planes of the current render device, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_temporal_accumulate_device(width: u32, height: u32, cam: *const RbrtCamera, d_hdr: *const f32, d_var: *const f32,
+                                               d_guides: *const RbrtAovOut, d_history: *const RbrtTemporalHistory,
+                                               opts: *const RbrtTemporalOpts, d_hdr_out: *mut f32, d_var_out: *mut f32,
+                                               d_len_out: *mut f32, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

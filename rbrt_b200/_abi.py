@@ -107,6 +107,14 @@ class DenoiseOptsC(C.Structure):  # rbrt_denoise_opts: 0 = default
     _fields_ = [("levels", C.c_uint32), ("sigma_depth", C.c_float), ("sigma_luminance", C.c_float)]
 
 
+class TemporalOptsC(C.Structure):  # rbrt_temporal_opts: every member used as given
+    _fields_ = [("alpha_min", C.c_float), ("sigma_depth", C.c_float), ("normal_min", C.c_float)]
+
+
+class TemporalHistoryC(C.Structure):  # rbrt_temporal_history: the previous call's outputs, that frame's guides and camera
+    _fields_ = [("cam", CameraC), ("hdr", C.c_void_p), ("var", C.c_void_p), ("length", C.c_void_p), ("guides", AovOutC)]
+
+
 class SceneInfoC(C.Structure):
     _fields_ = [("num_spheres", C.c_uint32), ("num_meshes", C.c_uint32), ("num_triangles", C.c_uint64),
                 ("num_triangles_tested", C.c_uint64), ("num_bvh_nodes", C.c_uint64),
@@ -182,6 +190,11 @@ GPU_SIGNATURES = {
                                             C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise_variance_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, P(AovOutC), P(DenoiseOptsC),
                                                    C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_temporal_accumulate": (C.c_int, [C.c_uint32, C.c_uint32, P(CameraC), C.c_void_p, C.c_void_p, P(AovOutC), P(TemporalHistoryC),
+                                               P(TemporalOptsC), C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_temporal_accumulate_device": (C.c_int, [C.c_uint32, C.c_uint32, P(CameraC), C.c_void_p, C.c_void_p, P(AovOutC),
+                                                      P(TemporalHistoryC), P(TemporalOptsC), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                      P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

@@ -16,6 +16,7 @@
 #include "multi.cuh"
 #include "query.cuh"
 #include "update.cuh"
+#include "temporal.cuh"
 #include "variance.cuh"
 
 namespace rbrt {
@@ -229,7 +230,8 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
 
 // ------------------------------------------------------------------ device modules
 // The refit kernels (librbrt_gpu_update.so), the AOV kernel (librbrt_gpu_aov.so), the ray queries (librbrt_gpu_query.so), the denoiser
-// (librbrt_gpu_denoise.so) and the variance kernels (librbrt_gpu_variance.so) live in their own device modules, loaded from this library's
+// (librbrt_gpu_denoise.so), the variance kernels (librbrt_gpu_variance.so) and the temporal accumulation (librbrt_gpu_temporal.so) live in
+// their own device modules, loaded from this library's
 // directory (or the path in the module's environment variable) on first use.  Without a module its calls are refused: there is no other
 // implementation.
 // Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
@@ -251,6 +253,7 @@ static Module g_aov_module = {"RBRT_GPU_AOV_LIB", "librbrt_gpu_aov.so", "AOV", n
 static Module g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "query", nullptr};
 static Module g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", nullptr};
 static Module g_variance_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", nullptr};
+static Module g_temporal_module = {"RBRT_GPU_TEMPORAL_LIB", "librbrt_gpu_temporal.so", "temporal", nullptr};
 // The entry point `symbol` of module m, which is opened on first use.  A failed dlopen is not remembered: the next call tries again.
 template <class F> static int module_entry(Module& m, const char* symbol, F* fn) {
     if (!m.h) {
@@ -388,9 +391,9 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
 
 // ------------------------------------------------------------------ per-device state of the calls into the device modules
 // Created on first use, freed by rbrt_gpu_release_cache.
-//  - The staging block that the host-pointer AOV and denoise calls carve their device planes from (grown, never shrunk).  One block
-//    serves both: each such call runs on the legacy default stream and synchronises it before returning.
-//  - The timing events of calls with stats (AOV, query, denoise, variance).  Each such call waits for `e1` or its stream before returning.
+//  - The staging block that the host-pointer AOV, denoise and temporal calls carve their device planes from (grown, never shrunk).  One
+//    block serves them all: each such call runs on the legacy default stream and synchronises it before returning.
+//  - The timing events of calls with stats (AOV, query, denoise, variance, temporal).  Each such call waits for `e1` or its stream before returning.
 //  - The AOV counters, used by calls with stats.
 //  - The query ring: QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
 //    block, zeroes it on its own stream and records `qry_used` behind its kernel, so calls on different streams never share a cursor.  A
@@ -685,6 +688,114 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
         CKA(cudaEventSynchronize(c.e1));
         float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
         stats->ms_device = ms; stats->launches = 1 + a.levels;
+        stats->ms_total = now_ms() - t0;
+    }
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ temporal accumulation (rbrt_gpu_temporal_accumulate*)
+// The host-pointer variant copies its planes into the device's staging block; the device variant launches on the caller's planes.
+static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float* hdr, const float* var, const rbrt_aov_out* guides,
+                    const rbrt_temporal_history* hist, const rbrt_temporal_opts* opts, float* hdr_out, float* var_out, float* len_out,
+                    bool host, cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!cam || !hdr || !guides) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!guides->depth || !guides->normal || !guides->hit_kind || !guides->elem_idx) {
+        set_error("null guide plane: depth, normal, hit_kind and elem_idx are read"); return RBRT_E_INVALID;
+    }
+    if (hist && (!hist->hdr || !hist->length || !hist->guides.depth || !hist->guides.normal || !hist->guides.hit_kind || !hist->guides.elem_idx)) {
+        set_error("null history plane: hdr, length and the guides' depth, normal, hit_kind and elem_idx are read"); return RBRT_E_INVALID;
+    }
+    if (!hdr_out && !var_out && !len_out) { set_error("no output requested (hdr_out, var_out and len_out are all NULL)"); return RBRT_E_INVALID; }
+    if (var_out && (!var || (hist && !hist->var))) { set_error("var_out needs var, and the history's var when there is a history"); return RBRT_E_INVALID; }
+    if (!W || !H) { set_error("empty image"); return RBRT_E_INVALID; }
+    const size_t n = (size_t)W * H;
+    if (n > 0x7FFFFFFFull) { set_error("image too large"); return RBRT_E_INVALID; }
+    if (cam->img_width_pix != W || cam->img_height_pix != H || (hist && (hist->cam.img_width_pix != W || hist->cam.img_height_pix != H))) {
+        set_error("a camera's image is not %u x %u", W, H); return RBRT_E_INVALID;
+    }
+    TemporalArgs a;
+    memset(&a, 0, sizeof(a));
+    a.W = W; a.H = H;
+    a.alpha_min = opts ? opts->alpha_min : TP_ALPHA_MIN;
+    a.sigma_z = opts ? opts->sigma_depth : TP_SIGMA_DEPTH;
+    a.n_min = opts ? opts->normal_min : TP_NORMAL_MIN;
+    if (!(a.alpha_min >= 0.0f && a.alpha_min <= 1.0f) || !(a.sigma_z >= 0.0f && a.sigma_z <= FLT_MAX) || !(a.n_min >= 0.0f && a.n_min <= FLT_MAX)) {
+        set_error("options must be finite and >= 0, alpha_min at most 1"); return RBRT_E_INVALID;
+    }
+    // inputs: what is read.  The history's var only with var_out.
+    const bool hv = hist && var_out;
+    const struct { const void* p; size_t b; } in[13] = {
+        {hdr, 12 * n}, {var, 12 * n}, {guides->depth, 4 * n}, {guides->normal, 12 * n}, {guides->hit_kind, 4 * n}, {guides->elem_idx, 4 * n},
+        {hist ? hist->hdr : nullptr, 12 * n}, {hv ? hist->var : nullptr, 12 * n}, {hist ? hist->length : nullptr, 4 * n},
+        {hist ? hist->guides.depth : nullptr, 4 * n}, {hist ? hist->guides.normal : nullptr, 12 * n},
+        {hist ? hist->guides.hit_kind : nullptr, 4 * n}, {hist ? hist->guides.elem_idx : nullptr, 4 * n}};
+    const struct { void* p; size_t b; } out[3] = {{hdr_out, 12 * n}, {var_out, 12 * n}, {len_out, 4 * n}};
+    for (int o = 0; o < 3; ++o) {
+        for (const auto& i : in)
+            if (overlap(out[o].p, out[o].b, i.p, i.b)) { set_error("an output overlaps an input"); return RBRT_E_INVALID; }
+        for (int k = o + 1; k < 3; ++k)
+            if (overlap(out[o].p, out[o].b, out[k].p, out[k].b)) { set_error("two outputs overlap"); return RBRT_E_INVALID; }
+    }
+    { int rc = ensure_device(); if (rc) return rc; }
+    const int dev = g_device;
+    if (!host) {
+        for (const auto& i : in) { int rc = check_usable_on({i.p}, dev, "planes must be device memory on the current device %d"); if (rc) return rc; }
+        int rc = check_usable_on({hdr_out, var_out, len_out}, dev, "planes must be device memory on the current device %d");
+        if (rc) return rc;
+    }
+    rbrt_temporal_launch_fn launch = nullptr;
+    { int rc = module_entry(g_temporal_module, "rbrt_temporal_launch", &launch); if (rc) return rc; }
+    const double t0 = now_ms();
+
+    a.cam = make_cam(*cam);
+    a.var = var;
+    if (hist) {
+        a.history = 1;
+        a.same_cam = memcmp(cam, &hist->cam, sizeof(rbrt_camera)) == 0;
+        a.prev = make_cam(hist->cam);
+    }
+    const void** dst[13] = {(const void**)&a.hdr, (const void**)&a.var, (const void**)&a.depth, (const void**)&a.normal, (const void**)&a.kind,
+                            (const void**)&a.elem, (const void**)&a.h_hdr, (const void**)&a.h_var, (const void**)&a.h_len,
+                            (const void**)&a.h_depth, (const void**)&a.h_normal, (const void**)&a.h_kind, (const void**)&a.h_elem};
+    DeviceCache& c = g_cache[dev & 63];
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
+    if (host) {                                                           // inputs and outputs carved from the staging block
+        size_t need = 0;
+        for (const auto& i : in) if (i.p) need += a256(i.b);
+        for (const auto& o : out) if (o.p) need += a256(o.b);
+        char* p = nullptr;
+        { int rc = staging_block(c, need, &p); if (rc) return rc; }
+        for (int k = 0; k < 13; ++k) {
+            if (!in[k].p) continue;
+            CKA(cudaMemcpyAsync(p, in[k].p, in[k].b, cudaMemcpyHostToDevice, st));
+            *dst[k] = p; p += a256(in[k].b);
+        }
+        if (hdr_out) { a.hdr_out = (float*)p; p += a256(12 * n); }
+        if (var_out) { a.var_out = (float*)p; p += a256(12 * n); }
+        if (len_out) a.len_out = (float*)p;
+    } else {
+        for (int k = 0; k < 13; ++k) *dst[k] = in[k].p;
+        a.hdr_out = hdr_out; a.var_out = var_out; a.len_out = len_out;
+    }
+    if (stats) CKA(cudaEventRecord(c.e0, st));
+    {
+        cudaError_t e = (cudaError_t)launch(&a, st);
+        if (e == cudaSuccess && stats) e = cudaEventRecord(c.e1, st);
+        if (e != cudaSuccess) return cuda_fail(e, "rbrt_temporal_launch");
+    }
+    if (host) {
+        if (hdr_out) CKA(cudaMemcpyAsync(hdr_out, a.hdr_out, 12 * n, cudaMemcpyDeviceToHost, st));
+        if (var_out) CKA(cudaMemcpyAsync(var_out, a.var_out, 12 * n, cudaMemcpyDeviceToHost, st));
+        if (len_out) CKA(cudaMemcpyAsync(len_out, a.len_out, 4 * n, cudaMemcpyDeviceToHost, st));
+        CKA(cudaStreamSynchronize(st));
+    } else if (!stats) {
+        return RBRT_OK;                                                   // enqueue only
+    }
+    if (stats) {
+        CKA(cudaEventSynchronize(c.e1));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
+        stats->ms_device = ms; stats->launches = 1;
         stats->ms_total = now_ms() - t0;
     }
     return RBRT_OK;
@@ -1277,6 +1388,22 @@ int rbrt_gpu_denoise_variance_device(uint32_t width, uint32_t height, const floa
                                      const rbrt_denoise_opts* opts, float* d_hdr_out, uint8_t* d_rgb_out, void* cuda_stream, rbrt_stats* stats) {
     LOCK;
     return denoise(width, height, d_hdr, d_var, d_guides, opts, d_hdr_out, d_rgb_out, true, false, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_temporal_accumulate(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* hdr, const float* var,
+                                 const rbrt_aov_out* guides, const rbrt_temporal_history* history, const rbrt_temporal_opts* opts,
+                                 float* hdr_out, float* var_out, float* len_out, rbrt_stats* stats) {
+    LOCK;
+    return temporal(width, height, cam, hdr, var, guides, history, opts, hdr_out, var_out, len_out, true, 0, stats);
+}
+
+int rbrt_gpu_temporal_accumulate_device(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* d_hdr, const float* d_var,
+                                        const rbrt_aov_out* d_guides, const rbrt_temporal_history* d_history,
+                                        const rbrt_temporal_opts* opts, float* d_hdr_out, float* d_var_out, float* d_len_out,
+                                        void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return temporal(width, height, cam, d_hdr, d_var, d_guides, d_history, opts, d_hdr_out, d_var_out, d_len_out, false,
+                    (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

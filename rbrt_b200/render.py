@@ -317,3 +317,78 @@ def denoise_variance_device(hdr, var, aovs, levels=0, sigma_depth=0.0, sigma_lum
     """The same on CUDA tensors of the current render device: returns (hdr_out [H,W,3] float32, rgb [H,W,3] uint8) tensors, enqueued on
     `stream` (default: the current stream) without synchronising."""
     return _denoise(hdr, var, aovs, levels, sigma_depth, sigma_luminance, True, stream=stream)
+
+
+# ---- temporal accumulation (rbrt_gpu_temporal_accumulate*; include/rbrt_gpu.h and DESIGN.md section 15) ----------------------------
+_TEMPORAL_GUIDES = (("depth", 1, "float32"), ("normal", 3, "float32"), ("hit_kind", 1, "int32"), ("elem_idx", 1, "uint32"))
+
+
+def _temporal_plane(what, v, H, W, k, dtype, device):
+    shape = (H, W, k) if k > 1 else (H, W)
+    if device:
+        import torch
+        ok = isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == getattr(torch, dtype) and v.is_contiguous()
+    else:
+        ok = isinstance(v, np.ndarray) and v.dtype == np.dtype(dtype) and v.flags.c_contiguous
+    if not ok or tuple(v.shape) != shape:
+        raise ValueError(f"{what} must be a contiguous {dtype} {'CUDA tensor' if device else 'numpy array'} of shape {shape}")
+    return v.data_ptr() if device else v.ctypes.data
+
+
+def _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, device, outs, stream=None, stats=None):
+    """temporal_accumulate (numpy) and, with device=True, temporal_accumulate_device; outs = (hdr_out, var_out, len_out) or None."""
+    W, H = cam.img_width_pix, cam.img_height_pix
+    if var is not None and history is not None and history.get("var") is None:
+        raise ValueError("with var, the history needs the var it returned")
+    ptr = lambda what, v, k=3, dt="float32": _temporal_plane(what, v, H, W, k, dt, device)
+    planes = [ptr("hdr", hdr), ptr("var", var) if var is not None else None]
+
+    def guides(what, g):
+        missing = [k for k, *_ in _TEMPORAL_GUIDES if k not in g]
+        if missing:
+            raise ValueError(f"the {what} need the AOVs {missing} (render_aovs with passes depth, normal and ids)")
+        return _abi.AovOutC(**{k: ptr(f"{what}[{k!r}]", g[k], n, dt) for k, n, dt in _TEMPORAL_GUIDES})
+
+    g = guides("guides", aovs)
+    h = None
+    if history is not None:
+        h = _abi.TemporalHistoryC(cam=history["cam"].to_c(), hdr=ptr("history hdr", history["hdr"]),
+                                  var=ptr("history var", history["var"]) if var is not None else None,
+                                  length=ptr("history length", history["length"], 1), guides=guides("history guides", history["aovs"]))
+    opts = _abi.TemporalOptsC(float(alpha_min), float(sigma_depth), float(normal_min))
+    if outs is None:
+        if device:
+            import torch
+            with torch.cuda.stream(stream):
+                outs = (torch.empty((H, W, 3), dtype=torch.float32, device=stream.device),
+                        torch.empty((H, W, 3), dtype=torch.float32, device=stream.device) if var is not None else None,
+                        torch.empty((H, W), dtype=torch.float32, device=stream.device))
+        else:
+            outs = (np.empty((H, W, 3), np.float32), np.empty((H, W, 3), np.float32) if var is not None else None, np.empty((H, W), np.float32))
+    optr = [ptr("hdr_out", outs[0]), ptr("var_out", outs[1]) if outs[1] is not None else None, ptr("len_out", outs[2], 1)]
+    lib = _abi.lib()
+    if device:
+        _abi.check(lib.rbrt_gpu_temporal_accumulate_device(W, H, cam.to_c(), *planes, g, h, opts, *optr, stream.cuda_stream, None))
+    else:
+        st = _abi.StatsC()
+        _abi.check(lib.rbrt_gpu_temporal_accumulate(W, H, cam.to_c(), *planes, g, h, opts, *optr, st))
+        if stats is not None:
+            stats.update(st.as_dict())
+    return outs
+
+
+def temporal_accumulate(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stats=None):
+    """Fold the frame hdr [H,W,3] (with its variance var [H,W,3], optional) rendered at camera `cam` into a history: each pixel's
+    history is reprojected through the previous camera and blended with the frame where depth, normal and sample 0's hit ids agree.
+    aovs: render_aovs planes of the same camera and seed with depth, normal, hit_kind and elem_idx.  history: None for the first frame,
+    else a dict with the previous call's results and inputs: cam, hdr, var (with var), length and aovs.  Returns (hdr_out, var_out or
+    None, length [H,W]) numpy float32 arrays; blocks until they are on the host."""
+    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, False, None, stats=stats)
+
+
+def temporal_accumulate_device(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stream=None):
+    """The same on CUDA tensors of the current render device (render_aovs_device's planes): returns (hdr_out, var_out or None, length)
+    tensors, enqueued on `stream` (default: the current stream) without synchronising."""
+    import torch
+    stream = stream or torch.cuda.current_stream()
+    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, True, None, stream=stream)
