@@ -37,11 +37,27 @@ def build(fn):
     return fn()
 
 
+def sample_shard_mean(scene, cam, spp, world, seed):
+    """What the PEER sample-sharded render computes: ((a_0 + a_1) + ... + a_{world-1}) * (1/spp) in f32 (k_sum_peers, then k_finalize),
+    a_r the sums of an explicit sample shard r of `world` rendered on one GPU."""
+    import torch
+    W, H = cam.img_width_pix, cam.img_height_pix
+    total = None
+    for r in range(world):
+        buf = torch.empty(H * W * 4, dtype=torch.float32, device="cuda")
+        _abi.check(_abi.lib().rbrt_gpu_render_accum_device(scene.handle(), cam.to_c(), spp, R.render.make_opts(
+            seed=seed, shard_mode=_abi.SHARD_SAMPLES, shard_rank=r, shard_count=world), buf.data_ptr(), torch.cuda.current_stream().cuda_stream, None))
+        a = buf.cpu().numpy().reshape(H, W, 4)[..., :3]
+        total = a if total is None else (total + a).astype(np.float32)
+    return (total * (np.float32(1.0) / np.float32(spp))).astype(np.float32)
+
+
 @pytest.mark.parametrize("world", [2, 3, 8])
 def test_collective_render_equals_one_gpu(gpu, comm, world):
     cam = S.example_camera(150, 101)                                   # ragged: partial tiles on both edges
     want_u8 = R.render_scene(cam, 5, S.small_mesh_scene(4), seed=12).pixels
     want_hdr = R.render_scene_hdr(cam, 5, S.small_mesh_scene(4), seed=12)
+    want_samples = sample_shard_mean(S.small_mesh_scene(4), cam, 5, world, seed=12)
     info = comm(world)
     assert info["active"] == 1 and info["world"] == world and info["local_devices"] == world and info["transport"] == _abi.TRANSPORT_PEER
     scene = S.small_mesh_scene(4)                                      # created under the communicator: built once, replicated
@@ -51,8 +67,9 @@ def test_collective_render_equals_one_gpu(gpu, comm, world):
     assert st["paths"] == 150 * 101 * 5
     hdr = R.render_scene_hdr(cam, 5, scene, seed=12)
     assert np.array_equal(hdr.view(np.uint32), want_hdr.view(np.uint32))
-    # sample-range shards: the per-rank partial sums are re-associated
+    # sample-range shards: rank 0's sums plus the other ranks' in rank order, then the 1/spp scale, all in f32
     hs = R.render_scene_hdr(cam, 5, scene, seed=12, shard_mode=_abi.SHARD_SAMPLES)
+    assert np.array_equal(hs.view(np.uint32), want_samples.view(np.uint32))
     assert np.allclose(hs, want_hdr, rtol=1e-5, atol=1e-6)
     # an explicit shard placed by the host still works under a communicator, and a LOCAL scene is not sharded
     one = R.render_scene_hdr(cam, 5, scene, seed=12, shard_mode=_abi.SHARD_TILES, shard_rank=1, shard_count=2)

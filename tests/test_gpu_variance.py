@@ -202,7 +202,9 @@ def test_render_on_side_streams_two_calls_in_flight(gpu):
     (different wavefront pools: frames in flight at the same time use different pools)."""
     import torch
     scene, cam = workload("c2", 128, 96)
-    want = [R.render_scene_hdr_variance(cam, 16, scene, splits=4, seed=s) for s in (5, 6)]
+    # the references run on the pools the device calls use, so that those find them large enough: a pool that has to grow frees its
+    # old buffers, and cudaFree waits for the whole device (the sleep queued on the other stream included)
+    want = [R.render_scene_hdr_variance(cam, 16, scene, splits=4, seed=s, pool=i) for i, s in enumerate((5, 6))]
     torch.cuda.synchronize()
     streams = [torch.cuda.Stream(), torch.cuda.Stream()]
     outs, busy = [], []
