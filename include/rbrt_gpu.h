@@ -586,7 +586,7 @@ int rbrt_gpu_denoise_variance_device(uint32_t width, uint32_t height, const floa
  *   5. α = max(1 / (n_h + 1), α_min);  hdr_out = c_h + α * (c - c_h);  var_out = ((1-α)*(1-α)) * v_h + (α*α) * v;  len_out = n_h + 1.
  * With α_min = 0, a static camera and scene, and independent frames (different seeds), hdr_out is the running mean of the frames and
  * var_out the variance of that mean.  A surface moving under a static camera keeps its history where id, depth and normal still agree,
- * so its shading lags by up to about 1 / α_min frames; there are no per-object motion vectors. */
+ * so its shading lags by up to about 1 / α_min frames unless the motion variant below reprojects it along its motion vectors. */
 typedef struct rbrt_temporal_opts {
     float alpha_min;           /* α_min, in [0, 1] (default 0.1) */
     float sigma_depth;         /* σ_z, >= 0 (default 0.02) */
@@ -621,6 +621,66 @@ int rbrt_gpu_temporal_accumulate_device(uint32_t width, uint32_t height, const r
                                         const rbrt_aov_out* d_guides, const rbrt_temporal_history* d_history,
                                         const rbrt_temporal_opts* opts, float* d_hdr_out, float* d_var_out, float* d_len_out,
                                         void* cuda_stream, rbrt_stats* stats);
+
+/* ---- per-object motion vectors (DESIGN.md section 16) ---------------------------------------------
+ * SNAPSHOT.  Records the scene's current geometry as "the previous frame", in device memory owned by the scene (allocated on the first
+ * snapshot, about 48 bytes per tested triangle, freed with the scene): for every mesh each tested triangle's record (v0, e1, e2 as the
+ * scene stores them) at its ORIGINAL triangle index, so RBRT_UPDATE_REBUILD, which permutes the records, does not mix them up; every
+ * element's sphere values (centre, radius); every BasicTriangle's v0, e1, e2.  Enqueue only, on cuda_stream (0 = default stream).
+ * Ordering: the snapshot sees every update enqueued before it, every later update waits for it, and it waits for every read of the
+ * scene enqueued before it (so a motion call still reading the previous snapshot finishes first).  Under a communicator it acts on
+ * replica 0 and is not collective.  An unchanged scene snapshots to the same bytes.  Refused with RBRT_E_INVALID: a NULL scene, a scene
+ * with a mesh whose tree was refused as too deep.  The kernel lives in librbrt_gpu_motion.so (RBRT_GPU_MOTION_LIB: another path);
+ * without it the call fails with RBRT_E_CUDA and a message. */
+int rbrt_gpu_scene_snapshot(rbrt_scene* scene, void* cuda_stream);
+
+/* MOTION PASS.  Per pixel p = (x, y) of cam's W x H image, each operation one correctly rounded f32 operation, products and sums left to
+ * right as written (rbrt_b200/csrc/motion.cuh holds steps 3-5; the camera arithmetic is the temporal section's):
+ *   1. The ray: origin pos, direction d = that of step 3 of the temporal accumulation (rbrt_gpu_primary_rays' direction for p with both
+ *      jitter draws at 0.5, the pixel centre).  No seed.
+ *   2. h = Scene::hit(ray), bit for bit what rbrt_gpu_trace_rays(RBRT_TRACE_BVH) reports.  A miss, or a NaN ray (counted in
+ *      stats->nan_rays), gives motion = (NaN, NaN) and prev_dist = +inf.
+ *   3. P = h.point = pos + h.t * d per component.
+ *   4. The previous point P'.  When the hit element is unchanged since the latest snapshot — a mesh triangle's v0, e1, e2, a sphere's
+ *      centre and radius, a BasicTriangle's v0, e1, e2, bit for bit equal to the snapshot's — P' = P.  Otherwise, for a mesh triangle or a
+ *      BasicTriangle, u and v are the Moller-Trumbore values of its intersection test for the current record and this ray (h = d x e2,
+ *      a = e1 . h, f = 1 / a, s = pos - v0, u = f * (s . h), q = s x e1, v = f * (d . q)) and P' = (v0' + u*e1') + v*e2' per component
+ *      (primes: the snapshot); for a sphere P' = c' + (P - c) * (r' / r) per component (negative radii as at creation).
+ *   5. q = the projection of D = P - pos into cam, q' = that of D' = P' - pos' into prev_cam, each as step 3 of the temporal accumulation
+ *      (Cramer's rule; px, py).  motion = (q'.x - q.x, q'.y - q.y), or (NaN, NaN) when either projection fails (s <= 0 or NaN) or gives a
+ *      coordinate that is not finite.  prev_dist = sqrt((D'.x*D'.x + D'.y*D'.y) + D'.z*D'.z).
+ * With nothing changed since the snapshot and prev_cam equal to cam bit for bit, every hit pixel has motion exactly (0, 0) and prev_dist
+ * the distance from pos to h.point.  Planes row-major: motion W*H*2 (x, y per pixel), prev_dist W*H; a NULL member is not written.
+ * Ordering: the call sees every update enqueued before it and the latest snapshot enqueued before it (on any stream); every later update
+ * and snapshot waits for it.  Under a communicator it runs on replica 0 and is not collective.  The kernel lives in
+ * librbrt_gpu_motion.so (RBRT_GPU_MOTION_LIB: another path); without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL scene, cam, prev_cam or out, both planes NULL; prev_cam's image not W x H; an
+ * empty image or W*H > 2^31 - 1; the planes overlapping; a scene without a snapshot; a scene with a mesh whose tree was refused as too
+ * deep.  stats may be NULL; it reports rays = W*H, nan_rays, node_visits / tri_tests, ms_device, ms_total and launches (1). */
+typedef struct rbrt_motion_out {
+    float* motion;      /* W*H*2 */
+    float* prev_dist;   /* W*H */
+} rbrt_motion_out;
+/* HOST pointers; blocks until the planes are on the host. */
+int rbrt_gpu_render_motion(const rbrt_scene* scene, const rbrt_camera* cam, const rbrt_camera* prev_cam, const rbrt_motion_out* out,
+                           rbrt_stats* stats);
+/* DEVICE pointers on the scene's first device, enqueued on cuda_stream (0 = default stream); stats == NULL: enqueue only, no
+ * synchronisation.  Also refused: planes in another device's memory or in unregistered host memory. */
+int rbrt_gpu_render_motion_device(const rbrt_scene* scene, const rbrt_camera* cam, const rbrt_camera* prev_cam, const rbrt_motion_out* d_out,
+                                  void* cuda_stream, rbrt_stats* stats);
+
+/* TEMPORAL ACCUMULATION ALONG THE MOTION.  rbrt_gpu_temporal_accumulate* with the current frame's motion pass against the history's
+ * camera (prev_cam = history->cam) and the snapshot taken at the history's frame.  Only step 3 changes: when both components of m =
+ * motion[p] are finite, (px, py) = (x + m.x, y + m.y) and r = prev_dist[p], and the tests of step 3 on r and on the bounds, and steps
+ * 4 and 5, run as there; otherwise step 3 runs as there (camera reprojection, the bitwise-equal camera included).  The motion planes are
+ * inputs: refused when NULL (either plane), or when an output overlaps them; everything else as rbrt_gpu_temporal_accumulate*. */
+int rbrt_gpu_temporal_accumulate_motion(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* hdr, const float* var,
+                                        const rbrt_aov_out* guides, const rbrt_temporal_history* history, const rbrt_motion_out* motion,
+                                        const rbrt_temporal_opts* opts, float* hdr_out, float* var_out, float* len_out, rbrt_stats* stats);
+int rbrt_gpu_temporal_accumulate_motion_device(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* d_hdr, const float* d_var,
+                                               const rbrt_aov_out* d_guides, const rbrt_temporal_history* d_history,
+                                               const rbrt_motion_out* d_motion, const rbrt_temporal_opts* opts, float* d_hdr_out,
+                                               float* d_var_out, float* d_len_out, void* cuda_stream, rbrt_stats* stats);
 
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
  * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters, the

@@ -53,6 +53,9 @@ pub struct RbrtTemporalOpts { pub alpha_min: f32, pub sigma_depth: f32, pub norm
 /// The previous temporal call's outputs (hdr, var, length), aligned to `cam`, and that frame's guides.
 #[repr(C)] #[derive(Copy, Clone, Debug)]
 pub struct RbrtTemporalHistory { pub cam: RbrtCamera, pub hdr: *const f32, pub var: *const f32, pub length: *const f32, pub guides: RbrtAovOut }
+/// Planes of the motion pass (rbrt_gpu_render_motion*): motion W*H*2 (x, y per pixel), prev_dist W*H; a null member is not produced.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtMotionOut { pub motion: *mut f32, pub prev_dist: *mut f32 }
 pub enum RbrtScene {}
 /// `kind` of a hit (rbrt_hit, rbrt_query_out)
 pub const RBRT_HIT_NONE: i32 = -1;
@@ -180,6 +183,26 @@ extern "C" {
                                                d_guides: *const RbrtAovOut, d_history: *const RbrtTemporalHistory,
                                                opts: *const RbrtTemporalOpts, d_hdr_out: *mut f32, d_var_out: *mut f32,
                                                d_len_out: *mut f32, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// Records the scene's geometry as "the previous frame" for the motion pass; enqueued on `stream`.
+    pub fn rbrt_gpu_scene_snapshot(scene: *mut RbrtScene, stream: *mut c_void) -> c_int;
+    /// Per-pixel screen motion from `cam` back to `prev_cam` along the geometry's change since the latest snapshot, and the distance
+    /// from prev_cam's position to the previous point; HOST pointers, blocks.
+    pub fn rbrt_gpu_render_motion(scene: *const RbrtScene, cam: *const RbrtCamera, prev_cam: *const RbrtCamera, out: *const RbrtMotionOut,
+                                  stats: *mut RbrtStats) -> c_int;
+    /// The same on DEVICE planes of the scene's first device, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_render_motion_device(scene: *const RbrtScene, cam: *const RbrtCamera, prev_cam: *const RbrtCamera,
+                                         d_out: *const RbrtMotionOut, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// rbrt_gpu_temporal_accumulate reprojecting along the frame's motion pass where it is finite; HOST pointers, blocks.
+    pub fn rbrt_gpu_temporal_accumulate_motion(width: u32, height: u32, cam: *const RbrtCamera, hdr: *const f32, var: *const f32,
+                                               guides: *const RbrtAovOut, history: *const RbrtTemporalHistory, motion: *const RbrtMotionOut,
+                                               opts: *const RbrtTemporalOpts, hdr_out: *mut f32, var_out: *mut f32, len_out: *mut f32,
+                                               stats: *mut RbrtStats) -> c_int;
+    /// The same on DEVICE planes of the current render device, enqueued on `stream` (stats = null: no synchronisation).
+    pub fn rbrt_gpu_temporal_accumulate_motion_device(width: u32, height: u32, cam: *const RbrtCamera, d_hdr: *const f32, d_var: *const f32,
+                                                      d_guides: *const RbrtAovOut, d_history: *const RbrtTemporalHistory,
+                                                      d_motion: *const RbrtMotionOut, opts: *const RbrtTemporalOpts, d_hdr_out: *mut f32,
+                                                      d_var_out: *mut f32, d_len_out: *mut f32, stream: *mut c_void,
+                                                      stats: *mut RbrtStats) -> c_int;
     pub fn rbrt_gpu_release_cache() -> c_int;
     pub fn rbrt_last_error() -> *const c_char;
     pub fn rbrt_gpu_version() -> *const c_char;

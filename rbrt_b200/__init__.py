@@ -16,8 +16,8 @@ from .materials import Dielectric, Lambertian, Metal
 from .mesh import TriangleMesh, load_mesh_vertices_from_file
 from .pipeline import FramePipeline
 from .render import (AOV_PASSES, ImageBuffer, denoise, denoise_device, denoise_variance, denoise_variance_device, primary_rays, render_aovs,
-                     render_aovs_device, render_hdr_variance_device, render_scene, render_scene_hdr, render_scene_hdr_variance,
-                     temporal_accumulate, temporal_accumulate_device)
+                     render_aovs_device, render_hdr_variance_device, render_motion, render_motion_device, render_scene, render_scene_hdr,
+                     render_scene_hdr_variance, temporal_accumulate, temporal_accumulate_device)
 from .scene import Scene
 from .temporal import TemporalAccumulator
 from .sphere import Sphere

@@ -115,6 +115,10 @@ class TemporalHistoryC(C.Structure):  # rbrt_temporal_history: the previous call
     _fields_ = [("cam", CameraC), ("hdr", C.c_void_p), ("var", C.c_void_p), ("length", C.c_void_p), ("guides", AovOutC)]
 
 
+class MotionOutC(C.Structure):  # rbrt_motion_out: device or host planes, NULL = not produced
+    _fields_ = [("motion", C.c_void_p), ("prev_dist", C.c_void_p)]
+
+
 class SceneInfoC(C.Structure):
     _fields_ = [("num_spheres", C.c_uint32), ("num_meshes", C.c_uint32), ("num_triangles", C.c_uint64),
                 ("num_triangles_tested", C.c_uint64), ("num_bvh_nodes", C.c_uint64),
@@ -195,6 +199,15 @@ GPU_SIGNATURES = {
     "rbrt_gpu_temporal_accumulate_device": (C.c_int, [C.c_uint32, C.c_uint32, P(CameraC), C.c_void_p, C.c_void_p, P(AovOutC),
                                                       P(TemporalHistoryC), P(TemporalOptsC), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                       P(StatsC)]),
+    "rbrt_gpu_scene_snapshot": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "rbrt_gpu_render_motion": (C.c_int, [C.c_void_p, P(CameraC), P(CameraC), P(MotionOutC), P(StatsC)]),
+    "rbrt_gpu_render_motion_device": (C.c_int, [C.c_void_p, P(CameraC), P(CameraC), P(MotionOutC), C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_temporal_accumulate_motion": (C.c_int, [C.c_uint32, C.c_uint32, P(CameraC), C.c_void_p, C.c_void_p, P(AovOutC),
+                                                      P(TemporalHistoryC), P(MotionOutC), P(TemporalOptsC), C.c_void_p, C.c_void_p,
+                                                      C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_temporal_accumulate_motion_device": (C.c_int, [C.c_uint32, C.c_uint32, P(CameraC), C.c_void_p, C.c_void_p, P(AovOutC),
+                                                             P(TemporalHistoryC), P(MotionOutC), P(TemporalOptsC), C.c_void_p, C.c_void_p,
+                                                             C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_release_cache": (C.c_int, []),
     "rbrt_last_error": (C.c_char_p, []),
     "rbrt_gpu_version": (C.c_char_p, []),

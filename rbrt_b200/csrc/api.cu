@@ -16,6 +16,7 @@
 #include "multi.cuh"
 #include "query.cuh"
 #include "update.cuh"
+#include "motion.cuh"
 #include "temporal.cuh"
 #include "variance.cuh"
 
@@ -167,6 +168,13 @@ void destroy_scene(Scene* sc) {
         s = Scene::Staging();
     }
     pinned_put(sc->res_h, 16ull * sc->n_meshes); sc->res_h = nullptr;
+    if (sc->snap) {                                                       // behind the snapshot and every read of it (the motion calls)
+        cudaSetDevice(sc->rep[0].device);
+        if (sc->snap_ev) cudaEventSynchronize(sc->snap_ev);
+        for (SceneUse& u : sc->uses) if (u.device == sc->rep[0].device && u.ev) cudaEventSynchronize(u.ev);
+        cudaFree(sc->snap); sc->snap = nullptr;
+    }
+    if (sc->snap_ev) { cudaEventDestroy(sc->snap_ev); sc->snap_ev = nullptr; }
     for (Replica& r : sc->rep) {
         if (!r.arena) { if (r.ready) cudaEventDestroy(r.ready); continue; }
         ArenaBlock b{r.arena, r.arena_bytes, r.device, {}};
@@ -230,8 +238,8 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
 
 // ------------------------------------------------------------------ device modules
 // The refit kernels (librbrt_gpu_update.so), the AOV kernel (librbrt_gpu_aov.so), the ray queries (librbrt_gpu_query.so), the denoiser
-// (librbrt_gpu_denoise.so), the variance kernels (librbrt_gpu_variance.so) and the temporal accumulation (librbrt_gpu_temporal.so) live in
-// their own device modules, loaded from this library's
+// (librbrt_gpu_denoise.so), the variance kernels (librbrt_gpu_variance.so), the temporal accumulation (librbrt_gpu_temporal.so) and the
+// snapshot with the motion pass (librbrt_gpu_motion.so) live in their own device modules, loaded from this library's
 // directory (or the path in the module's environment variable) on first use.  Without a module its calls are refused: there is no other
 // implementation.
 // Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
@@ -254,6 +262,7 @@ static Module g_query_module = {"RBRT_GPU_QUERY_LIB", "librbrt_gpu_query.so", "q
 static Module g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.so", "denoise", nullptr};
 static Module g_variance_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", nullptr};
 static Module g_temporal_module = {"RBRT_GPU_TEMPORAL_LIB", "librbrt_gpu_temporal.so", "temporal", nullptr};
+static Module g_motion_module = {"RBRT_GPU_MOTION_LIB", "librbrt_gpu_motion.so", "motion", nullptr};
 // The entry point `symbol` of module m, which is opened on first use.  A failed dlopen is not remembered: the next call tries again.
 template <class F> static int module_entry(Module& m, const char* symbol, F* fn) {
     if (!m.h) {
@@ -391,10 +400,11 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
 
 // ------------------------------------------------------------------ per-device state of the calls into the device modules
 // Created on first use, freed by rbrt_gpu_release_cache.
-//  - The staging block that the host-pointer AOV, denoise and temporal calls carve their device planes from (grown, never shrunk).  One
+//  - The staging block that the host-pointer AOV, denoise, temporal and motion calls carve their device planes from (grown, never shrunk).  One
 //    block serves them all: each such call runs on the legacy default stream and synchronises it before returning.
-//  - The timing events of calls with stats (AOV, query, denoise, variance, temporal).  Each such call waits for `e1` or its stream before returning.
-//  - The AOV counters, used by calls with stats.
+//  - The timing events of calls with stats (AOV, query, denoise, variance, temporal, motion).  Each such call waits for `e1` or its stream
+//    before returning.
+//  - The AOV counters, used by AOV and motion calls with stats.
 //  - The query ring: QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
 //    block, zeroes it on its own stream and records `qry_used` behind its kernel, so calls on different streams never share a cursor.  A
 //    block is reused QRY_RING calls later; the host waits for its previous call only if that one has still not run by then.
@@ -695,11 +705,13 @@ static int denoise(uint32_t W, uint32_t H, const float* hdr, const float* var, c
 
 // ------------------------------------------------------------------ temporal accumulation (rbrt_gpu_temporal_accumulate*)
 // The host-pointer variant copies its planes into the device's staging block; the device variant launches on the caller's planes.
+// with_motion: rbrt_gpu_temporal_accumulate_motion*, reading the planes of `mo`.
 static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float* hdr, const float* var, const rbrt_aov_out* guides,
-                    const rbrt_temporal_history* hist, const rbrt_temporal_opts* opts, float* hdr_out, float* var_out, float* len_out,
-                    bool host, cudaStream_t st, rbrt_stats* stats) {
+                    const rbrt_temporal_history* hist, const rbrt_motion_out* mo, bool with_motion, const rbrt_temporal_opts* opts,
+                    float* hdr_out, float* var_out, float* len_out, bool host, cudaStream_t st, rbrt_stats* stats) {
     if (stats) memset(stats, 0, sizeof(*stats));
     if (!cam || !hdr || !guides) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (with_motion && (!mo || !mo->motion || !mo->prev_dist)) { set_error("null motion plane: motion and prev_dist are read"); return RBRT_E_INVALID; }
     if (!guides->depth || !guides->normal || !guides->hit_kind || !guides->elem_idx) {
         set_error("null guide plane: depth, normal, hit_kind and elem_idx are read"); return RBRT_E_INVALID;
     }
@@ -725,11 +737,12 @@ static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float*
     }
     // inputs: what is read.  The history's var only with var_out.
     const bool hv = hist && var_out;
-    const struct { const void* p; size_t b; } in[13] = {
+    const struct { const void* p; size_t b; } in[15] = {
         {hdr, 12 * n}, {var, 12 * n}, {guides->depth, 4 * n}, {guides->normal, 12 * n}, {guides->hit_kind, 4 * n}, {guides->elem_idx, 4 * n},
         {hist ? hist->hdr : nullptr, 12 * n}, {hv ? hist->var : nullptr, 12 * n}, {hist ? hist->length : nullptr, 4 * n},
         {hist ? hist->guides.depth : nullptr, 4 * n}, {hist ? hist->guides.normal : nullptr, 12 * n},
-        {hist ? hist->guides.hit_kind : nullptr, 4 * n}, {hist ? hist->guides.elem_idx : nullptr, 4 * n}};
+        {hist ? hist->guides.hit_kind : nullptr, 4 * n}, {hist ? hist->guides.elem_idx : nullptr, 4 * n},
+        {with_motion ? mo->motion : nullptr, 8 * n}, {with_motion ? mo->prev_dist : nullptr, 4 * n}};
     const struct { void* p; size_t b; } out[3] = {{hdr_out, 12 * n}, {var_out, 12 * n}, {len_out, 4 * n}};
     for (int o = 0; o < 3; ++o) {
         for (const auto& i : in)
@@ -755,9 +768,10 @@ static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float*
         a.same_cam = memcmp(cam, &hist->cam, sizeof(rbrt_camera)) == 0;
         a.prev = make_cam(hist->cam);
     }
-    const void** dst[13] = {(const void**)&a.hdr, (const void**)&a.var, (const void**)&a.depth, (const void**)&a.normal, (const void**)&a.kind,
+    const void** dst[15] = {(const void**)&a.hdr, (const void**)&a.var, (const void**)&a.depth, (const void**)&a.normal, (const void**)&a.kind,
                             (const void**)&a.elem, (const void**)&a.h_hdr, (const void**)&a.h_var, (const void**)&a.h_len,
-                            (const void**)&a.h_depth, (const void**)&a.h_normal, (const void**)&a.h_kind, (const void**)&a.h_elem};
+                            (const void**)&a.h_depth, (const void**)&a.h_normal, (const void**)&a.h_kind, (const void**)&a.h_elem,
+                            (const void**)&a.motion, (const void**)&a.prev_dist};
     DeviceCache& c = g_cache[dev & 63];
     if (stats) { int rc = timing_events(c); if (rc) return rc; }
     if (host) {                                                           // inputs and outputs carved from the staging block
@@ -766,7 +780,7 @@ static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float*
         for (const auto& o : out) if (o.p) need += a256(o.b);
         char* p = nullptr;
         { int rc = staging_block(c, need, &p); if (rc) return rc; }
-        for (int k = 0; k < 13; ++k) {
+        for (int k = 0; k < 15; ++k) {
             if (!in[k].p) continue;
             CKA(cudaMemcpyAsync(p, in[k].p, in[k].b, cudaMemcpyHostToDevice, st));
             *dst[k] = p; p += a256(in[k].b);
@@ -775,7 +789,7 @@ static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float*
         if (var_out) { a.var_out = (float*)p; p += a256(12 * n); }
         if (len_out) a.len_out = (float*)p;
     } else {
-        for (int k = 0; k < 13; ++k) *dst[k] = in[k].p;
+        for (int k = 0; k < 15; ++k) *dst[k] = in[k].p;
         a.hdr_out = hdr_out; a.var_out = var_out; a.len_out = len_out;
     }
     if (stats) CKA(cudaEventRecord(c.e0, st));
@@ -795,6 +809,111 @@ static int temporal(uint32_t W, uint32_t H, const rbrt_camera* cam, const float*
     if (stats) {
         CKA(cudaEventSynchronize(c.e1));
         float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
+        stats->ms_device = ms; stats->launches = 1;
+        stats->ms_total = now_ms() - t0;
+    }
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ per-object motion vectors (rbrt_gpu_scene_snapshot, rbrt_gpu_render_motion*)
+// The snapshot block: 3 float4 per tested triangle slot of the scene (indexed tri_base + original index), one per element, 3 per
+// BasicTriangle.
+static size_t snapshot_tri_slots(const Scene& sc) {
+    size_t n = 0;
+    for (const MeshDev& m : sc.meshes_h) n = std::max(n, (size_t)m.tri_base + m.n_tris);
+    return n;
+}
+static size_t snapshot_bytes(const Scene& sc) { return a256(48 * snapshot_tri_slots(sc)) + a256(16ull * sc.n_elems) + a256(48ull * sc.n_etris); }
+static SnapshotDev snapshot_dev(const Scene& sc) {
+    SnapshotDev s;
+    s.tris = (float4*)sc.snap;
+    s.elems = (float4*)(sc.snap + a256(48 * snapshot_tri_slots(sc)));
+    s.etris = (float4*)((char*)s.elems + a256(16ull * sc.n_elems));
+    return s;
+}
+
+static int scene_snapshot(rbrt_scene* scene, cudaStream_t st) {
+    if (!scene) { set_error("null argument"); return RBRT_E_INVALID; }
+    Scene& sc = *reinterpret_cast<Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device
+    CKA(cudaSetDevice(rp.device));
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    rbrt_snapshot_launch_fn launch = nullptr;
+    { int rc = module_entry(g_motion_module, "rbrt_snapshot_launch", &launch); if (rc) return rc; }
+    if (!sc.snap) CKA(cudaMalloc((void**)&sc.snap, std::max(snapshot_bytes(sc), (size_t)256)));
+    { int rc = ensure_event(&sc.snap_ev); if (rc) return rc; }
+    int smc = 148;
+    { int rc = device_sm_count(rp.device, &smc); if (rc) return rc; }
+    SnapshotArgs a;
+    a.S = rp.dev; a.snap = snapshot_dev(sc); a.blocks = (uint32_t)smc * 4;
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    wait_scene_uses(sc, rp.device, st);                                   // and every read enqueued so far: motion calls may still read the block
+    CKA((cudaError_t)launch(&a, st));
+    CKA(cudaEventRecord(sc.snap_ev, st));                                 // motion calls from now on read this snapshot
+    note_scene_use(sc, rp.device, st);                                    // later updates wait for it
+    return RBRT_OK;
+}
+
+static int render_motion(const rbrt_scene* scene, const rbrt_camera* cam, const rbrt_camera* prev, const rbrt_motion_out* out, bool host,
+                         cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!scene || !cam || !prev || !out) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!out->motion && !out->prev_dist) { set_error("no output requested (motion and prev_dist are both NULL)"); return RBRT_E_INVALID; }
+    const uint32_t W = cam->img_width_pix, H = cam->img_height_pix;
+    const size_t n = (size_t)W * H;
+    if (!n) { set_error("empty image"); return RBRT_E_INVALID; }
+    if (n > 0x7FFFFFFFull) { set_error("image too large"); return RBRT_E_INVALID; }
+    if (prev->img_width_pix != W || prev->img_height_pix != H) { set_error("prev_cam's image is not %u x %u", W, H); return RBRT_E_INVALID; }
+    if (overlap(out->motion, 8 * n, out->prev_dist, 4 * n)) { set_error("motion and prev_dist overlap"); return RBRT_E_INVALID; }
+    const Scene& sc = *reinterpret_cast<const Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device, whole image
+    CKA(cudaSetDevice(rp.device));
+    if (!host) {
+        int rc = check_usable_on({out->motion, out->prev_dist}, rp.device, "planes must be device memory on the scene's device %d");
+        if (rc) return rc;
+    }
+    rbrt_motion_launch_fn launch = nullptr;
+    { int rc = module_entry(g_motion_module, "rbrt_motion_launch", &launch); if (rc) return rc; }
+    if (!sc.snap_ev) { set_error("the scene has no snapshot (rbrt_gpu_scene_snapshot)"); return RBRT_E_INVALID; }
+    const double t0 = now_ms();
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+
+    static_assert((int)MV_ST_COUNT <= (int)AOV_ST_COUNT, "the motion counters live in the AOV counter block");
+    DeviceCache& c = g_cache[rp.device & 63];
+    MotionArgs a;
+    memset(&a, 0, sizeof(a));
+    a.S = rp.dev; a.snap = snapshot_dev(sc); a.cam = make_cam(*cam); a.prev = make_cam(*prev);
+    a.tiles_x = (W + 7) / 8; a.tiles_total = a.tiles_x * ((H + 3) / 4);
+    a.out = *out;
+    if (host) {                                                           // the requested planes, carved from the staging block
+        char* p = nullptr;
+        { int rc = staging_block(c, (out->motion ? a256(8 * n) : 0) + (out->prev_dist ? a256(4 * n) : 0), &p); if (rc) return rc; }
+        if (out->motion) { a.out.motion = (float*)p; p += a256(8 * n); }
+        if (out->prev_dist) a.out.prev_dist = (float*)p;
+    }
+    if (stats) {
+        if (!c.aov_ctr) CKA(cudaMalloc(&c.aov_ctr, 8 * AOV_ST_COUNT));
+        { int rc = timing_events(c); if (rc) return rc; }
+        a.stats = c.aov_ctr;
+    }
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    CKA(cudaStreamWaitEvent(st, sc.snap_ev, 0));                          // and the latest snapshot
+    if (stats) { CKA(cudaMemsetAsync(c.aov_ctr, 0, 8 * AOV_ST_COUNT, st)); CKA(cudaEventRecord(c.e0, st)); }
+    CKA((cudaError_t)launch(&a, st));
+    if (stats) CKA(cudaEventRecord(c.e1, st));
+    note_scene_use(sc, rp.device, st);                                    // later updates and snapshots wait for this read
+    if (!host && !stats) return RBRT_OK;                                  // enqueue only
+
+    if (host) {
+        if (out->motion) CKA(cudaMemcpyAsync(out->motion, a.out.motion, 8 * n, cudaMemcpyDeviceToHost, st));
+        if (out->prev_dist) CKA(cudaMemcpyAsync(out->prev_dist, a.out.prev_dist, 4 * n, cudaMemcpyDeviceToHost, st));
+    }
+    CKA(cudaStreamSynchronize(st));
+    if (stats) {
+        unsigned long long h[MV_ST_COUNT];
+        CKA(cudaMemcpy(h, c.aov_ctr, sizeof(h), cudaMemcpyDeviceToHost));
+        float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
+        stats->rays = n; stats->nan_rays = h[MV_ST_NAN]; stats->node_visits = h[MV_ST_NODES]; stats->tri_tests = h[MV_ST_TRIS];
         stats->ms_device = ms; stats->launches = 1;
         stats->ms_total = now_ms() - t0;
     }
@@ -1394,7 +1513,7 @@ int rbrt_gpu_temporal_accumulate(uint32_t width, uint32_t height, const rbrt_cam
                                  const rbrt_aov_out* guides, const rbrt_temporal_history* history, const rbrt_temporal_opts* opts,
                                  float* hdr_out, float* var_out, float* len_out, rbrt_stats* stats) {
     LOCK;
-    return temporal(width, height, cam, hdr, var, guides, history, opts, hdr_out, var_out, len_out, true, 0, stats);
+    return temporal(width, height, cam, hdr, var, guides, history, nullptr, false, opts, hdr_out, var_out, len_out, true, 0, stats);
 }
 
 int rbrt_gpu_temporal_accumulate_device(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* d_hdr, const float* d_var,
@@ -1402,8 +1521,41 @@ int rbrt_gpu_temporal_accumulate_device(uint32_t width, uint32_t height, const r
                                         const rbrt_temporal_opts* opts, float* d_hdr_out, float* d_var_out, float* d_len_out,
                                         void* cuda_stream, rbrt_stats* stats) {
     LOCK;
-    return temporal(width, height, cam, d_hdr, d_var, d_guides, d_history, opts, d_hdr_out, d_var_out, d_len_out, false,
+    return temporal(width, height, cam, d_hdr, d_var, d_guides, d_history, nullptr, false, opts, d_hdr_out, d_var_out, d_len_out, false,
                     (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_temporal_accumulate_motion(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* hdr, const float* var,
+                                        const rbrt_aov_out* guides, const rbrt_temporal_history* history, const rbrt_motion_out* motion,
+                                        const rbrt_temporal_opts* opts, float* hdr_out, float* var_out, float* len_out, rbrt_stats* stats) {
+    LOCK;
+    return temporal(width, height, cam, hdr, var, guides, history, motion, true, opts, hdr_out, var_out, len_out, true, 0, stats);
+}
+
+int rbrt_gpu_temporal_accumulate_motion_device(uint32_t width, uint32_t height, const rbrt_camera* cam, const float* d_hdr, const float* d_var,
+                                               const rbrt_aov_out* d_guides, const rbrt_temporal_history* d_history,
+                                               const rbrt_motion_out* d_motion, const rbrt_temporal_opts* opts, float* d_hdr_out,
+                                               float* d_var_out, float* d_len_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return temporal(width, height, cam, d_hdr, d_var, d_guides, d_history, d_motion, true, opts, d_hdr_out, d_var_out, d_len_out, false,
+                    (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_scene_snapshot(rbrt_scene* scene, void* cuda_stream) {
+    LOCK;
+    return scene_snapshot(scene, (cudaStream_t)cuda_stream);
+}
+
+int rbrt_gpu_render_motion(const rbrt_scene* scene, const rbrt_camera* cam, const rbrt_camera* prev_cam, const rbrt_motion_out* out,
+                           rbrt_stats* stats) {
+    LOCK;
+    return render_motion(scene, cam, prev_cam, out, true, 0, stats);
+}
+
+int rbrt_gpu_render_motion_device(const rbrt_scene* scene, const rbrt_camera* cam, const rbrt_camera* prev_cam, const rbrt_motion_out* d_out,
+                                  void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return render_motion(scene, cam, prev_cam, d_out, false, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_scatter(const rbrt_scatter_in* items, uint64_t n, uint64_t seed, rbrt_scatter_out* out) {

@@ -79,6 +79,10 @@ struct Scene {
     struct Staging { void* p = nullptr; size_t bytes = 0; cudaEvent_t done = nullptr; };
     Staging stage[2];                       // pinned host staging of element / material values, alternating; `done`: its copy has run
     int stage_next = 0;
+    // ---- rbrt_gpu_scene_snapshot: the geometry of "the previous frame" on replica 0's device (api.cu, snapshot_dev), allocated on the
+    // first snapshot; snap_ev is recorded behind the latest snapshot, and every motion call waits for it
+    char* snap = nullptr;
+    cudaEvent_t snap_ev = nullptr;
 };
 int resolve_scene_info(const Scene& sc, bool wait);   // api.cu: fills info from the build results once they are there (wait: block for them); returns RBRT_E_* if the build refused a mesh
 void wait_scene_ready(const Scene& sc, int li, cudaStream_t st);   // makes `st` wait for replica li's data

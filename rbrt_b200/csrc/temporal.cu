@@ -1,6 +1,7 @@
 // temporal.cu — temporal accumulation of a frame sequence (rbrt_gpu_temporal_accumulate*): each pixel's history, aligned to the previous
 // camera, is reprojected through that camera, resampled from the bilinear taps whose depth, normal and hit ids agree with the pixel, and
-// blended with the current frame in colour, variance and history length.
+// blended with the current frame in colour, variance and history length.  The motion variant reprojects along the frame's per-object
+// motion pass (motion.cu) where that is finite.
 //
 // Built into its own shared object (librbrt_gpu_temporal.so), which librbrt_gpu.so loads at run time like the other device modules: the
 // device code of librbrt_gpu.so stays exactly the build the GPU tests verified.  The per-pixel arithmetic is temporal.cuh's, so the kernel

@@ -25,8 +25,8 @@ __host__ __device__ __forceinline__ f3 tp_sub(f3 a, f3 b) { return mk3(XSUB(a.x,
 __host__ __device__ __forceinline__ f3 tp_v(const float* v) { return mk3(v[0], v[1], v[2]); }
 __host__ __device__ __forceinline__ f3 tp_load3(const float* a, size_t p) { return mk3(a[3 * p], a[3 * p + 1], a[3 * p + 2]); }
 
-// The world point of pixel (x, y) at depth z: pos + z * d, d = camera_ray's direction (shade.cuh) with both jitter draws at 0.5.
-__host__ __device__ __forceinline__ f3 tp_world_point(const CamDev& c, uint32_t x, uint32_t y, float z) {
+// The direction of pixel (x, y)'s centre ray: camera_ray's direction (shade.cuh) with both jitter draws at 0.5, v / |v| per component.
+__host__ __device__ __forceinline__ f3 tp_pixel_dir(const CamDev& c, uint32_t x, uint32_t y) {
     const float col_off = XSUB((float)x, (float)(c.width / 2));
     const float row_off = XSUB((float)y, (float)(c.height / 2));
     const float col_mm = XMUL(XSUB(XADD(col_off, 0.5f), 0.5f), c.mm_per_pix_hor);
@@ -37,7 +37,13 @@ __host__ __device__ __forceinline__ f3 tp_world_point(const CamDev& c, uint32_t 
                      XSUB(XADD(c.center[2], XMUL(ch, c.right[2])), XMUL(cv, c.up[2])));
     const f3 v = tp_sub(t, tp_v(c.pos));
     const float l = XSQRT(tp_dot(v, v));
-    return mk3(XADD(c.pos[0], XMUL(z, XDIV(v.x, l))), XADD(c.pos[1], XMUL(z, XDIV(v.y, l))), XADD(c.pos[2], XMUL(z, XDIV(v.z, l))));
+    return mk3(XDIV(v.x, l), XDIV(v.y, l), XDIV(v.z, l));
+}
+
+// The world point of pixel (x, y) at depth z: pos + z * d, d = tp_pixel_dir.
+__host__ __device__ __forceinline__ f3 tp_world_point(const CamDev& c, uint32_t x, uint32_t y, float z) {
+    const f3 d = tp_pixel_dir(c, x, y);
+    return mk3(XADD(c.pos[0], XMUL(z, d.x)), XADD(c.pos[1], XMUL(z, d.y)), XADD(c.pos[2], XMUL(z, d.z)));
 }
 
 // X projected into camera c: the continuous pixel coordinates (*px, *py), integers at pixel centres.  Solves
@@ -81,51 +87,13 @@ struct TemporalArgs {
     float* hdr_out;              // W*H*3 or NULL
     float* var_out;              // W*H*3 or NULL
     float* len_out;              // W*H or NULL
+    const float* motion;         // motion variant: W*H*2, the frame's motion pass against prev and the history's snapshot
+    const float* prev_dist;      // motion variant: W*H
 };
 
-// Pixel (x, y):
-//  1. p is VALID when its colour and depth are finite and, with a variance, each component of it is finite and >= 0 (-0 is).  An
-//     invalid p gives (hdr, var, 0).
-//  2. Without a history, or when the reprojection below finds none: (hdr, var, 1).
-//  3. X = tp_world_point(cam, x, y, z_p); D = X - prev.pos; r = sqrt(D . D).  There is no history when r is not finite, when
-//     tp_project fails or gives a non-finite coordinate, or when the point lies outside [0, W-1] x [0, H-1] (the borders are inside).
-//     same_cam: (px, py) = (x, y) exactly and tp_project is not called.
-//  4. x0 = floor(px), fx = px - x0 (likewise y); taps (x0, y0), (x0+1, y0), (x0, y0+1), (x0+1, y0+1) in that order with the bilinear
-//     weights (1-fx)*(1-fy), fx*(1-fy), (1-fx)*fy, fx*fy.  A tap q is skipped when its weight is 0, when it lies outside the image,
-//     and unless it is CONSISTENT: length_q > 0, hit_kind_q == hit_kind_p, elem_idx_q == elem_idx_p, |z_q - r| <= σ_z * r and
-//     n_p . n_q >= n_min * (|n_p| * |n_q|) (tp_dot, |n| = sqrt(n . n): the AOV normals are means, not unit vectors).  Σw, Σ w*c_q,
-//     Σ (w*w)*v_q and Σ w*length_q are sums from +0 in tap order.  Σw < TP_MIN_WEIGHT: no history.  c_h = Σ w*c_q / Σw, v_h = Σ (w*w)*v_q / (Σw * Σw), n_h = Σ w*length_q / Σw.
-//  5. α = max(1 / (n_h + 1), α_min); out = c_h + α * (c - c_h); var_out = ((1-α)*(1-α)) * v_h + (α*α) * v; len_out = n_h + 1.
-// v takes part in the validity when var is given; v_h and var_out are formed only when h_var is given (var_out requested with a history).
-__host__ __device__ __forceinline__ void tp_pixel(const TemporalArgs& A, uint32_t x, uint32_t y, f3* out, f3* vout, float* lout) {
-    const size_t p = (size_t)y * A.W + x;
-    const f3 c = tp_load3(A.hdr, p);
-    const f3 v = A.var ? tp_load3(A.var, p) : mk3(0.0f, 0.0f, 0.0f);
-    const float z = A.depth[p];
-    *out = c;
-    *vout = v;
-    const bool valid = dn_finite(c.x) && dn_finite(c.y) && dn_finite(c.z) && dn_finite(z) &&
-                       (!A.var || (v.x >= 0.0f && dn_finite(v.x) && v.y >= 0.0f && dn_finite(v.y) && v.z >= 0.0f && dn_finite(v.z)));
-    if (!valid) { *lout = 0.0f; return; }
-    *lout = 1.0f;
-    if (!A.history) return;
-
-    const f3 X = tp_world_point(A.cam, x, y, z);
-    const f3 D = tp_sub(X, tp_v(A.prev.pos));
-    const float r = XSQRT(tp_dot(D, D));
-    if (!dn_finite(r)) return;
-    uint32_t x0, y0;
-    float fx, fy;
-    if (A.same_cam) {
-        x0 = x; y0 = y; fx = 0.0f; fy = 0.0f;
-    } else {
-        float px, py;
-        if (!tp_project(A.prev, D, &px, &py)) return;
-        if (!(px >= 0.0f && px <= (float)(A.W - 1) && py >= 0.0f && py <= (float)(A.H - 1))) return;   // (NaN fails too)
-        const float fx0 = floorf(px), fy0 = floorf(py);
-        x0 = (uint32_t)fx0; y0 = (uint32_t)fy0;
-        fx = XSUB(px, fx0); fy = XSUB(py, fy0);
-    }
+// Steps 4 and 5 for a valid pixel p with a history: the taps around (x0 + fx, y0 + fy), their consistency with depth r, and the blend.
+__host__ __device__ __forceinline__ void tp_resample(const TemporalArgs& A, size_t p, f3 c, f3 v, float r, uint32_t x0, uint32_t y0, float fx,
+                                                     float fy, f3* out, f3* vout, float* lout) {
     const f3 n = tp_load3(A.normal, p);
     const float ln = XSQRT(tp_dot(n, n));
     const int32_t kp = A.kind[p];
@@ -167,6 +135,66 @@ __host__ __device__ __forceinline__ void tp_pixel(const TemporalArgs& A, uint32_
                     XADD(XMUL(k1, XDIV(sv2, sw2)), XMUL(k2, v.z)));
     }
     *lout = XADD(nh, 1.0f);
+}
+
+// Pixel (x, y):
+//  1. p is VALID when its colour and depth are finite and, with a variance, each component of it is finite and >= 0 (-0 is).  An
+//     invalid p gives (hdr, var, 0).
+//  2. Without a history, or when the reprojection below finds none: (hdr, var, 1).
+//  3. X = tp_world_point(cam, x, y, z_p); D = X - prev.pos; r = sqrt(D . D).  There is no history when r is not finite, when
+//     tp_project fails or gives a non-finite coordinate, or when the point lies outside [0, W-1] x [0, H-1] (the borders are inside).
+//     same_cam: (px, py) = (x, y) exactly and tp_project is not called.
+//     With motion planes (rbrt_gpu_temporal_accumulate_motion*): when both components of m = motion[p] are finite, (px, py) = (x + m.x, y + m.y) and
+//     r = prev_dist[p] instead, with the same tests on r and on the bounds; otherwise step 3 as above.
+//  4. x0 = floor(px), fx = px - x0 (likewise y); taps (x0, y0), (x0+1, y0), (x0, y0+1), (x0+1, y0+1) in that order with the bilinear
+//     weights (1-fx)*(1-fy), fx*(1-fy), (1-fx)*fy, fx*fy.  A tap q is skipped when its weight is 0, when it lies outside the image,
+//     and unless it is CONSISTENT: length_q > 0, hit_kind_q == hit_kind_p, elem_idx_q == elem_idx_p, |z_q - r| <= σ_z * r and
+//     n_p . n_q >= n_min * (|n_p| * |n_q|) (tp_dot, |n| = sqrt(n . n): the AOV normals are means, not unit vectors).  Σw, Σ w*c_q,
+//     Σ (w*w)*v_q and Σ w*length_q are sums from +0 in tap order.  Σw < TP_MIN_WEIGHT: no history.  c_h = Σ w*c_q / Σw, v_h = Σ (w*w)*v_q / (Σw * Σw), n_h = Σ w*length_q / Σw.
+//  5. α = max(1 / (n_h + 1), α_min); out = c_h + α * (c - c_h); var_out = ((1-α)*(1-α)) * v_h + (α*α) * v; len_out = n_h + 1.
+// v takes part in the validity when var is given; v_h and var_out are formed only when h_var is given (var_out requested with a history).
+__host__ __device__ __forceinline__ void tp_pixel(const TemporalArgs& A, uint32_t x, uint32_t y, f3* out, f3* vout, float* lout) {
+    const size_t p = (size_t)y * A.W + x;
+    const f3 c = tp_load3(A.hdr, p);
+    const f3 v = A.var ? tp_load3(A.var, p) : mk3(0.0f, 0.0f, 0.0f);
+    const float z = A.depth[p];
+    *out = c;
+    *vout = v;
+    const bool valid = dn_finite(c.x) && dn_finite(c.y) && dn_finite(c.z) && dn_finite(z) &&
+                       (!A.var || (v.x >= 0.0f && dn_finite(v.x) && v.y >= 0.0f && dn_finite(v.y) && v.z >= 0.0f && dn_finite(v.z)));
+    if (!valid) { *lout = 0.0f; return; }
+    *lout = 1.0f;
+    if (!A.history) return;
+
+    float r;
+    uint32_t x0, y0;
+    float fx, fy;
+    const float mx = A.motion ? A.motion[2 * p] : 0.0f, my = A.motion ? A.motion[2 * p + 1] : 0.0f;
+    if (A.motion && dn_finite(mx) && dn_finite(my)) {
+        r = A.prev_dist[p];
+        if (!dn_finite(r)) return;
+        const float px = XADD((float)x, mx), py = XADD((float)y, my);
+        if (!(px >= 0.0f && px <= (float)(A.W - 1) && py >= 0.0f && py <= (float)(A.H - 1))) return;
+        const float fx0 = floorf(px), fy0 = floorf(py);
+        x0 = (uint32_t)fx0; y0 = (uint32_t)fy0;
+        fx = XSUB(px, fx0); fy = XSUB(py, fy0);
+    } else {
+        const f3 X = tp_world_point(A.cam, x, y, z);
+        const f3 D = tp_sub(X, tp_v(A.prev.pos));
+        r = XSQRT(tp_dot(D, D));
+        if (!dn_finite(r)) return;
+        if (A.same_cam) {
+            x0 = x; y0 = y; fx = 0.0f; fy = 0.0f;
+        } else {
+            float px, py;
+            if (!tp_project(A.prev, D, &px, &py)) return;
+            if (!(px >= 0.0f && px <= (float)(A.W - 1) && py >= 0.0f && py <= (float)(A.H - 1))) return;   // (NaN fails too)
+            const float fx0 = floorf(px), fy0 = floorf(py);
+            x0 = (uint32_t)fx0; y0 = (uint32_t)fy0;
+            fx = XSUB(px, fx0); fy = XSUB(py, fy0);
+        }
+    }
+    tp_resample(A, p, c, v, r, x0, y0, fx, fy, out, vout, lout);
 }
 
 }  // namespace rbrt

@@ -335,8 +335,9 @@ def _temporal_plane(what, v, H, W, k, dtype, device):
     return v.data_ptr() if device else v.ctypes.data
 
 
-def _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, device, outs, stream=None, stats=None):
-    """temporal_accumulate (numpy) and, with device=True, temporal_accumulate_device; outs = (hdr_out, var_out, len_out) or None."""
+def _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, device, outs, stream=None, stats=None, motion=None):
+    """temporal_accumulate (numpy) and, with device=True, temporal_accumulate_device; outs = (hdr_out, var_out, len_out) or None.
+    motion: None, or (motion [H,W,2], prev_dist [H,W]) of render_motion*: the _motion variants."""
     W, H = cam.img_width_pix, cam.img_height_pix
     if var is not None and history is not None and history.get("var") is None:
         raise ValueError("with var, the history needs the var it returned")
@@ -367,28 +368,69 @@ def _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, 
             outs = (np.empty((H, W, 3), np.float32), np.empty((H, W, 3), np.float32) if var is not None else None, np.empty((H, W), np.float32))
     optr = [ptr("hdr_out", outs[0]), ptr("var_out", outs[1]) if outs[1] is not None else None, ptr("len_out", outs[2], 1)]
     lib = _abi.lib()
+    mo = None if motion is None else _abi.MotionOutC(ptr("motion", motion[0], 2), ptr("prev_dist", motion[1], 1))
     if device:
-        _abi.check(lib.rbrt_gpu_temporal_accumulate_device(W, H, cam.to_c(), *planes, g, h, opts, *optr, stream.cuda_stream, None))
+        if mo is None:
+            _abi.check(lib.rbrt_gpu_temporal_accumulate_device(W, H, cam.to_c(), *planes, g, h, opts, *optr, stream.cuda_stream, None))
+        else:
+            _abi.check(lib.rbrt_gpu_temporal_accumulate_motion_device(W, H, cam.to_c(), *planes, g, h, mo, opts, *optr, stream.cuda_stream,
+                                                                      None))
     else:
         st = _abi.StatsC()
-        _abi.check(lib.rbrt_gpu_temporal_accumulate(W, H, cam.to_c(), *planes, g, h, opts, *optr, st))
+        if mo is None:
+            _abi.check(lib.rbrt_gpu_temporal_accumulate(W, H, cam.to_c(), *planes, g, h, opts, *optr, st))
+        else:
+            _abi.check(lib.rbrt_gpu_temporal_accumulate_motion(W, H, cam.to_c(), *planes, g, h, mo, opts, *optr, st))
         if stats is not None:
             stats.update(st.as_dict())
     return outs
 
 
-def temporal_accumulate(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stats=None):
+def temporal_accumulate(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stats=None, motion=None):
     """Fold the frame hdr [H,W,3] (with its variance var [H,W,3], optional) rendered at camera `cam` into a history: each pixel's
     history is reprojected through the previous camera and blended with the frame where depth, normal and sample 0's hit ids agree.
     aovs: render_aovs planes of the same camera and seed with depth, normal, hit_kind and elem_idx.  history: None for the first frame,
     else a dict with the previous call's results and inputs: cam, hdr, var (with var), length and aovs.  Returns (hdr_out, var_out or
-    None, length [H,W]) numpy float32 arrays; blocks until they are on the host."""
-    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, False, None, stats=stats)
+    None, length [H,W]) numpy float32 arrays; blocks until they are on the host.  motion: (motion, prev_dist) of render_motion for cam
+    against the history's camera and the snapshot taken at the history's frame: each pixel is reprojected along its motion where
+    that is finite (moving objects keep their history), through the cameras otherwise."""
+    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, False, None, stats=stats, motion=motion)
 
 
-def temporal_accumulate_device(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stream=None):
-    """The same on CUDA tensors of the current render device (render_aovs_device's planes): returns (hdr_out, var_out or None, length)
-    tensors, enqueued on `stream` (default: the current stream) without synchronising."""
+def temporal_accumulate_device(cam, hdr, aovs, var=None, history=None, alpha_min=0.1, sigma_depth=0.02, normal_min=0.9, stream=None,
+                               motion=None):
+    """The same on CUDA tensors of the current render device (render_aovs_device's planes; motion: render_motion_device's): returns
+    (hdr_out, var_out or None, length) tensors, enqueued on `stream` (default: the current stream) without synchronising."""
     import torch
     stream = stream or torch.cuda.current_stream()
-    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, True, None, stream=stream)
+    return _temporal(cam, hdr, var, aovs, history, alpha_min, sigma_depth, normal_min, True, None, stream=stream, motion=motion)
+
+
+# ---- per-object motion vectors (rbrt_gpu_render_motion*; include/rbrt_gpu.h and DESIGN.md section 16) -------------------------------
+def render_motion(cam, prev_cam, scene, stats=None):
+    """Per pixel of cam's image, the screen motion [H,W,2] f32 from the pixel-centre ray's hit in cam to where that surface point was
+    in prev_cam at the scene's latest snapshot (Scene.snapshot), and the distance [H,W] f32 from prev_cam's position to that previous
+    point; (NaN, NaN) and +inf for a miss.  Returns (motion, prev_dist); blocks until they are on the host."""
+    W, H = cam.img_width_pix, cam.img_height_pix
+    motion = np.empty((H, W, 2), dtype=np.float32)
+    prev_dist = np.empty((H, W), dtype=np.float32)
+    st = _abi.StatsC()
+    _abi.check(_abi.lib().rbrt_gpu_render_motion(scene.handle(), cam.to_c(), prev_cam.to_c(), _abi.MotionOutC(motion.ctypes.data, prev_dist.ctypes.data),
+                                                 st))
+    if stats is not None:
+        stats.update(st.as_dict())
+    return motion, prev_dist
+
+
+def render_motion_device(cam, prev_cam, scene, stream=None):
+    """The same as CUDA tensors on the scene's first device, enqueued on `stream` (default: the current stream) without synchronising."""
+    import torch
+    stream = stream or torch.cuda.current_stream()
+    W, H = cam.img_width_pix, cam.img_height_pix
+    handle = scene.handle()
+    with torch.cuda.stream(stream):
+        motion = torch.empty((H, W, 2), dtype=torch.float32, device=stream.device)
+        prev_dist = torch.empty((H, W), dtype=torch.float32, device=stream.device)
+    _abi.check(_abi.lib().rbrt_gpu_render_motion_device(handle, cam.to_c(), prev_cam.to_c(),
+                                                        _abi.MotionOutC(motion.data_ptr(), prev_dist.data_ptr()), stream.cuda_stream, None))
+    return motion, prev_dist

@@ -138,6 +138,12 @@ class Scene:
             _abi.check(_abi.lib().rbrt_gpu_scene_update_elements(self._handle, order, ne, spheres, ns, tris, nt))
         self.elements = elements
 
+    # ---- motion vectors (rbrt_gpu_scene_snapshot, DESIGN.md section 16) ---------------------------
+    def snapshot(self, stream=None):
+        """Record the scene's current geometry as "the previous frame" of render_motion*, enqueued on `stream` (a torch.cuda.Stream;
+        default: the legacy default stream).  It sees every update made before it; later updates wait for it."""
+        _abi.check(_abi.lib().rbrt_gpu_scene_snapshot(self.handle(), stream.cuda_stream if stream is not None else None))
+
     # ---- Scene::hit (scene.rs:19-43) for caller-supplied rays ----------------------------------
     def hit(self, rays, trace_mode=_abi.TRACE_BVH, stats=None):
         """rays: [N,6] f32 (origin xyz, direction xyz). Returns a structured array (HIT_DTYPE)."""

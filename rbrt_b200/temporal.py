@@ -10,6 +10,7 @@ camera and guides.
         hdr, var = render_hdr_variance_device(cam, spp, scene, splits=4, seed=seed)
         aovs = render_aovs_device(cam, aov_spp, scene, seed=seed, passes=("depth", "normal", "ids"))
         hdr_t, var_t, length = acc.step(cam, hdr, var, aovs)      # valid until the step after next
+                                                                  # (motion=render_motion_device(cam, acc.camera, scene): per-object motion)
         out, _ = denoise_variance_device(hdr_t, var_t, {**aovs, **albedo}, ...)
 
 The returned tensors are the accumulator's own: they are overwritten two steps later, so clone what must outlive that.
@@ -41,10 +42,16 @@ class TemporalAccumulator:
         self._next ^= 1
         return s
 
-    def step(self, cam, hdr, var, aovs):
+    @property
+    def camera(self):
+        """The history's camera (None before the first step or after reset): the prev_cam of the next frame's render_motion*."""
+        return self._history["cam"] if self._history is not None else None
+
+    def step(self, cam, hdr, var, aovs, motion=None):
         """Fold the frame at camera `cam` (hdr, var [H,W,3] CUDA tensors, var may be None; aovs with depth, normal, hit_kind and
-        elem_idx) into the history.  Returns (hdr, var or None, length) tensors, enqueued on the accumulator's stream (default: the
-        current stream)."""
+        elem_idx) into the history.  motion: None, or (motion, prev_dist) of render_motion_device for cam against the history's camera
+        and the snapshot taken at the history's frame; the history is then reprojected along each pixel's motion where it is finite.
+        Returns (hdr, var or None, length) tensors, enqueued on the accumulator's stream (default: the current stream)."""
         import torch
         if (cam.img_width_pix, cam.img_height_pix) != (self.width, self.height):
             raise ValueError(f"the camera's image is {cam.img_width_pix} x {cam.img_height_pix}, the accumulator's {self.width} x {self.height}")
@@ -53,7 +60,7 @@ class TemporalAccumulator:
             self._history = None                                            # a change between with and without variance restarts
         with torch.cuda.stream(stream):
             outs = self._outputs(torch, var is not None, stream.device)
-        out = render._temporal(cam, hdr, var, aovs, self._history, **self.opts, device=True, outs=outs, stream=stream)
+        out = render._temporal(cam, hdr, var, aovs, self._history, **self.opts, device=True, outs=outs, stream=stream, motion=motion)
         guides = {k: aovs[k] for k in ("depth", "normal", "hit_kind", "elem_idx")}
         self._history = {"cam": cam, "hdr": out[0], "var": out[1], "length": out[2], "aovs": guides}
         return out
