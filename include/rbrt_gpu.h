@@ -452,6 +452,47 @@ int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_ra
                                    const float* d_max_dist,
                                    uint8_t* d_occluded, void* cuda_stream, rbrt_stats* stats);
 
+/* ---- nearest-surface queries on device memory (DESIGN.md section 17) ------------------------
+ * For each point p (n points, f32 xyz, contiguous) the nearest surface of the scene, as the scene stores it.  Each operation is one
+ * correctly rounded f32 operation, in the order rbrt_b200/csrc/point.cuh writes it.
+ *   Candidates: every element of Scene.elements, and every TESTED triangle of every mesh (the N_eff triangles of the tail rule, as
+ *   rbrt_scene_info.num_triangles_tested counts them; tail-dropped triangles are not candidates).
+ *     sphere {c, r}: the surface |x - c| = |r| (a negative radius is the same surface, r = 0 the point c);
+ *                    q = c + (p - c) * (|r| / |p - c|) per component, q = c + (|r|, 0, 0) when p = c; uv = (0, 0).
+ *     triangle (a BasicTriangle or a mesh triangle): the real triangle v0 + u*e1 + v*e2 (u, v >= 0, u + v <= 1) of its stored record
+ *                    {v0, e1 = b - a, e2 = c - a}; q and (u, v) by Ericson's ClosestPtPointTriangle on the record (point.cuh).  A degenerate
+ *                    record (cross(e1, e2) exactly 0: collinear vertices, a zero-length edge, three equal vertices) is the closest of its
+ *                    three segments: never NaN for finite inputs.
+ *     d2 = (dx*dx + dy*dy) + dz*dz with d = p - q.  A candidate whose d2 is not finite (NaN or inf values, overflow) is never recorded.
+ *   A candidate is ACCEPTED when sqrt(d2) < max_dist (strict; d_max_dist NULL = +inf; a NaN, zero or negative bound accepts nothing).
+ *   The winner is the accepted candidate with the least (d2, scene order): elements by index, then meshes in order, then original
+ *   triangle index within a mesh (the first minimum of a brute-force loop with a strict <).  The answer does not depend on the tree.
+ *   Planes for the winner: dist = sqrt(d2); point = q; normal as the ray query reports it at q (a sphere q - c un-normalised, a
+ *   BasicTriangle or mesh triangle its stored unit normal); uv = (u, v); kind, elem_idx, tri_idx as rbrt_query_out.  No accepted
+ *   candidate: kind = RBRT_HIT_NONE, dist = +inf, zeros elsewhere.  A point with a NaN coordinate is such a miss and is counted in
+ *   stats->nan_rays.  A point farther than about 1.8e19 from every surface overflows d2 and is a miss too.
+ * There is no signed distance: meshes are triangle soups without adjacency.
+ * Points, bounds and planes are DEVICE memory on the scene's first device.  Enqueued on cuda_stream (0 = default stream): stats == NULL
+ * returns without synchronising; with stats the call waits and fills rays (= n), nan_rays, node_visits, tri_tests, ms_device, ms_total
+ * and launches.  Ordered like a render: the call sees every update of the scene enqueued before it, and every later update waits for
+ * it.  Under a communicator it runs on replica 0 and is not collective.  n = 0 returns RBRT_OK, nothing written.
+ * The kernel lives in librbrt_gpu_point.so, loaded at run time from this library's directory (RBRT_GPU_POINT_LIB: another path);
+ * without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL scene, points or output with n > 0, every plane of the output NULL,
+ * n > 2^32 - 1, points, bounds or planes in another device's memory or in unregistered host memory, a scene with a mesh whose tree was
+ * refused as too deep. */
+typedef struct rbrt_nearest_out {    /* device planes, n entries each (point / normal: n*3, uv: n*2); NULL = not produced, not written */
+    float*    dist;
+    int32_t*  kind;                  /* RBRT_HIT_* */
+    uint32_t* elem_idx;
+    uint32_t* tri_idx;
+    float*    point;
+    float*    normal;
+    float*    uv;
+} rbrt_nearest_out;
+int rbrt_gpu_query_nearest_device(const rbrt_scene* scene, const float* d_points, uint64_t n, const float* d_max_dist,
+                                  const rbrt_nearest_out* d_out, void* cuda_stream, rbrt_stats* stats);
+
 /* ---- guided denoising (DESIGN.md section 13) -----------------------------------------------
  * An edge-aware à-trous filter of the HDR mean colour, guided by the first-hit AOVs of the same camera and seed (the spatial filter of
  * SVGF, Schied et al. 2017, without variance or temporal terms).  Inputs are row-major W x H planes: c = hdr (W*H*3, what
@@ -683,7 +724,7 @@ int rbrt_gpu_temporal_accumulate_motion_device(uint32_t width, uint32_t height, 
                                                float* d_var_out, float* d_len_out, void* cuda_stream, rbrt_stats* stats);
 
 /* The wavefront state (ray / hit / queue buffers, tens of GB at full batch size) is pooled per device and kept
- * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query counters, the
+ * between renders and across scenes; this releases it (and the pooled scene blocks, the build scratch, the query and nearest-surface counters, the
  * denoiser's host-call block and the variance call's internal stream). */
 int rbrt_gpu_release_cache(void);
 

@@ -44,6 +44,10 @@ pub struct RbrtAovOut { pub depth: *mut f32, pub normal: *mut f32, pub albedo: *
 #[repr(C)] #[derive(Copy, Clone, Debug)]
 pub struct RbrtQueryOut { pub t: *mut f32, pub dist: *mut f32, pub kind: *mut i32, pub elem_idx: *mut u32, pub tri_idx: *mut u32,
                           pub point: *mut f32, pub normal: *mut f32 }
+/// Nearest-surface planes in device memory (n values each; n*3 for point and normal, n*2 for uv); a null member is not produced.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtNearestOut { pub dist: *mut f32, pub kind: *mut i32, pub elem_idx: *mut u32, pub tri_idx: *mut u32, pub point: *mut f32,
+                            pub normal: *mut f32, pub uv: *mut f32 }
 /// Options of the guided denoiser (rbrt_gpu_denoise*); 0 = default (4 levels, at most 8).
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct RbrtDenoiseOpts { pub levels: u32, pub sigma_depth: f32, pub sigma_luminance: f32 }
@@ -149,6 +153,11 @@ extern "C" {
     /// RBRT_QUERY_NAN_RAY for a NaN ray, else RBRT_QUERY_CLEAR.
     pub fn rbrt_gpu_query_occluded_device(scene: *const RbrtScene, d_rays: *const RbrtRay, n: u64, d_max_dist: *const f32,
                                           d_occluded: *mut u8, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// The nearest surface of the scene to each point (n points, f32 xyz, in device memory): the least (d2, scene order) over every
+    /// element and every tested mesh triangle closer than d_max_dist (null = +inf, strict); enqueued on `stream` (stats = null: no
+    /// synchronisation).  Not collective: replica 0.
+    pub fn rbrt_gpu_query_nearest_device(scene: *const RbrtScene, d_points: *const f32, n: u64, d_max_dist: *const f32,
+                                         d_out: *const RbrtNearestOut, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     /// Edge-aware à-trous denoise of a render_hdr image guided by render_aov depth / normal / albedo of the same camera and seed; HOST
     /// pointers, blocks.  hdr_out (W*H*3 f32) and / or rgb_out (W*H*3 u8, k_finalize's tonemap); opts may be null.
     pub fn rbrt_gpu_denoise(width: u32, height: u32, hdr: *const f32, guides: *const RbrtAovOut, opts: *const RbrtDenoiseOpts,

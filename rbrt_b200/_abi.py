@@ -103,6 +103,11 @@ class QueryOutC(C.Structure):  # rbrt_query_out: device planes, NULL = not produ
                 ("point", C.c_void_p), ("normal", C.c_void_p)]
 
 
+class NearestOutC(C.Structure):  # rbrt_nearest_out: device planes, NULL = not produced
+    _fields_ = [("dist", C.c_void_p), ("kind", C.c_void_p), ("elem_idx", C.c_void_p), ("tri_idx", C.c_void_p), ("point", C.c_void_p),
+                ("normal", C.c_void_p), ("uv", C.c_void_p)]
+
+
 class DenoiseOptsC(C.Structure):  # rbrt_denoise_opts: 0 = default
     _fields_ = [("levels", C.c_uint32), ("sigma_depth", C.c_float), ("sigma_luminance", C.c_float)]
 
@@ -183,6 +188,7 @@ GPU_SIGNATURES = {
     "rbrt_gpu_render_aov_device": (C.c_int, [C.c_void_p, P(CameraC), C.c_uint32, C.c_uint64, P(AovOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_closest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, P(QueryOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_occluded_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_query_nearest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, P(NearestOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, C.c_void_p,
                                           P(StatsC)]),

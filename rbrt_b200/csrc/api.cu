@@ -15,6 +15,7 @@
 #include "engine.cuh"
 #include "multi.cuh"
 #include "query.cuh"
+#include "point.cuh"
 #include "update.cuh"
 #include "motion.cuh"
 #include "temporal.cuh"
@@ -239,7 +240,7 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
 // ------------------------------------------------------------------ device modules
 // The refit kernels (librbrt_gpu_update.so), the AOV kernel (librbrt_gpu_aov.so), the ray queries (librbrt_gpu_query.so), the denoiser
 // (librbrt_gpu_denoise.so), the variance kernels (librbrt_gpu_variance.so), the temporal accumulation (librbrt_gpu_temporal.so) and the
-// snapshot with the motion pass (librbrt_gpu_motion.so) live in their own device modules, loaded from this library's
+// snapshot with the motion pass (librbrt_gpu_motion.so) and the nearest-surface queries (librbrt_gpu_point.so) live in their own device modules, loaded from this library's
 // directory (or the path in the module's environment variable) on first use.  Without a module its calls are refused: there is no other
 // implementation.
 // Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
@@ -263,6 +264,7 @@ static Module g_denoise_module = {"RBRT_GPU_DENOISE_LIB", "librbrt_gpu_denoise.s
 static Module g_variance_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_variance.so", "variance", nullptr};
 static Module g_temporal_module = {"RBRT_GPU_TEMPORAL_LIB", "librbrt_gpu_temporal.so", "temporal", nullptr};
 static Module g_motion_module = {"RBRT_GPU_MOTION_LIB", "librbrt_gpu_motion.so", "motion", nullptr};
+static Module g_point_module = {"RBRT_GPU_POINT_LIB", "librbrt_gpu_point.so", "nearest-surface", nullptr};
 // The entry point `symbol` of module m, which is opened on first use.  A failed dlopen is not remembered: the next call tries again.
 template <class F> static int module_entry(Module& m, const char* symbol, F* fn) {
     if (!m.h) {
@@ -405,7 +407,8 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
 //  - The timing events of calls with stats (AOV, query, denoise, variance, temporal, motion).  Each such call waits for `e1` or its stream
 //    before returning.
 //  - The AOV counters, used by AOV and motion calls with stats.
-//  - The query ring: QRY_RING counter blocks (the ray cursor of the persistent kernel and the stats counters).  Each call takes the next
+//  - The query ring: QRY_RING counter blocks (the ray or point cursor of the persistent kernel and the stats counters), shared by the ray
+//    and the nearest-surface queries (query_ring_slot).  Each call takes the next
 //    block, zeroes it on its own stream and records `qry_used` behind its kernel, so calls on different streams never share a cursor.  A
 //    block is reused QRY_RING calls later; the host waits for its previous call only if that one has still not run by then.
 //  - The variance lane: an internal stream and the events that fork a call's shards onto it and join them back (render_variance).
@@ -538,6 +541,19 @@ static int render_aov(const rbrt_scene* scene, const rbrt_camera* cam, uint32_t 
 }
 
 // ------------------------------------------------------------------ ray queries on device memory (rbrt_gpu_query_*_device)
+// The next block of the device's query ring: QRY_ST_COUNT counters (the persistent kernel's cursor first) and the event the caller records
+// behind its kernel.  The block's previous call has run when this returns.
+static_assert((int)PT_ST_COUNT == (int)QRY_ST_COUNT && (int)PT_ST_HEAD == (int)QRY_ST_HEAD, "the nearest-surface query shares the ring's blocks");
+static int query_ring_slot(DeviceCache& c, unsigned long long** ctr, cudaEvent_t* used) {
+    if (!c.qry_ctr) CKA(cudaMalloc(&c.qry_ctr, 8ull * QRY_ST_COUNT * QRY_RING));
+    const uint32_t slot = c.qry_next++ % QRY_RING;
+    cudaEvent_t& e = c.qry_used[slot];
+    if (e) CKA(cudaEventSynchronize(e));
+    else CKA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    *ctr = c.qry_ctr + QRY_ST_COUNT * slot; *used = e;
+    return RBRT_OK;
+}
+
 // occ: an occlusion query into occluded[]; else a closest query into *out.
 static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool occ, const rbrt_query_out* out, const float* max_dist,
                  uint8_t* occluded, cudaStream_t st, rbrt_stats* stats) {
@@ -560,16 +576,13 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     { int rc = module_entry(g_query_module, "rbrt_query_launch", &launch); if (rc) return rc; }
 
     DeviceCache& c = g_cache[rp.device & 63];
-    if (!c.qry_ctr) CKA(cudaMalloc(&c.qry_ctr, 8ull * QRY_ST_COUNT * QRY_RING));
-    const uint32_t slot = c.qry_next++ % QRY_RING;
-    cudaEvent_t& used = c.qry_used[slot];
-    if (used) CKA(cudaEventSynchronize(used));
-    else CKA(cudaEventCreateWithFlags(&used, cudaEventDisableTiming));
+    unsigned long long* ctr = nullptr; cudaEvent_t used = nullptr;
+    { int rc = query_ring_slot(c, &ctr, &used); if (rc) return rc; }
     if (stats) { int rc = timing_events(c); if (rc) return rc; }
 
     QueryArgs a;
     memset(&a, 0, sizeof(a));
-    a.S = rp.dev; a.rays = rays; a.n = n; a.max_dist = max_dist; a.occluded = occluded; a.ctr = c.qry_ctr + QRY_ST_COUNT * slot;
+    a.S = rp.dev; a.rays = rays; a.n = n; a.max_dist = max_dist; a.occluded = occluded; a.ctr = ctr;
     a.out = o;
     a.count = stats != nullptr;
     {
@@ -591,6 +604,60 @@ static int query(const rbrt_scene* scene, const rbrt_ray* rays, uint64_t n, bool
     CKA(cudaStreamSynchronize(st));
     float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
     stats->rays = n; stats->nan_rays = h[QRY_ST_NAN]; stats->node_visits = h[QRY_ST_NODES]; stats->tri_tests = h[QRY_ST_TRIS];
+    stats->ms_device = ms; stats->launches = 1;
+    stats->ms_total = now_ms() - t0;
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ nearest-surface queries on device memory (rbrt_gpu_query_nearest_device)
+static int nearest(const rbrt_scene* scene, const float* points, uint64_t n, const float* max_dist, const rbrt_nearest_out* out,
+                   cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!n) return RBRT_OK;
+    if (!scene || !points || !out) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!out->dist && !out->kind && !out->elem_idx && !out->tri_idx && !out->point && !out->normal && !out->uv) {
+        set_error("no output requested (every plane of the output is NULL)"); return RBRT_E_INVALID;
+    }
+    if (n > 0xFFFFFFFFull) { set_error("more than 2^32 - 1 points"); return RBRT_E_INVALID; }
+    const Scene& sc = *reinterpret_cast<const Scene*>(scene);
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device
+    CKA(cudaSetDevice(rp.device));
+    const double t0 = now_ms();
+    const rbrt_nearest_out& o = *out;
+    { int rc = check_usable_on({points, max_dist, o.dist, o.kind, o.elem_idx, o.tri_idx, o.point, o.normal, o.uv}, rp.device,
+                               "points, bounds and outputs must be device memory on the scene's device %d"); if (rc) return rc; }
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    rbrt_point_launch_fn launch = nullptr;
+    { int rc = module_entry(g_point_module, "rbrt_point_launch", &launch); if (rc) return rc; }
+
+    DeviceCache& c = g_cache[rp.device & 63];
+    unsigned long long* ctr = nullptr; cudaEvent_t used = nullptr;
+    { int rc = query_ring_slot(c, &ctr, &used); if (rc) return rc; }
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
+
+    PointArgs a;
+    memset(&a, 0, sizeof(a));
+    a.S = rp.dev; a.points = points; a.n = n; a.max_dist = max_dist; a.out = o; a.ctr = ctr;
+    a.count = stats != nullptr;
+    {
+        const uint64_t blocks = (n + 127) / 128;                          // persistent: at most the resident blocks (8 per SM, point.cu)
+        const uint64_t resident = 8ull * (uint64_t)rp.sm_count;
+        a.blocks = (uint32_t)(blocks < resident ? blocks : resident);
+    }
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    CKA(cudaMemsetAsync(a.ctr, 0, 8 * PT_ST_COUNT, st));
+    if (stats) CKA(cudaEventRecord(c.e0, st));
+    CKA((cudaError_t)launch(&a, st));
+    if (stats) CKA(cudaEventRecord(c.e1, st));
+    CKA(cudaEventRecord(used, st));
+    note_scene_use(sc, rp.device, st);                                    // later updates wait for this read
+    if (!stats) return RBRT_OK;                                           // enqueue only
+
+    unsigned long long h[PT_ST_COUNT];
+    CKA(cudaMemcpyAsync(h, a.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CKA(cudaStreamSynchronize(st));
+    float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
+    stats->rays = n; stats->nan_rays = h[PT_ST_NAN]; stats->node_visits = h[PT_ST_NODES]; stats->tri_tests = h[PT_ST_TRIS];
     stats->ms_device = ms; stats->launches = 1;
     stats->ms_total = now_ms() - t0;
     return RBRT_OK;
@@ -1471,6 +1538,12 @@ int rbrt_gpu_query_occluded_device(const rbrt_scene* scene, const rbrt_ray* d_ra
                                    void* cuda_stream, rbrt_stats* stats) {
     LOCK;
     return query(scene, d_rays, n, true, nullptr, d_max_dist, d_occluded, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_query_nearest_device(const rbrt_scene* scene, const float* d_points, uint64_t n, const float* d_max_dist,
+                                  const rbrt_nearest_out* d_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return nearest(scene, d_points, n, d_max_dist, d_out, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,

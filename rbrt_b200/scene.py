@@ -47,6 +47,7 @@ def element_arrays(elements):
 
 
 QUERY_PASSES = ("t", "dist", "kind", "elem_idx", "tri_idx", "point", "normal")
+NEAREST_PASSES = ("dist", "kind", "elem_idx", "tri_idx", "point", "normal", "uv")
 
 
 class Scene:
@@ -215,6 +216,42 @@ class Scene:
                                                          occ.data_ptr(), stream.cuda_stream, st if stats is not None else None)
         self._query_check(rc, stats, st)
         return occ
+
+    # ---- nearest-surface queries on device memory (rbrt_gpu_query_nearest_device, DESIGN.md section 17) ----------
+    def nearest_device(self, points, max_dist=None, passes=None, stream=None, stats=None):
+        """The nearest surface of the scene to each point of a contiguous float32 CUDA tensor [N,3] on the scene's device: a dict of CUDA
+        tensors dist, kind (RBRT_HIT_*), elem_idx, tri_idx [N], point, normal [N,3] and uv [N,2] (`passes`: a subset of those names).
+        max_dist: None (+inf) or a float32 CUDA tensor [N]; only surfaces closer than it (strict) count, and a point without one gets
+        kind RBRT_HIT_NONE and dist +inf.  Enqueued on `stream` (default: the points' current stream); returns without synchronising
+        unless `stats` (a dict) is given."""
+        import torch
+        if not (isinstance(points, torch.Tensor) and points.is_cuda and points.dtype == torch.float32 and points.dim() == 2
+                and points.shape[1] == 3 and points.is_contiguous()):
+            raise ValueError("points must be a contiguous float32 CUDA tensor of shape [N,3]")
+        stream = stream or torch.cuda.current_stream(points.device)
+        if stream.device != points.device:
+            raise ValueError(f"points are on {points.device}, the stream on {stream.device}")
+        n = points.shape[0]
+        if max_dist is not None and not (isinstance(max_dist, torch.Tensor) and max_dist.device == points.device
+                                         and max_dist.dtype == torch.float32 and tuple(max_dist.shape) == (n,) and max_dist.is_contiguous()):
+            raise ValueError("max_dist must be None or a contiguous float32 CUDA tensor [N] on the points' device")
+        names = NEAREST_PASSES if passes is None else ((passes,) if isinstance(passes, str) else tuple(dict.fromkeys(passes)))
+        unknown = [p for p in names if p not in NEAREST_PASSES]
+        if unknown or not names:
+            raise ValueError(f"unknown or no pass(es) {unknown}; choose from {NEAREST_PASSES}")
+        handle = self.handle()
+        out, tensors = _abi.NearestOutC(), {}
+        with torch.cuda.stream(stream):
+            for name in names:
+                dt = torch.int32 if name == "kind" else (torch.uint32 if name in ("elem_idx", "tri_idx") else torch.float32)
+                shape = (n, 3) if name in ("point", "normal") else ((n, 2) if name == "uv" else (n,))
+                tensors[name] = torch.empty(shape, dtype=dt, device=points.device)
+                setattr(out, name, tensors[name].data_ptr())
+        st = _abi.StatsC()
+        rc = _abi.lib().rbrt_gpu_query_nearest_device(handle, points.data_ptr(), n, max_dist.data_ptr() if max_dist is not None else None,
+                                                       out, stream.cuda_stream, st if stats is not None else None)
+        self._query_check(rc, stats, st)
+        return tensors
 
 
 def scatter(items, seed=0):
