@@ -493,6 +493,52 @@ typedef struct rbrt_nearest_out {    /* device planes, n entries each (point / n
 int rbrt_gpu_query_nearest_device(const rbrt_scene* scene, const float* d_points, uint64_t n, const float* d_max_dist,
                                   const rbrt_nearest_out* d_out, void* cuda_stream, rbrt_stats* stats);
 
+/* ---- inside tests on device memory: generalized winding numbers (DESIGN.md section 18) -------
+ * For each point p (n points, f32 xyz, contiguous) the generalized winding number w(p) of the scene (Jacobson et al. 2013): 1 inside a
+ * closed surface whose corners run counter-clockwise seen from outside, 0 outside, fractional near a hole.  It is defined on triangle
+ * soups, so meshes need no adjacency.  rbrt_b200/csrc/winding.cuh holds the terms.
+ *   Candidates: those of rbrt_gpu_query_nearest_device: every element of Scene.elements and every TESTED mesh triangle (N_eff;
+ *   tail-dropped triangles are not candidates).  Each contributes a term, in f32:
+ *     triangle (a BasicTriangle or a mesh triangle), its stored record {v0, e1, e2}: a = v0 - p, b = a + e1, c = a + e2, scaled by one
+ *       power of two (exact); Omega = 2 atan2(det, |a||b||c| + (a.b)|c| + (a.c)|b| + (b.c)|a|) with det = a.(b x c) (van Oosterom and
+ *       Strackee).  The sign follows the corner order.  det exactly 0 (p in the triangle's plane, a degenerate record, p on a vertex)
+ *       gives 0, and so does a non-finite term (NaN or inf vertices, overflow): a NaN triangle never poisons a sum.
+ *     sphere {c, r}: with d = p - c, d2 = (dx*dx + dy*dy) + dz*dz and r2 = r*r, a full turn (4 pi) when d2 < r2, half of one when
+ *       d2 == r2, 0 otherwise.  The sign of r is ignored; r = 0 gives 0.
+ *   The terms are summed in f64 per point, and the sum is divided by 4 pi once in f64 and rounded to f32: the result does not depend on the
+ *   order of the terms beyond f64 rounding.
+ *   Fast evaluation (Barill et al. 2018), parameter beta: every child slot of every 4-wide node, and every mesh root, carries the moments
+ *   of its subtree's triangles: the area-weighted centroid c, a radius R >= the distance from c to every vertex of the subtree (rounded
+ *   up), N = sum 1/2 (e1 x e2) and the 3 x 3 tensor T = sum N_t (x) (c_t - c).  A child (or a mesh root) with |p - c| > beta R (the f32
+ *   difference, its length in f64) adds the expansion ((N.u) + (tr T - 3 u.T.u) / |r|) / |r|^2 of its subtree (r = c - p, u = r / |r|)
+ *   instead of its triangles' terms; any other child is descended, a leaf's triangles summed exactly.  A subtree whose moments are not
+ *   finite (NaN or inf vertices, overflow) is always descended.  beta = +inf is the exact sum over every candidate.
+ *   Outputs: winding (f32) = w; inside (u8) = |w| > 0.5 (the absolute value: a mesh whose faces all point inward still classifies; strict:
+ *   a point on a closed surface, w = 1/2, is outside).  A point with a NaN coordinate gives winding NaN, inside 0, and is counted in
+ *   stats->nan_rays.
+ * The moments live in a block the scene owns, allocated on the first call (64 bytes per node child slot and per mesh, plus scratch).  A
+ * mesh update (rbrt_gpu_scene_update_mesh*, refit or rebuild) marks the mesh's moments stale; the next call recomputes them on its own
+ * stream, behind every update and every read of the scene enqueued before it, and every later call waits for that.  Element updates do not
+ * touch moments.
+ * Points and planes are DEVICE memory on the scene's first device.  Enqueued on cuda_stream (0 = default stream): stats == NULL returns
+ * without synchronising; with stats the call waits and fills rays (= n), nan_rays, node_visits, tri_tests (exact mesh triangle terms),
+ * ms_device, ms_total and launches.  Ordered like a render: the call sees every update of the scene enqueued before it, and every later
+ * update waits for it.  Under a communicator it runs on replica 0 and is not collective.  n = 0 returns RBRT_OK, nothing written.
+ * The kernels live in librbrt_gpu_wind.so, loaded at run time from this library's directory (RBRT_GPU_WIND_LIB: another path);
+ * without it the call fails with RBRT_E_CUDA and a message.
+ * Refused with RBRT_E_INVALID, nothing written: a NULL scene, points or output with n > 0, both planes NULL, n > 2^32 - 1, points or
+ * planes in another device's memory or in unregistered host memory, a scene with a mesh whose tree was refused as too deep, and beta <= 1,
+ * negative or NaN other than 0 (the expansion does not converge within its sphere). */
+typedef struct rbrt_winding_opts {
+    float beta;                      /* far-field factor: 0 = the default 2.0; +inf = exact; otherwise > 1 */
+} rbrt_winding_opts;
+typedef struct rbrt_winding_out {    /* device planes, n entries each; NULL = not produced, not written */
+    float*    winding;
+    uint8_t*  inside;
+} rbrt_winding_out;
+int rbrt_gpu_query_winding_device(const rbrt_scene* scene, const float* d_points, uint64_t n, const rbrt_winding_opts* opts,
+                                  const rbrt_winding_out* d_out, void* cuda_stream, rbrt_stats* stats);
+
 /* ---- guided denoising (DESIGN.md section 13) -----------------------------------------------
  * An edge-aware à-trous filter of the HDR mean colour, guided by the first-hit AOVs of the same camera and seed (the spatial filter of
  * SVGF, Schied et al. 2017, without variance or temporal terms).  Inputs are row-major W x H planes: c = hdr (W*H*3, what

@@ -48,6 +48,12 @@ pub struct RbrtQueryOut { pub t: *mut f32, pub dist: *mut f32, pub kind: *mut i3
 #[repr(C)] #[derive(Copy, Clone, Debug)]
 pub struct RbrtNearestOut { pub dist: *mut f32, pub kind: *mut i32, pub elem_idx: *mut u32, pub tri_idx: *mut u32, pub point: *mut f32,
                             pub normal: *mut f32, pub uv: *mut f32 }
+/// Options of the winding-number query (rbrt_gpu_query_winding_device): beta 0 = the default 2.0, +inf = the exact sum, else > 1.
+#[repr(C)] #[derive(Copy, Clone, Debug, Default)]
+pub struct RbrtWindingOpts { pub beta: f32 }
+/// Winding-number planes in device memory (n values each); a null member is not produced.
+#[repr(C)] #[derive(Copy, Clone, Debug)]
+pub struct RbrtWindingOut { pub winding: *mut f32, pub inside: *mut u8 }
 /// Options of the guided denoiser (rbrt_gpu_denoise*); 0 = default (4 levels, at most 8).
 #[repr(C)] #[derive(Copy, Clone, Debug, Default)]
 pub struct RbrtDenoiseOpts { pub levels: u32, pub sigma_depth: f32, pub sigma_luminance: f32 }
@@ -158,6 +164,11 @@ extern "C" {
     /// synchronisation).  Not collective: replica 0.
     pub fn rbrt_gpu_query_nearest_device(scene: *const RbrtScene, d_points: *const f32, n: u64, d_max_dist: *const f32,
                                          d_out: *const RbrtNearestOut, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
+    /// The generalized winding number of the scene at each point (n points, f32 xyz, in device memory) over the nearest query's
+    /// candidates, and inside = |w| > 0.5; far subtrees by their moments unless opts.beta = +inf (opts may be null: beta 2);
+    /// enqueued on `stream` (stats = null: no synchronisation).  Not collective: replica 0.
+    pub fn rbrt_gpu_query_winding_device(scene: *const RbrtScene, d_points: *const f32, n: u64, opts: *const RbrtWindingOpts,
+                                         d_out: *const RbrtWindingOut, stream: *mut c_void, stats: *mut RbrtStats) -> c_int;
     /// Edge-aware à-trous denoise of a render_hdr image guided by render_aov depth / normal / albedo of the same camera and seed; HOST
     /// pointers, blocks.  hdr_out (W*H*3 f32) and / or rgb_out (W*H*3 u8, k_finalize's tonemap); opts may be null.
     pub fn rbrt_gpu_denoise(width: u32, height: u32, hdr: *const f32, guides: *const RbrtAovOut, opts: *const RbrtDenoiseOpts,

@@ -108,6 +108,14 @@ class NearestOutC(C.Structure):  # rbrt_nearest_out: device planes, NULL = not p
                 ("normal", C.c_void_p), ("uv", C.c_void_p)]
 
 
+class WindingOptsC(C.Structure):  # rbrt_winding_opts: beta 0 = default 2.0, +inf = exact
+    _fields_ = [("beta", C.c_float)]
+
+
+class WindingOutC(C.Structure):  # rbrt_winding_out: device planes, NULL = not produced
+    _fields_ = [("winding", C.c_void_p), ("inside", C.c_void_p)]
+
+
 class DenoiseOptsC(C.Structure):  # rbrt_denoise_opts: 0 = default
     _fields_ = [("levels", C.c_uint32), ("sigma_depth", C.c_float), ("sigma_luminance", C.c_float)]
 
@@ -189,6 +197,7 @@ GPU_SIGNATURES = {
     "rbrt_gpu_query_closest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, P(QueryOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_occluded_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_query_nearest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, P(NearestOutC), C.c_void_p, P(StatsC)]),
+    "rbrt_gpu_query_winding_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, P(WindingOptsC), P(WindingOutC), C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, P(StatsC)]),
     "rbrt_gpu_denoise_device": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, P(AovOutC), P(DenoiseOptsC), C.c_void_p, C.c_void_p, C.c_void_p,
                                           P(StatsC)]),

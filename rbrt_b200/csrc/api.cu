@@ -16,6 +16,7 @@
 #include "multi.cuh"
 #include "query.cuh"
 #include "point.cuh"
+#include "winding.cuh"
 #include "update.cuh"
 #include "motion.cuh"
 #include "temporal.cuh"
@@ -176,6 +177,13 @@ void destroy_scene(Scene* sc) {
         cudaFree(sc->snap); sc->snap = nullptr;
     }
     if (sc->snap_ev) { cudaEventDestroy(sc->snap_ev); sc->snap_ev = nullptr; }
+    if (sc->wind) {                                                       // behind the moments' computation and every read of them
+        cudaSetDevice(sc->rep[0].device);
+        if (sc->wind_ev) cudaEventSynchronize(sc->wind_ev);
+        for (SceneUse& u : sc->uses) if (u.device == sc->rep[0].device && u.ev) cudaEventSynchronize(u.ev);
+        cudaFree(sc->wind); sc->wind = nullptr;
+    }
+    if (sc->wind_ev) { cudaEventDestroy(sc->wind_ev); sc->wind_ev = nullptr; }
     for (Replica& r : sc->rep) {
         if (!r.arena) { if (r.ready) cudaEventDestroy(r.ready); continue; }
         ArenaBlock b{r.arena, r.arena_bytes, r.device, {}};
@@ -240,7 +248,8 @@ static void pack_elements(const rbrt_element_ref* order, uint32_t ns, const rbrt
 // ------------------------------------------------------------------ device modules
 // The refit kernels (librbrt_gpu_update.so), the AOV kernel (librbrt_gpu_aov.so), the ray queries (librbrt_gpu_query.so), the denoiser
 // (librbrt_gpu_denoise.so), the variance kernels (librbrt_gpu_variance.so), the temporal accumulation (librbrt_gpu_temporal.so) and the
-// snapshot with the motion pass (librbrt_gpu_motion.so) and the nearest-surface queries (librbrt_gpu_point.so) live in their own device modules, loaded from this library's
+// snapshot with the motion pass (librbrt_gpu_motion.so), the nearest-surface queries (librbrt_gpu_point.so) and the winding numbers
+// (librbrt_gpu_wind.so) live in their own device modules, loaded from this library's
 // directory (or the path in the module's environment variable) on first use.  Without a module its calls are refused: there is no other
 // implementation.
 // Path of a device module shipped next to this library (`file`), or the value of the environment variable `env` if that is set.
@@ -265,6 +274,7 @@ static Module g_variance_module = {"RBRT_GPU_VARIANCE_LIB", "librbrt_gpu_varianc
 static Module g_temporal_module = {"RBRT_GPU_TEMPORAL_LIB", "librbrt_gpu_temporal.so", "temporal", nullptr};
 static Module g_motion_module = {"RBRT_GPU_MOTION_LIB", "librbrt_gpu_motion.so", "motion", nullptr};
 static Module g_point_module = {"RBRT_GPU_POINT_LIB", "librbrt_gpu_point.so", "nearest-surface", nullptr};
+static Module g_wind_module = {"RBRT_GPU_WIND_LIB", "librbrt_gpu_wind.so", "winding-number", nullptr};
 // The entry point `symbol` of module m, which is opened on first use.  A failed dlopen is not remembered: the next call tries again.
 template <class F> static int module_entry(Module& m, const char* symbol, F* fn) {
     if (!m.h) {
@@ -391,6 +401,7 @@ static int update_mesh(rbrt_scene* scene, uint32_t mi, const float* verts, bool 
         }
     }
     { int rc = update_end(sc, ctx); if (rc) return rc; }
+    ++sc->mesh_gen[mi];                                                   // its winding moments are stale (refit and rebuild alike)
     if (on_device && !receiver) {                                         // the caller's stream continues behind the update
         { int rc = ensure_event(&sc->upd_out); if (rc) return rc; }
         CKA(cudaEventRecord(sc->upd_out, ctx.build));
@@ -658,6 +669,119 @@ static int nearest(const rbrt_scene* scene, const float* points, uint64_t n, con
     CKA(cudaStreamSynchronize(st));
     float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
     stats->rays = n; stats->nan_rays = h[PT_ST_NAN]; stats->node_visits = h[PT_ST_NODES]; stats->tri_tests = h[PT_ST_TRIS];
+    stats->ms_device = ms; stats->launches = 1;
+    stats->ms_total = now_ms() - t0;
+    return RBRT_OK;
+}
+
+// ------------------------------------------------------------------ winding numbers on device memory (rbrt_gpu_query_winding_device)
+// The moment block: 4 records of 64 bytes per node slot of the scene (a mesh's node j at node_base + j), one record per mesh root, and the
+// scratch of k_wind_moments for the largest mesh (parent, need, arrive per node, one f64 area per child slot).
+struct WindLayout { size_t mom, root, parent, need, arrive, area, total; };
+static WindLayout wind_layout(const Scene& sc) {
+    size_t slots = 0, most = 1;
+    for (const MeshDev& m : sc.meshes_h) { slots = std::max(slots, (size_t)m.node_base + m.n_tris); most = std::max(most, (size_t)m.n_tris); }
+    WindLayout L; size_t off = 0;
+    L.mom = off; off += a256(256 * slots);
+    L.root = off; off += a256(64ull * std::max<uint32_t>(sc.n_meshes, 1));
+    L.parent = off; off += a256(4 * most);
+    L.need = off; off += a256(4 * most);
+    L.arrive = off; off += a256(4 * most);
+    L.area = off; off += a256(32 * most);
+    L.total = off;
+    return L;
+}
+
+// The moments of every mesh updated since they were last computed, on `st`: behind the scene's updates (ready) and every read of the
+// scene enqueued so far (no winding call in flight still reads the old records).  wind_ev is recorded behind them.
+static int wind_refresh(Scene& sc, cudaStream_t st) {
+    const Replica& rp = sc.rep[0];
+    const WindLayout L = wind_layout(sc);
+    if (!sc.wind) {
+        CKA(cudaMalloc((void**)&sc.wind, L.total));
+        sc.wind_gen.assign(sc.n_meshes, ~0ull);
+    }
+    { int rc = ensure_event(&sc.wind_ev); if (rc) return rc; }
+    bool stale = false;
+    for (uint32_t i = 0; i < sc.n_meshes; ++i) stale = stale || sc.wind_gen[i] != sc.mesh_gen[i];
+    if (!stale) return RBRT_OK;
+    rbrt_wind_moments_launch_fn launch = nullptr;
+    { int rc = module_entry(g_wind_module, "rbrt_wind_moments_launch", &launch); if (rc) return rc; }
+    wait_scene_ready(sc, 0, st);
+    wait_scene_uses(sc, rp.device, st);
+    for (uint32_t i = 0; i < sc.n_meshes; ++i) {
+        if (sc.wind_gen[i] == sc.mesh_gen[i]) continue;
+        const MeshDev& md = sc.meshes_h[i];
+        WindMomentArgs a;
+        a.nodes = reinterpret_cast<const uint4*>(rp.arena + sc.lay.nodes) + 4ull * md.node_base;
+        a.tris = reinterpret_cast<const float4*>(rp.arena + sc.lay.tris) + 3ull * md.tri_base;
+        a.mesh = reinterpret_cast<const MeshDev*>(rp.arena + sc.lay.mesh) + i;
+        a.live_nodes = &(reinterpret_cast<const BuildResult*>(rp.arena + sc.lay.result) + i)->live_nodes;
+        a.mom = reinterpret_cast<float4*>(sc.wind + L.mom) + 16ull * md.node_base;
+        a.root = reinterpret_cast<float4*>(sc.wind + L.root) + 4ull * i;
+        a.parent = (uint32_t*)(sc.wind + L.parent); a.need = (uint32_t*)(sc.wind + L.need); a.arrive = (uint32_t*)(sc.wind + L.arrive);
+        a.area = (double*)(sc.wind + L.area);
+        a.n_tris = md.n_tris;
+        CKA((cudaError_t)launch(&a, st));
+        sc.wind_gen[i] = sc.mesh_gen[i];
+    }
+    CKA(cudaEventRecord(sc.wind_ev, st));
+    return RBRT_OK;
+}
+
+static int winding(const rbrt_scene* scene, const float* points, uint64_t n, const rbrt_winding_opts* opts, const rbrt_winding_out* out,
+                   cudaStream_t st, rbrt_stats* stats) {
+    if (stats) memset(stats, 0, sizeof(*stats));
+    if (!n) return RBRT_OK;
+    if (!scene || !points || !out) { set_error("null argument"); return RBRT_E_INVALID; }
+    if (!out->winding && !out->inside) { set_error("no output requested (winding and inside are both NULL)"); return RBRT_E_INVALID; }
+    if (n > 0xFFFFFFFFull) { set_error("more than 2^32 - 1 points"); return RBRT_E_INVALID; }
+    float beta = opts ? opts->beta : 0.0f;
+    if (beta == 0.0f) beta = 2.0f;
+    if (!(beta > 1.0f)) { set_error("beta must be > 1 (or 0 for the default 2, +inf for the exact sum)"); return RBRT_E_INVALID; }
+    Scene& sc = *reinterpret_cast<Scene*>(const_cast<rbrt_scene*>(scene));   // the moment block is a cache behind the handle
+    const Replica& rp = sc.rep[0];                                        // under a communicator: this process's first device
+    CKA(cudaSetDevice(rp.device));
+    const double t0 = now_ms();
+    { int rc = check_usable_on({points, out->winding, out->inside}, rp.device,
+                               "points and outputs must be device memory on the scene's device %d"); if (rc) return rc; }
+    { int rc = resolve_scene_info(sc, true); if (rc) return rc; }         // a refused mesh is known before anything is written
+    rbrt_wind_query_launch_fn launch = nullptr;
+    { int rc = module_entry(g_wind_module, "rbrt_wind_query_launch", &launch); if (rc) return rc; }
+    { int rc = wind_refresh(sc, st); if (rc) return rc; }
+
+    DeviceCache& c = g_cache[rp.device & 63];
+    unsigned long long* ctr = nullptr; cudaEvent_t used = nullptr;
+    { int rc = query_ring_slot(c, &ctr, &used); if (rc) return rc; }
+    if (stats) { int rc = timing_events(c); if (rc) return rc; }
+
+    static_assert((int)WD_ST_COUNT == (int)QRY_ST_COUNT && (int)WD_ST_HEAD == (int)QRY_ST_HEAD, "the winding query shares the ring's blocks");
+    const WindLayout L = wind_layout(sc);
+    WindQueryArgs a;
+    memset(&a, 0, sizeof(a));
+    a.S = rp.dev; a.mom = (const float4*)(sc.wind + L.mom); a.root = (const float4*)(sc.wind + L.root);
+    a.points = points; a.n = n; a.beta = beta; a.out = *out; a.ctr = ctr;
+    a.count = stats != nullptr;
+    {
+        const uint64_t blocks = (n + 127) / 128;                          // persistent: at most the resident blocks (8 per SM, wind.cu)
+        const uint64_t resident = 8ull * (uint64_t)rp.sm_count;
+        a.blocks = (uint32_t)(blocks < resident ? blocks : resident);
+    }
+    wait_scene_ready(sc, 0, st);                                          // behind the scene's build and every update enqueued so far
+    CKA(cudaStreamWaitEvent(st, sc.wind_ev, 0));                          // and the latest moments
+    CKA(cudaMemsetAsync(a.ctr, 0, 8 * WD_ST_COUNT, st));
+    if (stats) CKA(cudaEventRecord(c.e0, st));
+    CKA((cudaError_t)launch(&a, st));
+    if (stats) CKA(cudaEventRecord(c.e1, st));
+    CKA(cudaEventRecord(used, st));
+    note_scene_use(sc, rp.device, st);                                    // later updates and recomputations wait for this read
+    if (!stats) return RBRT_OK;                                           // enqueue only
+
+    unsigned long long h[WD_ST_COUNT];
+    CKA(cudaMemcpyAsync(h, a.ctr, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CKA(cudaStreamSynchronize(st));
+    float ms = 0; CKA(cudaEventElapsedTime(&ms, c.e0, c.e1));
+    stats->rays = n; stats->nan_rays = h[WD_ST_NAN]; stats->node_visits = h[WD_ST_NODES]; stats->tri_tests = h[WD_ST_TRIS];
     stats->ms_device = ms; stats->launches = 1;
     stats->ms_total = now_ms() - t0;
     return RBRT_OK;
@@ -1166,6 +1290,7 @@ int rbrt_gpu_scene_create_elements(const rbrt_element_ref* order, uint32_t ne, c
     sc->info.num_triangles = total_tris; sc->info.num_triangles_tested = total_eff;
     sc->pad_rel = pad_rel; sc->leaf_size = leaf_size; sc->sah = !(sflags & RBRT_SCENE_NO_SAH); sc->replicated = replicate;
     sc->mesh_n_all.resize(nm);
+    sc->mesh_gen.assign(nm, 0);
     for (uint32_t i = 0; i < nm; ++i) sc->mesh_n_all[i] = meshes[i].num_triangles;
     sc->elem_kind_h.resize(ns);
     for (uint32_t i = 0; i < ns; ++i) sc->elem_kind_h[i] = order[i].kind;
@@ -1544,6 +1669,12 @@ int rbrt_gpu_query_nearest_device(const rbrt_scene* scene, const float* d_points
                                   const rbrt_nearest_out* d_out, void* cuda_stream, rbrt_stats* stats) {
     LOCK;
     return nearest(scene, d_points, n, d_max_dist, d_out, (cudaStream_t)cuda_stream, stats);
+}
+
+int rbrt_gpu_query_winding_device(const rbrt_scene* scene, const float* d_points, uint64_t n, const rbrt_winding_opts* opts,
+                                  const rbrt_winding_out* d_out, void* cuda_stream, rbrt_stats* stats) {
+    LOCK;
+    return winding(scene, d_points, n, opts, d_out, (cudaStream_t)cuda_stream, stats);
 }
 
 int rbrt_gpu_denoise(uint32_t width, uint32_t height, const float* hdr, const rbrt_aov_out* guides, const rbrt_denoise_opts* opts,

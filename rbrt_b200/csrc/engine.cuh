@@ -83,6 +83,12 @@ struct Scene {
     // first snapshot; snap_ev is recorded behind the latest snapshot, and every motion call waits for it
     char* snap = nullptr;
     cudaEvent_t snap_ev = nullptr;
+    // ---- rbrt_gpu_query_winding_device: the moment block on replica 0's device (api.cu, wind_layout), allocated on the first call.
+    // mesh_gen counts the updates of each mesh, wind_gen the generation its moments were computed for; wind_ev is recorded behind the
+    // latest recomputation, and every winding call waits for it
+    std::vector<uint64_t> mesh_gen, wind_gen;
+    char* wind = nullptr;
+    cudaEvent_t wind_ev = nullptr;
 };
 int resolve_scene_info(const Scene& sc, bool wait);   // api.cu: fills info from the build results once they are there (wait: block for them); returns RBRT_E_* if the build refused a mesh
 void wait_scene_ready(const Scene& sc, int li, cudaStream_t st);   // makes `st` wait for replica li's data

@@ -48,6 +48,7 @@ def element_arrays(elements):
 
 QUERY_PASSES = ("t", "dist", "kind", "elem_idx", "tri_idx", "point", "normal")
 NEAREST_PASSES = ("dist", "kind", "elem_idx", "tri_idx", "point", "normal", "uv")
+WINDING_PASSES = ("winding", "inside")
 
 
 class Scene:
@@ -225,12 +226,7 @@ class Scene:
         kind RBRT_HIT_NONE and dist +inf.  Enqueued on `stream` (default: the points' current stream); returns without synchronising
         unless `stats` (a dict) is given."""
         import torch
-        if not (isinstance(points, torch.Tensor) and points.is_cuda and points.dtype == torch.float32 and points.dim() == 2
-                and points.shape[1] == 3 and points.is_contiguous()):
-            raise ValueError("points must be a contiguous float32 CUDA tensor of shape [N,3]")
-        stream = stream or torch.cuda.current_stream(points.device)
-        if stream.device != points.device:
-            raise ValueError(f"points are on {points.device}, the stream on {stream.device}")
+        points, stream = self._device_points(points, stream)
         n = points.shape[0]
         if max_dist is not None and not (isinstance(max_dist, torch.Tensor) and max_dist.device == points.device
                                          and max_dist.dtype == torch.float32 and tuple(max_dist.shape) == (n,) and max_dist.is_contiguous()):
@@ -252,6 +248,58 @@ class Scene:
                                                        out, stream.cuda_stream, st if stats is not None else None)
         self._query_check(rc, stats, st)
         return tensors
+
+    @staticmethod
+    def _device_points(points, stream):
+        """(points, stream) of a query on points: a contiguous float32 CUDA tensor [N,3], and the stream (default: its current one)."""
+        import torch
+        if not (isinstance(points, torch.Tensor) and points.is_cuda and points.dtype == torch.float32 and points.dim() == 2
+                and points.shape[1] == 3 and points.is_contiguous()):
+            raise ValueError("points must be a contiguous float32 CUDA tensor of shape [N,3]")
+        stream = stream or torch.cuda.current_stream(points.device)
+        if stream.device != points.device:
+            raise ValueError(f"points are on {points.device}, the stream on {stream.device}")
+        return points, stream
+
+    # ---- inside tests on device memory (rbrt_gpu_query_winding_device, DESIGN.md section 18) ---------------------------
+    def winding_device(self, points, beta=None, passes=None, stream=None, stats=None):
+        """The generalized winding number of the scene at each point of a contiguous float32 CUDA tensor [N,3] on the scene's device: a
+        dict of CUDA tensors winding (float32 [N]) and inside (uint8 [N], |winding| > 0.5); `passes`: a subset of those names.  beta: None
+        (the default 2.0), > 1, or float('inf') for the exact sum over every triangle.  Enqueued on `stream` (default: the points'
+        current stream); returns without synchronising unless `stats` (a dict) is given."""
+        import torch
+        points, stream = self._device_points(points, stream)
+        n = points.shape[0]
+        names = WINDING_PASSES if passes is None else ((passes,) if isinstance(passes, str) else tuple(dict.fromkeys(passes)))
+        unknown = [p for p in names if p not in WINDING_PASSES]
+        if unknown or not names:
+            raise ValueError(f"unknown or no pass(es) {unknown}; choose from {WINDING_PASSES}")
+        handle = self.handle()
+        out, tensors = _abi.WindingOutC(), {}
+        with torch.cuda.stream(stream):
+            for name in names:
+                tensors[name] = torch.empty(n, dtype=torch.float32 if name == "winding" else torch.uint8, device=points.device)
+                setattr(out, name, tensors[name].data_ptr())
+        st = _abi.StatsC()
+        rc = _abi.lib().rbrt_gpu_query_winding_device(handle, points.data_ptr(), n, _abi.WindingOptsC(0.0 if beta is None else float(beta)),
+                                                       out, stream.cuda_stream, st if stats is not None else None)
+        self._query_check(rc, stats, st)
+        return tensors
+
+    def signed_distance_device(self, points, max_dist=None, beta=None, stream=None):
+        """The signed distance to the scene at each point (float32 CUDA tensor [N]): nearest_device's `dist`, negated where
+        winding_device's `inside` is set; both calls run on one stream.  max_dist (None, a float, or a float32 CUDA tensor [N]) bounds
+        the nearest search: a point with no surface closer than it gets +inf outside and -inf inside, which narrow-band SDF sampling
+        can take as "beyond the band, on this side"."""
+        import torch
+        points, stream = self._device_points(points, stream)
+        if max_dist is not None and not isinstance(max_dist, torch.Tensor):
+            with torch.cuda.stream(stream):
+                max_dist = torch.full((points.shape[0],), float(max_dist), dtype=torch.float32, device=points.device)
+        dist = self.nearest_device(points, max_dist=max_dist, passes="dist", stream=stream)["dist"]
+        inside = self.winding_device(points, beta=beta, passes="inside", stream=stream)["inside"]
+        with torch.cuda.stream(stream):
+            return torch.where(inside.bool(), -dist, dist)
 
 
 def scatter(items, seed=0):
